@@ -2,6 +2,7 @@
 """bench.py -- ICM sweeps/s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3|c1|c5|ijac|palomar] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one ICM sweep (iterations_process_offline, sensors.py:125-168) over the whole
 trajectory: projection, association, landmark statistics, pose update, map filter.  Scan
@@ -20,6 +21,8 @@ throughput is reported separately (`extraction`).
                baseline/setup_ref.py; imported through oracle/ref_runner.py) on the host cores, on a
                bounded prefix of the same workload against the full map; extrapolated numbers say so.
 * `result_sha256`: hash of poses + map + labels after warm-up + steps: identical for 1/2/4/8 GPUs.
+* `--dump-outputs DIR`: the same poses, map and labels as .npy files (dump_outputs), so that two builds can be
+               compared array by array; the inputs of a workload are the same on every run.
 
 Workloads: c4 (default, the metric's configuration), c3, c1 (synthetic smoke), c5 (4096 independent
 trajectories), ijac / palomar (the reference's two real logs: pass 0 + sweeps, as shipped).
@@ -104,6 +107,24 @@ def result_hash(x, mapa, c):
     h.update(np.ascontiguousarray(mapa, dtype=np.float64).tobytes())
     h.update(np.ascontiguousarray(c, dtype=np.int32).tobytes())
     return h.hexdigest()
+
+
+DUMP_COLUMNS = 1 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """Writes each array as <out_dir>/<name>.npy in float64 (exact for the int32 labels).  An array of more than DUMP_COLUMNS
+    columns keeps a sample of them drawn with SEED (the same columns for the same length), and the sampled column indices go
+    to <name>_index.npy.  C4: the full 3 x 1M poses, the full map, 2^20 of the 25M labels; about 42 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        n = a.shape[-1]
+        if n > DUMP_COLUMNS:
+            idx = np.sort(np.random.default_rng(SEED).choice(n, DUMP_COLUMNS, replace=False))
+            a = a[..., idx]
+            np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 class ClockSampler:
@@ -314,11 +335,11 @@ def run_gpu(args, rank, world, local_rank):
     name = args.workload
     if name == "c5":
         from icm_slam_b200 import batch
-        return batch.bench(args, rank, world, local_rank, SEED, METRIC, peaks, ClockSampler, sweep_bytes)
+        return batch.bench(args, rank, world, local_rank, SEED, METRIC, peaks, ClockSampler, sweep_bytes, dump_outputs=dump_outputs)
     if world > 1:
         from icm_slam_b200 import multigpu
         return multigpu.bench(args, rank, world, local_rank, WORKLOADS, SEED, METRIC, sweep_bytes, peaks, ClockSampler, make_data,
-                              config_for, result_hash, runs_bytes)
+                              config_for, result_hash, runs_bytes, dump_outputs)
 
     L_true, T, desc = WORKLOADS[name]
     real = name in REAL_LOGS
@@ -385,7 +406,8 @@ def run_gpu(args, rank, world, local_rank):
     ms = ev0.elapsed_time(ev1) / args.steps
     launches = (eng.launch_count() - lc0) // max(args.steps, 1)
     L_now = eng.landmarks_actuales
-    sha = result_hash(eng.get_poses(), eng.get_map(), eng.associations())
+    outputs = dict(poses=eng.get_poses(), map=eng.get_map(), associations=eng.associations())
+    sha = result_hash(outputs["poses"], outputs["map"], outputs["associations"])
     t_load = time.perf_counter()          # the same load, untimed, for the clock sampler
     while time.perf_counter() - t_load < 0.15:
         eng.iterate(x_dev, x0, 20, **mode)
@@ -479,6 +501,8 @@ def run_gpu(args, rank, world, local_rank):
                                "note": "whole sweep (all kernels of the graph replay) against the sweep's algorithmic bytes"}},
         "cpu_baseline": cpu,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, **outputs)
     print(json.dumps(out), flush=True)
 
 
@@ -491,12 +515,20 @@ def main():
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
     ap.add_argument("--ref-poses", type=int, default=None, help="prefix length for the CPU arm")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the poses, map and labels of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "b200":
         args.warmup = max(args.warmup, 3)          # the first sweeps build the run records; steady state needs them
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU implementation computes; the reference arm times a prefix only")
+    if args.dump_outputs and args.workload == "c5" and world > 1:
+        ap.error("--dump-outputs with c5 needs one rank: each rank holds only its own trajectories")
     if args.impl == "reference":
         return run_reference(args, rank, world)
     return run_gpu(args, rank, world, local_rank)

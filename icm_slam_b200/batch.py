@@ -179,7 +179,8 @@ def gather_results(local: dict, group=None):
 
 
 # ---- bench arm for the batch workload (called by bench.py --workload c5; one rank per GPU, no data-path collective) ---------
-def bench(args, rank, world, local_rank, SEED, METRIC, peaks, ClockSampler, sweep_bytes, per_gpu=512, Tk=2048, L_true=16):
+def bench(args, rank, world, local_rank, SEED, METRIC, peaks, ClockSampler, sweep_bytes, per_gpu=512, Tk=2048, L_true=16,
+          dump_outputs=None):
     import json
     import time
 
@@ -237,6 +238,7 @@ def bench(args, rank, world, local_rank, SEED, METRIC, peaks, ClockSampler, swee
     else:
         n_tot = n_obs
     launches = (b.engine.launch_count() - lc0) // max(args.steps, 1)
+    outputs = dict(poses=b.engine.get_poses(), map=b.engine.get_map(), associations=b.engine.associations()) if args.dump_outputs else None
     t_load = time.perf_counter()          # the same load, untimed, for the clock sampler
     while time.perf_counter() - t_load < 0.15:
         b.iterate(20)
@@ -287,6 +289,8 @@ def bench(args, rank, world, local_rank, SEED, METRIC, peaks, ClockSampler, swee
                          "algorithmic_bytes": int(B_sweep)},
             "cpu_baseline": None,
         }
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, **outputs)
         print(json.dumps(out), flush=True)
     if dist is not None:
         dist.barrier()

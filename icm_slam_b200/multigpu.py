@@ -479,7 +479,7 @@ class SegmentedSolver:
 
 # ---- bench arm for N > 1 (called by bench.py under torchrun) -----------------------------------------------------
 def bench(args, rank, world, local_rank, WORKLOADS, SEED, METRIC, sweep_bytes, peaks, ClockSampler, make_data, config_for, result_hash,
-          runs_bytes):
+          runs_bytes, dump_outputs):
     import json
     import time
 
@@ -623,6 +623,8 @@ def bench(args, rank, world, local_rank, WORKLOADS, SEED, METRIC, sweep_bytes, p
                                    "note": "whole job: all segments' bytes over the max-over-ranks sweep time, vs %d x the HBM peak" % world}},
             "cpu_baseline": None,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, poses=x_all, map=m_all, associations=c_all)
         print(json.dumps(out), flush=True)
     dist.barrier()
     sol.close()

@@ -1,16 +1,21 @@
-"""CPU checks of bench.py's reference arm (the unmodified reference from baseline/_ref or /root/reference, driven through
-oracle/ref_runner.py -- the one place besides tests/ and smoke() that may execute oracle/) and of the result writers: the JSON
-contract the driver parses, no GPU needed."""
+"""CPU checks of bench.py's reference arm (the unmodified reference copied to baseline/_ref, driven through
+oracle/ref_runner.py -- the one place besides tests/ and smoke() that may execute oracle/), of its argument checks and output
+dump, and of the result writers: the JSON line bench.py prints, no GPU needed."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
+
+import bench
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+@pytest.mark.skipif(bench.ref_dir() is None, reason="the unmodified reference is not part of the repository; "
+                                                     "baseline/setup_ref.py copies it to baseline/_ref where it is installed")
 def test_reference_arm_prints_one_contract_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "c1", "--steps", "1",
                           "--warmup", "0", "--ref-poses", "200"], capture_output=True, text=True, timeout=300, cwd=ROOT)
@@ -36,3 +41,28 @@ def test_result_writers_round_trip(tmp_path):
         for k in ("x", "mapa", "cambios", "mapa_inicial", "x_inicial"):
             assert np.array_equal(np.asarray(back[k]), res[k]), (ext, k)
         assert np.array_equal(np.asarray(back["labels"]).ravel(), res["labels"])
+
+
+def test_steps_below_one_is_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120,
+                         cwd=ROOT)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+def test_dump_outputs_writes_float64_and_a_seeded_sample(tmp_path):
+    rng = np.random.default_rng(3)
+    poses = rng.normal(size=(3, 1000))
+    labels = rng.integers(-1, 1 << 20, size=bench.DUMP_COLUMNS + 17).astype(np.int32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), poses=poses, associations=labels)
+    assert sorted(os.listdir(tmp_path / "a")) == ["associations.npy", "associations_index.npy", "poses.npy"]
+    p = np.load(tmp_path / "a" / "poses.npy")
+    assert p.dtype == np.float64 and np.array_equal(p, poses)
+    idx = np.load(tmp_path / "a" / "associations_index.npy")
+    c = np.load(tmp_path / "a" / "associations.npy")
+    assert idx.dtype == c.dtype == np.float64 and c.shape == idx.shape == (bench.DUMP_COLUMNS,)
+    assert np.all(np.diff(idx) > 0) and np.array_equal(c, labels[idx.astype(np.int64)])
+    for f in os.listdir(tmp_path / "a"):
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f
+    # the largest single-GPU workload (c4: 1M poses, ~100k landmarks, ~25M labels) stays under 64 MB
+    assert (3 * 1_000_000 + 2 * 2 * 316 * 316 + 2 * bench.DUMP_COLUMNS) * 8 < 64 << 20
