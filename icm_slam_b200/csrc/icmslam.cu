@@ -115,9 +115,6 @@ struct icmslam_handle {
     GraphSlot graphs[4];
     int use_graph = 1, graph_launches = 0;
     int runs_occ = 24;           // resident one-warp blocks per SM k_runs is compiled for (24: 80 registers; ICMSLAM_RUNS_OCC=32: 64)
-    size_t solve_pad = 0;        // unused dynamic shared memory of k_solve_tile: caps its resident blocks per SM so that the tail's kernels,
-                                 // which run beside it, find free registers at once (ICMSLAM_SOLVE_PAD, bytes)
-    int solve_occ = 5;           // resident 128-thread blocks per SM k_solve_tile is compiled for (ICMSLAM_SOLVE_OCC=4|5|6)
     int use_runs = 1;            // ICMSLAM_RUNS=0: every tile goes through the association kernel every sweep (no steady-state shortcut)
     int assoc_blocks = 0;        // grid of the (persistent) association kernel
     double2* d_bxy = nullptr;    // interleaved (bx, by) records for the TMA staging
@@ -388,18 +385,7 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
     if (e == cudaSuccess && h->trace_on) { const int one = 1; e = cudaMemcpy(&h->d_ts->trace_on, &one, sizeof one, cudaMemcpyHostToDevice); }
     { const char* eg = getenv("ICMSLAM_GRAPH"); if (eg) h->use_graph = atoi(eg); }
     { const char* er = getenv("ICMSLAM_RUNS"); if (er) h->use_runs = atoi(er) != 0; }
-    { const char* er = getenv("ICMSLAM_SOLVE_OCC"); if (er && (atoi(er) == 4 || atoi(er) == 6)) h->solve_occ = atoi(er); }
     { const char* er = getenv("ICMSLAM_RUNS_OCC"); if (er && atoi(er) == 32) h->runs_occ = 32; }
-    {
-        const char* ep = getenv("ICMSLAM_SOLVE_PAD");
-        if (ep && atoi(ep) > 0) h->solve_pad = (size_t)atoi(ep);
-        if (h->solve_pad > 0) {
-            cudaFuncSetAttribute(k_solve_tile<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->solve_pad);
-            cudaFuncSetAttribute(k_solve_tile<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->solve_pad);
-            cudaFuncSetAttribute(k_solve_tile<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->solve_pad);
-            cudaGetLastError();
-        }
-    }
     if (e == cudaSuccess) {
         int sms = 0;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
@@ -964,9 +950,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (ready > h->n_solve_tiles) ready = h->n_solve_tiles;
             if (ready > solved) {
                 P.tile0 = solved;
-                if (h->solve_occ == 4) k_solve_tile<4><<<ready - solved, ST_THREADS, h->solve_pad, s>>>(P);
-                else if (h->solve_occ == 6) k_solve_tile<6><<<ready - solved, ST_THREADS, h->solve_pad, s>>>(P);
-                else k_solve_tile<5><<<ready - solved, ST_THREADS, h->solve_pad, s>>>(P);
+                k_solve_tile<<<ready - solved, ST_THREADS, 0, s>>>(P);
                 CK(cudaGetLastError());
                 h->n_launch += 1;
                 CK(cudaEventRecord(h->ev_out[c], s));
@@ -1015,9 +999,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             CK(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
             ss = h->side_stream;
         }
-        if (h->solve_occ == 4) k_solve_tile<4><<<h->n_solve_tiles, ST_THREADS, h->solve_pad, ss>>>(P);
-        else if (h->solve_occ == 6) k_solve_tile<6><<<h->n_solve_tiles, ST_THREADS, h->solve_pad, ss>>>(P);
-        else k_solve_tile<5><<<h->n_solve_tiles, ST_THREADS, h->solve_pad, ss>>>(P);
+        k_solve_tile<<<h->n_solve_tiles, ST_THREADS, 0, ss>>>(P);
         CK(cudaGetLastError());
         if (h->d2h_x) {      // a host-memory caller: its poses start their way back as soon as they are solved, beside the tail
             CK(cudaMemcpy2DAsync(h->d2h_x, (size_t)h->d2h_ld * 8, kout, (size_t)kld * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, ss));
