@@ -118,6 +118,7 @@ def lib():
     L.icmslam_filtrar_obs.argtypes = [vp, vp, i32, i32, i64, dbl, i32, vp, i64, i32]
     L.icmslam_associate.argtypes = [vp, vp, i32, i64, vp, vp, i32, vp, i32, i64, vp, i32]
     L.icmslam_iterate_until.argtypes = [vp, vp, i32, dbl, C.POINTER(SweepOpts), vp, _ip]
+    L.icmslam_batch_iterate_until.argtypes = [vp, i32, dbl, dbl, i32, C.POINTER(SweepOpts), vp, _ip, _ip]
     for name in EXPORTS:
         getattr(L, name)  # fail loudly if the header and the library disagree
         if name not in ("icmslam_strerror", "icmslam_last_error"):
@@ -134,6 +135,7 @@ EXPORTS = [
     "icmslam_calc_cambio", "icmslam_filtrar_obs", "icmslam_set_map", "icmslam_get_map", "icmslam_iterate",
     "icmslam_get_kernel_ms", "icmslam_get_launch_count", "icmslam_get_transfer_bytes", "icmslam_set_poses", "icmslam_get_poses", "icmslam_set_segment", "icmslam_device_ptr", "icmslam_seg_begin",
     "icmslam_seg_exchange", "icmslam_seg_halo", "icmslam_p2p_export", "icmslam_p2p_import", "icmslam_get_trace", "icmslam_pose_eval", "icmslam_seg_finish", "icmslam_fcluster", "icmslam_pass0", "icmslam_associate", "icmslam_iterate_until", "icmslam_set_counts", "icmslam_set_batch",
+    "icmslam_batch_iterate_until",
 ]
 
 

@@ -8,7 +8,9 @@ sweeps of a rank's handles are enqueued back to back on their own streams, so sm
     for i in batch.owned(n_traj):
         batch.add(i, z_i, odo_i, u_i, map_i, x_i)
     batch.finalize()                                  # (ConcatBatch only)
-    batch.iterate(30)
+    batch.iterate(30)                                 # a fixed number of sweeps of every trajectory, or
+    conv = batch.iterate_until(60, tol)               # each trajectory until its own largest landmark change is <= tol (the
+                                                      # reference's stop rule, sensors.py:302-315): {i: (n_done, cambios (n_done, 3))}
     res = batch.results()          # {i: (x (3 x T), mapa (2 x L))}
     allres = gather_results(res)   # optional, for output only (torch.distributed all_gather_object)
 """
@@ -54,6 +56,10 @@ class TrajectoryBatch:
         for _ in range(int(n_sweeps)):
             for idx, e in self._eng.items():
                 e.iterate(None, self._x0[idx], 1, **mode)
+
+    def iterate_until(self, max_sweeps: int, tol: float):
+        """Engine.iterate_until of every owned trajectory: {trajectory index: (n_done, cambios (n_done, 3))}."""
+        return {idx: e.iterate_until(self._x0[idx], int(max_sweeps), float(tol)) for idx, e in self._eng.items()}
 
     def results(self):
         return {idx: (e.get_poses(), e.get_map()) for idx, e in self._eng.items()}
@@ -141,6 +147,13 @@ class ConcatBatch:
 
     def iterate(self, n_sweeps: int = 1, **mode):
         self.engine.iterate(None, self.x0s[:, 0], int(n_sweeps), **mode)
+
+    def iterate_until(self, max_sweeps: int, tol: float):
+        """Each trajectory sweeps until its own largest landmark change is <= tol (at most max_sweeps), exactly as
+        Engine.iterate_until on it alone; a trajectory that has stopped is frozen on the device while the others sweep on
+        (Engine.batch_iterate_until).  {trajectory index: (n_done, cambios (n_done, 3))}, keyed like results()."""
+        _, n_done, cam = self.engine.batch_iterate_until(int(max_sweeps), float(tol), self.spacing, 64)
+        return {it[0]: (int(n_done[k]), cam[k, : n_done[k]].copy()) for k, it in enumerate(self._items)}
 
     def results(self):
         """{trajectory index: (x (3 x T), mapa (2 x L))} in each trajectory's own frame; a landmark belongs to the region it lies in."""

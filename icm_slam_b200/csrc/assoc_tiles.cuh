@@ -408,7 +408,7 @@ k_assoc_tiles(const AssocParams p)
         __syncthreads();     // the block's records and slot table are visible to its warps
         tile_stage(R, S.tile, tile, nslots);
         __syncthreads();
-        if (warp < RT_SLICES) process_slice<false>(R, S.tile, tile * RT_SLICES + warp, tile, commit_all);
+        if (warp < RT_SLICES) process_slice<false, true>(R, S.tile, tile * RT_SLICES + warp, tile, commit_all);
         __syncthreads();
         stats_flush(R, S.tile, tile, nslots);
         __syncthreads();

@@ -19,6 +19,37 @@ struct DevCfg {
     int L;
 };
 
+// Per-trajectory freezing of a batch handle (icmslam_batch_iterate_until).  frozen == nullptr on every other path, where every
+// test below is one uniform branch.  Landmark ownership is stateless: region k = rint(y / pitch) * cols + rint(x / pitch).
+#define FZ_SLOTS 5     // per-trajectory results of a sweep: min, max, sum of the resolved changes, new landmarks, unresolved ones
+struct Freeze {
+    const unsigned char* frozen;   // K bytes: trajectory k is frozen
+    int traj_T;                    // columns per trajectory: scan t belongs to trajectory t / traj_T
+    int K, cols;
+    double pitch;
+    double* slots;                 // FZ_SLOTS x K (row r, trajectory k): calc_cambio of each trajectory's landmarks
+    __device__ __forceinline__ int region(double x, double y) const
+    {
+        const double k = rint(y / pitch) * (double)cols + rint(x / pitch);
+        return (k >= 0.0 && k < (double)K) ? (int)k : -1;
+    }
+    __device__ __forceinline__ bool scan(int t) const { return frozen != nullptr && frozen[t / traj_T] != 0; }
+    __device__ __forceinline__ bool landmark(double x, double y) const
+    {
+        if (frozen == nullptr) return false;
+        const int k = region(x, y);
+        return k >= 0 && frozen[k] != 0;
+    }
+    // (grid-stride over the trajectories by thread i of n)
+    __device__ __forceinline__ void reset_slots(int i, int n) const
+    {
+        for (int k = i; k < K; k += n) {
+            slots[k] = INFINITY;
+            for (int r = 1; r < FZ_SLOTS; ++r) slots[(size_t)r * K + k] = 0.0;
+        }
+    }
+};
+
 // Status word written by kernels (checked by the host after the sweep).
 enum { ST_OK = 0, ST_LABEL_CAP = 1, /* 4: empty map */ ST_P2P_TIMEOUT = 8 };
 

@@ -109,9 +109,13 @@ struct icmslam_handle {
     int* d_remap = nullptr;             // label of the last sweep -> label in the current map
     int* d_klab = nullptr;              // raw label of each kept landmark (fast tail)
     int traj_T = 0, traj_K = 0; double* d_x0s = nullptr;   // batch of independent trajectories laid end to end (icmslam_set_batch)
+    // per-trajectory freezing (icmslam_batch_iterate_until): fz.frozen is null outside that call
+    Freeze fz = {};
+    unsigned char *d_fz_mask = nullptr, *d_fz_need = nullptr; double* d_fz_slots = nullptr; int* d_fz_reg = nullptr; int fz_K = 0;
+    int fz_fallbacks = 0;      // sweeps of the last icmslam_batch_iterate_until that needed the full calc_cambio search
     double* d_aobs = nullptr; int* d_ac = nullptr;   // icmslam_associate: one scan's observations (2 x ASSOC_MAX_OBS) and labels
     double thr1sq = 0.0;
-    struct GraphSlot { cudaGraphExec_t exec = nullptr; const double* src = nullptr; const double* map_in = nullptr; double x0[3] = {0, 0, 0}; double tol = 0; int maxit = 0; int lm = 0; };
+    struct GraphSlot { cudaGraphExec_t exec = nullptr; const double* src = nullptr; const double* map_in = nullptr; double x0[3] = {0, 0, 0}; double tol = 0; int maxit = 0; int lm = 0; Freeze fz = {}; };
     GraphSlot graphs[4];
     int use_graph = 1, graph_launches = 0;
     int runs_occ = 24;           // resident one-warp blocks per SM k_runs is compiled for (24: 80 registers; ICMSLAM_RUNS_OCC=32: 64)
@@ -197,6 +201,12 @@ extern "C" const char* icmslam_strerror(int s)
 
 extern "C" const char* icmslam_last_error(const icmslam_handle* h) { return h ? h->err : "null handle"; }
 
+// (a captured sweep holds the freeze arguments it was captured with)
+static bool same_freeze(const Freeze& a, const Freeze& b)
+{
+    return a.frozen == b.frozen && a.traj_T == b.traj_T && a.K == b.K && a.cols == b.cols && a.pitch == b.pitch && a.slots == b.slots;
+}
+
 static void drop_graphs(icmslam_handle* h)
 {
     for (auto& g : h->graphs) { if (g.exec) cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
@@ -218,6 +228,7 @@ static void free_dataset(icmslam_handle* h)
     h->last_map_L = -1;
     h->traj_T = 0; h->traj_K = 0;
     DFREE(h->d_x0s);
+    DFREE(h->d_fz_mask); DFREE(h->d_fz_need); DFREE(h->d_fz_slots); DFREE(h->d_fz_reg); h->fz_K = 0;
     h->fused_ok = false;
     h->extracted = false;
     h->n = 0;
@@ -864,6 +875,13 @@ struct HostPipe { double* x; int64_t ld; int chunks; };      // the caller's hos
 
 static bool pipe_ready(icmslam_handle* h);
 
+static void launch_runs(icmslam_handle* h, int blocks, cudaStream_t s, const RunParams& R)
+{
+    const bool fz = R.fz.frozen != nullptr;
+    if (h->runs_occ == 32) { if (fz) k_runs<32, true><<<blocks, RUNS_THREADS, 0, s>>>(R); else k_runs<32, false><<<blocks, RUNS_THREADS, 0, s>>>(R); }
+    else { if (fz) k_runs<24, true><<<blocks, RUNS_THREADS, 0, s>>>(R); else k_runs<24, false><<<blocks, RUNS_THREADS, 0, s>>>(R); }
+}
+
 static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, double* kout, int64_t kld, const double* x0,
                         const icmslam_sweep_opts& o, int n_search_cap, bool overlap = false, const HostPipe* hp = nullptr)
 {
@@ -900,7 +918,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     R.far_list = h->d_far_list; R.ts = h->d_ts; R.farbits = h->d_farbits;
     R.scan_dirty = h->d_scan_dirty; R.tile_flag = h->d_tile_flag; R.dirty_list = h->d_dirty_list;
     R.geom = h->d_fg_geom; R.cell_start = h->d_fg_start; R.gpts = h->d_fg_pts; R.dist_thr = h->dcfg.dist_thr;
-    R.st = st; R.L_in = h->begin_L; R.slice0 = 0;
+    R.st = st; R.L_in = h->begin_L; R.slice0 = 0; R.fz = h->fz;
     AssocParams A;
     A.first_halo = h->seg_first ? 0 : 1; A.T = T; A.off = h->d_off; A.bxy = h->d_bxy; A.cfg = h->dcfg; A.thr2_hi = h->thr2_hi; A.st = st; A.geom = h->d_fg_geom;
     A.cell_start = h->d_fg_start; A.gpts = h->d_fg_pts; A.gidx = h->d_fg_idx; A.remap = h->d_remap;
@@ -916,7 +934,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
         P.xin = xin; P.ldin = ldin; P.xout = kout; P.ldout = kld;
         P.inc = h->d_inc; P.ldinc = T; P.u = h->d_u; P.ldu = T; P.bm = h->d_bm; P.ldbm = T; P.dyn = h->d_dyn;
         P.ppin = pp_in; P.ppout = pp_out; P.cfg = h->dcfg; P.tol = o.newton_tol; P.maxit = o.newton_maxit; P.iters = nullptr; P.tile0 = 0;
-        P.trace_row = nullptr; P.trace_seq = nullptr;
+        P.trace_row = nullptr; P.trace_seq = nullptr; P.fz = h->fz;
         const int C = hp->chunks, per = (h->n_tiles + C - 1) / C;
         cudaStream_t sin = h->h2d_stream, sout = h->side_stream;
         CK(cudaEventRecord(h->ev_fork, s));
@@ -937,8 +955,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (tile_b > tile_a) {
                 k_ppar_init<<<nblk(b - a, 256), 256, 0, s>>>(xin, ldin, a, b, P.lay, pp_in);
                 R.slice0 = tile_a * RT_SLICES;
-                if (h->runs_occ == 32) k_runs<32><<<(tile_b - tile_a) * RT_SLICES, RUNS_THREADS, 0, s>>>(R);
-                else k_runs<24><<<(tile_b - tile_a) * RT_SLICES, RUNS_THREADS, 0, s>>>(R);
+                launch_runs(h, (tile_b - tile_a) * RT_SLICES, s, R);
                 h->n_launch += 2;
             }
             A.final = last ? 1 : 0;
@@ -950,7 +967,8 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (ready > h->n_solve_tiles) ready = h->n_solve_tiles;
             if (ready > solved) {
                 P.tile0 = solved;
-                k_solve_tile<<<ready - solved, ST_THREADS, 0, s>>>(P);
+                if (P.fz.frozen) k_solve_tile<true><<<ready - solved, ST_THREADS, 0, s>>>(P);
+                else k_solve_tile<false><<<ready - solved, ST_THREADS, 0, s>>>(P);
                 CK(cudaGetLastError());
                 h->n_launch += 1;
                 CK(cudaEventRecord(h->ev_out[c], s));
@@ -969,8 +987,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     }
     if (timing) CK(cudaEventRecord(h->ev[0], s));
     if (h->use_runs) {
-        if (h->runs_occ == 32) k_runs<32><<<h->n_tiles * RT_SLICES, RUNS_THREADS, 0, s>>>(R);
-        else k_runs<24><<<h->n_tiles * RT_SLICES, RUNS_THREADS, 0, s>>>(R);
+        launch_runs(h, h->n_tiles * RT_SLICES, s, R);
     } else {
         k_all_dirty<<<nblk(h->n_tiles, 256), 256, 0, s>>>(h->d_tile_flag, h->d_dirty_list, h->d_ts, h->n_tiles, st, h->begin_L);
     }
@@ -992,6 +1009,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
         P.ppin = pp_in; P.ppout = pp_out; P.cfg = h->dcfg; P.tol = o.newton_tol; P.maxit = o.newton_maxit;
         P.iters = (o.reserved & 1) ? &st->newton_iters : nullptr; P.tile0 = 0;
         P.trace_row = h->trace_on ? &h->d_ts->trace[0][0] : nullptr; P.trace_seq = h->p2p.on ? &h->d_ts->halo_seq : &h->d_ts->sweep_no;
+        P.fz = h->fz;
         cudaStream_t ss = s;
         const bool fork = overlap && h->overlap_solve && !timing && h->side_stream;
         if (fork) {      // the tail does not depend on the new poses: solve beside it
@@ -999,7 +1017,8 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             CK(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
             ss = h->side_stream;
         }
-        k_solve_tile<<<h->n_solve_tiles, ST_THREADS, 0, ss>>>(P);
+        if (P.fz.frozen) k_solve_tile<true><<<h->n_solve_tiles, ST_THREADS, 0, ss>>>(P);
+        else k_solve_tile<false><<<h->n_solve_tiles, ST_THREADS, 0, ss>>>(P);
         CK(cudaGetLastError());
         if (h->d2h_x) {      // a host-memory caller: its poses start their way back as soon as they are solved, beside the tail
             CK(cudaMemcpy2DAsync(h->d2h_x, (size_t)h->d2h_ld * 8, kout, (size_t)kld * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, ss));
@@ -1063,7 +1082,7 @@ static int fused_part_c(icmslam_handle* h, double* dmap_out, int out_cap, int64_
         a.gbuild = h->d_gbuild; a.nnd0 = h->d_nnd0; a.gslots = h->d_gslots; a.gpts = h->d_fg_pts;
         a.raw_x = raw_x; a.raw_y = raw_y; a.rawcnt = h->d_rawcnt;
         a.map_out = dmap_out; a.cap_out = out_cap; a.ld_out = out_ld; a.counts_state = h->d_counts; a.remap = h->d_remap; a.Lcap = L;
-        a.cpart = h->d_cpart;
+        a.cpart = h->d_cpart; a.fz = h->fz;
         a.sh_x = h->d_sh_x; a.sh_y = h->d_sh_y; a.sh_k = h->d_sh_k; a.farbits = h->d_farbits; a.n_far_words = h->n_tiles * 4;
         a.use_cond = 0;
         memset(&a.cond, 0, sizeof a.cond);
@@ -1080,7 +1099,8 @@ static int fused_part_c(icmslam_handle* h, double* dmap_out, int out_cap, int64_
                 a.use_cond = 1;
             else { cudaGetLastError(); cgraph = nullptr; }
         }
-        k_tail_steady<<<nblk(L, 256), 256, 0, s>>>(st, ts, a, h->p2p);
+        if (a.fz.frozen) k_tail_steady<true><<<nblk(L, 256), 256, 0, s>>>(st, ts, a, h->p2p);
+        else k_tail_steady<false><<<nblk(L, 256), 256, 0, s>>>(st, ts, a, h->p2p);
         CK(cudaGetLastError());
         h->n_launch += 1;
         if (a.use_cond) {
@@ -1129,7 +1149,7 @@ static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t 
     {
     k_fused_means<<<nblk(L, 256), 256, 0, s>>>(st, h->d_fsum_x, h->d_fsum_y, h->d_cnt, min_x, min_y, 1.0 / h->fix_scale, h->dcfg.cota,
                                                h->d_newraw, raw_x, raw_y, h->d_kflag, L, h->d_blk_kept, h->d_farbits, h->n_tiles * 4, h->p2p, ts,
-                                               h->d_cnt, st, h->d_sh_x, h->d_sh_y, h->d_sh_k);
+                                               h->d_cnt, st, h->d_sh_x, h->d_sh_y, h->d_sh_k, h->fz, h->d_counts);
     CK(cudaGetLastError());
     k_tail_compact<<<nblk(L, 256), 256, 0, s>>>(st, h->d_kflag, h->d_blk_kept, h->d_kpos, raw_x, raw_y, h->d_cnt, h->d_kx, h->d_ky, h->d_kc,
                                                 h->d_parent, h->d_bb, L, h->d_klab, h->d_rawcnt, ts);
@@ -1146,7 +1166,7 @@ static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t 
         sa.dist_thr = h->dcfg.dist_thr; sa.parent = h->d_parent; sa.ind_pos = h->d_indpos; sa.ind = h->d_ind; sa.lab = h->d_lab; sa.used = h->d_used;
         sa.rank = h->d_rank; sa.ox = h->d_ox; sa.oy = h->d_oy; sa.oc = h->d_oc; sa.max_cells = h->fg_cells; sa.geom = h->d_fg_geom;
         sa.cell_cnt = h->d_fg_cnt; sa.cell_start = h->d_fg_start; sa.pts = h->d_fg_pts; sa.gidx = h->d_fg_idx;
-        sa.gbuild = h->d_gbuild; sa.nnd0 = h->d_nnd0; sa.steady_enable = h->steady_enable;
+        sa.gbuild = h->d_gbuild; sa.nnd0 = h->d_nnd0; sa.steady_enable = h->steady_enable; sa.fz = h->fz;
         k_tail_nn<<<nblk(L, 256), 256, 0, s>>>(st, ts, h->d_kx, h->d_ky, h->d_kc, h->d_fg_geom, h->d_fg_start, h->d_fg_pts, h->d_fg_idx, h->thr2_lt,
                                                h->d_nn, h->d_indflag, L, h->d_klab, h->d_kflag, h->d_kpos, h->d_lmrec2[h->lm_cur],
                                                h->d_lmrec2[h->lm_cur ^ 1], dmap_out, out_cap, out_ld, h->d_counts, h->thr1sq, h->thr2_hi, h->d_remap, sa);
@@ -1518,7 +1538,7 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
             icmslam_handle::GraphSlot* slot = nullptr;
             for (auto& g : h->graphs)
                 if (g.exec && g.src == src && g.map_in == h->d_map_in && g.x0[0] == x0[0] && g.x0[1] == x0[1] && g.x0[2] == x0[2] &&
-                    g.tol == o.newton_tol && g.maxit == o.newton_maxit && g.lm == h->lm_cur) slot = &g;
+                    g.tol == o.newton_tol && g.maxit == o.newton_maxit && g.lm == h->lm_cur && same_freeze(g.fz, h->fz)) slot = &g;
             if (!slot) {
                 for (auto& g : h->graphs) if (!g.exec) { slot = &g; break; }
                 if (!slot) { drop_graphs(h); slot = &h->graphs[0]; }
@@ -1549,7 +1569,7 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
                 cudaGraphDestroy(graph);
                 if (ce != cudaSuccess) { slot->exec = nullptr; snprintf(h->err, sizeof h->err, "cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return ICMSLAM_ERR_CUDA; }
                 slot->src = src; slot->map_in = h->d_map_in; slot->x0[0] = x0[0]; slot->x0[1] = x0[1]; slot->x0[2] = x0[2];
-                slot->tol = o.newton_tol; slot->maxit = o.newton_maxit; slot->lm = lm;
+                slot->tol = o.newton_tol; slot->maxit = o.newton_maxit; slot->lm = lm; slot->fz = h->fz;
             }
             CK(cudaGraphLaunch(slot->exec, s));
             h->n_launch += h->graph_launches;    // kernels of this library inside the graph
@@ -2005,9 +2025,10 @@ extern "C" int icmslam_get_sweep_stats(icmslam_handle* h, int64_t* stats, int32_
     const DevState* s = h->h_st;
     TailState hts;
     CK(cudaMemcpy(&hts, h->d_ts, sizeof(TailState), cudaMemcpyDeviceToHost));
-    int64_t v[16] = {(int64_t)s->newton_iters, s->n_far_scans, s->raw_l, s->kept, s->new_l, s->n_ind, s->lsearch, s->status, s->dirty_tiles,
-                     hts.epoch, (int64_t)h->n_tiles, hts.remap_identity, (int64_t)(h->last_runs_ms * 1e6), hts.n_dirty, hts.far_count, hts.steady_sweeps};
-    for (int i = 0; i < n && i < 16; ++i) stats[i] = v[i];
+    int64_t v[17] = {(int64_t)s->newton_iters, s->n_far_scans, s->raw_l, s->kept, s->new_l, s->n_ind, s->lsearch, s->status, s->dirty_tiles,
+                     hts.epoch, (int64_t)h->n_tiles, hts.remap_identity, (int64_t)(h->last_runs_ms * 1e6), hts.n_dirty, hts.far_count, hts.steady_sweeps,
+                     h->fz_fallbacks};
+    for (int i = 0; i < n && i < 17; ++i) stats[i] = v[i];
     return ICMSLAM_OK;
 }
 
@@ -2233,6 +2254,115 @@ extern "C" int icmslam_iterate_until(icmslam_handle* h, const double* x0, int32_
         if (tol_max_change > 0.0 && tri[1] <= tol_max_change) break;
     }
     return ICMSLAM_OK;
+}
+
+// ---- the same driver loop for a batch handle, one monitor per trajectory -------------------------------------------------
+// Each trajectory stops at its own first sweep whose largest landmark change is <= tol: from the next sweep on it is frozen on the
+// device (Freeze: its scans commit nothing, its poses and landmarks pass through unchanged) while the others sweep on.
+__global__ void k_fz_reset(const Freeze fz) { fz.reset_slots(blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x); }
+
+static int batch_until_loop(icmslam_handle* h, int max_sweeps, double tol, const icmslam_sweep_opts& o, double* cambios, int32_t* n_done,
+                            int32_t* n_run)
+{
+    const int K = h->traj_K, L = h->Lcap;
+    cudaStream_t s = h->stream;
+    double x0[3];
+    for (int r = 0; r < 3; ++r) CK(cudaMemcpyAsync(x0 + r, h->d_x0s + (size_t)r * K, sizeof(double), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    std::vector<unsigned char> frozen((size_t)K, 0);
+    std::vector<double> sl((size_t)FZ_SLOTS * K);
+    int active = K;
+    for (int it = 0; it < max_sweeps && active > 0; ++it) {
+        int rc = sync_state(h);
+        if (rc) return rc;
+        const int L_old = h->h_st->lact;
+        k_fz_reset<<<nblk(K, 256), 256, 0, s>>>(h->fz);
+        CK(cudaGetLastError());
+        rc = icmslam_iterate(h, nullptr, 0, x0, 1, &o, ICMSLAM_DEVICE);
+        if (rc) return rc;
+        rc = sync_state(h);
+        if (rc) return rc;
+        rc = status_from_state(h->h_st);
+        if (rc) return rc;
+        const int L_new = h->h_st->new_l;
+        CK(cudaMemcpyAsync(sl.data(), h->d_fz_slots, sl.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        bool need = false;
+        for (int k = 0; k < K; ++k) need = need || (!frozen[k] && sl[(size_t)4 * K + k] > 0.0);
+        if (need && L_new > 0 && L_old > 0) {      // the full search for the trajectories the tail could not settle (new map = d_map_in)
+            k_fz_regions<<<nblk(L_old, 256), 256, 0, s>>>(h->fz, h->d_map_out, h->d_map_out + L, L_old, h->d_fz_reg);
+            CK(cudaGetLastError());
+            k_fz_need<<<nblk(K, 256), 256, 0, s>>>(h->fz, h->d_fz_need);
+            CK(cudaGetLastError());
+            k_cambio_regions<<<nblk(L_new, 128), 128, 0, s>>>(h->fz, h->d_fz_need, h->d_map_in, h->d_map_in + L, L_new, h->d_map_out,
+                                                              h->d_map_out + L, h->d_fz_reg, L_old);
+            CK(cudaGetLastError());
+            h->n_launch += 3;
+            h->fz_fallbacks += 1;
+            CK(cudaMemcpyAsync(sl.data(), h->d_fz_slots, sl.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
+            CK(cudaStreamSynchronize(s));
+        }
+        for (int k = 0; k < K; ++k) {
+            if (frozen[k]) continue;
+            const double tri[3] = {sl[k], sl[(size_t)K + k], sl[(size_t)2 * K + k] / sl[(size_t)3 * K + k]};
+            if (cambios)
+                for (int r = 0; r < 3; ++r) cambios[((size_t)r * K + k) * max_sweeps + it] = tri[r];
+            n_done[k] = it + 1;
+            if (tol > 0.0 && tri[1] <= tol) { frozen[k] = 1; --active; }
+        }
+        *n_run = it + 1;
+        if (active > 0 && it + 1 < max_sweeps) CK(cudaMemcpyAsync(h->d_fz_mask, frozen.data(), (size_t)K, cudaMemcpyHostToDevice, s));
+    }
+    CK(cudaStreamSynchronize(s));      // (the staging vector of the last mask upload goes away)
+    return ICMSLAM_OK;
+}
+
+extern "C" int icmslam_batch_iterate_until(icmslam_handle* h, int32_t max_sweeps, double tol_max_change, double region_pitch,
+                                           int32_t region_cols, const icmslam_sweep_opts* opts, double* cambios, int32_t* n_done,
+                                           int32_t* n_run)
+{
+    if (!h || !n_done || !n_run || max_sweeps < 0 || !(region_pitch > 0.0) || region_cols <= 0 || h->traj_T <= 0 || !h->d_x0s)
+        return ICMSLAM_ERR_INVALID;
+    icmslam_sweep_opts o;
+    default_opts(o, opts);
+    if (!(h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON && o.map_view == ICMSLAM_VIEW_PREV) ||
+        h->p2p.on || !h->seg_first || !h->seg_last)
+        return ICMSLAM_ERR_UNSUPPORTED;
+    CK(cudaSetDevice(h->cfg.device));
+    const int K = h->traj_K, L = h->Lcap;
+    cudaStream_t s = h->stream;
+    *n_run = 0;
+    for (int k = 0; k < K; ++k) n_done[k] = 0;
+    {   // every landmark of the starting map belongs to one of the K regions
+        int rc = sync_state(h);
+        if (rc) return rc;
+        const int L0 = h->h_st->lact;
+        std::vector<double> m((size_t)2 * L0);
+        if (L0 > 0) CK(cudaMemcpy2DAsync(m.data(), (size_t)L0 * 8, h->d_map_in, (size_t)L * 8, (size_t)L0 * 8, 2, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        for (int l = 0; l < L0; ++l) {
+            const double k = rint(m[(size_t)L0 + l] / region_pitch) * (double)region_cols + rint(m[l] / region_pitch);
+            if (!(k >= 0.0 && k < (double)K)) {
+                snprintf(h->err, sizeof h->err, "landmark %d at (%g, %g) lies outside the %d trajectory regions", l, m[l], m[(size_t)L0 + l], K);
+                return ICMSLAM_ERR_INVALID;
+            }
+        }
+    }
+    if (h->fz_K != K) {
+        DFREE(h->d_fz_mask); DFREE(h->d_fz_need); DFREE(h->d_fz_slots); DFREE(h->d_fz_reg);
+        h->fz_K = 0;
+        drop_graphs(h);      // (graphs of an earlier call hold the old buffers)
+        CK(dalloc(&h->d_fz_mask, (size_t)K)); CK(dalloc(&h->d_fz_need, (size_t)K));
+        CK(dalloc(&h->d_fz_slots, (size_t)FZ_SLOTS * K)); CK(dalloc(&h->d_fz_reg, (size_t)L));
+        h->fz_K = K;
+    }
+    CK(cudaMemsetAsync(h->d_fz_mask, 0, (size_t)K, s));
+    h->fz.frozen = h->d_fz_mask; h->fz.traj_T = h->traj_T; h->fz.K = K; h->fz.cols = region_cols; h->fz.pitch = region_pitch;
+    h->fz.slots = h->d_fz_slots;
+    h->fz_fallbacks = 0;
+    const int rc = batch_until_loop(h, max_sweeps, tol_max_change, o, cambios, n_done, n_run);
+    h->fz = Freeze{};      // every trajectory unfrozen: later sweeps run the plain batch path
+    return rc;
 }
 
 extern "C" int icmslam_filtrar_obs(icmslam_handle* h, const double* obs, int32_t B, int32_t T, int64_t ld, double max_dist,

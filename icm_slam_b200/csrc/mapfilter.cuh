@@ -229,3 +229,45 @@ __global__ void k_cambio(DevState* st, const double* __restrict__ nx_, const dou
         atomicAdd(acc + 2, sm);
     }
 }
+
+// ---- calc_cambio per trajectory of a batch handle (icmslam_batch_iterate_until) --------------------------------------------
+// The tail (k_tail_nn / k_tail_steady) fills each trajectory's slots (Freeze::slots) with the changes it could certify.  A
+// trajectory with an uncertified change (a landmark that left its proven radius, appeared or merged) gets the full search here,
+// as calc_cambio computes it for the trajectory alone: every new landmark against every old landmark of the same region.  Brute
+// force over the old map: it runs only on the sweeps that need it.
+__global__ void k_fz_regions(const Freeze fz, const double* __restrict__ x, const double* __restrict__ y, int n, int* __restrict__ reg)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) reg[i] = fz.region(x[i], y[i]);
+}
+
+// the active trajectories with uncertified changes: need[k] = 1 and their min / max / sum / count slots cleared
+__global__ void k_fz_need(const Freeze fz, unsigned char* __restrict__ need)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= fz.K) return;
+    const bool nd = !fz.frozen[k] && fz.slots[4 * (size_t)fz.K + k] > 0.0;
+    need[k] = nd ? 1 : 0;
+    if (nd) {
+        fz.slots[k] = INFINITY;
+        for (int r = 1; r < 4; ++r) fz.slots[(size_t)r * fz.K + k] = 0.0;
+    }
+}
+
+__global__ void k_cambio_regions(const Freeze fz, const unsigned char* __restrict__ need, const double* __restrict__ nx_,
+                                 const double* __restrict__ ny_, int Ln, const double* __restrict__ oldx, const double* __restrict__ oldy,
+                                 const int* __restrict__ oreg, int Lo)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= Ln) return;
+    const double xj = nx_[j], yj = ny_[j];
+    const int k = fz.region(xj, yj);
+    if (k < 0 || !need[k]) return;
+    double best = INFINITY;
+    for (int i = 0; i < Lo; ++i)
+        if (__ldg(oreg + i) == k) best = fmin(best, dist_rn(__ldg(oldx + i) - xj, __ldg(oldy + i) - yj));
+    atomic_min_pos(fz.slots + k, best);
+    atomic_max_pos(fz.slots + (size_t)fz.K + k, best);
+    atomicAdd(fz.slots + 2 * (size_t)fz.K + k, best);
+    atomicAdd(fz.slots + 3 * (size_t)fz.K + k, 1.0);
+}

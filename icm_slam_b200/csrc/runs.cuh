@@ -103,6 +103,7 @@ struct RunParams {
     int* scan_dirty; int* tile_flag; int* dirty_list;     // steady state: what failed validation (tile_flag: 1 some scans, 2 all)
     const FGeom* geom; const int* cell_start; const double2* gpts;   // the landmark grid (fastgrid.cuh), for the far runs
     double dist_thr;
+    Freeze fz;                            // a frozen trajectory's scans commit nothing (no moments, statistics or far records)
 };
 
 // A far run stays far if no landmark can be within the gate of any of its observations.  Every observation lies within rho of
@@ -203,8 +204,8 @@ __device__ __forceinline__ RunEval run_eval(const RunParams& p, const TileSmem& 
 // One slice (32 scans, one per lane) by one warp.  STEADY: every run is certified before it is committed; a scan with a run
 // that cannot be certified takes back what it committed, is marked dirty and returns false for its lane.  !STEADY (the
 // association kernel has just written the records): no certification; only the scans with commit_all or a dirty flag are
-// committed.
-template <bool STEADY>
+// committed.  FZ: the scans of frozen trajectories (p.fz) commit nothing (compiled out of the steady kernel of the plain sweep).
+template <bool STEADY, bool FZ>
 __device__ __forceinline__ bool process_slice(const RunParams& p, TileSmem& S, int slice, int tile, bool commit_all, SliceRing* ring = nullptr)
 {
     const int lane = threadIdx.x & 31;
@@ -219,7 +220,7 @@ __device__ __forceinline__ bool process_slice(const RunParams& p, TileSmem& S, i
     const int lt = p.tile_perm[ppos];
     const int nr0 = p.pos_nruns[ppos];
     const int t = p.t_start + tile * RT_TILE + lt;
-    const bool in = t < p.t_hi;
+    const bool in = t < p.t_hi && !(FZ && p.fz.scan(t));
     const int nr = in ? nr0 : 0;
     const bool halo = t == p.halo_t;
     bool commit = in && nr > 0;
@@ -313,7 +314,7 @@ __device__ __forceinline__ bool process_slice(const RunParams& p, TileSmem& S, i
 
 // steady state: one WARP per slice and block (no block barrier: a slice that needs more steps than its neighbours holds nobody
 // up); every block stages its tile's slot table
-template <int MINB>      // resident blocks per SM the kernel is compiled for
+template <int MINB, bool FZ>      // resident blocks per SM the kernel is compiled for; FZ: a batch with frozen trajectories
 __global__ void __launch_bounds__(RUNS_THREADS, MINB)
 k_runs(const RunParams p)
 {
@@ -327,7 +328,7 @@ k_runs(const RunParams p)
         return;
     }
     tile_stage(p, S, tile, nslots);      // (its two dependent loads overlap those of process_slice's prologue: no barrier in between)
-    process_slice<true>(p, S, slice, tile, true, &ring);
+    process_slice<true, FZ>(p, S, slice, tile, true, &ring);
     __syncwarp();
     stats_flush(p, S, tile, nslots);
 }

@@ -226,6 +226,7 @@ struct SolveParams {
     int tile0;                            // first tile of this launch
     unsigned long long* trace_row;        // instrumentation: ring of %globaltimer marks (or null), indexed by *trace_seq
     const unsigned* trace_seq;
+    Freeze fz;                            // a frozen trajectory's poses (and projection parameters) are copied through, not solved
 };
 
 struct __align__(16) SolveSmem {
@@ -243,6 +244,7 @@ struct SlotMom {
     int t, li;
 };
 
+template <bool FZ>
 __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb, int q, int phase)
 {
     SlotMom s;
@@ -251,7 +253,9 @@ __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb,
     // (phase 0, slot 0 = the odd pose tb-1 left of the tile: re-solved here because the even pose tb needs its NEW value;
     //  phase 1, last slot = tb+ST_OWN: the next tile's)
     s.valid = s.t >= 0 && s.t < p.t_hi && (phase == 0 ? (q == 0 || s.t >= p.t_lo) : (q != ST_SLOTS - 1 && s.t >= p.t_lo));
-    s.pinned = s.valid && p.lay.pinned(s.t);
+    // (a frozen pose is handled like a pinned one: its input value passes through; the trajectory's first pose is pinned and its
+    //  last has no successor, so no pose of another trajectory reads it)
+    s.pinned = s.valid && (p.lay.pinned(s.t) || (FZ && p.fz.scan(s.t)));
     Mom& M = s.M;
     M.n = M.Bx = M.By = M.Bxx = M.Byy = M.Bxy = M.Yx = M.Yy = M.Mxx = M.Mxy = M.Myx = M.Myy = 0.0;
     if (s.valid && !s.pinned) {
@@ -267,6 +271,8 @@ __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb,
     return s;
 }
 
+// FZ: a batch with frozen trajectories (p.fz); the plain sweep launches the instance without the test
+template <bool FZ>
 __global__ void __launch_bounds__(ST_THREADS, ST_MINB)
 k_solve_tile(const SolveParams p)
 {
@@ -275,7 +281,7 @@ k_solve_tile(const SolveParams p)
     if (p.trace_row && blockIdx.x == 0 && q == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); p.trace_row[((*p.trace_seq) & 31) * 8 + 5] = t; }
     const int tb = p.t_lo + (p.tile0 + blockIdx.x) * ST_OWN;      // t_lo is even: colours stay aligned with the global time index
     const int T = p.T;
-    SlotMom cur = solve_slot_load(p, tb, q, 0);      // (in flight while the tile is staged)
+    SlotMom cur = solve_slot_load<FZ>(p, tb, q, 0);      // (in flight while the tile is staged)
     for (int li = q; li < ST_XT; li += ST_THREADS) {
         const int t = tb - 2 + li;
         const bool ok = t >= 0 && t < T;
@@ -340,7 +346,7 @@ k_solve_tile(const SolveParams p)
             if (solve) { rx = x2; ry = y2; th = th2; my_iters += it; }
         }
         SlotMom nxt = cur;
-        if (phase == 0) nxt = solve_slot_load(p, tb, q, 1);      // (the even pose's moments arrive during the barrier)
+        if (phase == 0) nxt = solve_slot_load<FZ>(p, tb, q, 1);      // (the even pose's moments arrive during the barrier)
         if (qvalid && !pinned) {
             // the new heading's sin/cos exactly as next sweep's projection forms them (one sincos per pose per sweep)
             double st, ct;
@@ -362,6 +368,7 @@ k_solve_tile(const SolveParams p)
     for (int k = q; k < n_own; k += ST_THREADS) {
         const int tt = tb + k, l2 = k + 2;
         if (p.lay.pinned(tt)) p.ppout[tt] = make_ppar(p.lay.x0_of(tt, 0), p.lay.x0_of(tt, 1), p.lay.x0_of(tt, 2));
+        else if (FZ && p.fz.scan(tt)) p.ppout[tt] = ldg_ppar(p.ppin + tt);
         else p.ppout[tt] = make_double4(S.xn[0][l2], S.xn[1][l2], -S.cs[l2], S.sn[l2]);
     }
 }

@@ -306,10 +306,12 @@ k_fused_means(const DevState* st, long long* fsum_x, long long* fsum_y, const in
                                 (old labels use a word as int64 sum, new labels as double mean: disjoint index ranges) */,
               double* __restrict__ raw_x, double* __restrict__ raw_y, int* __restrict__ flag, int Lcap, int* __restrict__ blk_kept,
               unsigned* __restrict__ farbits, int n_far_words, const P2PDev p2p, const TailState* ts, int* cnt_w, DevState* st_w,
-              const long long* __restrict__ sh_x, const long long* __restrict__ sh_y, const int* __restrict__ sh_k)
+              const long long* __restrict__ sh_x, const long long* __restrict__ sh_y, const int* __restrict__ sh_k,
+              const Freeze fz, const double* __restrict__ counts_prev)
 {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (ts->steady_ok) return;      // the steady tail closed the sweep (and cleared the statistics for the next one)
+    if (fz.frozen) fz.reset_slots(l, gridDim.x * blockDim.x);      // (k_tail_steady may have filled them; k_tail_nn fills them again)
     const bool shadow = ts->steady_cleared != 0;      // k_tail_steady ran and said no: the (reduced) statistics are in its shadow arrays
     if (p2p.on && !shadow) {      // every segment's slice of the reduced statistics is in place (and nobody reads this segment's block any more)
         __shared__ int s_ok;
@@ -349,6 +351,13 @@ k_fused_means(const DevState* st, long long* fsum_x, long long* fsum_y, const in
     newraw[l] = 0.0; newraw[Lcap + l] = 0.0;
     fsum_x[l] = 0; fsum_y[l] = 0;
     keep = (l < raw_l && !((double)k < cota)) ? 1 : 0;      // ICM_SLAM.py:232-236
+    if (fz.frozen && l < ls && fz.landmark(map_x[l], map_y[l])) {
+        // a frozen trajectory's landmark: no observation reached it; it keeps its position and its count, hence survives cota
+        const int kp = (int)counts_prev[l];
+        raw_x[l] = map_x[l]; raw_y[l] = map_y[l];
+        cnt_w[l] = kp;
+        keep = 1;
+    }
     flag[l] = keep;
     }
     const int total = __syncthreads_count(keep);
@@ -510,12 +519,24 @@ struct SlowArgs {
     double* ox; double* oy; double* oc;
     int max_cells; FGeom* geom; int* cell_cnt; int* cell_start; double2* pts; int* gidx;
     double2* gbuild; double* nnd0; int steady_enable;      // for the steady tail of the next sweeps
+    Freeze fz;
 };
+
+// one landmark's calc_cambio term in its trajectory's slots (resolved: the change cd; not: it needs the fallback search)
+__device__ __forceinline__ void fz_add(const Freeze& fz, int k, bool resolved, double cd)
+{
+    atomicAdd(fz.slots + 3 * (size_t)fz.K + k, 1.0);
+    if (resolved) {
+        atomic_min_pos(fz.slots + k, cd); atomic_max_pos(fz.slots + (size_t)fz.K + k, cd); atomicAdd(fz.slots + 2 * (size_t)fz.K + k, cd);
+    } else {
+        atomicAdd(fz.slots + 4 * (size_t)fz.K + k, 1.0);
+    }
+}
 
 __device__ void tail_slow_body(DevState* st, TailState* ts, double dist_thr, double* kx, double* ky, double* kc, int* parent, int* nn, int* ind_flag,
             int* ind_pos, int* ind, int* lab, int* used, int* rank, double* ox, double* oy, double* oc, double* map_out, int cap_out,
             int64_t ld_out, double* counts_state, int Lcap, int max_cells, FGeom* geom, int* cell_cnt, int* cell_start, double2* pts, int* gidx,
-            const int* kflag, const int* kpos, double thr1sq, double thr2_hi, LmRec* lmrec, int* remap);
+            const int* kflag, const int* kpos, double thr1sq, double thr2_hi, LmRec* lmrec, int* remap, const Freeze& fz);
 
 // Nearest OTHER survivor (zero distances are never neighbours, ICM_SLAM.py:242) within dist_thr, searched in the 3 x 3 block
 // of cells around the survivor (three contiguous runs of the cell-sorted arrays, one per row of cells): the block holds
@@ -542,7 +563,13 @@ k_tail_nn(DevState* st, TailState* ts, double* __restrict__ kx, double* __restri
     const bool act = j < Lcap && j < K && !ts->degenerate;
     double cd = 0.0, wide = 0.0;
     int cres = 0, cun = 0, nind = 0;
-    if (j < Lcap && !act) { ind_flag[j] = 0; if (j == 0 && K > 0) cun = K; }
+    const Freeze& fz = sa.fz;
+    // a frozen trajectory's landmark keeps its exact position and never merges (every landmark near it is frozen as well)
+    const bool frz = fz.frozen && j < Lcap && j < K && fz.landmark(kx[j], ky[j]);
+    if (j < Lcap && !act) {
+        ind_flag[j] = 0;
+        if (j == 0 && K > 0) { cun = K; if (fz.frozen) for (int k = 0; k < fz.K; ++k) atomicAdd(fz.slots + 4 * (size_t)fz.K + k, 1.0); }
+    }
     if (act) {
         const int l = klab[j];
         const double xj = kx[j], yj = ky[j];
@@ -584,15 +611,19 @@ k_tail_nn(DevState* st, TailState* ts, double* __restrict__ kx, double* __restri
                 }
                 if (take) { best = s2; arg = id; lo = s2 * (1.0 - 8.8817841970012523e-16); hi = s2 * (1.0 + 8.8817841970012523e-16); }
             }
-        const int f = (arg >= 0 && best <= thr2_lt) ? 1 : 0;      // amin < dist_thr (strict, :245)
+        const int f = (arg >= 0 && best <= thr2_lt && !frz) ? 1 : 0;      // amin < dist_thr (strict, :245)
         nn[j] = arg < 0 ? 0 : arg;
         ind_flag[j] = f;
         nind = f;
+        if (fz.frozen && !frz) {      // the trajectory's calc_cambio; a merge in its region needs the fallback search
+            const int k = fz.region(xj, yj);
+            if (k >= 0) { fz_add(fz, k, cres != 0, cd); if (f) atomicAdd(fz.slots + 4 * (size_t)fz.K + k, 1.0); }
+        }
     }
     if (j < Lcap) {      // the new map if nothing merges
         const bool have = j < K;
         const double c = have ? kc[j] : 0.0;
-        const double mx = have ? mul_rn(kx[j], c) / c : 0.0, my = have ? mul_rn(ky[j], c) / c : 0.0;
+        const double mx = have ? (frz ? kx[j] : mul_rn(kx[j], c) / c) : 0.0, my = have ? (frz ? ky[j] : mul_rn(ky[j], c) / c) : 0.0;
         if (j < cap_out) { map_out[j] = mx; map_out[ld_out + j] = my; }
         counts_state[j] = c;
         LmRec rec;
@@ -643,7 +674,7 @@ k_tail_nn(DevState* st, TailState* ts, double* __restrict__ kx, double* __restri
     if (!s_last || !s_slow) return;
     tail_slow_body(st, ts, sa.dist_thr, kx, ky, kc, sa.parent, nn, ind_flag, sa.ind_pos, sa.ind, sa.lab, sa.used, sa.rank, sa.ox, sa.oy, sa.oc,
                    map_out, cap_out, ld_out, counts_state, Lcap, sa.max_cells, sa.geom, sa.cell_cnt, sa.cell_start, sa.pts, sa.gidx, kflag, kpos,
-                   thr1sq, thr2_hi, lmrec_new, remap);
+                   thr1sq, thr2_hi, lmrec_new, remap, fz);
 }
 
 
@@ -671,8 +702,10 @@ struct SteadyArgs {
     double* raw_x; double* raw_y; int* rawcnt;
     double* map_out; int cap_out; int64_t ld_out; double* counts_state; int* remap; int Lcap;
     double* cpart;      // 5 doubles per block: calc_cambio partials (min, max, sum, resolved?, unresolved)
+    Freeze fz;
 };
 
+template <bool FZ>      // FZ: a batch with frozen trajectories (a.fz); the plain sweep launches the instance without the tests
 __global__ void __launch_bounds__(256)
 k_tail_steady(DevState* st, TailState* ts, const SteadyArgs a, const P2PDev p2p)
 {
@@ -722,16 +755,24 @@ k_tail_steady(DevState* st, TailState* ts, const SteadyArgs a, const P2PDev p2p)
         rec.x = 0.0; rec.y = 0.0; rec.r2 = 0.0; rec.r = 0.0;
         double mx = 0.0, my = 0.0, c = 0.0, rx = 0.0, ry = 0.0;
         if (l < ls) {
-            if ((double)k < a.cota) fail = 1;                      // the landmark would be dropped (ICM_SLAM.py:232-236)
+            const bool frz = FZ && a.fz.landmark(a.map_x[l], a.map_y[l]);
+            if (!frz && (double)k < a.cota) fail = 1;                      // the landmark would be dropped (ICM_SLAM.py:232-236)
             else {
-                c = (double)k;
-                rx = a.map_x[l] + ((double)wx * a.inv_scale) / c;      // k_fused_means
-                ry = a.map_y[l] + ((double)wy * a.inv_scale) / c;
-                mx = mul_rn(rx, c) / c; my = mul_rn(ry, c) / c;      // k_tail_nn (count-weighted mean of one member, :258-260)
-                const LmRec o = a.lmrec_old[l];
-                const double d = dist_rn(mx - o.x, my - o.y);
-                if (d < o.r * (1.0 - 1e-9)) { cres = 1; cd = d; }
-                cun = 1 - cres;
+                if (frz) {      // (k_fused_means / k_tail_nn: position and count as they were)
+                    c = a.counts_state[l];
+                    kg = (int)c;
+                    rx = a.map_x[l]; ry = a.map_y[l]; mx = rx; my = ry;
+                } else {
+                    c = (double)k;
+                    rx = a.map_x[l] + ((double)wx * a.inv_scale) / c;      // k_fused_means
+                    ry = a.map_y[l] + ((double)wy * a.inv_scale) / c;
+                    mx = mul_rn(rx, c) / c; my = mul_rn(ry, c) / c;      // k_tail_nn (count-weighted mean of one member, :258-260)
+                    const LmRec o = a.lmrec_old[l];
+                    const double d = dist_rn(mx - o.x, my - o.y);
+                    if (d < o.r * (1.0 - 1e-9)) { cres = 1; cd = d; }
+                    cun = 1 - cres;
+                    if (FZ) { const int kk = a.fz.region(mx, my); if (kk >= 0) fz_add(a.fz, kk, cres != 0, cd); }
+                }
                 const double2 gb = a.gbuild[l];
                 const double D = dist_rn(mx - gb.x, my - gb.y) * (1.0 + 1e-12);
                 const double nb = a.nnd0[l] - D - margin;             // lower bound of the distance to any other landmark now
@@ -861,7 +902,7 @@ __device__ void tail_slow_body(DevState* st, TailState* ts, double dist_thr, dou
             int64_t ld_out, double* counts_state, int Lcap,
             // grid rebuild over the merged map
             int max_cells, FGeom* geom, int* cell_cnt, int* cell_start, double2* pts, int* gidx,
-            const int* kflag, const int* kpos, double thr1sq, double thr2_hi, LmRec* lmrec, int* remap)
+            const int* kflag, const int* kpos, double thr1sq, double thr2_hi, LmRec* lmrec, int* remap, const Freeze& fz)
 {
     // (runs in the last block of k_tail_nn: everything it reads was written by other blocks of the same launch or before)
     __shared__ int wsum[34];
@@ -931,6 +972,11 @@ __device__ void tail_slow_body(DevState* st, TailState* ts, double dist_thr, dou
         counts_state[r] = c;
     }
     for (int l = tid; l < Lcap; l += nth) remap[l] = (l < st->raw_l && kflag[l]) ? rank[lab[kpos[l]]] : -1;
+    if (fz.frozen) {      // a frozen landmark is a class of its own: its exact position, not the rounded count-weighted mean
+        __syncthreads();
+        for (int j = tid; j < K; j += nth)
+            if (fz.landmark(kx[j], ky[j])) { const int r = rank[lab[j]]; if (r < cap_out) { map_out[r] = kx[j]; map_out[ld_out + r] = ky[j]; } }
+    }
     if (tid == 0) { st->new_l = newL; st->lact = newL; st->n_ind = n_ind; ts->remap_identity = 0; st->cambio_unres += 1; }   // (merged map: calc_cambio needs the full search)
     __syncthreads();
     // ---- rebuild the landmark grid over the merged map (it is the next sweep's association grid) -------------

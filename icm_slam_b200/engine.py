@@ -141,9 +141,11 @@ class Engine:
         switches back to one trajectory."""
         if not traj_T:
             check(self.lib.icmslam_set_batch(self._h, 0, None, 0, 0), self._h)
+            self.batch_K = 0
             return
         x0s = np.ascontiguousarray(x0s, dtype=np.float64)
         check(self.lib.icmslam_set_batch(self._h, int(traj_T), _ptr(x0s)[0], _rows(x0s, 3), int(x0s.shape[1])), self._h)
+        self.batch_K = int(x0s.shape[1])
 
     def set_counts(self, counts=None):
         """cant_obs_i <- counts (rest zero); None: Mapa.clear_obs."""
@@ -224,6 +226,22 @@ class Engine:
         check(self.lib.icmslam_iterate_until(self._h, C.c_void_p(x0.ctypes.data), int(max_sweeps), float(tol_max_change), C.byref(opts),
                                              _ptr(cam)[0], C.byref(n)), self._h)
         return int(n.value), np.ascontiguousarray(cam[:, : n.value].T)
+
+    def batch_iterate_until(self, max_sweeps, tol_max_change, region_pitch, region_cols, newton_tol=0.0, newton_maxit=0):
+        """iterate_until for every trajectory of a batch handle (set_batch) on its own: trajectory k stops -- and is frozen on the
+        device while the others sweep on -- after its first sweep whose largest landmark change is <= tol_max_change.  A landmark
+        belongs to trajectory rint(y / region_pitch) * region_cols + rint(x / region_pitch).  Returns (sweeps the handle ran,
+        n_done (K,), cambios (K, max_sweeps, 3): min / max / mean of trajectory k's sweep s for s < n_done[k])."""
+        K = int(getattr(self, "batch_K", 0))
+        opts = SweepOpts(_lib.SCHED["redblack"], _lib.SOLVER["newton"], _lib.VIEW["prev"], int(newton_maxit), float(newton_tol), 1, 0)
+        m = max(int(max_sweeps), 1)
+        cam = np.zeros((3, max(K, 1), m))
+        n_done = np.zeros(max(K, 1), np.int32)
+        n_run = C.c_int32(0)
+        check(self.lib.icmslam_batch_iterate_until(self._h, int(max_sweeps), float(tol_max_change), float(region_pitch), int(region_cols),
+                                                   C.byref(opts), _ptr(cam)[0], n_done.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                   C.byref(n_run)), self._h)
+        return int(n_run.value), n_done[:K].copy(), np.ascontiguousarray(cam[:, :K, :].transpose(1, 2, 0))
 
     def associate(self, mapa, mapa_referencia, obs):
         """Mapa.actualizar for one scan (ICM_SLAM.py:128-201): `mapa` (2 x L, updated in place), `mapa_referencia` (2 x Lref),
@@ -321,10 +339,10 @@ class Engine:
         return int(a.value), int(b.value)
 
     def sweep_stats(self):
-        v = (C.c_int64 * 16)()
-        check(self.lib.icmslam_get_sweep_stats(self._h, v, 16), self._h)
+        v = (C.c_int64 * 17)()
+        check(self.lib.icmslam_get_sweep_stats(self._h, v, 17), self._h)
         keys = ["newton_iters", "n_far_scans", "raw_L", "kept", "new_L", "n_ind", "lsearch", "status", "dirty_tiles", "epoch",
-                "n_tiles", "stable_ids", "k_runs_ns", "n_dirty_now", "far_count", "steady_sweeps"]
+                "n_tiles", "stable_ids", "k_runs_ns", "n_dirty_now", "far_count", "steady_sweeps", "batch_until_fallbacks"]
         return dict(zip(keys, [int(t) for t in v]))
 
     # -- map utilities --------------------------------------------------------------------------

@@ -276,6 +276,23 @@ int icmslam_associate(icmslam_handle* h, const double* map_ref, int32_t L_ref, i
 int icmslam_iterate_until(icmslam_handle* h, const double* x0, int32_t max_sweeps, double tol_max_change,
                           const icmslam_sweep_opts* opts, double* cambios, int32_t* n_done);
 
+/* -- the same driver loop on a batch handle (icmslam_set_batch), one convergence monitor per trajectory.  Trajectory k gets
+ * exactly what icmslam_iterate_until gives it alone from the same poses and map: n_done[k] (HOST, K) sweeps, its calc_cambio
+ * history in cambios (HOST, 3 x K x max_sweeps, element (r, k, s) at (r * K + k) * max_sweeps + s, rows min / max / mean; may be
+ * NULL), its poses and landmarks.  After its first sweep whose own largest change is <= tol_max_change (<= 0: never) the
+ * trajectory is FROZEN on the device: none of its scans is associated or contributes statistics or labels, none of its poses is
+ * solved, and its poses, landmarks and landmark counts stay bit for bit as they were.  The call returns when every trajectory is
+ * frozen or after max_sweeps sweeps (*n_run: sweeps the handle ran), with every trajectory unfrozen again: later sweeps continue
+ * each one as its own handle would.
+ * A landmark belongs to region k = rint(y / region_pitch) * region_cols + rint(x / region_pitch) (icm_slam_b200/batch.py lays the
+ * trajectories out so); ICMSLAM_ERR_INVALID for a handle that is not a batch handle, region_pitch <= 0, region_cols <= 0,
+ * max_sweeps < 0 or a landmark of the starting map outside regions 0 .. K-1.  (REDBLACK, NEWTON, PREV) sweeps on one GPU only
+ * (ICMSLAM_ERR_UNSUPPORTED otherwise).  Element 16 of icmslam_get_sweep_stats: sweeps of the last call that needed the full
+ * calc_cambio search for some trajectory (a landmark appeared, merged or left its proven radius). */
+int icmslam_batch_iterate_until(icmslam_handle* h, int32_t max_sweeps, double tol_max_change, double region_pitch,
+                                int32_t region_cols, const icmslam_sweep_opts* opts, double* cambios, int32_t* n_done,
+                                int32_t* n_run);
+
 /* -- filtrar_obs.m (scripts/filtrar_obs.m:6-50), the offline scan gate: keep the k(t) nearest
  * returns per scan.  obs / out: B x T. */
 int icmslam_filtrar_obs(icmslam_handle* h, const double* obs, int32_t B, int32_t T, int64_t ld, double max_dist,
