@@ -64,8 +64,7 @@ struct icmslam_handle {
     // state
     DevState* d_st = nullptr;
     DevState* h_st = nullptr;   // pinned mirror
-    int lact_host = 0;          // mirror of landmarks_actuales (valid when !lact_dirty)
-    bool lact_dirty = false;
+    int lact_host = 0;          // mirror of landmarks_actuales (valid when !ch.lact_dirty)
     void* d_cub = nullptr;
     size_t cub_bytes = 0;
     void* d_sort_ws = nullptr;
@@ -74,7 +73,6 @@ struct icmslam_handle {
     bool fused_ok = false;
     double *d_bm = nullptr /*6 x T static body-frame moments + beam count*/, *d_inc = nullptr /*3 x T odometry increments*/, *d_x2 = nullptr /*3 x T, pose double buffer*/;
     double4* d_ppar[2] = {nullptr, nullptr};   // projection parameters of the poses in d_x / d_x2 (solve.cuh make_ppar)
-    const double* ppar_of = nullptr;           // the pose buffer whose projection parameters are current (nullptr: recompute)
     FarRec* d_far_list = nullptr;
     int* d_blk_prefix = nullptr;
     unsigned* d_farbits = nullptr;             // 4 words per record tile: scans that created a label this sweep
@@ -91,10 +89,8 @@ struct icmslam_handle {
     double* d_dyn = nullptr;                   // 6 landmark moments per pose
     TailState* d_ts = nullptr;
     double thr2_lt = 0.0;        // largest s with sqrt_rn(s) < dist_thr
-    const double* grid_map = nullptr;   // the map buffer the fast grid currently indexes (nullptr: rebuild)
-    const double* hint_map = nullptr;   // the map buffer for which c[] (through d_remap) holds last sweep's labels
     LmRec* d_lmrec2[2] = {nullptr, nullptr};   // landmarks of a map by label (position + hint radius): the current map's in
-    int lm_cur = 0;                            // d_lmrec2[lm_cur], the tail writes the new map's into the other one
+                                               // d_lmrec2[ch.lm_cur], the tail writes the new map's into the other one
     // the steady tail (tail.cuh k_tail_steady): where every landmark was when the grid was built, a lower bound of its distance to
     // any other landmark then, the positions of its grid entries, per-block calc_cambio partials
     double2* d_gbuild = nullptr; double* d_nnd0 = nullptr; int4* d_gslots = nullptr; double* d_cpart = nullptr; int steady_enable = 1;
@@ -103,9 +99,7 @@ struct icmslam_handle {
     bool in_own_capture = false; int use_cond = 1; cudaStream_t cap_stream = nullptr;
     int* d_blk_kept = nullptr;                 // kept landmarks per block of k_fused_means
     int* d_rawcnt = nullptr;                   // observation counts of the last fused sweep's raw map (the tail clears d_cnt)
-    bool rawcnt_valid = false;
     unsigned long long* d_scan_state = nullptr; // block totals of k_cell_scan
-    bool stats_clean = false;                  // statistics / counts / far bits are all zero (the fused tail leaves them so)
     int* d_remap = nullptr;             // label of the last sweep -> label in the current map
     int* d_klab = nullptr;              // raw label of each kept landmark (fast tail)
     int traj_T = 0, traj_K = 0; double* d_x0s = nullptr;   // batch of independent trajectories laid end to end (icmslam_set_batch)
@@ -115,10 +109,10 @@ struct icmslam_handle {
     int fz_fallbacks = 0;      // sweeps of the last icmslam_batch_iterate_until that needed the full calc_cambio search
     double* d_aobs = nullptr; int* d_ac = nullptr;   // icmslam_associate: one scan's observations (2 x ASSOC_MAX_OBS) and labels
     double thr1sq = 0.0;
-    struct GraphSlot { cudaGraphExec_t exec = nullptr; const double* src = nullptr; const double* map_in = nullptr; double x0[3] = {0, 0, 0}; double tol = 0; int maxit = 0; int lm = 0; Freeze fz = {}; };
+    struct GraphSlot { cudaGraphExec_t exec = nullptr; const double* src = nullptr; const double* map_in = nullptr; double x0[3] = {0, 0, 0}; double tol = 0; int maxit = 0; int lm = 0; Freeze fz = {};
+                       int launches = 0; };      // kernels of this library in the graph
     GraphSlot graphs[4];
-    int use_graph = 1, graph_launches = 0;
-    int runs_occ = 24;           // resident one-warp blocks per SM k_runs is compiled for (24: 80 registers; ICMSLAM_RUNS_OCC=32: 64)
+    int use_graph = 1;
     int use_runs = 1;            // ICMSLAM_RUNS=0: every tile goes through the association kernel every sweep (no steady-state shortcut)
     int assoc_blocks = 0;        // grid of the (persistent) association kernel
     double2* d_bxy = nullptr;    // interleaved (bx, by) records for the TMA staging
@@ -157,10 +151,21 @@ struct icmslam_handle {
     size_t fused_smem = 0;
     double thr2_hi = 0.0, fix_scale = 1.0;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    bool timed_fused = false;
     double last_runs_ms = 0.0;   // k_runs alone in the last timed fused sweep
     int64_t n_launch = 0;   // kernels of this library launched so far (cub's not counted)
-    int x_cur = 0;          // which pose buffer (d_x / d_x2) holds the resident poses
+    // what the host knows of the state the device carries from one sweep to the next (a graph capture leaves it as it found it)
+    struct Chain {
+        int x_cur = 0;                      // which pose buffer (d_x / d_x2) holds the resident poses
+        const double* ppar_of = nullptr;    // the pose buffer whose projection parameters are current (nullptr: recompute)
+        const double* grid_map = nullptr;   // the map buffer the fast grid currently indexes (nullptr: rebuild)
+        const double* hint_map = nullptr;   // the map buffer for which c[] (through d_remap) holds last sweep's labels
+        int lm_cur = 0;                     // d_lmrec2[lm_cur] holds the current map's landmarks
+        bool stats_clean = false;           // statistics / counts / far bits are all zero (the fused tail leaves them so)
+        bool rawcnt_valid = false;          // d_rawcnt holds the counts of the raw map
+        bool timed_fused = false;           // the last sweep was a fused one (icmslam_get_kernel_ms reads its events)
+        bool lact_dirty = false;            // lact_host is stale: the device changed landmarks_actuales
+    };
+    Chain ch;
 };
 
 #define CK(call)                                                                                         \
@@ -180,6 +185,35 @@ static cudaError_t dalloc(Tp** p, size_t count)
 #define DFREE(p) do { if (p) { cudaFree(p); p = nullptr; } } while (0)
 
 static inline int nblk(int64_t n, int b) { return (int)((n + b - 1) / b); }
+
+// the resident poses, the buffer the next sweep writes, and the projection parameters of a pose buffer (they ping-pong with it)
+static double* cur_x(const icmslam_handle* h) { return h->ch.x_cur ? h->d_x2 : h->d_x; }
+static double* next_x(const icmslam_handle* h) { return h->ch.x_cur ? h->d_x : h->d_x2; }
+static double4* ppar_for(const icmslam_handle* h, const double* x) { return h->d_ppar[x == h->d_x2 ? 1 : 0]; }
+
+// the default sweep (REDBLACK, NEWTON, PREV) on the fused path: run records, association of dirty tiles, tile solve, fused tail
+static bool fused_mode(const icmslam_handle* h, const icmslam_sweep_opts& o)
+{
+    return h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON && o.map_view == ICMSLAM_VIEW_PREV;
+}
+
+// a fused sweep has been issued: its solve writes the poses in `xout` and their projection parameters (a segment's halo columns
+// come from the exchange), its tail the map in `map_out` (nullptr: a buffer the grid does not index) and the raw counts
+static void chain_advance(icmslam_handle* h, const double* xout, const double* map_out)
+{
+    icmslam_handle::Chain& c = h->ch;
+    c.ppar_of = xout;
+    c.grid_map = c.hint_map = map_out;      // the grid indexes the new map, and c[] / d_remap carry this sweep's labels into it
+    c.lm_cur ^= 1;
+    c.stats_clean = c.rawcnt_valid = c.timed_fused = c.lact_dirty = true;
+}
+
+// after a sweep of the resident poses: its poses become the resident ones, and mapa_viejo = mapa_refinado (sensors.py:315)
+static void end_sweep(icmslam_handle* h)
+{
+    h->ch.x_cur ^= 1;
+    double* t = h->d_map_in; h->d_map_in = h->d_map_out; h->d_map_out = t;
+}
 
 extern "C" int icmslam_abi_version(void) { return ICMSLAM_ABI_VERSION; }
 
@@ -221,10 +255,10 @@ static void free_dataset(icmslam_handle* h)
     DFREE(h->d_inc); DFREE(h->d_bm); DFREE(h->d_dyn); DFREE(h->d_x2); DFREE(h->d_far_list); DFREE(h->d_blk_prefix); DFREE(h->d_bxy);
     DFREE(h->d_ppar[0]); DFREE(h->d_ppar[1]); DFREE(h->d_farbits); DFREE(h->d_rec_sb); DFREE(h->d_rec_meta); DFREE(h->d_nruns); DFREE(h->d_tile_epoch);
     DFREE(h->d_tile_flag); DFREE(h->d_dirty_list); DFREE(h->d_scan_dirty); DFREE(h->d_tile_slots); DFREE(h->d_tile_nslots); DFREE(h->d_tile_perm); DFREE(h->d_pos_nruns);
-    h->ppar_of = nullptr;
+    h->ch.ppar_of = nullptr;
     drop_graphs(h);
-    h->grid_map = nullptr;
-    h->hint_map = nullptr;
+    h->ch.grid_map = nullptr;
+    h->ch.hint_map = nullptr;
     h->last_map_L = -1;
     h->traj_T = 0; h->traj_K = 0;
     DFREE(h->d_x0s);
@@ -396,7 +430,6 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
     if (e == cudaSuccess && h->trace_on) { const int one = 1; e = cudaMemcpy(&h->d_ts->trace_on, &one, sizeof one, cudaMemcpyHostToDevice); }
     { const char* eg = getenv("ICMSLAM_GRAPH"); if (eg) h->use_graph = atoi(eg); }
     { const char* er = getenv("ICMSLAM_RUNS"); if (er) h->use_runs = atoi(er) != 0; }
-    { const char* er = getenv("ICMSLAM_RUNS_OCC"); if (er && atoi(er) == 32) h->runs_occ = 32; }
     if (e == cudaSuccess) {
         int sms = 0;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
@@ -569,7 +602,7 @@ extern "C" int icmslam_extract(icmslam_handle* h)
     {   // run records and their bookkeeping (runs.cuh): slice s (32 scans) owns slots [s * maxr * 32, (s + 1) * maxr * 32)
         const size_t nt = (size_t)nblk(T + 1, RT_TILE) + 2;      // (+1 scan: a segment's tiling may start one scan earlier)
         h->n_tiles_alloc = (int)nt;
-        h->stats_clean = false;
+        h->ch.stats_clean = false;
         h->rec_maxr = h->max_per_scan > 0 ? h->max_per_scan : 1;
         h->rec_slots = (int64_t)(nt * RT_SLICES) * h->rec_maxr * 32;
         CK(dalloc(&h->d_rec_sb, (size_t)h->rec_slots)); CK(dalloc(&h->d_rec_meta, (size_t)h->rec_slots));
@@ -588,7 +621,7 @@ extern "C" int icmslam_extract(icmslam_handle* h)
         CK(cudaMemsetAsync(h->d_tile_flag, 0, nt * sizeof(int), h->stream));
         CK(cudaMemsetAsync(h->d_farbits, 0, nt * 4 * sizeof(unsigned), h->stream));
         CK(cudaMemsetAsync(h->d_scan_dirty, 0, nt * RT_TILE * sizeof(int), h->stream));
-        h->ppar_of = nullptr;
+        h->ch.ppar_of = nullptr;
     }
     CK(dalloc(&h->d_bm, (size_t)6 * T));
     CK(dalloc(&h->d_dyn, (size_t)6 * T));
@@ -662,7 +695,7 @@ static int sync_state(icmslam_handle* h)
     CK(cudaMemcpyAsync(h->h_st, h->d_st, sizeof(DevState), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->lact_host = h->h_st->lact;
-    h->lact_dirty = false;
+    h->ch.lact_dirty = false;
     return ICMSLAM_OK;
 }
 
@@ -676,11 +709,11 @@ extern "C" int icmslam_set_landmarks_actuales(icmslam_handle* h, int32_t lact)
     }
     k_set_lact<<<1, 1, 0, h->stream>>>(h->d_st, lact);
     CK(cudaGetLastError());
-    h->grid_map = nullptr;
-    h->hint_map = nullptr;
+    h->ch.grid_map = nullptr;
+    h->ch.hint_map = nullptr;
     h->last_map_L = -1;
     h->lact_host = lact;
-    h->lact_dirty = false;
+    h->ch.lact_dirty = false;
     return ICMSLAM_OK;
 }
 
@@ -689,7 +722,7 @@ extern "C" int icmslam_get_landmarks_actuales(const icmslam_handle* hc, int32_t*
     icmslam_handle* h = const_cast<icmslam_handle*>(hc);
     if (!h || !lact) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
-    if (h->lact_dirty) { int rc = sync_state(h); if (rc) return rc; }
+    if (h->ch.lact_dirty) { int rc = sync_state(h); if (rc) return rc; }
     *lact = h->lact_host;
     return ICMSLAM_OK;
 }
@@ -846,11 +879,11 @@ static TrajLayout traj_layout(const icmslam_handle* h, const double* x0)
 // projection parameters (solve.cuh make_ppar) of the poses in `x`, unless the solve of the previous sweep already left them
 static int ensure_ppar(icmslam_handle* h, const double* x, int64_t ldx, const double* x0, double4* dst)
 {
-    if (h->ppar_of == x && x != nullptr) return ICMSLAM_OK;
+    if (h->ch.ppar_of == x && x != nullptr) return ICMSLAM_OK;
     k_ppar_init<<<nblk(h->T, 256), 256, 0, h->stream>>>(x, ldx, 0, h->T, traj_layout(h, x0), dst);
     CK(cudaGetLastError());
     h->n_launch += 1;
-    h->ppar_of = x;
+    h->ch.ppar_of = x;
     return ICMSLAM_OK;
 }
 
@@ -858,12 +891,12 @@ static int ensure_ppar(icmslam_handle* h, const double* x, int64_t ldx, const do
 // wrote them (the reference-mode sweep, pass 0, a fresh extraction) leaves a memset to the next fused sweep.
 static int ensure_stats_clean(icmslam_handle* h)
 {
-    if (h->stats_clean) return ICMSLAM_OK;
+    if (h->ch.stats_clean) return ICMSLAM_OK;
     cudaStream_t s = h->stream;
     CK(cudaMemsetAsync(h->d_cnt, 0, ((size_t)h->Lcap + 1) * sizeof(int), s));
     if (h->d_fsum_x) CK(cudaMemsetAsync(h->d_fsum_x, 0, (size_t)2 * h->Lcap * sizeof(long long), s));
     if (h->d_farbits) CK(cudaMemsetAsync(h->d_farbits, 0, (size_t)h->n_tiles_alloc * 4 * sizeof(unsigned), s));
-    h->stats_clean = true;
+    h->ch.stats_clean = true;
     return ICMSLAM_OK;
 }
 
@@ -875,11 +908,16 @@ struct HostPipe { double* x; int64_t ld; int chunks; };      // the caller's hos
 
 static bool pipe_ready(icmslam_handle* h);
 
-static void launch_runs(icmslam_handle* h, int blocks, cudaStream_t s, const RunParams& R)
+static void launch_runs(int blocks, cudaStream_t s, const RunParams& R)
 {
-    const bool fz = R.fz.frozen != nullptr;
-    if (h->runs_occ == 32) { if (fz) k_runs<32, true><<<blocks, RUNS_THREADS, 0, s>>>(R); else k_runs<32, false><<<blocks, RUNS_THREADS, 0, s>>>(R); }
-    else { if (fz) k_runs<24, true><<<blocks, RUNS_THREADS, 0, s>>>(R); else k_runs<24, false><<<blocks, RUNS_THREADS, 0, s>>>(R); }
+    if (R.fz.frozen) k_runs<true><<<blocks, RUNS_THREADS, 0, s>>>(R);
+    else k_runs<false><<<blocks, RUNS_THREADS, 0, s>>>(R);
+}
+
+static void launch_solve(int blocks, cudaStream_t s, const SolveParams& P)
+{
+    if (P.fz.frozen) k_solve_tile<true><<<blocks, ST_THREADS, 0, s>>>(P);
+    else k_solve_tile<false><<<blocks, ST_THREADS, 0, s>>>(P);
 }
 
 static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, double* kout, int64_t kld, const double* x0,
@@ -892,27 +930,26 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     const double* min_x = h->d_map_in;
     const double* min_y = h->d_map_in + L;
     const bool timing = (o.reserved & 2) != 0;
-    if (h->grid_map != h->d_map_in) {      // the grid of the previous sweep's tail does not index this map: build it
+    if (h->ch.grid_map != h->d_map_in) {      // the grid of the previous sweep's tail does not index this map: build it
         int rc = build_fgrid(h, min_x, min_y, &st->lsearch, n_search_cap);
         if (rc) return rc;
         k_lmrec_build<<<nblk(n_search_cap, 256), 256, 0, s>>>(min_x, min_y, &st->lsearch, h->d_fg_geom, h->d_fg_start, h->d_fg_pts, h->d_fg_idx,
-                                                              h->thr1sq, h->thr2_hi, h->d_lmrec2[h->lm_cur]);
+                                                              h->thr1sq, h->thr2_hi, h->d_lmrec2[h->ch.lm_cur]);
         CK(cudaGetLastError());
         k_epoch_bump<<<1, 1, 0, s>>>(h->d_ts);      // a map from outside: its labels are a new numbering, run records are void
         CK(cudaGetLastError());
         h->n_launch += 2;
-        h->hint_map = nullptr;
+        h->ch.hint_map = nullptr;
     }
-    // the pose buffers ping-pong, and so do their projection parameters
-    double4* pp_in = h->d_ppar[xin == h->d_x2 ? 1 : 0];
-    double4* pp_out = h->d_ppar[xin == h->d_x2 ? 0 : 1];
+    double4* pp_in = ppar_for(h, xin);
+    double4* pp_out = h->d_ppar[pp_in == h->d_ppar[0] ? 1 : 0];      // (the other one, whatever buffer kout is)
     if (!hp) {
         int rc = ensure_ppar(h, xin, ldin, x0, pp_in);
         if (rc) return rc;
     }
     const int t_start = h->seg_lo - (h->seg_first ? 0 : 1);     // a later segment also forms the moments of its odd halo pose
     RunParams R;
-    R.t_start = t_start; R.t_hi = h->seg_hi; R.halo_t = h->seg_first ? -1 : t_start; R.maxr = h->rec_maxr; R.ppar = pp_in; R.lmrec = h->d_lmrec2[h->lm_cur];
+    R.t_start = t_start; R.t_hi = h->seg_hi; R.halo_t = h->seg_first ? -1 : t_start; R.maxr = h->rec_maxr; R.ppar = pp_in; R.lmrec = h->d_lmrec2[h->ch.lm_cur];
     R.rec_sb = h->d_rec_sb; R.rec_meta = h->d_rec_meta; R.nruns = h->d_nruns; R.tile_perm = h->d_tile_perm; R.pos_nruns = h->d_pos_nruns; R.tile_epoch = h->d_tile_epoch; R.dyn = h->d_dyn;
     R.fsum_x = h->d_fsum_x; R.fsum_y = h->d_fsum_y; R.cnt = h->d_cnt; R.fix_scale = h->fix_scale; R.tile_slots = h->d_tile_slots; R.tile_nslots = h->d_tile_nslots;
     R.far_list = h->d_far_list; R.ts = h->d_ts; R.farbits = h->d_farbits;
@@ -923,18 +960,22 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     A.first_halo = h->seg_first ? 0 : 1; A.T = T; A.off = h->d_off; A.bxy = h->d_bxy; A.cfg = h->dcfg; A.thr2_hi = h->thr2_hi; A.st = st; A.geom = h->d_fg_geom;
     A.cell_start = h->d_fg_start; A.gpts = h->d_fg_pts; A.gidx = h->d_fg_idx; A.remap = h->d_remap;
     { const char* eh = getenv("ICMSLAM_HINTS"); A.skip_hints = (eh && atoi(eh) == 0) ? 1 : 0; }
-    A.hints = (h->hint_map == h->d_map_in) ? 1 : 0;
+    A.hints = (h->ch.hint_map == h->d_map_in) ? 1 : 0;
     A.c = h->d_c; A.obs_cap = h->obs_cap; A.R = R;
     A.n_tiles = h->n_tiles; A.blk_prefix = h->d_blk_prefix; A.Lcap = L; A.bb = h->d_bb; A.stw = st; A.final = 1; A.p2p = h->p2p;
+    const int nb = h->assoc_blocks < h->n_tiles ? h->assoc_blocks : h->n_tiles;      // grid of the association kernel
+    SolveParams P;
+    P.T = T; P.t_lo = h->seg_lo; P.t_hi = h->seg_hi; P.lay = traj_layout(h, x0);
+    P.xin = xin; P.ldin = ldin; P.xout = kout; P.ldout = kld;
+    P.inc = h->d_inc; P.ldinc = T; P.u = h->d_u; P.ldu = T; P.bm = h->d_bm; P.ldbm = T; P.dyn = h->d_dyn;
+    P.ppin = pp_in; P.ppout = pp_out; P.cfg = h->dcfg; P.tol = o.newton_tol; P.maxit = o.newton_maxit;
+    P.iters = (o.reserved & 1) ? &st->newton_iters : nullptr; P.tile0 = 0;
+    P.trace_row = h->trace_on ? &h->d_ts->trace[0][0] : nullptr; P.trace_seq = h->p2p.on ? &h->d_ts->halo_seq : &h->d_ts->sweep_no;
+    P.fz = h->fz;
     if (hp) {
         // ---- chunks of tiles: upload | projection parameters, run kernel, association of the tiles it hands over, solve of the
         //      poses whose moments are complete | read-back, on three streams ---------------------------------------------------
-        SolveParams P;
-        P.T = T; P.t_lo = h->seg_lo; P.t_hi = h->seg_hi; P.lay = traj_layout(h, x0);
-        P.xin = xin; P.ldin = ldin; P.xout = kout; P.ldout = kld;
-        P.inc = h->d_inc; P.ldinc = T; P.u = h->d_u; P.ldu = T; P.bm = h->d_bm; P.ldbm = T; P.dyn = h->d_dyn;
-        P.ppin = pp_in; P.ppout = pp_out; P.cfg = h->dcfg; P.tol = o.newton_tol; P.maxit = o.newton_maxit; P.iters = nullptr; P.tile0 = 0;
-        P.trace_row = nullptr; P.trace_seq = nullptr; P.fz = h->fz;
+        P.iters = nullptr; P.trace_row = nullptr; P.trace_seq = nullptr;
         const int C = hp->chunks, per = (h->n_tiles + C - 1) / C;
         cudaStream_t sin = h->h2d_stream, sout = h->side_stream;
         CK(cudaEventRecord(h->ev_fork, s));
@@ -945,7 +986,6 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (b > a) CK(cudaMemcpy2DAsync((double*)xin + a, (size_t)ldin * 8, hp->x + a, (size_t)hp->ld * 8, (size_t)(b - a) * 8, 3, cudaMemcpyHostToDevice, sin));
             CK(cudaEventRecord(h->ev_in[c], sin));
         }
-        const int nb = h->assoc_blocks < h->n_tiles ? h->assoc_blocks : h->n_tiles;
         int solved = 0;
         for (int c = 0; c < C; ++c) {
             const int tile_a = c * per, tile_b = (c + 1) * per < h->n_tiles ? (c + 1) * per : h->n_tiles;
@@ -955,7 +995,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (tile_b > tile_a) {
                 k_ppar_init<<<nblk(b - a, 256), 256, 0, s>>>(xin, ldin, a, b, P.lay, pp_in);
                 R.slice0 = tile_a * RT_SLICES;
-                launch_runs(h, (tile_b - tile_a) * RT_SLICES, s, R);
+                launch_runs((tile_b - tile_a) * RT_SLICES, s, R);
                 h->n_launch += 2;
             }
             A.final = last ? 1 : 0;
@@ -967,8 +1007,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (ready > h->n_solve_tiles) ready = h->n_solve_tiles;
             if (ready > solved) {
                 P.tile0 = solved;
-                if (P.fz.frozen) k_solve_tile<true><<<ready - solved, ST_THREADS, 0, s>>>(P);
-                else k_solve_tile<false><<<ready - solved, ST_THREADS, 0, s>>>(P);
+                launch_solve(ready - solved, s, P);
                 CK(cudaGetLastError());
                 h->n_launch += 1;
                 CK(cudaEventRecord(h->ev_out[c], s));
@@ -982,61 +1021,45 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
         CK(cudaEventRecord(h->ev_fork, s));      // (what a tail on another stream waits for: the last chunk's kernels)
         h->join_pending = true;
         h->d2h_done = true;
-        h->ppar_of = kout;
         return ICMSLAM_OK;
     }
     if (timing) CK(cudaEventRecord(h->ev[0], s));
     if (h->use_runs) {
-        launch_runs(h, h->n_tiles * RT_SLICES, s, R);
+        launch_runs(h->n_tiles * RT_SLICES, s, R);
     } else {
         k_all_dirty<<<nblk(h->n_tiles, 256), 256, 0, s>>>(h->d_tile_flag, h->d_dirty_list, h->d_ts, h->n_tiles, st, h->begin_L);
     }
     CK(cudaGetLastError());
     if (timing) CK(cudaEventRecord(h->ev[2], s));
-    {
-        int nb = h->assoc_blocks < h->n_tiles ? h->assoc_blocks : h->n_tiles;
-        k_assoc_tiles<<<nb, AT_THREADS, h->fused_smem, s>>>(A);
-        CK(cudaGetLastError());
-    }
+    k_assoc_tiles<<<nb, AT_THREADS, h->fused_smem, s>>>(A);
+    CK(cudaGetLastError());
     if (o.reserved & 1) { k_note_dirty<<<1, 1, 0, s>>>(st, h->d_ts); CK(cudaGetLastError()); }
     if (timing) CK(cudaEventRecord(h->ev[3], s));
     h->n_launch += 2;
-    {
-        SolveParams P;
-        P.T = T; P.t_lo = h->seg_lo; P.t_hi = h->seg_hi; P.lay = traj_layout(h, x0);
-        P.xin = xin; P.ldin = ldin; P.xout = kout; P.ldout = kld;
-        P.inc = h->d_inc; P.ldinc = T; P.u = h->d_u; P.ldu = T; P.bm = h->d_bm; P.ldbm = T; P.dyn = h->d_dyn;
-        P.ppin = pp_in; P.ppout = pp_out; P.cfg = h->dcfg; P.tol = o.newton_tol; P.maxit = o.newton_maxit;
-        P.iters = (o.reserved & 1) ? &st->newton_iters : nullptr; P.tile0 = 0;
-        P.trace_row = h->trace_on ? &h->d_ts->trace[0][0] : nullptr; P.trace_seq = h->p2p.on ? &h->d_ts->halo_seq : &h->d_ts->sweep_no;
-        P.fz = h->fz;
-        cudaStream_t ss = s;
-        const bool fork = overlap && h->overlap_solve && !timing && h->side_stream;
-        if (fork) {      // the tail does not depend on the new poses: solve beside it
-            CK(cudaEventRecord(h->ev_fork, s));
-            CK(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
-            ss = h->side_stream;
-        }
-        if (P.fz.frozen) k_solve_tile<true><<<h->n_solve_tiles, ST_THREADS, 0, ss>>>(P);
-        else k_solve_tile<false><<<h->n_solve_tiles, ST_THREADS, 0, ss>>>(P);
-        CK(cudaGetLastError());
-        if (h->d2h_x) {      // a host-memory caller: its poses start their way back as soon as they are solved, beside the tail
-            CK(cudaMemcpy2DAsync(h->d2h_x, (size_t)h->d2h_ld * 8, kout, (size_t)kld * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, ss));
-            h->d2h_done = true;
-        }
-        if (h->p2p.on) {     // the segment's boundary poses to its neighbours, theirs into the halo columns: behind the solve
-            k_p2p_halo<<<1, 32, 0, ss>>>(h->p2p, &h->d_ts->halo_seq, kout, kld, T, h->seg_lo, h->seg_hi, pp_out, st,
-                                         h->trace_on ? &h->d_ts->trace[0][0] : nullptr);
-            CK(cudaGetLastError());
-            h->n_launch += 1;
-        }
-        if (fork) {
-            CK(cudaEventRecord(h->ev_join, ss));
-            h->join_pending = true;
-        }
-        h->n_launch += 1;
-        h->ppar_of = kout;      // the solve leaves the projection parameters of the new poses (all columns but a segment's halo)
+    cudaStream_t ss = s;
+    const bool fork = overlap && h->overlap_solve && !timing && h->side_stream;
+    if (fork) {      // the tail does not depend on the new poses: solve beside it
+        CK(cudaEventRecord(h->ev_fork, s));
+        CK(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
+        ss = h->side_stream;
     }
+    launch_solve(h->n_solve_tiles, ss, P);
+    CK(cudaGetLastError());
+    if (h->d2h_x) {      // a host-memory caller: its poses start their way back as soon as they are solved, beside the tail
+        CK(cudaMemcpy2DAsync(h->d2h_x, (size_t)h->d2h_ld * 8, kout, (size_t)kld * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, ss));
+        h->d2h_done = true;
+    }
+    if (h->p2p.on) {     // the segment's boundary poses to its neighbours, theirs into the halo columns: behind the solve
+        k_p2p_halo<<<1, 32, 0, ss>>>(h->p2p, &h->d_ts->halo_seq, kout, kld, T, h->seg_lo, h->seg_hi, pp_out, st,
+                                     h->trace_on ? &h->d_ts->trace[0][0] : nullptr);
+        CK(cudaGetLastError());
+        h->n_launch += 1;
+    }
+    if (fork) {
+        CK(cudaEventRecord(h->ev_join, ss));
+        h->join_pending = true;
+    }
+    h->n_launch += 1;
     if (timing) CK(cudaEventRecord(h->ev[1], s));
     return ICMSLAM_OK;
 }
@@ -1062,10 +1085,11 @@ static int fused_part_b(icmslam_handle* h, cudaStream_t s)
     return ICMSLAM_OK;
 }
 
-// part C: landmark update, Mapa.filtrar and the grid of the new map (needs the statistics of ALL segments)
+// part C: landmark update, Mapa.filtrar and the grid of the new map (needs the statistics of ALL segments); `xout` is the pose
+// buffer part A's solve wrote
 static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t out_ld, cudaStream_t s);
 
-static int fused_part_c(icmslam_handle* h, double* dmap_out, int out_cap, int64_t out_ld, cudaStream_t s)
+static int fused_part_c(icmslam_handle* h, const double* xout, double* dmap_out, int out_cap, int64_t out_ld, cudaStream_t s)
 {
     const int L = h->Lcap;
     DevState* st = h->d_st;
@@ -1078,7 +1102,7 @@ static int fused_part_c(icmslam_handle* h, double* dmap_out, int out_cap, int64_
         SteadyArgs a;
         a.fsum_x = h->d_fsum_x; a.fsum_y = h->d_fsum_y; a.cnt = h->d_cnt; a.map_x = min_x; a.map_y = min_y;
         a.inv_scale = 1.0 / h->fix_scale; a.cota = h->dcfg.cota; a.dist_thr = h->dcfg.dist_thr; a.thr1sq = h->thr1sq; a.thr2_hi = h->thr2_hi;
-        a.lmrec_old = h->d_lmrec2[h->lm_cur]; a.lmrec_new = h->d_lmrec2[h->lm_cur ^ 1];
+        a.lmrec_old = h->d_lmrec2[h->ch.lm_cur]; a.lmrec_new = h->d_lmrec2[h->ch.lm_cur ^ 1];
         a.gbuild = h->d_gbuild; a.nnd0 = h->d_nnd0; a.gslots = h->d_gslots; a.gpts = h->d_fg_pts;
         a.raw_x = raw_x; a.raw_y = raw_y; a.rawcnt = h->d_rawcnt;
         a.map_out = dmap_out; a.cap_out = out_cap; a.ld_out = out_ld; a.counts_state = h->d_counts; a.remap = h->d_remap; a.Lcap = L;
@@ -1125,13 +1149,7 @@ static int fused_part_c(icmslam_handle* h, double* dmap_out, int out_cap, int64_
             h->n_launch += 6;
         }
     }
-    h->lm_cur ^= 1;
-    h->stats_clean = true;
-    h->rawcnt_valid = true;
-    h->grid_map = (out_ld == L && out_cap == L) ? dmap_out : nullptr;   // the grid now indexes the new map
-    h->hint_map = h->grid_map;                                          // ... and c[] / d_remap carry this sweep's labels into it
-    h->timed_fused = true;
-    h->lact_dirty = true;
+    chain_advance(h, xout, (out_ld == L && out_cap == L) ? dmap_out : nullptr);
     if (h->join_pending) { CK(cudaStreamWaitEvent(s, h->ev_join, 0)); h->join_pending = false; }
     return ICMSLAM_OK;
 }
@@ -1168,8 +1186,8 @@ static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t 
         sa.cell_cnt = h->d_fg_cnt; sa.cell_start = h->d_fg_start; sa.pts = h->d_fg_pts; sa.gidx = h->d_fg_idx;
         sa.gbuild = h->d_gbuild; sa.nnd0 = h->d_nnd0; sa.steady_enable = h->steady_enable; sa.fz = h->fz;
         k_tail_nn<<<nblk(L, 256), 256, 0, s>>>(st, ts, h->d_kx, h->d_ky, h->d_kc, h->d_fg_geom, h->d_fg_start, h->d_fg_pts, h->d_fg_idx, h->thr2_lt,
-                                               h->d_nn, h->d_indflag, L, h->d_klab, h->d_kflag, h->d_kpos, h->d_lmrec2[h->lm_cur],
-                                               h->d_lmrec2[h->lm_cur ^ 1], dmap_out, out_cap, out_ld, h->d_counts, h->thr1sq, h->thr2_hi, h->d_remap, sa);
+                                               h->d_nn, h->d_indflag, L, h->d_klab, h->d_kflag, h->d_kpos, h->d_lmrec2[h->ch.lm_cur],
+                                               h->d_lmrec2[h->ch.lm_cur ^ 1], dmap_out, out_cap, out_ld, h->d_counts, h->thr1sq, h->thr2_hi, h->d_remap, sa);
         CK(cudaGetLastError());
     }
     }
@@ -1207,12 +1225,11 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
     const bool timing = (o.reserved & 2) != 0;
     const bool collect = (o.reserved & 1) != 0;
     unsigned long long* iters = collect ? &st->newton_iters : nullptr;
-    const bool use_fused = h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON &&
-                           o.map_view == ICMSLAM_VIEW_PREV;
+    const bool use_fused = fused_mode(h, o);
     const int n_search_cap = L_in < 0 ? L : (L_in > 0 ? L_in : 1);
 
     h->begin_L = L_in < 0 ? L : L_in;
-    if (!(use_fused && h->grid_map == h->d_map_in)) {
+    if (!(use_fused && h->ch.grid_map == h->d_map_in)) {
         k_sweep_begin<<<1, 1, 0, s>>>(st, h->d_ts, h->begin_L);
         CK(cudaGetLastError());
         h->n_launch += 1;
@@ -1238,13 +1255,13 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         }
         rc = fused_part_b(h, ts_);
         if (rc) return rc;
-        rc = fused_part_c(h, dmap_out, out_cap, out_ld, ts_);
+        rc = fused_part_c(h, kout, dmap_out, out_cap, out_ld, ts_);
         if (rc) return rc;
         if (ts_ != s) { CK(cudaEventRecord(h->ev_tail, ts_)); CK(cudaStreamWaitEvent(s, h->ev_tail, 0)); }
         return ICMSLAM_OK;
     } else {
-        h->stats_clean = false;
-        h->rawcnt_valid = false;
+        h->ch.stats_clean = false;
+        h->ch.rawcnt_valid = false;
         CK(cudaMemsetAsync(h->d_cnt, 0, ((size_t)L + 1) * sizeof(int), s));
         CK(cudaMemsetAsync(h->d_counts, 0, (size_t)L * sizeof(double), s));
         if (xin != xout) CK(cudaMemcpy2DAsync(xout, (size_t)ldout * 8, xin, (size_t)ldin * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToDevice, s));
@@ -1327,14 +1344,14 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         }
         if (timing) CK(cudaEventRecord(h->ev[3], s));
     }
-    h->timed_fused = false;
-    h->grid_map = nullptr;
-    h->hint_map = nullptr;
+    h->ch.timed_fused = false;
+    h->ch.grid_map = nullptr;
+    h->ch.hint_map = nullptr;
     // Mapa.filtrar (sensors.py:165-166)
     rc = run_filter(h, raw_x, raw_y, h->d_cnt, nullptr, dmap_out, out_cap, out_ld, nullptr, 1);
     if (rc) return rc;
     h->n_launch += 11;   // filter grid build (3) + filter kernels (8)
-    h->lact_dirty = true;
+    h->ch.lact_dirty = true;
     return ICMSLAM_OK;
 }
 
@@ -1366,7 +1383,7 @@ extern "C" int icmslam_sweep(icmslam_handle* h, const double* map_in, int32_t L_
     double* xout = x;
     int64_t ldin = ld_x, ldout = ld_x;
     bool continued = false;
-    if (memspace == ICMSLAM_HOST && L_in > 0 && L_in == h->last_map_L && h->grid_map != nullptr && h->grid_map == h->d_map_in &&
+    if (memspace == ICMSLAM_HOST && L_in > 0 && L_in == h->last_map_L && h->ch.grid_map != nullptr && h->ch.grid_map == h->d_map_in &&
         h->h_map_pin && memcmp(map_in, h->h_map_pin, (size_t)L_in * 8) == 0 &&
         memcmp(map_in + ld_map_in, h->h_map_pin + L, (size_t)L_in * 8) == 0) {
         // the caller hands back the map the previous sweep returned: it is already on the device (the current map buffer),
@@ -1376,13 +1393,12 @@ extern "C" int icmslam_sweep(icmslam_handle* h, const double* map_in, int32_t L_
     h->last_map_L = -1;
     // a link of a map chain in the default mode: the poses go up, through the kernels and back in chunks (fused_part_a)
     HostPipe pipe;
-    const bool piped = continued && h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON &&
-                       o.map_view == ICMSLAM_VIEW_PREV && o.reserved == 0 && h->use_runs && h->side_stream && h->seg_first && h->seg_last &&
+    const bool piped = continued && fused_mode(h, o) && o.reserved == 0 && h->use_runs && h->side_stream && h->seg_first && h->seg_last &&
                        h->seg_lo == 0 && h->pipe_chunks > 1 && h->n_tiles >= h->pipe_tiles_min * h->pipe_chunks && pipe_ready(h);
     if (memspace == ICMSLAM_HOST) {
         if (!piped) CK(cudaMemcpy2DAsync(h->d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyHostToDevice, s));
         h->bytes_h2d += (int64_t)3 * T * 8;
-        h->ppar_of = nullptr;
+        h->ch.ppar_of = nullptr;
         xin = h->d_x; ldin = T;
         xout = h->d_x2; ldout = T;
         pipe.x = x; pipe.ld = ld_x; pipe.chunks = h->pipe_chunks;
@@ -1392,8 +1408,8 @@ extern "C" int icmslam_sweep(icmslam_handle* h, const double* map_in, int32_t L_
             CK(cudaMemcpy2DAsync(h->d_map_in, (size_t)L * 8, map_in, (size_t)ld_map_in * 8, (size_t)L_in * 8, 2, cudaMemcpyDefault, s));
             if (memspace == ICMSLAM_HOST) h->bytes_h2d += (int64_t)2 * L_in * 8;
         }
-        h->grid_map = nullptr;
-        h->hint_map = nullptr;
+        h->ch.grid_map = nullptr;
+        h->ch.hint_map = nullptr;
     }
     const bool own_out = (memspace == ICMSLAM_HOST || !map_out);
     h->d2h_done = false;
@@ -1450,8 +1466,8 @@ extern "C" int icmslam_set_map(icmslam_handle* h, const double* map, int32_t L_m
     if (L_map > 0)
         CK(cudaMemcpy2DAsync(h->d_map_in, (size_t)h->Lcap * 8, map, (size_t)ld * 8, (size_t)L_map * 8, 2, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    h->grid_map = nullptr;
-    h->hint_map = nullptr;
+    h->ch.grid_map = nullptr;
+    h->ch.hint_map = nullptr;
     return icmslam_set_landmarks_actuales(h, L_map);
 }
 
@@ -1484,8 +1500,8 @@ extern "C" int icmslam_set_poses(icmslam_handle* h, const double* x, int64_t ld_
     const int T = h->T;
     CK(cudaMemcpy2DAsync(h->d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    h->x_cur = 0;
-    h->ppar_of = nullptr;
+    h->ch.x_cur = 0;
+    h->ch.ppar_of = nullptr;
     return ICMSLAM_OK;
 }
 
@@ -1495,8 +1511,7 @@ extern "C" int icmslam_get_poses(icmslam_handle* h, double* x, int64_t ld_x, int
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
     const int T = h->T;
-    const double* src = h->x_cur ? h->d_x2 : h->d_x;
-    CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, src, (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, cur_x(h), (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return ICMSLAM_OK;
 }
@@ -1513,52 +1528,44 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
     h->last_map_L = -1;
     if (h->seg_first && h->first_empty) return ICMSLAM_EMPTY_FIRST_SCAN;
     if (h->seg_last && h->last_empty && T > 1) return ICMSLAM_ERR_EMPTY_LAST;
-    if (h->p2p.on && !(h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON &&
-                       o.map_view == ICMSLAM_VIEW_PREV))
-        return ICMSLAM_ERR_UNSUPPORTED;      // only the restated parallel sweep partitions in time
+    const bool fused = fused_mode(h, o);
+    if (h->p2p.on && !fused) return ICMSLAM_ERR_UNSUPPORTED;      // only the restated parallel sweep partitions in time
     if (x) {
         CK(cudaMemcpy2DAsync(h->d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, s));
-        h->x_cur = 0;
-        h->ppar_of = nullptr;
+        h->ch.x_cur = 0;
+        h->ch.ppar_of = nullptr;
     }
-    const bool fused_mode = h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON &&
-                            o.map_view == ICMSLAM_VIEW_PREV;
-    const bool graph_ok = fused_mode && h->use_graph && s != nullptr && (o.reserved & 3) == 0;
+    const bool graph_ok = fused && h->use_graph && s != nullptr && (o.reserved & 3) == 0;
     for (int k = 0; k < n_sweeps; ++k) {
-        double* src = h->x_cur ? h->d_x2 : h->d_x;
-        double* dst = h->x_cur ? h->d_x : h->d_x2;
-        bool launched = false;
-        if (fused_mode) {      // projection parameters of poses that did not come out of the previous sweep's solve (outside the graph)
-            int rc = ensure_ppar(h, src, T, x0, h->d_ppar[src == h->d_x2 ? 1 : 0]);
+        double* src = cur_x(h);
+        double* dst = next_x(h);
+        if (fused) {      // (outside the graph) projection parameters of poses that did not come out of the previous sweep's solve, and
+                          // clean statistics after a sweep of another mode
+            int rc = ensure_ppar(h, src, T, x0, ppar_for(h, src));
+            if (rc) return rc;
+            rc = ensure_stats_clean(h);
             if (rc) return rc;
         }
-        if (fused_mode) { int rc = ensure_stats_clean(h); if (rc) return rc; }
-        if (graph_ok && h->grid_map == h->d_map_in) {
+        if (graph_ok && h->ch.grid_map == h->d_map_in) {
             // steady state: the whole sweep (memsets + 15 kernels) replays as one CUDA graph
             icmslam_handle::GraphSlot* slot = nullptr;
             for (auto& g : h->graphs)
                 if (g.exec && g.src == src && g.map_in == h->d_map_in && g.x0[0] == x0[0] && g.x0[1] == x0[1] && g.x0[2] == x0[2] &&
-                    g.tol == o.newton_tol && g.maxit == o.newton_maxit && g.lm == h->lm_cur && same_freeze(g.fz, h->fz)) slot = &g;
+                    g.tol == o.newton_tol && g.maxit == o.newton_maxit && g.lm == h->ch.lm_cur && same_freeze(g.fz, h->fz)) slot = &g;
             if (!slot) {
                 for (auto& g : h->graphs) if (!g.exec) { slot = &g; break; }
                 if (!slot) { drop_graphs(h); slot = &h->graphs[0]; }
                 cudaGraph_t graph = nullptr;
                 const int64_t nl0 = h->n_launch;
-                const double* pof = h->ppar_of;
-                const double* gm = h->grid_map;
-                const double* hm = h->hint_map;
-                const int lm = h->lm_cur;
+                const icmslam_handle::Chain ch0 = h->ch;      // (the capture only records the sweep: each launch below advances the chain)
                 CK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
                 h->in_own_capture = true;
                 int rc = sweep_core(h, src, T, dst, T, x0, o, -1, h->d_map_out, L, L);
                 cudaError_t ce = cudaStreamEndCapture(s, &graph);
                 h->in_own_capture = false;
-                h->graph_launches = (int)(h->n_launch - nl0);
+                h->ch = ch0;
+                const int launches = (int)(h->n_launch - nl0);
                 h->n_launch = nl0;
-                h->ppar_of = pof;
-                h->grid_map = gm;
-                h->hint_map = hm;
-                h->lm_cur = lm;
                 if (rc || ce != cudaSuccess || !graph) {
                     if (graph) cudaGraphDestroy(graph);
                     cudaGetLastError();
@@ -1569,30 +1576,19 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
                 cudaGraphDestroy(graph);
                 if (ce != cudaSuccess) { slot->exec = nullptr; snprintf(h->err, sizeof h->err, "cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return ICMSLAM_ERR_CUDA; }
                 slot->src = src; slot->map_in = h->d_map_in; slot->x0[0] = x0[0]; slot->x0[1] = x0[1]; slot->x0[2] = x0[2];
-                slot->tol = o.newton_tol; slot->maxit = o.newton_maxit; slot->lm = lm; slot->fz = h->fz;
+                slot->tol = o.newton_tol; slot->maxit = o.newton_maxit; slot->lm = h->ch.lm_cur; slot->fz = h->fz; slot->launches = launches;
             }
             CK(cudaGraphLaunch(slot->exec, s));
-            h->n_launch += h->graph_launches;    // kernels of this library inside the graph
-            h->ppar_of = dst;
-            h->grid_map = h->d_map_out;
-            h->hint_map = h->d_map_out;
-            h->lm_cur ^= 1;
-            h->stats_clean = true;
-            h->rawcnt_valid = true;
-            h->timed_fused = true;
-            h->lact_dirty = true;
-            launched = true;
-        }
-        if (!launched) {
+            h->n_launch += slot->launches;
+            chain_advance(h, dst, h->d_map_out);
+        } else {
             int rc = sweep_core(h, src, T, dst, T, x0, o, -1, h->d_map_out, L, L);
             if (rc) return rc;
         }
-        h->x_cur ^= 1;
-        double* t = h->d_map_in; h->d_map_in = h->d_map_out; h->d_map_out = t;   // mapa_viejo = mapa_refinado (sensors.py:315)
+        end_sweep(h);
     }
     if (x) {
-        const double* src = h->x_cur ? h->d_x2 : h->d_x;
-        CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, src, (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDefault, s));
+        CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, cur_x(h), (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDefault, s));
         if (memspace == ICMSLAM_HOST) {
             int rc = sync_state(h);
             if (rc) return rc;
@@ -1607,7 +1603,7 @@ extern "C" int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double
 {
     if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
-    if (traj_T <= 0) { h->traj_T = 0; h->traj_K = 0; DFREE(h->d_x0s); h->ppar_of = nullptr; drop_graphs(h); return ICMSLAM_OK; }
+    if (traj_T <= 0) { h->traj_T = 0; h->traj_K = 0; DFREE(h->d_x0s); h->ch.ppar_of = nullptr; drop_graphs(h); return ICMSLAM_OK; }
     if (!x0s || K <= 0 || ld_x0s < K || (int64_t)traj_T * K != h->T || traj_T < 3 || !h->fused_ok) return ICMSLAM_ERR_INVALID;
     // every trajectory needs a non-empty first and last scan (the reference returns early / raises otherwise, sensors.py:137, :148)
     std::vector<int> off((size_t)h->T + 1);
@@ -1623,7 +1619,7 @@ extern "C" int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double
     CK(cudaStreamSynchronize(h->stream));
     h->traj_T = traj_T; h->traj_K = K;
     h->first_empty = false; h->last_empty = false;
-    h->ppar_of = nullptr;
+    h->ch.ppar_of = nullptr;
     drop_graphs(h);
     return ICMSLAM_OK;
 }
@@ -1652,7 +1648,7 @@ extern "C" int icmslam_device_ptr(icmslam_handle* h, int32_t which, void** ptr, 
     case ICMSLAM_PTR_STAT_Y: *ptr = h->d_fsum_y; *count = L; break;
     case ICMSLAM_PTR_STAT_N: *ptr = h->d_cnt; *count = L; break;
     case ICMSLAM_PTR_NEW_LABELS: *ptr = h->d_newraw; *count = 2 * L; break;
-    case ICMSLAM_PTR_POSES: *ptr = h->x_cur ? h->d_x2 : h->d_x; *count = 3 * (int64_t)h->T; break;
+    case ICMSLAM_PTR_POSES: *ptr = cur_x(h); *count = 3 * (int64_t)h->T; break;
     case ICMSLAM_PTR_EXCHANGE: *ptr = h->d_exch; *count = h->exch_words; break;
     case ICMSLAM_PTR_SEG_REC_POSE: *ptr = h->d_seg_rec_pose; *count = SEG_REC; break;
     case ICMSLAM_PTR_SIDE_STREAM: *ptr = (void*)h->side_stream; *count = 1; break;
@@ -1725,8 +1721,7 @@ extern "C" int icmslam_seg_begin(icmslam_handle* h, const double* x0, const icms
     if (!h || !h->extracted || !x0 || !h->fused_ok) return ICMSLAM_ERR_INVALID;
     icmslam_sweep_opts o;
     default_opts(o, opts);
-    if (!(o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON && o.map_view == ICMSLAM_VIEW_PREV))
-        return ICMSLAM_ERR_UNSUPPORTED;     // only the restated parallel sweep partitions in time (DESIGN.md)
+    if (!fused_mode(h, o)) return ICMSLAM_ERR_UNSUPPORTED;     // only the restated parallel sweep partitions in time (DESIGN.md)
     if (h->p2p.on) return ICMSLAM_ERR_UNSUPPORTED;      // (peer-memory exchange: the sweeps go through icmslam_iterate)
     h->last_map_L = -1;
     CK(cudaSetDevice(h->cfg.device));
@@ -1734,12 +1729,12 @@ extern "C" int icmslam_seg_begin(icmslam_handle* h, const double* x0, const icms
     cudaStream_t s = h->stream;
     if (h->seg_first && h->first_empty) return ICMSLAM_EMPTY_FIRST_SCAN;
     if (h->seg_last && h->last_empty && T > 1) return ICMSLAM_ERR_EMPTY_LAST;
-    double* src = h->x_cur ? h->d_x2 : h->d_x;
-    double* dst = h->x_cur ? h->d_x : h->d_x2;
+    double* src = cur_x(h);
+    double* dst = next_x(h);
     int rc = ensure_stats_clean(h);
     if (rc) return rc;
     h->begin_L = L;
-    if (h->grid_map != h->d_map_in) {
+    if (h->ch.grid_map != h->d_map_in) {
         k_sweep_begin<<<1, 1, 0, s>>>(h->d_st, h->d_ts, L);
         CK(cudaGetLastError());
     }
@@ -1772,7 +1767,7 @@ extern "C" int icmslam_seg_halo(icmslam_handle* h, const double* gathered, int32
     if (!h || !gathered || !h->seg_dst || !h->seg_split || rank < 0 || rank >= world) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
     k_seg_unpack<<<1, 32, 0, h->side_stream>>>(gathered, rank, world, h->seg_dst, h->T, h->T, h->d_st, h->d_ts, h->Lcap,
-                                               h->d_ppar[h->seg_dst == h->d_x2 ? 1 : 0], 1, 0);
+                                               ppar_for(h, h->seg_dst), 1, 0);
     CK(cudaGetLastError());
     CK(cudaEventRecord(h->ev_join, h->side_stream));
     h->n_launch += 1;
@@ -1787,7 +1782,7 @@ extern "C" int icmslam_seg_exchange(icmslam_handle* h, const double* gathered, i
     if (!h || !gathered || !h->seg_dst || rank < 0 || rank >= world) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
     k_seg_unpack<<<1, 32, 0, h->stream>>>(gathered, rank, world, h->seg_dst, h->T, h->T, h->d_st, h->d_ts, h->Lcap,
-                                          h->d_ppar[h->seg_dst == h->d_x2 ? 1 : 0], h->seg_split ? 0 : 1, 1);
+                                          ppar_for(h, h->seg_dst), h->seg_split ? 0 : 1, 1);
     CK(cudaGetLastError());
     h->n_launch += 1;
     return fused_part_b(h, h->stream);
@@ -1799,11 +1794,10 @@ extern "C" int icmslam_seg_finish(icmslam_handle* h)
     if (!h || !h->seg_dst) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
     const int L = h->Lcap;
-    int rc = fused_part_c(h, h->d_map_out, L, L, h->stream);
+    int rc = fused_part_c(h, h->seg_dst, h->d_map_out, L, L, h->stream);
     if (rc) return rc;
     h->seg_dst = nullptr;
-    h->x_cur ^= 1;
-    double* t = h->d_map_in; h->d_map_in = h->d_map_out; h->d_map_out = t;   // mapa_viejo = mapa_refinado (sensors.py:315)
+    end_sweep(h);
     return ICMSLAM_OK;
 }
 
@@ -1815,7 +1809,7 @@ extern "C" int icmslam_get_kernel_ms(icmslam_handle* h, double* out2)
     CK(cudaSetDevice(h->cfg.device));
     CK(cudaStreamSynchronize(h->stream));
     float a = 0.f, b = 0.f;
-    if (h->timed_fused) {      // fused path: k_runs + k_assoc_tiles | k_solve_tile
+    if (h->ch.timed_fused) {      // fused path: k_runs + k_assoc_tiles | k_solve_tile
         CK(cudaEventElapsedTime(&a, h->ev[0], h->ev[3]));
         CK(cudaEventElapsedTime(&b, h->ev[3], h->ev[1]));
         float r = 0.f;
@@ -1823,7 +1817,7 @@ extern "C" int icmslam_get_kernel_ms(icmslam_handle* h, double* out2)
         h->last_runs_ms = r;
     } else {
         CK(cudaEventElapsedTime(&a, h->ev[0], h->ev[1]));
-        if (!h->timed_fused) CK(cudaEventElapsedTime(&b, h->ev[2], h->ev[3]));
+        if (!h->ch.timed_fused) CK(cudaEventElapsedTime(&b, h->ev[2], h->ev[3]));
     }
     out2[0] = a; out2[1] = b;
     return ICMSLAM_OK;
@@ -1879,7 +1873,7 @@ extern "C" int icmslam_get_raw_map(icmslam_handle* h, double* raw_map, int32_t c
     if (raw_map && w > 0)
         CK(cudaMemcpy2DAsync(raw_map, (size_t)ld * 8, h->d_raw, (size_t)h->Lcap * 8, (size_t)w * 8, 2, cudaMemcpyDefault, h->stream));
     if (raw_counts && w > 0) {
-        k_counts_to_double<<<nblk(w, 256), 256, 0, h->stream>>>(h->rawcnt_valid ? h->d_rawcnt : h->d_cnt, w, h->d_tmp_a);
+        k_counts_to_double<<<nblk(w, 256), 256, 0, h->stream>>>(h->ch.rawcnt_valid ? h->d_rawcnt : h->d_cnt, w, h->d_tmp_a);
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(raw_counts, h->d_tmp_a, (size_t)w * 8, cudaMemcpyDefault, h->stream));
     }
@@ -2050,7 +2044,7 @@ extern "C" int icmslam_filter_map(icmslam_handle* h, const double* map_in, int64
     CK(cudaGetLastError());
     // (the result goes through the handle's spare map buffer and rewrites the Mapa state: whatever map chain the handle was
     //  continuing -- grid, hints, run records, the copy of the last returned map -- no longer describes that buffer)
-    h->grid_map = nullptr; h->hint_map = nullptr; h->last_map_L = -1;
+    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr; h->last_map_L = -1;
     int rc = run_filter(h, h->d_tmp_a, h->d_tmp_a + L, nullptr, h->d_tmp_b, h->d_map_out, L, L, h->d_tmp_b + L, 1);
     if (rc) return rc;
     rc = sync_state(h);
@@ -2171,7 +2165,7 @@ extern "C" int icmslam_associate(icmslam_handle* h, const double* map_ref, int32
     int rc = sync_state(h);
     if (rc) return rc;
     const int lact = h->h_st->lact;
-    h->grid_map = nullptr; h->hint_map = nullptr; h->last_map_L = -1;      // (the Mapa state changes under any map chain in flight)
+    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr; h->last_map_L = -1;      // (the Mapa state changes under any map chain in flight)
     if (lact == 0) {
         // Branch A (ICM_SLAM.py:160-165): clusters of the first scan, on the host like icmslam_pass0's first step
         std::vector<double> wx(n_obs), wy(n_obs);
@@ -2195,7 +2189,7 @@ extern "C" int icmslam_associate(icmslam_handle* h, const double* map_ref, int32
         k_set_lact<<<1, 1, 0, s>>>(h->d_st, k0);
         CK(cudaGetLastError());
         CK(cudaStreamSynchronize(s));
-        h->lact_host = k0; h->lact_dirty = false;
+        h->lact_host = k0; h->ch.lact_dirty = false;
         (void)memspace;
         return ICMSLAM_OK;
     }
@@ -2243,7 +2237,7 @@ extern "C" int icmslam_iterate_until(icmslam_handle* h, const double* x0, int32_
         if (rc) return rc;
         const DevState* st = h->h_st;
         double tri[3];
-        if (h->timed_fused && st->cambio_unres == 0 && st->new_l > 0) {
+        if (h->ch.timed_fused && st->cambio_unres == 0 && st->new_l > 0) {
             tri[0] = st->cambio[0]; tri[1] = st->cambio[1]; tri[2] = st->cambio[2] / (double)st->new_l;
         } else {        // landmarks merged / appeared, or another sweep mode: the full search (new map = d_map_in, old = d_map_out)
             rc = icmslam_calc_cambio(h, h->d_map_in, st->new_l, L, h->d_map_out, L_old > 0 ? L_old : 1, L, tri, ICMSLAM_DEVICE);
@@ -2325,8 +2319,7 @@ extern "C" int icmslam_batch_iterate_until(icmslam_handle* h, int32_t max_sweeps
         return ICMSLAM_ERR_INVALID;
     icmslam_sweep_opts o;
     default_opts(o, opts);
-    if (!(h->fused_ok && o.fused && o.schedule == ICMSLAM_SCHED_REDBLACK && o.solver == ICMSLAM_SOLVER_NEWTON && o.map_view == ICMSLAM_VIEW_PREV) ||
-        h->p2p.on || !h->seg_first || !h->seg_last)
+    if (!fused_mode(h, o) || h->p2p.on || !h->seg_first || !h->seg_last)
         return ICMSLAM_ERR_UNSUPPORTED;
     CK(cudaSetDevice(h->cfg.device));
     const int K = h->traj_K, L = h->Lcap;
@@ -2408,7 +2401,7 @@ extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int
     const int64_t n = h->n;
     cudaStream_t s = h->stream;
     if (h->first_empty) return ICMSLAM_EMPTY_FIRST_SCAN;        // (the reference would fail inside tras_rot_z / linkage)
-    h->grid_map = nullptr; h->hint_map = nullptr;
+    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr;
     if (!h->d_seen_x) { CK(dalloc(&h->d_seen_x, (size_t)n)); CK(dalloc(&h->d_seen_y, (size_t)n)); }
     // ---- step 0: Branch A of Mapa.actualizar on the first scan (ICM_SLAM.py:160-165), on the host ------------------
     std::vector<int> off2(2);
@@ -2457,11 +2450,11 @@ extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int
     if (rc) return rc;
     if (h->h_st->status & ST_LABEL_CAP) return ICMSLAM_ERR_LABEL_CAP;
     const int lact = h->h_st->lact;
-    h->x_cur = 0;
-    h->ppar_of = nullptr;
+    h->ch.x_cur = 0;
+    h->ch.ppar_of = nullptr;
     // ---- Mapa.filtrar on the map that was built (sensors.py:99-100) ---------------------------------------------------
-    h->stats_clean = false;
-    h->rawcnt_valid = false;
+    h->ch.stats_clean = false;
+    h->ch.rawcnt_valid = false;
     k_counts_to_int<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, L, h->d_cnt);      // (get_raw_map reports integer counts)
     CK(cudaGetLastError());
     k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, lact, h->dcfg.cota, h->d_kflag, L);

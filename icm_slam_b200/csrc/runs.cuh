@@ -314,8 +314,8 @@ __device__ __forceinline__ bool process_slice(const RunParams& p, TileSmem& S, i
 
 // steady state: one WARP per slice and block (no block barrier: a slice that needs more steps than its neighbours holds nobody
 // up); every block stages its tile's slot table
-template <int MINB, bool FZ>      // resident blocks per SM the kernel is compiled for; FZ: a batch with frozen trajectories
-__global__ void __launch_bounds__(RUNS_THREADS, MINB)
+template <bool FZ>      // FZ: a batch with frozen trajectories; 24 resident blocks per SM (80 registers)
+__global__ void __launch_bounds__(RUNS_THREADS, 24)
 k_runs(const RunParams p)
 {
     __shared__ TileSmem S;
