@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <utility>
 #include <vector>
 
 #include "common.cuh"
@@ -25,132 +26,171 @@
 #define MAX_CELLS (1 << 22)
 #define ASSOC_MAX_OBS 4096      // observations of one scan icmslam_associate accepts (a scan has at most B <= 1024 beams)
 
+// ---- owners of the handle's CUDA resources: each is released by exactly one destructor ------------------------------------
+// Nothing is allocated, freed or reassigned inside a graph capture (sweep_core and the fused_part_* functions under
+// icmslam_iterate, and the icmslam_seg_* calls a caller captures together with its collectives): a captured graph holds the raw
+// pointers, so whatever replaces a buffer a graph can hold calls drop_graphs before the old buffer is freed.
+template <typename H, auto Release>
+struct Owner {
+    H p{};
+    Owner() = default;
+    Owner(Owner&& o) noexcept : p(o.p) { o.p = H{}; }
+    Owner& operator=(Owner&& o) noexcept { if (this != &o) { reset(); p = o.p; o.p = H{}; } return *this; }
+    ~Owner() { reset(); }
+    void reset() { if (p) Release(p); p = H{}; }
+    operator H() const { return p; }
+};
+using Stream = Owner<cudaStream_t, cudaStreamDestroy>;
+using Event = Owner<cudaEvent_t, cudaEventDestroy>;
+using GraphExec = Owner<cudaGraphExec_t, cudaGraphExecDestroy>;
+using IpcMapping = Owner<void*, cudaIpcCloseMemHandle>;
+
+// `count` elements of T in device memory (or, released with cudaFreeHost, in pinned host memory); alloc() frees what it held first
+template <typename T, auto Release>
+struct Buf : Owner<T*, Release> {
+    cudaError_t alloc(size_t count)
+    {
+        this->reset();
+        const size_t bytes = (count ? count : 1) * sizeof(T);
+        const cudaError_t e = Release == cudaFreeHost ? cudaMallocHost((void**)&this->p, bytes) : cudaMalloc((void**)&this->p, bytes);
+        if (e != cudaSuccess) this->p = nullptr;
+        return e;
+    }
+    T* operator->() const { return this->p; }
+};
+template <typename T> using DevBuf = Buf<T, cudaFree>;
+template <typename T> using PinnedBuf = Buf<T, cudaFreeHost>;
+
 struct icmslam_handle {
     icmslam_config cfg;
     DevCfg dcfg;
     cudaStream_t stream = nullptr;
-    cudaStream_t own_stream = nullptr;   // created with the handle; replaced by icmslam_set_stream
+    Stream own_stream;                   // created with the handle; replaced by icmslam_set_stream
     // the pose solve does not feed the tail (labels, landmark update, Mapa.filtrar): on one GPU the two run concurrently,
     // the solve forked onto a side stream after the association kernel and joined at the end of the sweep (also inside the CUDA graph)
-    cudaStream_t side_stream = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_tail = nullptr; bool join_pending = false; int overlap_solve = 1;
+    Stream side_stream; Event ev_fork, ev_join, ev_tail; bool join_pending = false; int overlap_solve = 1;
     char err[512];
     // dataset
     int B = 0, T = 0, precondition = 0;
-    double *d_scans = nullptr, *d_odo = nullptr, *d_u = nullptr, *d_cos = nullptr, *d_sin = nullptr, *d_ang = nullptr;
+    struct Dataset {      // what icmslam_load allocates, sized by T and B
+        DevBuf<double> d_scans, d_odo, d_u, d_cos, d_sin, d_ang;
+        DevBuf<int> d_nfar, d_flag, d_prefix;       // per scan workspace
+        DevBuf<double> d_x /*3 x T*/, d_x2 /*3 x T, pose double buffer*/, d_inc /*3 x T odometry increments*/;
+        DevBuf<FarRec> d_far_list;
+        DevBuf<int> d_blk_prefix;
+    } ds;
     // extraction
     bool extracted = false;
     int64_t n = 0;
     int n_empty = 0, max_per_scan = 0;
     bool first_empty = false, last_empty = false;
-    int *d_off = nullptr, *d_beam = nullptr, *d_scan_of = nullptr;
-    double *d_d = nullptr, *d_bx = nullptr, *d_by = nullptr;
-    // per observation workspace
-    int *d_c = nullptr, *d_keys_out = nullptr, *d_iota = nullptr, *d_sorted = nullptr;
-    double *d_seen_x = nullptr, *d_seen_y = nullptr;
-    // per scan workspace
-    int *d_nfar = nullptr, *d_flag = nullptr, *d_prefix = nullptr;
+    struct Extraction {   // what icmslam_extract allocates (some of it on first use), sized by n and the tile count
+        DevBuf<int> d_off, d_beam, d_scan_of;
+        DevBuf<double> d_d, d_bx, d_by;
+        DevBuf<double2> d_bxy;               // interleaved (bx, by) records for the TMA staging
+        // per observation workspace
+        DevBuf<int> d_c, d_keys_out, d_iota, d_sorted;
+        DevBuf<double> d_seen_x, d_seen_y;
+        // fused (REDBLACK, NEWTON, PREV) path: run records (runs.cuh) + association of dirty tiles (assoc_tiles.cuh) + solve (solve.cuh)
+        DevBuf<double> d_bm;                 // 6 x T static body-frame moments + beam count
+        DevBuf<double4> d_ppar[2];           // projection parameters of the poses in d_x / d_x2 (solve.cuh make_ppar)
+        DevBuf<unsigned> d_farbits;          // 4 words per record tile: scans that created a label this sweep
+        DevBuf<double2> d_rec_sb; DevBuf<int2> d_rec_meta;   // run records (runs.cuh)
+        DevBuf<unsigned short> d_nruns;      // runs of each scan
+        DevBuf<unsigned char> d_tile_perm;   // RT_TILE scan positions per record tile (runs.cuh)
+        DevBuf<unsigned short> d_pos_nruns;  // ... and the runs of the scan at each position
+        DevBuf<int> d_tile_slots, d_tile_nslots;   // RS_SLOTS labels per record tile, slots in use
+        DevBuf<int> d_tile_epoch, d_tile_flag, d_dirty_list, d_scan_dirty;
+        DevBuf<double> d_dyn;                // 6 landmark moments per pose
+    } ex;
     // per label workspace (capacity Lcap)
     int Lcap = 0;
-    double *d_sum_x = nullptr, *d_sum_y = nullptr, *d_raw = nullptr /*2 x Lcap*/, *d_counts = nullptr;
-    int *d_cnt = nullptr, *d_seg = nullptr;
-    int *d_kflag = nullptr, *d_kpos = nullptr, *d_parent = nullptr, *d_nn = nullptr, *d_indflag = nullptr, *d_indpos = nullptr,
-        *d_ind = nullptr, *d_lab = nullptr, *d_used = nullptr, *d_rank = nullptr;
-    double *d_kx = nullptr, *d_ky = nullptr, *d_kc = nullptr, *d_ox = nullptr, *d_oy = nullptr, *d_oc = nullptr, *d_acc = nullptr;
-    double *d_map_in = nullptr /*2 x Lcap*/, *d_map_out = nullptr /*2 x Lcap*/, *d_x = nullptr /*3 x T*/;
-    double *d_tmp_a = nullptr, *d_tmp_b = nullptr; /* 2 x Lcap scratch for filter_map / calc_cambio inputs */
+    DevBuf<double> d_sum_x, d_sum_y, d_raw /*2 x Lcap*/, d_counts;
+    int* d_cnt = nullptr; DevBuf<int> d_seg;
+    DevBuf<int> d_kflag, d_kpos, d_parent, d_nn, d_indflag, d_indpos, d_ind, d_lab, d_used, d_rank;
+    DevBuf<double> d_kx, d_ky, d_kc, d_ox, d_oy, d_oc, d_acc;
+    DevBuf<double> d_map_in /*2 x Lcap*/, d_map_out /*2 x Lcap*/;
+    DevBuf<double> d_tmp_a, d_tmp_b; /* 2 x Lcap scratch for filter_map / calc_cambio inputs */
     // grid
-    int *d_cell_start = nullptr, *d_cell_fill = nullptr, *d_cell_id = nullptr, *d_gidx = nullptr;
-    double *d_glx = nullptr, *d_gly = nullptr;
+    DevBuf<int> d_cell_start, d_cell_fill, d_cell_id, d_gidx;
+    DevBuf<double> d_glx, d_gly;
     // state
-    DevState* d_st = nullptr;
-    DevState* h_st = nullptr;   // pinned mirror
+    DevBuf<DevState> d_st;
+    PinnedBuf<DevState> h_st;   // pinned mirror
     int lact_host = 0;          // mirror of landmarks_actuales (valid when !ch.lact_dirty)
-    void* d_cub = nullptr;
+    DevBuf<unsigned char> d_cub;
     size_t cub_bytes = 0;
-    void* d_sort_ws = nullptr;
+    DevBuf<unsigned char> d_sort_ws;
     size_t sort_bytes = 0;
-    // fused (REDBLACK, NEWTON, PREV) path: run records (runs.cuh) + association of dirty tiles (assoc_tiles.cuh) + solve (solve.cuh)
     bool fused_ok = false;
-    double *d_bm = nullptr /*6 x T static body-frame moments + beam count*/, *d_inc = nullptr /*3 x T odometry increments*/, *d_x2 = nullptr /*3 x T, pose double buffer*/;
-    double4* d_ppar[2] = {nullptr, nullptr};   // projection parameters of the poses in d_x / d_x2 (solve.cuh make_ppar)
-    FarRec* d_far_list = nullptr;
-    int* d_blk_prefix = nullptr;
-    unsigned* d_farbits = nullptr;             // 4 words per record tile: scans that created a label this sweep
     int trace_on = 0;                          // ICMSLAM_TRACE=1: %globaltimer marks of the sweep's kernels (icmslam_get_trace)
     int begin_L = 0;                           // landmarks_actuales bound of the sweep being issued (k_sweep_begin / sweep_begin_state)
     int n_tiles_alloc = 0;                     // tiles the per-tile arrays were allocated for
     int n_tiles = 0, n_solve_tiles = 0;        // record tiles (RT_TILE scans) / solve tiles (ST_OWN poses)
-    double2* d_rec_sb = nullptr; int2* d_rec_meta = nullptr; int64_t rec_slots = 0; int rec_maxr = 1;   // run records (runs.cuh)
-    unsigned short* d_nruns = nullptr;         // runs of each scan
-    unsigned char* d_tile_perm = nullptr;      // RT_TILE scan positions per record tile (runs.cuh)
-    unsigned short* d_pos_nruns = nullptr;     // ... and the runs of the scan at each position
-    int* d_tile_slots = nullptr; int* d_tile_nslots = nullptr;   // RS_SLOTS labels per record tile, slots in use
-    int *d_tile_epoch = nullptr, *d_tile_flag = nullptr, *d_dirty_list = nullptr, *d_scan_dirty = nullptr;
-    double* d_dyn = nullptr;                   // 6 landmark moments per pose
-    TailState* d_ts = nullptr;
+    int64_t rec_slots = 0; int rec_maxr = 1;   // run records (runs.cuh)
+    DevBuf<TailState> d_ts;
     double thr2_lt = 0.0;        // largest s with sqrt_rn(s) < dist_thr
-    LmRec* d_lmrec2[2] = {nullptr, nullptr};   // landmarks of a map by label (position + hint radius): the current map's in
+    DevBuf<LmRec> d_lmrec2[2];                 // landmarks of a map by label (position + hint radius): the current map's in
                                                // d_lmrec2[ch.lm_cur], the tail writes the new map's into the other one
     // the steady tail (tail.cuh k_tail_steady): where every landmark was when the grid was built, a lower bound of its distance to
     // any other landmark then, the positions of its grid entries, per-block calc_cambio partials
-    double2* d_gbuild = nullptr; double* d_nnd0 = nullptr; int4* d_gslots = nullptr; double* d_cpart = nullptr; int steady_enable = 1;
-    long long *d_sh_x = nullptr, *d_sh_y = nullptr; int* d_sh_k = nullptr;      // shadow of the statistics (k_tail_steady clears the live ones)
+    DevBuf<double2> d_gbuild; DevBuf<double> d_nnd0; DevBuf<int4> d_gslots; DevBuf<double> d_cpart; int steady_enable = 1;
+    DevBuf<long long> d_sh_x, d_sh_y; DevBuf<int> d_sh_k;      // shadow of the statistics (k_tail_steady clears the live ones)
     // inside the library's own CUDA graph the full chain is the body of an IF node (cudaGraphSetConditional in k_tail_steady)
-    bool in_own_capture = false; int use_cond = 1; cudaStream_t cap_stream = nullptr;
-    int* d_blk_kept = nullptr;                 // kept landmarks per block of k_fused_means
-    int* d_rawcnt = nullptr;                   // observation counts of the last fused sweep's raw map (the tail clears d_cnt)
-    unsigned long long* d_scan_state = nullptr; // block totals of k_cell_scan
-    int* d_remap = nullptr;             // label of the last sweep -> label in the current map
-    int* d_klab = nullptr;              // raw label of each kept landmark (fast tail)
-    int traj_T = 0, traj_K = 0; double* d_x0s = nullptr;   // batch of independent trajectories laid end to end (icmslam_set_batch)
+    bool in_own_capture = false; int use_cond = 1; Stream cap_stream;
+    DevBuf<int> d_blk_kept;                    // kept landmarks per block of k_fused_means
+    DevBuf<int> d_rawcnt;                      // observation counts of the last fused sweep's raw map (the tail clears d_cnt)
+    DevBuf<unsigned long long> d_scan_state;   // block totals of k_cell_scan
+    DevBuf<int> d_remap;                // label of the last sweep -> label in the current map
+    DevBuf<int> d_klab;                 // raw label of each kept landmark (fast tail)
+    int traj_T = 0, traj_K = 0; DevBuf<double> d_x0s;   // batch of independent trajectories laid end to end (icmslam_set_batch)
     // per-trajectory freezing (icmslam_batch_iterate_until): fz.frozen is null outside that call
     Freeze fz = {};
-    unsigned char *d_fz_mask = nullptr, *d_fz_need = nullptr; double* d_fz_slots = nullptr; int* d_fz_reg = nullptr; int fz_K = 0;
+    DevBuf<unsigned char> d_fz_mask, d_fz_need; DevBuf<double> d_fz_slots; DevBuf<int> d_fz_reg; int fz_K = 0;
     int fz_fallbacks = 0;      // sweeps of the last icmslam_batch_iterate_until that needed the full calc_cambio search
-    double* d_aobs = nullptr; int* d_ac = nullptr;   // icmslam_associate: one scan's observations (2 x ASSOC_MAX_OBS) and labels
+    DevBuf<double> d_aobs; DevBuf<int> d_ac;   // icmslam_associate: one scan's observations (2 x ASSOC_MAX_OBS) and labels
     double thr1sq = 0.0;
-    struct GraphSlot { cudaGraphExec_t exec = nullptr; const double* src = nullptr; const double* map_in = nullptr; double x0[3] = {0, 0, 0}; double tol = 0; int maxit = 0; int lm = 0; Freeze fz = {};
+    struct GraphSlot { GraphExec exec; const double* src = nullptr; const double* map_in = nullptr; double x0[3] = {0, 0, 0}; double tol = 0; int maxit = 0; int lm = 0; Freeze fz = {};
                        int launches = 0; };      // kernels of this library in the graph
     GraphSlot graphs[4];
     int use_graph = 1;
     int use_runs = 1;            // ICMSLAM_RUNS=0: every tile goes through the association kernel every sweep (no steady-state shortcut)
     int assoc_blocks = 0;        // grid of the (persistent) association kernel
-    double2* d_bxy = nullptr;    // interleaved (bx, by) records for the TMA staging
     long long *d_fsum_x = nullptr, *d_fsum_y = nullptr;
     int fg_cells = 0;            // cell budget of the fast grid (host constant)
-    int *d_fg_cnt = nullptr, *d_fg_start = nullptr, *d_fg_idx = nullptr;
-    double2* d_fg_pts = nullptr;
-    FGeom* d_fg_geom = nullptr;
-    unsigned long long* d_bb = nullptr;
+    DevBuf<int> d_fg_cnt, d_fg_start, d_fg_idx;
+    DevBuf<double2> d_fg_pts;
+    DevBuf<FGeom> d_fg_geom;
+    DevBuf<unsigned long long> d_bb;
     int obs_cap = 0, max_tile_obs = 0;
     // host-memspace sweeps: copy of the map returned by the last one (a caller that feeds it back continues the device-side
     // map chain: grid, hints and labels stay valid, sensors.py:315 `mapa_viejo = mapa_refinado`)
-    double* h_map_pin = nullptr;      // pinned 2 x Lcap: the map the last host-memory sweep returned (read back in one async copy; what
+    PinnedBuf<double> h_map_pin;      // pinned 2 x Lcap: the map the last host-memory sweep returned (read back in one async copy; what
     int last_map_L = -1;              // the next call's mapa_viejo is compared with to continue the device-side map chain)
     int64_t bytes_h2d = 0, bytes_d2h = 0;      // copied by host-memspace sweeps (icmslam_get_transfer_bytes)
     // a host-memory sweep of a map chain goes through in chunks of tiles: upload, run kernel, solve and read-back of successive
     // chunks overlap (fused_part_a, HostPipe)
-    cudaStream_t h2d_stream = nullptr; cudaEvent_t ev_in[16] = {}, ev_out[16] = {}; int pipe_chunks = 8; bool pipe_events = false;
+    Stream h2d_stream; Event ev_in[16], ev_out[16]; int pipe_chunks = 8; bool pipe_events = false;
     bool tail_wait_fork = false;
     int pipe_tiles_min = 64;
     double* d2h_x = nullptr; int64_t d2h_ld = 0; bool d2h_done = false;   // host destination of the sweep in flight's poses (fused path)
     // time-segment partition (icmslam_set_segment): this handle owns columns [seg_lo, seg_hi) of its T columns
     int seg_lo = 0, seg_hi = 0, seg_first = 1, seg_last = 1;
     double* d_newraw = nullptr;   // 2 x Lcap: means of the sweep's new labels (zero elsewhere)
-    long long* d_exch = nullptr;  // ONE block [fsum_x | fsum_y | cnt] (newraw aliases the first two): what the segments sum-reduce, viewed as int64
+    DevBuf<long long> d_exch;     // ONE block [fsum_x | fsum_y | cnt] (newraw aliases the first two): what the segments sum-reduce, viewed as int64
     int64_t exch_words = 0;
-    double* d_seg_rec = nullptr;  // SEG_REC doubles: what this segment tells its neighbours
-    double* d_seg_rec_pose = nullptr;   // ... the boundary poses on their own when they are gathered beside the tail (icmslam_seg_halo)
+    DevBuf<double> d_seg_rec;     // SEG_REC doubles: what this segment tells its neighbours
+    DevBuf<double> d_seg_rec_pose;      // ... the boundary poses on their own when they are gathered beside the tail (icmslam_seg_halo)
     // peer-memory exchange of a time-segmented run (p2p.cuh): this rank's window and result buffer, every rank's pointers
     P2PDev p2p = {0, 0, 1, nullptr, nullptr, nullptr, nullptr, 0, 0};
-    P2PWin* d_win = nullptr; long long* d_res = nullptr;
-    void* p2p_opened[3 * P2P_MAX_WORLD] = {};      // mappings of the other ranks' buffers (cudaIpcOpenMemHandle)
-    void** d_p2p_ptrs = nullptr;                   // device copy of the three pointer tables
+    DevBuf<P2PWin> d_win; DevBuf<long long> d_res;
+    IpcMapping p2p_opened[3 * P2P_MAX_WORLD];      // mappings of the other ranks' buffers (cudaIpcOpenMemHandle)
+    DevBuf<void*> d_p2p_ptrs;                      // device copy of the three pointer tables
     bool seg_split = false;       // the sweep in flight exchanges its halo poses through icmslam_seg_halo
     double* seg_dst = nullptr;    // output pose buffer of the segment sweep in flight
     size_t fused_smem = 0;
     double thr2_hi = 0.0, fix_scale = 1.0;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    Event ev[4];
     double last_runs_ms = 0.0;   // k_runs alone in the last timed fused sweep
     int64_t n_launch = 0;   // kernels of this library launched so far (cub's not counted)
     // what the host knows of the state the device carries from one sweep to the next (a graph capture leaves it as it found it)
@@ -177,19 +217,12 @@ struct icmslam_handle {
         }                                                                                                \
     } while (0)
 
-template <typename Tp>
-static cudaError_t dalloc(Tp** p, size_t count)
-{
-    return cudaMalloc((void**)p, (count ? count : 1) * sizeof(Tp));
-}
-#define DFREE(p) do { if (p) { cudaFree(p); p = nullptr; } } while (0)
-
 static inline int nblk(int64_t n, int b) { return (int)((n + b - 1) / b); }
 
 // the resident poses, the buffer the next sweep writes, and the projection parameters of a pose buffer (they ping-pong with it)
-static double* cur_x(const icmslam_handle* h) { return h->ch.x_cur ? h->d_x2 : h->d_x; }
-static double* next_x(const icmslam_handle* h) { return h->ch.x_cur ? h->d_x : h->d_x2; }
-static double4* ppar_for(const icmslam_handle* h, const double* x) { return h->d_ppar[x == h->d_x2 ? 1 : 0]; }
+static double* cur_x(const icmslam_handle* h) { return h->ch.x_cur ? h->ds.d_x2 : h->ds.d_x; }
+static double* next_x(const icmslam_handle* h) { return h->ch.x_cur ? h->ds.d_x : h->ds.d_x2; }
+static double4* ppar_for(const icmslam_handle* h, const double* x) { return h->ex.d_ppar[x == h->ds.d_x2 ? 1 : 0]; }
 
 // the default sweep (REDBLACK, NEWTON, PREV) on the fused path: run records, association of dirty tiles, tile solve, fused tail
 static bool fused_mode(const icmslam_handle* h, const icmslam_sweep_opts& o)
@@ -212,7 +245,7 @@ static void chain_advance(icmslam_handle* h, const double* xout, const double* m
 static void end_sweep(icmslam_handle* h)
 {
     h->ch.x_cur ^= 1;
-    double* t = h->d_map_in; h->d_map_in = h->d_map_out; h->d_map_out = t;
+    std::swap(h->d_map_in, h->d_map_out);
 }
 
 extern "C" int icmslam_abi_version(void) { return ICMSLAM_ABI_VERSION; }
@@ -243,28 +276,29 @@ static bool same_freeze(const Freeze& a, const Freeze& b)
 
 static void drop_graphs(icmslam_handle* h)
 {
-    for (auto& g : h->graphs) { if (g.exec) cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
+    for (auto& g : h->graphs) g.exec.reset();
+}
+
+// a fresh extraction: graphs that hold the old buffers go first, and nothing the host knew of the old observations stays
+static void reset_extraction(icmslam_handle* h)
+{
+    drop_graphs(h);
+    h->ex = icmslam_handle::Extraction();
+    h->ch.ppar_of = nullptr;
+    h->ch.grid_map = nullptr;
+    h->ch.hint_map = nullptr;
+    h->fused_ok = false;
+    h->extracted = false;
 }
 
 static void free_dataset(icmslam_handle* h)
 {
-    DFREE(h->d_scans); DFREE(h->d_odo); DFREE(h->d_u); DFREE(h->d_cos); DFREE(h->d_sin); DFREE(h->d_ang);
-    DFREE(h->d_off); DFREE(h->d_beam); DFREE(h->d_scan_of); DFREE(h->d_d); DFREE(h->d_bx); DFREE(h->d_by);
-    DFREE(h->d_c); DFREE(h->d_keys_out); DFREE(h->d_iota); DFREE(h->d_sorted); DFREE(h->d_seen_x); DFREE(h->d_seen_y);
-    DFREE(h->d_nfar); DFREE(h->d_flag); DFREE(h->d_prefix); DFREE(h->d_x);
-    DFREE(h->d_inc); DFREE(h->d_bm); DFREE(h->d_dyn); DFREE(h->d_x2); DFREE(h->d_far_list); DFREE(h->d_blk_prefix); DFREE(h->d_bxy);
-    DFREE(h->d_ppar[0]); DFREE(h->d_ppar[1]); DFREE(h->d_farbits); DFREE(h->d_rec_sb); DFREE(h->d_rec_meta); DFREE(h->d_nruns); DFREE(h->d_tile_epoch);
-    DFREE(h->d_tile_flag); DFREE(h->d_dirty_list); DFREE(h->d_scan_dirty); DFREE(h->d_tile_slots); DFREE(h->d_tile_nslots); DFREE(h->d_tile_perm); DFREE(h->d_pos_nruns);
-    h->ch.ppar_of = nullptr;
-    drop_graphs(h);
-    h->ch.grid_map = nullptr;
-    h->ch.hint_map = nullptr;
+    reset_extraction(h);
+    h->ds = icmslam_handle::Dataset();
     h->last_map_L = -1;
     h->traj_T = 0; h->traj_K = 0;
-    DFREE(h->d_x0s);
-    DFREE(h->d_fz_mask); DFREE(h->d_fz_need); DFREE(h->d_fz_slots); DFREE(h->d_fz_reg); h->fz_K = 0;
-    h->fused_ok = false;
-    h->extracted = false;
+    h->d_x0s.reset();
+    h->d_fz_mask.reset(); h->d_fz_need.reset(); h->d_fz_slots.reset(); h->d_fz_reg.reset(); h->fz_K = 0;
     h->n = 0;
 }
 
@@ -272,32 +306,6 @@ extern "C" int icmslam_destroy(icmslam_handle* h)
 {
     if (!h) return ICMSLAM_OK;
     cudaSetDevice(h->cfg.device);
-    free_dataset(h);
-    DFREE(h->d_sum_x); DFREE(h->d_sum_y); DFREE(h->d_raw); DFREE(h->d_counts); DFREE(h->d_seg);
-    DFREE(h->d_kflag); DFREE(h->d_kpos); DFREE(h->d_parent); DFREE(h->d_nn); DFREE(h->d_indflag); DFREE(h->d_indpos);
-    DFREE(h->d_ind); DFREE(h->d_lab); DFREE(h->d_used); DFREE(h->d_rank);
-    DFREE(h->d_kx); DFREE(h->d_ky); DFREE(h->d_kc); DFREE(h->d_ox); DFREE(h->d_oy); DFREE(h->d_oc); DFREE(h->d_acc);
-    DFREE(h->d_map_in); DFREE(h->d_map_out); DFREE(h->d_tmp_a); DFREE(h->d_tmp_b);
-    DFREE(h->d_cell_start); DFREE(h->d_cell_fill); DFREE(h->d_cell_id); DFREE(h->d_gidx); DFREE(h->d_glx); DFREE(h->d_gly);
-    DFREE(h->d_st); DFREE(h->d_cub); DFREE(h->d_sort_ws);
-    DFREE(h->d_exch); DFREE(h->d_fg_cnt); DFREE(h->d_fg_start); DFREE(h->d_fg_idx);
-    DFREE(h->d_fg_pts); DFREE(h->d_fg_geom); DFREE(h->d_bb); DFREE(h->d_ts); DFREE(h->d_seg_rec); DFREE(h->d_seg_rec_pose);
-    DFREE(h->d_lmrec2[0]); DFREE(h->d_lmrec2[1]); DFREE(h->d_blk_kept); DFREE(h->d_rawcnt); DFREE(h->d_gbuild); DFREE(h->d_nnd0); DFREE(h->d_gslots); DFREE(h->d_cpart);
-    DFREE(h->d_sh_x); DFREE(h->d_sh_y); DFREE(h->d_sh_k);
-    DFREE(h->d_scan_state); DFREE(h->d_remap); DFREE(h->d_klab); DFREE(h->d_aobs); DFREE(h->d_ac);
-    if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
-    if (h->h_st) cudaFreeHost(h->h_st);
-    for (int i = 0; i < 4; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
-    if (h->own_stream) cudaStreamDestroy(h->own_stream);
-    if (h->side_stream) cudaStreamDestroy(h->side_stream);
-    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    if (h->ev_join) cudaEventDestroy(h->ev_join);
-    if (h->ev_tail) cudaEventDestroy(h->ev_tail);
-    if (h->h_map_pin) cudaFreeHost(h->h_map_pin);
-    for (void*& q : h->p2p_opened) if (q) { cudaIpcCloseMemHandle(q); q = nullptr; }
-    DFREE(h->d_win); DFREE(h->d_res); DFREE(h->d_p2p_ptrs);
-    if (h->h2d_stream) cudaStreamDestroy(h->h2d_stream);
-    for (int i = 0; i < 16; ++i) { if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]); if (h->ev_out[i]) cudaEventDestroy(h->ev_out[i]); }
     delete h;
     return ICMSLAM_OK;
 }
@@ -312,9 +320,8 @@ static int ensure_cub(icmslam_handle* h, size_t bytes)
         return ICMSLAM_ERR_CUDA;
     }
     drop_graphs(h);
-    DFREE(h->d_cub);
     h->cub_bytes = 0;
-    CK(cudaMalloc(&h->d_cub, bytes));
+    CK(h->d_cub.alloc(bytes));
     h->cub_bytes = bytes;
     return ICMSLAM_OK;
 }
@@ -346,10 +353,10 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
     h->Lcap = cfg->L;
     const size_t L = (size_t)h->Lcap;
     cudaError_t e = cudaSetDevice(cfg->device);
-    if (e == cudaSuccess) e = dalloc(&h->d_sum_x, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_sum_y, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_raw, 2 * L);
-    if (e == cudaSuccess) e = dalloc(&h->d_counts, L);
+    if (e == cudaSuccess) e = h->d_sum_x.alloc(L);
+    if (e == cudaSuccess) e = h->d_sum_y.alloc(L);
+    if (e == cudaSuccess) e = h->d_raw.alloc(2 * L);
+    if (e == cudaSuccess) e = h->d_counts.alloc(L);
     {   // exchange block (see icmslam_device_ptr): 64-bit words
         const size_t wcnt = (L + 2) / 2;
         // [fsum_x | fsum_y | cnt].  The means of the sweep's NEW labels (doubles, indices >= lsearch) live in the same words as the
@@ -357,68 +364,68 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
         // written by exactly one segment, and adding the all-zero words of the other segments to a double's bit pattern as an
         // integer leaves it unchanged -- so the segments sum-reduce 2.5 words per landmark instead of 4.5.
         h->exch_words = (int64_t)(2 * L + wcnt);
-        if (e == cudaSuccess) e = dalloc(&h->d_exch, (size_t)h->exch_words);
+        if (e == cudaSuccess) e = h->d_exch.alloc((size_t)h->exch_words);
         if (e == cudaSuccess) e = cudaMemset(h->d_exch, 0, (size_t)h->exch_words * 8);
-        h->d_fsum_x = h->d_exch; h->d_fsum_y = h->d_exch + L; h->d_newraw = (double*)h->d_exch; h->d_cnt = (int*)(h->d_exch + 2 * L);
+        h->d_fsum_x = h->d_exch; h->d_fsum_y = h->d_exch + L; h->d_newraw = (double*)h->d_exch.p; h->d_cnt = (int*)(h->d_exch + 2 * L);
     }
-    if (e == cudaSuccess) e = dalloc(&h->d_seg, L + 1);
-    if (e == cudaSuccess) e = dalloc(&h->d_kflag, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_kpos, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_parent, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_nn, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_indflag, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_indpos, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_ind, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_lab, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_used, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_rank, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_kx, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_ky, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_kc, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_ox, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_oy, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_oc, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_acc, 8);
-    if (e == cudaSuccess) e = dalloc(&h->d_map_in, 2 * L);
-    if (e == cudaSuccess) e = dalloc(&h->d_map_out, 2 * L);
-    if (e == cudaSuccess) e = dalloc(&h->d_tmp_a, 2 * L);
-    if (e == cudaSuccess) e = dalloc(&h->d_tmp_b, 2 * L);
-    if (e == cudaSuccess) e = dalloc(&h->d_cell_start, (size_t)MAX_CELLS + 2);
-    if (e == cudaSuccess) e = dalloc(&h->d_cell_fill, (size_t)MAX_CELLS + 2);
-    if (e == cudaSuccess) e = dalloc(&h->d_cell_id, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_gidx, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_glx, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_gly, L);
+    if (e == cudaSuccess) e = h->d_seg.alloc(L + 1);
+    if (e == cudaSuccess) e = h->d_kflag.alloc(L);
+    if (e == cudaSuccess) e = h->d_kpos.alloc(L);
+    if (e == cudaSuccess) e = h->d_parent.alloc(L);
+    if (e == cudaSuccess) e = h->d_nn.alloc(L);
+    if (e == cudaSuccess) e = h->d_indflag.alloc(L);
+    if (e == cudaSuccess) e = h->d_indpos.alloc(L);
+    if (e == cudaSuccess) e = h->d_ind.alloc(L);
+    if (e == cudaSuccess) e = h->d_lab.alloc(L);
+    if (e == cudaSuccess) e = h->d_used.alloc(L);
+    if (e == cudaSuccess) e = h->d_rank.alloc(L);
+    if (e == cudaSuccess) e = h->d_kx.alloc(L);
+    if (e == cudaSuccess) e = h->d_ky.alloc(L);
+    if (e == cudaSuccess) e = h->d_kc.alloc(L);
+    if (e == cudaSuccess) e = h->d_ox.alloc(L);
+    if (e == cudaSuccess) e = h->d_oy.alloc(L);
+    if (e == cudaSuccess) e = h->d_oc.alloc(L);
+    if (e == cudaSuccess) e = h->d_acc.alloc(8);
+    if (e == cudaSuccess) e = h->d_map_in.alloc(2 * L);
+    if (e == cudaSuccess) e = h->d_map_out.alloc(2 * L);
+    if (e == cudaSuccess) e = h->d_tmp_a.alloc(2 * L);
+    if (e == cudaSuccess) e = h->d_tmp_b.alloc(2 * L);
+    if (e == cudaSuccess) e = h->d_cell_start.alloc((size_t)MAX_CELLS + 2);
+    if (e == cudaSuccess) e = h->d_cell_fill.alloc((size_t)MAX_CELLS + 2);
+    if (e == cudaSuccess) e = h->d_cell_id.alloc(L);
+    if (e == cudaSuccess) e = h->d_gidx.alloc(L);
+    if (e == cudaSuccess) e = h->d_glx.alloc(L);
+    if (e == cudaSuccess) e = h->d_gly.alloc(L);
     h->fg_cells = (int)(4 * L > 4096 ? 4 * L : 4096);
-    if (e == cudaSuccess) e = dalloc(&h->d_fg_cnt, (size_t)h->fg_cells + 2);
-    if (e == cudaSuccess) e = dalloc(&h->d_fg_start, (size_t)h->fg_cells + 2);
-    if (e == cudaSuccess) e = dalloc(&h->d_fg_idx, 4 * L);    // replicated binning: <= 4 cells per landmark
-    if (e == cudaSuccess) e = dalloc(&h->d_fg_pts, 4 * L);
-    if (e == cudaSuccess) e = dalloc(&h->d_fg_geom, 1);
-    if (e == cudaSuccess) e = dalloc(&h->d_bb, 4);
-    if (e == cudaSuccess) e = dalloc(&h->d_ts, 1);
-    if (e == cudaSuccess) e = dalloc(&h->d_seg_rec, SEG_REC);
-    if (e == cudaSuccess) e = dalloc(&h->d_seg_rec_pose, SEG_REC);
+    if (e == cudaSuccess) e = h->d_fg_cnt.alloc((size_t)h->fg_cells + 2);
+    if (e == cudaSuccess) e = h->d_fg_start.alloc((size_t)h->fg_cells + 2);
+    if (e == cudaSuccess) e = h->d_fg_idx.alloc(4 * L);    // replicated binning: <= 4 cells per landmark
+    if (e == cudaSuccess) e = h->d_fg_pts.alloc(4 * L);
+    if (e == cudaSuccess) e = h->d_fg_geom.alloc(1);
+    if (e == cudaSuccess) e = h->d_bb.alloc(4);
+    if (e == cudaSuccess) e = h->d_ts.alloc(1);
+    if (e == cudaSuccess) e = h->d_seg_rec.alloc(SEG_REC);
+    if (e == cudaSuccess) e = h->d_seg_rec_pose.alloc(SEG_REC);
     if (e == cudaSuccess) e = cudaMemset(h->d_seg_rec_pose, 0, SEG_REC * sizeof(double));
-    if (e == cudaSuccess) e = dalloc(&h->d_lmrec2[0], L);
-    if (e == cudaSuccess) e = dalloc(&h->d_lmrec2[1], L);
-    if (e == cudaSuccess) e = dalloc(&h->d_blk_kept, (size_t)nblk((int)L, 256) + 1);
-    if (e == cudaSuccess) e = dalloc(&h->d_rawcnt, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_gbuild, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_nnd0, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_gslots, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_cpart, (size_t)4 * (nblk((int)L, 256) + 1));
-    if (e == cudaSuccess) e = dalloc(&h->d_sh_x, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_sh_y, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_sh_k, L);
+    if (e == cudaSuccess) e = h->d_lmrec2[0].alloc(L);
+    if (e == cudaSuccess) e = h->d_lmrec2[1].alloc(L);
+    if (e == cudaSuccess) e = h->d_blk_kept.alloc((size_t)nblk((int)L, 256) + 1);
+    if (e == cudaSuccess) e = h->d_rawcnt.alloc(L);
+    if (e == cudaSuccess) e = h->d_gbuild.alloc(L);
+    if (e == cudaSuccess) e = h->d_nnd0.alloc(L);
+    if (e == cudaSuccess) e = h->d_gslots.alloc(L);
+    if (e == cudaSuccess) e = h->d_cpart.alloc((size_t)4 * (nblk((int)L, 256) + 1));
+    if (e == cudaSuccess) e = h->d_sh_x.alloc(L);
+    if (e == cudaSuccess) e = h->d_sh_y.alloc(L);
+    if (e == cudaSuccess) e = h->d_sh_k.alloc(L);
     { const char* es = getenv("ICMSLAM_STEADY"); if (es) h->steady_enable = atoi(es) != 0; }
     { const char* es = getenv("ICMSLAM_TRACE"); if (es && atoi(es)) h->trace_on = 1; }
     { const char* es = getenv("ICMSLAM_COND"); if (es) h->use_cond = atoi(es) != 0; }
-    if (e == cudaSuccess) e = dalloc(&h->d_scan_state, (size_t)nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS) + 1);
-    if (e == cudaSuccess) e = dalloc(&h->d_remap, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_klab, L);
-    if (e == cudaSuccess) e = dalloc(&h->d_aobs, (size_t)2 * ASSOC_MAX_OBS);
-    if (e == cudaSuccess) e = dalloc(&h->d_ac, (size_t)ASSOC_MAX_OBS);
+    if (e == cudaSuccess) e = h->d_scan_state.alloc((size_t)nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS) + 1);
+    if (e == cudaSuccess) e = h->d_remap.alloc(L);
+    if (e == cudaSuccess) e = h->d_klab.alloc(L);
+    if (e == cudaSuccess) e = h->d_aobs.alloc((size_t)2 * ASSOC_MAX_OBS);
+    if (e == cudaSuccess) e = h->d_ac.alloc((size_t)ASSOC_MAX_OBS);
     if (e == cudaSuccess) e = cudaMemset(h->d_lmrec2[0], 0, L * sizeof(LmRec));
     if (e == cudaSuccess) e = cudaMemset(h->d_lmrec2[1], 0, L * sizeof(LmRec));
     if (e == cudaSuccess) e = cudaMemset(h->d_scan_state, 0, ((size_t)nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS) + 1) * sizeof(unsigned long long));
@@ -449,28 +456,28 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
         int ex = thr > 1.0 ? ilogb(thr) + 1 : 0;
         h->fix_scale = ldexp(1.0, 34 - ex);      // 2^-34 m per unit: a run's sum fits the two 32-bit limbs of runs.cuh
     }
-    if (e == cudaSuccess) e = dalloc(&h->d_st, 1);
-    if (e == cudaSuccess) e = cudaMallocHost((void**)&h->h_st, sizeof(DevState));
-    for (int i = 0; i < 4 && e == cudaSuccess; ++i) e = cudaEventCreate(&h->ev[i]);
+    if (e == cudaSuccess) e = h->d_st.alloc(1);
+    if (e == cudaSuccess) e = h->h_st.alloc(1);
+    for (int i = 0; i < 4 && e == cudaSuccess; ++i) e = cudaEventCreate(&h->ev[i].p);
     if (e == cudaSuccess) {     // the tail's small kernels (main stream, highest priority) are dispatched ahead of the waves of the solve
         int lo = 0, hi = 0;     // (side stream, lowest): with equal priorities the solve's pending blocks keep the tail out until it ends
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        e = cudaStreamCreateWithPriority(&h->own_stream, cudaStreamNonBlocking, hi);
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&h->side_stream, cudaStreamNonBlocking, lo);
+        e = cudaStreamCreateWithPriority(&h->own_stream.p, cudaStreamNonBlocking, hi);
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&h->side_stream.p, cudaStreamNonBlocking, lo);
     }
     { const char* ec = getenv("ICMSLAM_PIPE_CHUNKS"); if (ec) { int c = atoi(ec); h->pipe_chunks = c < 1 ? 1 : (c > 16 ? 16 : c); } }
     { const char* ec = getenv("ICMSLAM_PIPE_TILES"); if (ec && atoi(ec) > 0) h->pipe_tiles_min = atoi(ec); }
 
     if (e == cudaSuccess) h->stream = h->own_stream;
-    if (e == cudaSuccess) { int lo = 0, hi = 0; cudaDeviceGetStreamPriorityRange(&lo, &hi); e = cudaStreamCreateWithPriority(&h->cap_stream, cudaStreamNonBlocking, hi); }
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_tail, cudaEventDisableTiming);
+    if (e == cudaSuccess) { int lo = 0, hi = 0; cudaDeviceGetStreamPriorityRange(&lo, &hi); e = cudaStreamCreateWithPriority(&h->cap_stream.p, cudaStreamNonBlocking, hi); }
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_fork.p, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_join.p, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_tail.p, cudaEventDisableTiming);
     { const char* eo = getenv("ICMSLAM_OVERLAP"); if (eo) h->overlap_solve = atoi(eo) != 0; }
     if (e == cudaSuccess) e = cudaMemset(h->d_st, 0, sizeof(DevState));
     if (e == cudaSuccess) e = cudaMemset(h->d_counts, 0, L * sizeof(double));
     if (e != cudaSuccess) {
-        icmslam_destroy(h);
+        delete h;
         return e == cudaErrorMemoryAllocation ? ICMSLAM_ERR_ALLOC : ICMSLAM_ERR_CUDA;
     }
     *out = h;
@@ -504,23 +511,23 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
     CK(cudaSetDevice(h->cfg.device));
     free_dataset(h);
     h->B = B; h->T = T; h->precondition = precondition;
-    CK(dalloc(&h->d_scans, (size_t)B * T));
-    CK(dalloc(&h->d_odo, (size_t)3 * T));
-    CK(dalloc(&h->d_u, (size_t)2 * T));
-    CK(dalloc(&h->d_cos, (size_t)B));
-    CK(dalloc(&h->d_sin, (size_t)B));
-    CK(dalloc(&h->d_ang, (size_t)B));
-    CK(dalloc(&h->d_x, (size_t)3 * T));
-    CK(dalloc(&h->d_nfar, (size_t)T + 1));
-    CK(dalloc(&h->d_flag, (size_t)T + 1));
-    CK(dalloc(&h->d_prefix, (size_t)T + 1));
-    CK(dalloc(&h->d_inc, (size_t)3 * T));
-    CK(dalloc(&h->d_x2, (size_t)3 * T));
+    CK(h->ds.d_scans.alloc((size_t)B * T));
+    CK(h->ds.d_odo.alloc((size_t)3 * T));
+    CK(h->ds.d_u.alloc((size_t)2 * T));
+    CK(h->ds.d_cos.alloc((size_t)B));
+    CK(h->ds.d_sin.alloc((size_t)B));
+    CK(h->ds.d_ang.alloc((size_t)B));
+    CK(h->ds.d_x.alloc((size_t)3 * T));
+    CK(h->ds.d_nfar.alloc((size_t)T + 1));
+    CK(h->ds.d_flag.alloc((size_t)T + 1));
+    CK(h->ds.d_prefix.alloc((size_t)T + 1));
+    CK(h->ds.d_inc.alloc((size_t)3 * T));
+    CK(h->ds.d_x2.alloc((size_t)3 * T));
     h->seg_lo = 0; h->seg_hi = T; h->seg_first = 1; h->seg_last = 1;
     h->n_tiles = nblk(T, RT_TILE);
     h->n_solve_tiles = nblk(T, ST_OWN);
-    CK(dalloc(&h->d_far_list, (size_t)T));
-    CK(dalloc(&h->d_blk_prefix, (size_t)nblk(T + 1, RT_TILE) + 2));
+    CK(h->ds.d_far_list.alloc((size_t)T));
+    CK(h->ds.d_blk_prefix.alloc((size_t)nblk(T + 1, RT_TILE) + 2));
     {   // scan workspace for the largest scan of a sweep, so that nothing allocates inside a graph capture
         size_t need = 0, b = 0;
         const int lens[4] = {h->Lcap + 1, h->fg_cells + 2, T + 1, MAX_CELLS + 2};      // (the generic grid scans MAX_CELLS + 1 cells)
@@ -529,49 +536,49 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
         if (rcw) return rcw;
     }
     const size_t w = (size_t)T * sizeof(double);
-    CK(cudaMemcpy2DAsync(h->d_scans, w, scans, (size_t)ld_scans * sizeof(double), w, B, cudaMemcpyDefault, h->stream));
-    CK(cudaMemcpy2DAsync(h->d_odo, w, odo, (size_t)ld_odo * sizeof(double), w, 3, cudaMemcpyDefault, h->stream));
-    CK(cudaMemcpy2DAsync(h->d_u, w, u, (size_t)ld_u * sizeof(double), w, 2, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(h->ds.d_scans, w, scans, (size_t)ld_scans * sizeof(double), w, B, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(h->ds.d_odo, w, odo, (size_t)ld_odo * sizeof(double), w, 3, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(h->ds.d_u, w, u, (size_t)ld_u * sizeof(double), w, 2, cudaMemcpyDefault, h->stream));
     std::vector<double> ang(B), cb(B), sb(B);
     for (int i = 0; i < B; ++i) {
         ang[i] = ((double)i * ICM_PI) / 180.0;                 // nind*np.pi/180.0 (ICM_SLAM.py:44,51)
         cb[i] = cos_tab ? cos_tab[i] : cos(ang[i]);
         sb[i] = sin_tab ? sin_tab[i] : sin(ang[i]);
     }
-    k_odo_increments<<<nblk(T, 256), 256, 0, h->stream>>>(h->d_odo, T, T, h->d_inc, T);
+    k_odo_increments<<<nblk(T, 256), 256, 0, h->stream>>>(h->ds.d_odo, T, T, h->ds.d_inc, T);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h->d_ang, ang.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(h->d_cos, cb.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(h->d_sin, sb.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->ds.d_ang, ang.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->ds.d_cos, cb.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->ds.d_sin, sb.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));   // the host staging vectors and caller buffers may go away
     return ICMSLAM_OK;
 }
 
 extern "C" int icmslam_extract(icmslam_handle* h)
 {
-    if (!h || !h->d_scans) return ICMSLAM_ERR_INVALID;
+    if (!h || !h->ds.d_scans) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
+    reset_extraction(h);
     const int B = h->B, T = h->T;
     const int nwords = (B + 31) / 32;
-    uint32_t* d_masks = nullptr;
-    int* d_counts = nullptr;
-    CK(dalloc(&d_masks, (size_t)T * nwords));
-    CK(dalloc(&d_counts, (size_t)T + 1));
-    DFREE(h->d_off);
-    CK(dalloc(&h->d_off, (size_t)T + 1));
+    DevBuf<uint32_t> d_masks;
+    DevBuf<int> d_counts;
+    CK(d_masks.alloc((size_t)T * nwords));
+    CK(d_counts.alloc((size_t)T + 1));
+    CK(h->ex.d_off.alloc((size_t)T + 1));
     CK(cudaMemsetAsync(d_counts, 0, ((size_t)T + 1) * sizeof(int), h->stream));
     const size_t smem = extract_smem_bytes(B);
     CK(cudaFuncSetAttribute(k_extract<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaFuncSetAttribute(k_extract<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int blocks = nblk(T, EX_TILE);
-    k_extract<1><<<blocks, EX_THREADS, smem, h->stream>>>(h->d_scans, B, T, T, h->d_cos, h->d_sin, h->dcfg, h->precondition,
+    k_extract<1><<<blocks, EX_THREADS, smem, h->stream>>>(h->ds.d_scans, B, T, T, h->ds.d_cos, h->ds.d_sin, h->dcfg, h->precondition,
                                                           nwords, d_masks, d_counts, nullptr, nullptr, nullptr, nullptr,
                                                           nullptr, nullptr);
     CK(cudaGetLastError());
-    int rc = exclusive_sum(h, d_counts, h->d_off, T + 1);
+    int rc = exclusive_sum(h, d_counts, h->ex.d_off, T + 1);
     if (rc) return rc;
     std::vector<int> off((size_t)T + 1);
-    CK(cudaMemcpyAsync(off.data(), h->d_off, ((size_t)T + 1) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(off.data(), h->ex.d_off, ((size_t)T + 1) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->n = off[T];
     h->n_empty = 0; h->max_per_scan = 0;
@@ -583,54 +590,46 @@ extern "C" int icmslam_extract(icmslam_handle* h)
     h->first_empty = off[1] == off[0];
     h->last_empty = off[T] == off[T - 1];
     const size_t n = (size_t)h->n;
-    DFREE(h->d_beam); DFREE(h->d_scan_of); DFREE(h->d_d); DFREE(h->d_bx); DFREE(h->d_by); DFREE(h->d_bxy);
-    DFREE(h->d_c); DFREE(h->d_keys_out); DFREE(h->d_iota); DFREE(h->d_sorted); DFREE(h->d_seen_x); DFREE(h->d_seen_y);
-    CK(dalloc(&h->d_beam, n)); CK(dalloc(&h->d_scan_of, n)); CK(dalloc(&h->d_d, n)); CK(dalloc(&h->d_bx, n + 2)); CK(dalloc(&h->d_by, n + 2));
-    CK(cudaMemsetAsync(h->d_bx, 0, (n + 2) * sizeof(double), h->stream));
-    CK(cudaMemsetAsync(h->d_by, 0, (n + 2) * sizeof(double), h->stream));
-    CK(dalloc(&h->d_c, n + 8));      // (+ slack: the fused kernel stages 16-byte aligned slices of it)
-    k_extract<2><<<blocks, EX_THREADS, smem, h->stream>>>(h->d_scans, B, T, T, h->d_cos, h->d_sin, h->dcfg, h->precondition,
-                                                          nwords, d_masks, nullptr, h->d_off, h->d_beam, h->d_d, h->d_bx,
-                                                          h->d_by, h->d_scan_of);
+    CK(h->ex.d_beam.alloc(n)); CK(h->ex.d_scan_of.alloc(n)); CK(h->ex.d_d.alloc(n)); CK(h->ex.d_bx.alloc(n + 2)); CK(h->ex.d_by.alloc(n + 2));
+    CK(cudaMemsetAsync(h->ex.d_bx, 0, (n + 2) * sizeof(double), h->stream));
+    CK(cudaMemsetAsync(h->ex.d_by, 0, (n + 2) * sizeof(double), h->stream));
+    CK(h->ex.d_c.alloc(n + 8));      // (+ slack: the fused kernel stages 16-byte aligned slices of it)
+    k_extract<2><<<blocks, EX_THREADS, smem, h->stream>>>(h->ds.d_scans, B, T, T, h->ds.d_cos, h->ds.d_sin, h->dcfg, h->precondition,
+                                                          nwords, d_masks, nullptr, h->ex.d_off, h->ex.d_beam, h->ex.d_d, h->ex.d_bx,
+                                                          h->ex.d_by, h->ex.d_scan_of);
     CK(cudaGetLastError());
-    CK(dalloc(&h->d_bxy, n + 2));
-    k_interleave<<<nblk((int64_t)n, 256), 256, 0, h->stream>>>(h->d_bx, h->d_by, (int64_t)n, h->d_bxy);
+    CK(h->ex.d_bxy.alloc(n + 2));
+    k_interleave<<<nblk((int64_t)n, 256), 256, 0, h->stream>>>(h->ex.d_bx, h->ex.d_by, (int64_t)n, h->ex.d_bxy);
     CK(cudaGetLastError());
-    DFREE(h->d_bm); DFREE(h->d_dyn);
-    DFREE(h->d_ppar[0]); DFREE(h->d_ppar[1]); DFREE(h->d_farbits); DFREE(h->d_rec_sb); DFREE(h->d_rec_meta); DFREE(h->d_nruns); DFREE(h->d_tile_epoch);
-    DFREE(h->d_tile_flag); DFREE(h->d_dirty_list); DFREE(h->d_scan_dirty); DFREE(h->d_tile_slots); DFREE(h->d_tile_nslots); DFREE(h->d_tile_perm); DFREE(h->d_pos_nruns);
     {   // run records and their bookkeeping (runs.cuh): slice s (32 scans) owns slots [s * maxr * 32, (s + 1) * maxr * 32)
         const size_t nt = (size_t)nblk(T + 1, RT_TILE) + 2;      // (+1 scan: a segment's tiling may start one scan earlier)
         h->n_tiles_alloc = (int)nt;
         h->ch.stats_clean = false;
         h->rec_maxr = h->max_per_scan > 0 ? h->max_per_scan : 1;
         h->rec_slots = (int64_t)(nt * RT_SLICES) * h->rec_maxr * 32;
-        CK(dalloc(&h->d_rec_sb, (size_t)h->rec_slots)); CK(dalloc(&h->d_rec_meta, (size_t)h->rec_slots));
-        CK(dalloc(&h->d_nruns, nt * RT_TILE));
-        CK(dalloc(&h->d_tile_perm, nt * RT_TILE));
-        CK(dalloc(&h->d_pos_nruns, nt * RT_TILE));
-        CK(cudaMemsetAsync(h->d_pos_nruns, 0, nt * RT_TILE * sizeof(unsigned short), h->stream));
-        CK(cudaMemsetAsync(h->d_tile_perm, 0, nt * RT_TILE, h->stream));      // (rewritten with every tile's records; never read before)
-        CK(dalloc(&h->d_ppar[0], (size_t)T)); CK(dalloc(&h->d_ppar[1], (size_t)T));
-        CK(dalloc(&h->d_farbits, nt * 4)); CK(dalloc(&h->d_tile_epoch, nt));
-        CK(dalloc(&h->d_tile_flag, nt)); CK(dalloc(&h->d_dirty_list, nt)); CK(dalloc(&h->d_tile_slots, nt * RS_SLOTS)); CK(dalloc(&h->d_tile_nslots, nt));
-        CK(cudaMemsetAsync(h->d_tile_nslots, 0, nt * sizeof(int), h->stream));
-        CK(dalloc(&h->d_scan_dirty, nt * RT_TILE));
-        CK(cudaMemsetAsync(h->d_nruns, 0, nt * RT_TILE * sizeof(unsigned short), h->stream));
-        CK(cudaMemsetAsync(h->d_tile_epoch, 0xff, nt * sizeof(int), h->stream));       // epoch -1: no tile holds records
-        CK(cudaMemsetAsync(h->d_tile_flag, 0, nt * sizeof(int), h->stream));
-        CK(cudaMemsetAsync(h->d_farbits, 0, nt * 4 * sizeof(unsigned), h->stream));
-        CK(cudaMemsetAsync(h->d_scan_dirty, 0, nt * RT_TILE * sizeof(int), h->stream));
-        h->ch.ppar_of = nullptr;
+        CK(h->ex.d_rec_sb.alloc((size_t)h->rec_slots)); CK(h->ex.d_rec_meta.alloc((size_t)h->rec_slots));
+        CK(h->ex.d_nruns.alloc(nt * RT_TILE));
+        CK(h->ex.d_tile_perm.alloc(nt * RT_TILE));
+        CK(h->ex.d_pos_nruns.alloc(nt * RT_TILE));
+        CK(cudaMemsetAsync(h->ex.d_pos_nruns, 0, nt * RT_TILE * sizeof(unsigned short), h->stream));
+        CK(cudaMemsetAsync(h->ex.d_tile_perm, 0, nt * RT_TILE, h->stream));      // (rewritten with every tile's records; never read before)
+        CK(h->ex.d_ppar[0].alloc((size_t)T)); CK(h->ex.d_ppar[1].alloc((size_t)T));
+        CK(h->ex.d_farbits.alloc(nt * 4)); CK(h->ex.d_tile_epoch.alloc(nt));
+        CK(h->ex.d_tile_flag.alloc(nt)); CK(h->ex.d_dirty_list.alloc(nt)); CK(h->ex.d_tile_slots.alloc(nt * RS_SLOTS)); CK(h->ex.d_tile_nslots.alloc(nt));
+        CK(cudaMemsetAsync(h->ex.d_tile_nslots, 0, nt * sizeof(int), h->stream));
+        CK(h->ex.d_scan_dirty.alloc(nt * RT_TILE));
+        CK(cudaMemsetAsync(h->ex.d_nruns, 0, nt * RT_TILE * sizeof(unsigned short), h->stream));
+        CK(cudaMemsetAsync(h->ex.d_tile_epoch, 0xff, nt * sizeof(int), h->stream));       // epoch -1: no tile holds records
+        CK(cudaMemsetAsync(h->ex.d_tile_flag, 0, nt * sizeof(int), h->stream));
+        CK(cudaMemsetAsync(h->ex.d_farbits, 0, nt * 4 * sizeof(unsigned), h->stream));
+        CK(cudaMemsetAsync(h->ex.d_scan_dirty, 0, nt * RT_TILE * sizeof(int), h->stream));
     }
-    CK(dalloc(&h->d_bm, (size_t)6 * T));
-    CK(dalloc(&h->d_dyn, (size_t)6 * T));
-    CK(cudaMemsetAsync(h->d_dyn, 0, (size_t)6 * T * sizeof(double), h->stream));
-    k_body_moments<<<nblk(T, 128), 128, 0, h->stream>>>(h->d_off, h->d_bxy, T, h->d_bm, T);
+    CK(h->ex.d_bm.alloc((size_t)6 * T));
+    CK(h->ex.d_dyn.alloc((size_t)6 * T));
+    CK(cudaMemsetAsync(h->ex.d_dyn, 0, (size_t)6 * T * sizeof(double), h->stream));
+    k_body_moments<<<nblk(T, 128), 128, 0, h->stream>>>(h->ex.d_off, h->ex.d_bxy, T, h->ex.d_bm, T);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));
-    cudaFree(d_masks);
-    cudaFree(d_counts);
     h->extracted = true;
     {   // shared-memory budget of the association kernel: observations of one tile of RT_TILE scans
         int mx = 0;
@@ -678,11 +677,11 @@ extern "C" int icmslam_get_extraction(icmslam_handle* h, int32_t* off, int32_t* 
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
     const size_t n = (size_t)h->n;
-    if (off) CK(cudaMemcpyAsync(off, h->d_off, ((size_t)h->T + 1) * sizeof(int), cudaMemcpyDefault, h->stream));
-    if (beam) CK(cudaMemcpyAsync(beam, h->d_beam, n * sizeof(int), cudaMemcpyDefault, h->stream));
-    if (d) CK(cudaMemcpyAsync(d, h->d_d, n * sizeof(double), cudaMemcpyDefault, h->stream));
-    if (bx) CK(cudaMemcpyAsync(bx, h->d_bx, n * sizeof(double), cudaMemcpyDefault, h->stream));
-    if (by) CK(cudaMemcpyAsync(by, h->d_by, n * sizeof(double), cudaMemcpyDefault, h->stream));
+    if (off) CK(cudaMemcpyAsync(off, h->ex.d_off, ((size_t)h->T + 1) * sizeof(int), cudaMemcpyDefault, h->stream));
+    if (beam) CK(cudaMemcpyAsync(beam, h->ex.d_beam, n * sizeof(int), cudaMemcpyDefault, h->stream));
+    if (d) CK(cudaMemcpyAsync(d, h->ex.d_d, n * sizeof(double), cudaMemcpyDefault, h->stream));
+    if (bx) CK(cudaMemcpyAsync(bx, h->ex.d_bx, n * sizeof(double), cudaMemcpyDefault, h->stream));
+    if (by) CK(cudaMemcpyAsync(by, h->ex.d_by, n * sizeof(double), cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return ICMSLAM_OK;
 }
@@ -809,7 +808,7 @@ static int run_filter(icmslam_handle* h, const double* raw_x, const double* raw_
                                                             h->d_oc);
     CK(cudaGetLastError());
     k_filter_finalize<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_used, h->d_rank, h->d_ox, h->d_oy, h->d_oc, map_out, cap_out,
-                                                           ld_out, update_state ? h->d_counts : nullptr, counts_out, L,
+                                                           ld_out, update_state ? h->d_counts.p : nullptr, counts_out, L,
                                                            update_state);
     CK(cudaGetLastError());
     return ICMSLAM_OK;
@@ -895,7 +894,7 @@ static int ensure_stats_clean(icmslam_handle* h)
     cudaStream_t s = h->stream;
     CK(cudaMemsetAsync(h->d_cnt, 0, ((size_t)h->Lcap + 1) * sizeof(int), s));
     if (h->d_fsum_x) CK(cudaMemsetAsync(h->d_fsum_x, 0, (size_t)2 * h->Lcap * sizeof(long long), s));
-    if (h->d_farbits) CK(cudaMemsetAsync(h->d_farbits, 0, (size_t)h->n_tiles_alloc * 4 * sizeof(unsigned), s));
+    if (h->ex.d_farbits) CK(cudaMemsetAsync(h->ex.d_farbits, 0, (size_t)h->n_tiles_alloc * 4 * sizeof(unsigned), s));
     h->ch.stats_clean = true;
     return ICMSLAM_OK;
 }
@@ -942,7 +941,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
         h->ch.hint_map = nullptr;
     }
     double4* pp_in = ppar_for(h, xin);
-    double4* pp_out = h->d_ppar[pp_in == h->d_ppar[0] ? 1 : 0];      // (the other one, whatever buffer kout is)
+    double4* pp_out = h->ex.d_ppar[pp_in == h->ex.d_ppar[0] ? 1 : 0];      // (the other one, whatever buffer kout is)
     if (!hp) {
         int rc = ensure_ppar(h, xin, ldin, x0, pp_in);
         if (rc) return rc;
@@ -950,24 +949,24 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     const int t_start = h->seg_lo - (h->seg_first ? 0 : 1);     // a later segment also forms the moments of its odd halo pose
     RunParams R;
     R.t_start = t_start; R.t_hi = h->seg_hi; R.halo_t = h->seg_first ? -1 : t_start; R.maxr = h->rec_maxr; R.ppar = pp_in; R.lmrec = h->d_lmrec2[h->ch.lm_cur];
-    R.rec_sb = h->d_rec_sb; R.rec_meta = h->d_rec_meta; R.nruns = h->d_nruns; R.tile_perm = h->d_tile_perm; R.pos_nruns = h->d_pos_nruns; R.tile_epoch = h->d_tile_epoch; R.dyn = h->d_dyn;
-    R.fsum_x = h->d_fsum_x; R.fsum_y = h->d_fsum_y; R.cnt = h->d_cnt; R.fix_scale = h->fix_scale; R.tile_slots = h->d_tile_slots; R.tile_nslots = h->d_tile_nslots;
-    R.far_list = h->d_far_list; R.ts = h->d_ts; R.farbits = h->d_farbits;
-    R.scan_dirty = h->d_scan_dirty; R.tile_flag = h->d_tile_flag; R.dirty_list = h->d_dirty_list;
+    R.rec_sb = h->ex.d_rec_sb; R.rec_meta = h->ex.d_rec_meta; R.nruns = h->ex.d_nruns; R.tile_perm = h->ex.d_tile_perm; R.pos_nruns = h->ex.d_pos_nruns; R.tile_epoch = h->ex.d_tile_epoch; R.dyn = h->ex.d_dyn;
+    R.fsum_x = h->d_fsum_x; R.fsum_y = h->d_fsum_y; R.cnt = h->d_cnt; R.fix_scale = h->fix_scale; R.tile_slots = h->ex.d_tile_slots; R.tile_nslots = h->ex.d_tile_nslots;
+    R.far_list = h->ds.d_far_list; R.ts = h->d_ts; R.farbits = h->ex.d_farbits;
+    R.scan_dirty = h->ex.d_scan_dirty; R.tile_flag = h->ex.d_tile_flag; R.dirty_list = h->ex.d_dirty_list;
     R.geom = h->d_fg_geom; R.cell_start = h->d_fg_start; R.gpts = h->d_fg_pts; R.dist_thr = h->dcfg.dist_thr;
     R.st = st; R.L_in = h->begin_L; R.slice0 = 0; R.fz = h->fz;
     AssocParams A;
-    A.first_halo = h->seg_first ? 0 : 1; A.T = T; A.off = h->d_off; A.bxy = h->d_bxy; A.cfg = h->dcfg; A.thr2_hi = h->thr2_hi; A.st = st; A.geom = h->d_fg_geom;
+    A.first_halo = h->seg_first ? 0 : 1; A.T = T; A.off = h->ex.d_off; A.bxy = h->ex.d_bxy; A.cfg = h->dcfg; A.thr2_hi = h->thr2_hi; A.st = st; A.geom = h->d_fg_geom;
     A.cell_start = h->d_fg_start; A.gpts = h->d_fg_pts; A.gidx = h->d_fg_idx; A.remap = h->d_remap;
     { const char* eh = getenv("ICMSLAM_HINTS"); A.skip_hints = (eh && atoi(eh) == 0) ? 1 : 0; }
     A.hints = (h->ch.hint_map == h->d_map_in) ? 1 : 0;
-    A.c = h->d_c; A.obs_cap = h->obs_cap; A.R = R;
-    A.n_tiles = h->n_tiles; A.blk_prefix = h->d_blk_prefix; A.Lcap = L; A.bb = h->d_bb; A.stw = st; A.final = 1; A.p2p = h->p2p;
+    A.c = h->ex.d_c; A.obs_cap = h->obs_cap; A.R = R;
+    A.n_tiles = h->n_tiles; A.blk_prefix = h->ds.d_blk_prefix; A.Lcap = L; A.bb = h->d_bb; A.stw = st; A.final = 1; A.p2p = h->p2p;
     const int nb = h->assoc_blocks < h->n_tiles ? h->assoc_blocks : h->n_tiles;      // grid of the association kernel
     SolveParams P;
     P.T = T; P.t_lo = h->seg_lo; P.t_hi = h->seg_hi; P.lay = traj_layout(h, x0);
     P.xin = xin; P.ldin = ldin; P.xout = kout; P.ldout = kld;
-    P.inc = h->d_inc; P.ldinc = T; P.u = h->d_u; P.ldu = T; P.bm = h->d_bm; P.ldbm = T; P.dyn = h->d_dyn;
+    P.inc = h->ds.d_inc; P.ldinc = T; P.u = h->ds.d_u; P.ldu = T; P.bm = h->ex.d_bm; P.ldbm = T; P.dyn = h->ex.d_dyn;
     P.ppin = pp_in; P.ppout = pp_out; P.cfg = h->dcfg; P.tol = o.newton_tol; P.maxit = o.newton_maxit;
     P.iters = (o.reserved & 1) ? &st->newton_iters : nullptr; P.tile0 = 0;
     P.trace_row = h->trace_on ? &h->d_ts->trace[0][0] : nullptr; P.trace_seq = h->p2p.on ? &h->d_ts->halo_seq : &h->d_ts->sweep_no;
@@ -1027,7 +1026,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     if (h->use_runs) {
         launch_runs(h->n_tiles * RT_SLICES, s, R);
     } else {
-        k_all_dirty<<<nblk(h->n_tiles, 256), 256, 0, s>>>(h->d_tile_flag, h->d_dirty_list, h->d_ts, h->n_tiles, st, h->begin_L);
+        k_all_dirty<<<nblk(h->n_tiles, 256), 256, 0, s>>>(h->ex.d_tile_flag, h->ex.d_dirty_list, h->d_ts, h->n_tiles, st, h->begin_L);
     }
     CK(cudaGetLastError());
     if (timing) CK(cudaEventRecord(h->ev[2], s));
@@ -1069,7 +1068,7 @@ static int fused_part_b(icmslam_handle* h, cudaStream_t s)
 {
     const int L = h->Lcap;
     const int t_start = h->seg_lo - (h->seg_first ? 0 : 1);
-    k_tail_labels<<<148, 256, 0, s>>>(h->d_ts, h->d_far_list, h->d_blk_prefix, h->d_farbits, RT_TILE, t_start, h->d_off, h->d_st, L, h->d_c,
+    k_tail_labels<<<148, 256, 0, s>>>(h->d_ts, h->ds.d_far_list, h->ds.d_blk_prefix, h->ex.d_farbits, RT_TILE, t_start, h->ex.d_off, h->d_st, L, h->ex.d_c,
                                               h->d_newraw, h->d_newraw + L, h->d_cnt, h->p2p);
     CK(cudaGetLastError());
     h->n_launch += 1;
@@ -1107,7 +1106,7 @@ static int fused_part_c(icmslam_handle* h, const double* xout, double* dmap_out,
         a.raw_x = raw_x; a.raw_y = raw_y; a.rawcnt = h->d_rawcnt;
         a.map_out = dmap_out; a.cap_out = out_cap; a.ld_out = out_ld; a.counts_state = h->d_counts; a.remap = h->d_remap; a.Lcap = L;
         a.cpart = h->d_cpart; a.fz = h->fz;
-        a.sh_x = h->d_sh_x; a.sh_y = h->d_sh_y; a.sh_k = h->d_sh_k; a.farbits = h->d_farbits; a.n_far_words = h->n_tiles * 4;
+        a.sh_x = h->d_sh_x; a.sh_y = h->d_sh_y; a.sh_k = h->d_sh_k; a.farbits = h->ex.d_farbits; a.n_far_words = h->n_tiles * 4;
         a.use_cond = 0;
         memset(&a.cond, 0, sizeof a.cond);
         // Inside the library's own graph capture the rest of the chain becomes the body of an IF node whose condition the steady
@@ -1166,7 +1165,7 @@ static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t 
     double* raw_y = h->d_raw + L;
     {
     k_fused_means<<<nblk(L, 256), 256, 0, s>>>(st, h->d_fsum_x, h->d_fsum_y, h->d_cnt, min_x, min_y, 1.0 / h->fix_scale, h->dcfg.cota,
-                                               h->d_newraw, raw_x, raw_y, h->d_kflag, L, h->d_blk_kept, h->d_farbits, h->n_tiles * 4, h->p2p, ts,
+                                               h->d_newraw, raw_x, raw_y, h->d_kflag, L, h->d_blk_kept, h->ex.d_farbits, h->n_tiles * 4, h->p2p, ts,
                                                h->d_cnt, st, h->d_sh_x, h->d_sh_y, h->d_sh_k, h->fz, h->d_counts);
     CK(cudaGetLastError());
     k_tail_compact<<<nblk(L, 256), 256, 0, s>>>(st, h->d_kflag, h->d_blk_kept, h->d_kpos, raw_x, raw_y, h->d_cnt, h->d_kx, h->d_ky, h->d_kc,
@@ -1198,12 +1197,21 @@ static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t 
 static bool pipe_ready(icmslam_handle* h)
 {
     if (h->pipe_events) return true;
-    if (cudaStreamCreateWithFlags(&h->h2d_stream, cudaStreamNonBlocking) != cudaSuccess) { h->pipe_chunks = 1; return false; }
+    if (cudaStreamCreateWithFlags(&h->h2d_stream.p, cudaStreamNonBlocking) != cudaSuccess) { h->pipe_chunks = 1; return false; }
     for (int i = 0; i < 16; ++i)
-        if (cudaEventCreateWithFlags(&h->ev_in[i], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->ev_out[i], cudaEventDisableTiming) != cudaSuccess) { h->pipe_chunks = 1; return false; }
+        if (cudaEventCreateWithFlags(&h->ev_in[i].p, cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&h->ev_out[i].p, cudaEventDisableTiming) != cudaSuccess) { h->pipe_chunks = 1; return false; }
     h->pipe_events = true;
     return true;
+}
+
+// the landmark each observation was matched with, for the RUNNING view (pass 0, reference-mode sweeps): allocated on first use
+static int ensure_seen(icmslam_handle* h)
+{
+    if (h->ex.d_seen_x && h->ex.d_seen_y) return ICMSLAM_OK;
+    CK(h->ex.d_seen_x.alloc((size_t)h->n));
+    CK(h->ex.d_seen_y.alloc((size_t)h->n));
+    return ICMSLAM_OK;
 }
 
 // One sweep on device-resident data.  The previous map is in h->d_map_in (2 x Lcap); L_in is its
@@ -1240,7 +1248,7 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         if (rc) return rc;
         double* kout = xout;
         int64_t kld = ldout;
-        if (xin == xout) { kout = (xin == h->d_x2) ? h->d_x : h->d_x2; kld = T; }
+        if (xin == xout) { kout = (xin == h->ds.d_x2) ? h->ds.d_x : h->ds.d_x2; kld = T; }
         rc = fused_part_a(h, xin, ldin, kout, kld, x0, o, n_search_cap, /*overlap=*/kout == xout, hp);
         if (rc) return rc;
         if (kout != xout) CK(cudaMemcpy2DAsync(xout, (size_t)ldout * 8, kout, (size_t)kld * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToDevice, s));
@@ -1273,49 +1281,49 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         if (rc) return rc;
         h->n_launch += 3;
         PoseArrays A;
-        A.x = dx; A.ldx = ldx; A.odo = h->d_odo; A.ldo = T; A.u = h->d_u; A.ldu = T;
+        A.x = dx; A.ldx = ldx; A.odo = h->ds.d_odo; A.ldo = T; A.u = h->ds.d_u; A.ldu = T;
         A.x0[0] = x0[0]; A.x0[1] = x0[1]; A.x0[2] = x0[2];
-        A.off = h->d_off; A.T = T;
+        A.off = h->ex.d_off; A.T = T;
         if (timing) CK(cudaEventRecord(h->ev[0], s));
-        k_assoc<<<148 * 8, 256, 0, s>>>(T, h->d_off, h->d_bx, h->d_by, dx, ldx, x0[0], x0[1], x0[2], st, h->d_cell_start, h->d_glx,
-                                        h->d_gly, h->d_gidx, h->dcfg.dist_thr, h->d_c, h->d_nfar, h->d_sum_x, h->d_sum_y, h->d_cnt);
+        k_assoc<<<148 * 8, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, x0[0], x0[1], x0[2], st, h->d_cell_start, h->d_glx,
+                                        h->d_gly, h->d_gidx, h->dcfg.dist_thr, h->ex.d_c, h->ds.d_nfar, h->d_sum_x, h->d_sum_y, h->d_cnt);
         CK(cudaGetLastError());
         h->n_launch += 1;
         if (timing) CK(cudaEventRecord(h->ev[1], s));
         // new labels: one per scan that has a far observation, numbered in time order
-        k_flag_positive<<<nblk(T, 256), 256, 0, s>>>(h->d_nfar, T, h->d_flag);
+        k_flag_positive<<<nblk(T, 256), 256, 0, s>>>(h->ds.d_nfar, T, h->ds.d_flag);
         CK(cudaGetLastError());
-        rc = exclusive_sum(h, h->d_flag, h->d_prefix, T);
+        rc = exclusive_sum(h, h->ds.d_flag, h->ds.d_prefix, T);
         if (rc) return rc;
-        k_new_labels<<<148 * 4, 256, 0, s>>>(T, h->d_off, h->d_bx, h->d_by, dx, ldx, x0[0], x0[1], x0[2], st, h->d_nfar, h->d_prefix,
-                                             L, h->d_c, h->d_sum_x, h->d_sum_y, h->d_cnt);
+        k_new_labels<<<148 * 4, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, x0[0], x0[1], x0[2], st, h->ds.d_nfar, h->ds.d_prefix,
+                                             L, h->ex.d_c, h->d_sum_x, h->d_sum_y, h->d_cnt);
         CK(cudaGetLastError());
         h->n_launch += 2;
         const bool running = o.map_view == ICMSLAM_VIEW_RUNNING;
         if (running) {
-            if (!h->d_sorted) {
-                CK(dalloc(&h->d_keys_out, (size_t)n)); CK(dalloc(&h->d_iota, (size_t)n)); CK(dalloc(&h->d_sorted, (size_t)n));
-                CK(dalloc(&h->d_seen_x, (size_t)n)); CK(dalloc(&h->d_seen_y, (size_t)n));
-                k_iota<<<nblk(n, 256), 256, 0, s>>>((int)n, h->d_iota);
+            if (!h->ex.d_sorted) {
+                CK(h->ex.d_keys_out.alloc((size_t)n)); CK(h->ex.d_iota.alloc((size_t)n)); CK(h->ex.d_sorted.alloc((size_t)n));
+                k_iota<<<nblk(n, 256), 256, 0, s>>>((int)n, h->ex.d_iota);
                 CK(cudaGetLastError());
             }
+            rc = ensure_seen(h);
+            if (rc) return rc;
             rc = exclusive_sum(h, h->d_cnt, h->d_seg, L);
             if (rc) return rc;
             int end_bit = 1;
             while ((1ll << end_bit) < (long long)L + 1 && end_bit < 32) ++end_bit;
             size_t bytes = 0;
-            CK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const unsigned*)h->d_c, (unsigned*)h->d_keys_out, h->d_iota, h->d_sorted,
+            CK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const unsigned*)h->ex.d_c.p, (unsigned*)h->ex.d_keys_out.p, h->ex.d_iota.p, h->ex.d_sorted.p,
                                                (int)n, 0, end_bit, s));
             if (bytes > h->sort_bytes) {      // (its own workspace: never invalidates the scans' one that captured graphs use)
-                DFREE(h->d_sort_ws);
                 h->sort_bytes = 0;
-                CK(cudaMalloc(&h->d_sort_ws, bytes));
+                CK(h->d_sort_ws.alloc(bytes));
                 h->sort_bytes = bytes;
             }
-            CK(cub::DeviceRadixSort::SortPairs(h->d_sort_ws, bytes, (const unsigned*)h->d_c, (unsigned*)h->d_keys_out, h->d_iota, h->d_sorted,
+            CK(cub::DeviceRadixSort::SortPairs(h->d_sort_ws, bytes, (const unsigned*)h->ex.d_c.p, (unsigned*)h->ex.d_keys_out.p, h->ex.d_iota.p, h->ex.d_sorted.p,
                                                (int)n, 0, end_bit, s));
-            k_running_mean<<<nblk(L, 128), 128, 0, s>>>(st, h->d_seg, h->d_cnt, h->d_sorted, h->d_scan_of, h->d_bx, h->d_by, dx, ldx,
-                                                        x0[0], x0[1], x0[2], h->d_seen_x, h->d_seen_y, raw_x, raw_y, L);
+            k_running_mean<<<nblk(L, 128), 128, 0, s>>>(st, h->d_seg, h->d_cnt, h->ex.d_sorted, h->ex.d_scan_of, h->ex.d_bx, h->ex.d_by, dx, ldx,
+                                                        x0[0], x0[1], x0[2], h->ex.d_seen_x, h->ex.d_seen_y, raw_x, raw_y, L);
             CK(cudaGetLastError());
             h->n_launch += 1;
         }
@@ -1324,9 +1332,9 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         CK(cudaGetLastError());
         h->n_launch += 1;
         ObsArrays O;
-        O.bx = h->d_bx; O.by = h->d_by; O.d = h->d_d; O.beam = h->d_beam; O.ang = h->d_ang;
+        O.bx = h->ex.d_bx; O.by = h->ex.d_by; O.d = h->ex.d_d; O.beam = h->ex.d_beam; O.ang = h->ds.d_ang;
         SeenSrc S;
-        S.view = o.map_view; S.c = h->d_c; S.seen_x = h->d_seen_x; S.seen_y = h->d_seen_y;
+        S.view = o.map_view; S.c = h->ex.d_c; S.seen_x = h->ex.d_seen_x; S.seen_y = h->ex.d_seen_y;
         S.raw_x = raw_x; S.raw_y = raw_y; S.min_x = min_x; S.min_y = min_y;
         S.lsearch_ptr = &st->lsearch;
         if (timing) CK(cudaEventRecord(h->ev[2], s));
@@ -1396,11 +1404,11 @@ extern "C" int icmslam_sweep(icmslam_handle* h, const double* map_in, int32_t L_
     const bool piped = continued && fused_mode(h, o) && o.reserved == 0 && h->use_runs && h->side_stream && h->seg_first && h->seg_last &&
                        h->seg_lo == 0 && h->pipe_chunks > 1 && h->n_tiles >= h->pipe_tiles_min * h->pipe_chunks && pipe_ready(h);
     if (memspace == ICMSLAM_HOST) {
-        if (!piped) CK(cudaMemcpy2DAsync(h->d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyHostToDevice, s));
+        if (!piped) CK(cudaMemcpy2DAsync(h->ds.d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyHostToDevice, s));
         h->bytes_h2d += (int64_t)3 * T * 8;
         h->ch.ppar_of = nullptr;
-        xin = h->d_x; ldin = T;
-        xout = h->d_x2; ldout = T;
+        xin = h->ds.d_x; ldin = T;
+        xout = h->ds.d_x2; ldout = T;
         pipe.x = x; pipe.ld = ld_x; pipe.chunks = h->pipe_chunks;
     }
     if (!continued) {
@@ -1419,14 +1427,14 @@ extern "C" int icmslam_sweep(icmslam_handle* h, const double* map_in, int32_t L_
     h->d2h_x = nullptr;
     if (rc) return rc;
     if (own_out) {      // mapa_refinado becomes the handle's current map (icmslam_get_map, and the map chain a caller may continue)
-        double* t = h->d_map_in; h->d_map_in = h->d_map_out; h->d_map_out = t;
+        std::swap(h->d_map_in, h->d_map_out);
     }
     if (memspace == ICMSLAM_HOST) {
         if (!h->d2h_done) CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, xout, (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, s));
         h->bytes_d2h += (int64_t)3 * T * 8 + (int64_t)sizeof(DevState);
         // the whole map buffer comes back with the state in ONE asynchronous copy into pinned memory (its width is only known on
         // the device until then); the caller's array -- usually pageable -- is then filled by a host copy
-        if (map_out && !h->h_map_pin) CK(cudaMallocHost((void**)&h->h_map_pin, (size_t)2 * L * sizeof(double)));
+        if (map_out && !h->h_map_pin) CK(h->h_map_pin.alloc((size_t)2 * L));
         if (map_out) {
             CK(cudaMemcpyAsync(h->h_map_pin, h->d_map_in, (size_t)2 * L * sizeof(double), cudaMemcpyDeviceToHost, s));
             h->bytes_d2h += (int64_t)2 * L * 8;       // (what actually crosses the bus: the whole buffer, not only the live columns)
@@ -1494,11 +1502,11 @@ extern "C" int icmslam_get_map(icmslam_handle* h, double* map, int32_t cap, int6
 // icmslam_get_poses reads them back.
 extern "C" int icmslam_set_poses(icmslam_handle* h, const double* x, int64_t ld_x, int32_t memspace)
 {
-    if (!h || !h->d_x || !x || ld_x < h->T) return ICMSLAM_ERR_INVALID;
+    if (!h || !h->ds.d_x || !x || ld_x < h->T) return ICMSLAM_ERR_INVALID;
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
     const int T = h->T;
-    CK(cudaMemcpy2DAsync(h->d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(h->ds.d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->ch.x_cur = 0;
     h->ch.ppar_of = nullptr;
@@ -1507,7 +1515,7 @@ extern "C" int icmslam_set_poses(icmslam_handle* h, const double* x, int64_t ld_
 
 extern "C" int icmslam_get_poses(icmslam_handle* h, double* x, int64_t ld_x, int32_t memspace)
 {
-    if (!h || !h->d_x || !x || ld_x < h->T) return ICMSLAM_ERR_INVALID;
+    if (!h || !h->ds.d_x || !x || ld_x < h->T) return ICMSLAM_ERR_INVALID;
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
     const int T = h->T;
@@ -1531,7 +1539,7 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
     const bool fused = fused_mode(h, o);
     if (h->p2p.on && !fused) return ICMSLAM_ERR_UNSUPPORTED;      // only the restated parallel sweep partitions in time
     if (x) {
-        CK(cudaMemcpy2DAsync(h->d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, s));
+        CK(cudaMemcpy2DAsync(h->ds.d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, s));
         h->ch.x_cur = 0;
         h->ch.ppar_of = nullptr;
     }
@@ -1572,9 +1580,9 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
                     if (!rc) snprintf(h->err, sizeof h->err, "graph capture of the sweep failed (%s)", cudaGetErrorString(ce));
                     return rc ? rc : ICMSLAM_ERR_CUDA;
                 }
-                ce = cudaGraphInstantiate(&slot->exec, graph, cudaGraphInstantiateFlagUseNodePriority);   // (nodes keep the priority of the stream they were captured on)
+                ce = cudaGraphInstantiate(&slot->exec.p, graph, cudaGraphInstantiateFlagUseNodePriority);   // (nodes keep the priority of the stream they were captured on)
                 cudaGraphDestroy(graph);
-                if (ce != cudaSuccess) { slot->exec = nullptr; snprintf(h->err, sizeof h->err, "cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return ICMSLAM_ERR_CUDA; }
+                if (ce != cudaSuccess) { slot->exec.p = nullptr; snprintf(h->err, sizeof h->err, "cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return ICMSLAM_ERR_CUDA; }
                 slot->src = src; slot->map_in = h->d_map_in; slot->x0[0] = x0[0]; slot->x0[1] = x0[1]; slot->x0[2] = x0[2];
                 slot->tol = o.newton_tol; slot->maxit = o.newton_maxit; slot->lm = h->ch.lm_cur; slot->fz = h->fz; slot->launches = launches;
             }
@@ -1603,24 +1611,23 @@ extern "C" int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double
 {
     if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
-    if (traj_T <= 0) { h->traj_T = 0; h->traj_K = 0; DFREE(h->d_x0s); h->ch.ppar_of = nullptr; drop_graphs(h); return ICMSLAM_OK; }
+    if (traj_T <= 0) { drop_graphs(h); h->traj_T = 0; h->traj_K = 0; h->d_x0s.reset(); h->ch.ppar_of = nullptr; return ICMSLAM_OK; }
     if (!x0s || K <= 0 || ld_x0s < K || (int64_t)traj_T * K != h->T || traj_T < 3 || !h->fused_ok) return ICMSLAM_ERR_INVALID;
     // every trajectory needs a non-empty first and last scan (the reference returns early / raises otherwise, sensors.py:137, :148)
     std::vector<int> off((size_t)h->T + 1);
-    CK(cudaMemcpyAsync(off.data(), h->d_off, ((size_t)h->T + 1) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(off.data(), h->ex.d_off, ((size_t)h->T + 1) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     for (int k = 0; k < K; ++k) {
         const int a = k * traj_T, b = (k + 1) * traj_T - 1;
         if (off[a + 1] == off[a] || off[b + 1] == off[b]) return ICMSLAM_ERR_UNSUPPORTED;
     }
-    DFREE(h->d_x0s);
-    CK(dalloc(&h->d_x0s, (size_t)3 * K));
+    drop_graphs(h);      // (before the old buffer goes: graphs hold it)
+    CK(h->d_x0s.alloc((size_t)3 * K));
     CK(cudaMemcpy2DAsync(h->d_x0s, (size_t)K * 8, x0s, (size_t)ld_x0s * 8, (size_t)K * 8, 3, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->traj_T = traj_T; h->traj_K = K;
     h->first_empty = false; h->last_empty = false;
     h->ch.ppar_of = nullptr;
-    drop_graphs(h);
     return ICMSLAM_OK;
 }
 
@@ -1633,7 +1640,7 @@ extern "C" int icmslam_set_segment(icmslam_handle* h, int32_t t_lo, int32_t t_hi
     h->n_tiles = nblk(t_hi - (t_lo - (is_first ? 0 : 1)), RT_TILE);
     h->n_solve_tiles = nblk(t_hi - t_lo, ST_OWN);
     // the record tiling moved: no tile holds records (epoch -1)
-    CK(cudaMemsetAsync(h->d_tile_epoch, 0xff, ((size_t)nblk(h->T + 1, RT_TILE) + 2) * sizeof(int), h->stream));
+    CK(cudaMemsetAsync(h->ex.d_tile_epoch, 0xff, ((size_t)nblk(h->T + 1, RT_TILE) + 2) * sizeof(int), h->stream));
     drop_graphs(h);
     return ICMSLAM_OK;
 }
@@ -1664,9 +1671,9 @@ extern "C" int icmslam_p2p_export(icmslam_handle* h, void* handles, int64_t cap_
     if (!h || !handles || cap_bytes < (int64_t)(3 * sizeof(cudaIpcMemHandle_t)) || !h->d_exch) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
     if (!h->d_win) {
-        CK(cudaMalloc((void**)&h->d_win, sizeof(P2PWin)));
+        CK(h->d_win.alloc(1));
         CK(cudaMemset(h->d_win, 0, sizeof(P2PWin)));
-        CK(cudaMalloc((void**)&h->d_res, (size_t)h->exch_words * 8));
+        CK(h->d_res.alloc((size_t)h->exch_words));
         CK(cudaMemset(h->d_res, 0, (size_t)h->exch_words * 8));
     }
     cudaIpcMemHandle_t* out = (cudaIpcMemHandle_t*)handles;
@@ -1686,6 +1693,7 @@ extern "C" int icmslam_p2p_import(icmslam_handle* h, int32_t rank, int32_t world
         return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
     CK(cudaStreamSynchronize(h->stream));
+    drop_graphs(h);      // (before the old mappings are closed: graphs of the old exchange hold them through the pointer table)
     const cudaIpcMemHandle_t* hs = (const cudaIpcMemHandle_t*)all;
     void* tab[3 * P2P_MAX_WORLD] = {};
     for (int r = 0; r < world; ++r) {
@@ -1693,24 +1701,23 @@ extern "C" int icmslam_p2p_import(icmslam_handle* h, int32_t rank, int32_t world
             void* ptr = nullptr;
             if (r == rank) ptr = k == 0 ? (void*)h->d_exch : (k == 1 ? (void*)h->d_win : (void*)h->d_res);
             else {
-                if (h->p2p_opened[3 * r + k]) { cudaIpcCloseMemHandle(h->p2p_opened[3 * r + k]); h->p2p_opened[3 * r + k] = nullptr; }
+                h->p2p_opened[3 * r + k].reset();
                 CK(cudaIpcOpenMemHandle(&ptr, hs[3 * r + k], cudaIpcMemLazyEnablePeerAccess));
-                h->p2p_opened[3 * r + k] = ptr;
+                h->p2p_opened[3 * r + k].p = ptr;
             }
             tab[k * P2P_MAX_WORLD + r] = ptr;      // three tables of P2P_MAX_WORLD pointers: exchange blocks, windows, result buffers
         }
     }
-    if (!h->d_p2p_ptrs) CK(cudaMalloc((void**)&h->d_p2p_ptrs, sizeof tab));
+    if (!h->d_p2p_ptrs) CK(h->d_p2p_ptrs.alloc(3 * P2P_MAX_WORLD));
     CK(cudaMemcpy(h->d_p2p_ptrs, tab, sizeof tab, cudaMemcpyHostToDevice));
     P2PDev& p = h->p2p;
     p.on = world > 1 ? 1 : 0; p.rank = rank; p.world = world;
-    p.exch = (const long long* const*)(h->d_p2p_ptrs);
+    p.exch = (const long long* const*)h->d_p2p_ptrs.p;
     p.win = (P2PWin* const*)(h->d_p2p_ptrs + P2P_MAX_WORLD);
     p.res = (const long long* const*)(h->d_p2p_ptrs + 2 * P2P_MAX_WORLD);
     p.my_res = h->d_res;
     p.words = h->exch_words;
     p.per = (h->exch_words + world - 1) / world;
-    drop_graphs(h);
     return ICMSLAM_OK;
 }
 
@@ -1842,7 +1849,7 @@ extern "C" int icmslam_get_associations(icmslam_handle* h, int32_t* c, int32_t m
     if (!h || !h->extracted || !c) return ICMSLAM_ERR_INVALID;
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
-    CK(cudaMemcpyAsync(c, h->d_c, (size_t)h->n * sizeof(int), cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpyAsync(c, h->ex.d_c, (size_t)h->n * sizeof(int), cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return ICMSLAM_OK;
 }
@@ -1956,22 +1963,20 @@ extern "C" int icmslam_pose_eval(icmslam_handle* h, int32_t model, int32_t op, i
     CK(cudaSetDevice(h->cfg.device));
     cudaStream_t s = h->stream;
     const size_t nn = (size_t)(n > 0 ? n : 1);
-    double* dbuf = nullptr;
-    int* ibuf = nullptr;
-    CK(cudaMalloc((void**)&dbuf, (6 * nn + 8) * sizeof(double)));
-    if (cudaMalloc((void**)&ibuf, nn * sizeof(int)) != cudaSuccess) { cudaFree(dbuf); return ICMSLAM_ERR_ALLOC; }
+    DevBuf<double> dbuf;
+    DevBuf<int> ibuf;
+    CK(dbuf.alloc(6 * nn + 8));
+    if (ibuf.alloc(nn) != cudaSuccess) return ICMSLAM_ERR_ALLOC;
     PoseEvalArgs a;
     memset(&a, 0, sizeof a);
     a.op = op; a.n = n; a.has_next = x_pos ? 1 : 0; a.maxit = o.newton_maxit; a.tol = o.newton_tol;
     double* dz = dbuf; double* dang = dbuf + nn; double* dsx = dbuf + 2 * nn; double* dsy = dbuf + 3 * nn;
     a.zd = dz; a.zang = dang; a.sx = dsx; a.sy = dsy; a.bx = dbuf + 4 * nn; a.by = dbuf + 5 * nn; a.out = dbuf + 6 * nn; a.iota = ibuf;
-    int rc = ICMSLAM_OK;
-    cudaError_t ce = cudaSuccess;
     if (n > 0) {
-        ce = cudaMemcpyAsync(dz, z_d, (size_t)n * 8, cudaMemcpyHostToDevice, s);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(dang, z_ang, (size_t)n * 8, cudaMemcpyHostToDevice, s);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(dsx, seen_x, (size_t)n * 8, cudaMemcpyHostToDevice, s);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(dsy, seen_y, (size_t)n * 8, cudaMemcpyHostToDevice, s);
+        CK(cudaMemcpyAsync(dz, z_d, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(dang, z_ang, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(dsx, seen_x, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(dsy, seen_y, (size_t)n * 8, cudaMemcpyHostToDevice, s));
     }
     for (int j = 0; j < 3; ++j) {
         a.x[j] = x[j];
@@ -1982,19 +1987,15 @@ extern "C" int icmslam_pose_eval(icmslam_handle* h, int32_t model, int32_t op, i
     if (u_ant) { a.ua[0] = u_ant[0]; a.ua[1] = u_ant[1]; }
     if (u_act) { a.uc[0] = u_act[0]; a.uc[1] = u_act[1]; }
     double out[5] = {0, 0, 0, 0, 0};
-    if (ce == cudaSuccess) {
-        k_pose_eval<<<1, 1, 0, s>>>(h->dcfg, a);
-        ce = cudaGetLastError();
-        h->n_launch += 1;
-    }
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(out, a.out, sizeof out, cudaMemcpyDeviceToHost, s);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
-    cudaFree(dbuf); cudaFree(ibuf);
-    if (ce != cudaSuccess) { snprintf(h->err, sizeof h->err, "icmslam_pose_eval: %s", cudaGetErrorString(ce)); return ICMSLAM_ERR_CUDA; }
+    k_pose_eval<<<1, 1, 0, s>>>(h->dcfg, a);
+    CK(cudaGetLastError());
+    h->n_launch += 1;
+    CK(cudaMemcpyAsync(out, a.out, sizeof out, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     if (op != ICMSLAM_POSE_ENERGY && op != ICMSLAM_POSE_H) { x[0] = out[0]; x[1] = out[1]; x[2] = out[2]; }
     if (f) *f = out[3];
     if (n_eval) *n_eval = (int32_t)out[4];
-    return rc;
+    return ICMSLAM_OK;
 }
 
 // instrumentation: the ring of %globaltimer marks (32 sweeps x 8 marks, nanoseconds; TailState::trace) and the sweep counters
@@ -2342,11 +2343,10 @@ extern "C" int icmslam_batch_iterate_until(icmslam_handle* h, int32_t max_sweeps
         }
     }
     if (h->fz_K != K) {
-        DFREE(h->d_fz_mask); DFREE(h->d_fz_need); DFREE(h->d_fz_slots); DFREE(h->d_fz_reg);
-        h->fz_K = 0;
         drop_graphs(h);      // (graphs of an earlier call hold the old buffers)
-        CK(dalloc(&h->d_fz_mask, (size_t)K)); CK(dalloc(&h->d_fz_need, (size_t)K));
-        CK(dalloc(&h->d_fz_slots, (size_t)FZ_SLOTS * K)); CK(dalloc(&h->d_fz_reg, (size_t)L));
+        h->fz_K = 0;
+        CK(h->d_fz_mask.alloc((size_t)K)); CK(h->d_fz_need.alloc((size_t)K));
+        CK(h->d_fz_slots.alloc((size_t)FZ_SLOTS * K)); CK(h->d_fz_reg.alloc((size_t)L));
         h->fz_K = K;
     }
     CK(cudaMemsetAsync(h->d_fz_mask, 0, (size_t)K, s));
@@ -2365,10 +2365,10 @@ extern "C" int icmslam_filtrar_obs(icmslam_handle* h, const double* obs, int32_t
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
     cudaStream_t s = h->stream;
-    double *d_in = nullptr, *d_out = nullptr;
-    int *d_a = nullptr, *d_keep = nullptr, *d_err = nullptr;
-    CK(dalloc(&d_in, (size_t)B * T)); CK(dalloc(&d_out, (size_t)B * T));
-    CK(dalloc(&d_a, (size_t)T)); CK(dalloc(&d_keep, (size_t)T)); CK(dalloc(&d_err, 1));
+    DevBuf<double> d_in, d_out;
+    DevBuf<int> d_a, d_keep, d_err;
+    CK(d_in.alloc((size_t)B * T)); CK(d_out.alloc((size_t)B * T));
+    CK(d_a.alloc((size_t)T)); CK(d_keep.alloc((size_t)T)); CK(d_err.alloc(1));
     CK(cudaMemcpy2DAsync(d_in, (size_t)T * 8, obs, (size_t)ld * 8, (size_t)T * 8, B, cudaMemcpyDefault, s));
     CK(cudaMemsetAsync(d_err, 0, sizeof(int), s));
     k_fo_count<<<nblk(T, 128), 128, 0, s>>>(d_in, B, T, T, max_dist, d_a);
@@ -2383,7 +2383,6 @@ extern "C" int icmslam_filtrar_obs(icmslam_handle* h, const double* obs, int32_t
     CK(cudaMemcpyAsync(&err, d_err, sizeof(int), cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpy2DAsync(out, (size_t)ld_out * 8, d_out, (size_t)T * 8, (size_t)T * 8, B, cudaMemcpyDefault, s));
     CK(cudaStreamSynchronize(s));
-    cudaFree(d_in); cudaFree(d_out); cudaFree(d_a); cudaFree(d_keep); cudaFree(d_err);
     return err ? ICMSLAM_ERR_INVALID : ICMSLAM_OK;
 }
 
@@ -2398,24 +2397,23 @@ extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int
     if (h->max_per_scan > 1024) return ICMSLAM_ERR_UNSUPPORTED;
     CK(cudaSetDevice(h->cfg.device));
     const int T = h->T, L = h->Lcap;
-    const int64_t n = h->n;
     cudaStream_t s = h->stream;
     if (h->first_empty) return ICMSLAM_EMPTY_FIRST_SCAN;        // (the reference would fail inside tras_rot_z / linkage)
     h->ch.grid_map = nullptr; h->ch.hint_map = nullptr;
-    if (!h->d_seen_x) { CK(dalloc(&h->d_seen_x, (size_t)n)); CK(dalloc(&h->d_seen_y, (size_t)n)); }
+    int rc = ensure_seen(h);
+    if (rc) return rc;
     // ---- step 0: Branch A of Mapa.actualizar on the first scan (ICM_SLAM.py:160-165), on the host ------------------
     std::vector<int> off2(2);
-    CK(cudaMemcpyAsync(off2.data(), h->d_off, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(off2.data(), h->ex.d_off, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     const int n0 = off2[1] - off2[0];
-    double *d_w = nullptr;
-    CK(dalloc(&d_w, (size_t)2 * n0));
-    k_project_scan<<<nblk(n0, 128), 128, 0, s>>>(h->d_off, 0, h->d_bx, h->d_by, x0[0], x0[1], x0[2], d_w, d_w + n0);
+    DevBuf<double> d_w;
+    CK(d_w.alloc((size_t)2 * n0));
+    k_project_scan<<<nblk(n0, 128), 128, 0, s>>>(h->ex.d_off, 0, h->ex.d_bx, h->ex.d_by, x0[0], x0[1], x0[2], d_w, d_w + n0);
     CK(cudaGetLastError());
     std::vector<double> w((size_t)2 * n0);
     CK(cudaMemcpyAsync(w.data(), d_w, (size_t)2 * n0 * 8, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    cudaFree(d_w);
     std::vector<int> lab0(n0);
     const int k0 = icm_fcluster::fcluster_inconsistent(w.data(), w.data() + n0, n0, h->cfg.dist_thr, lab0.data());
     if (k0 > L) return ICMSLAM_ERR_LABEL_CAP;
@@ -2428,16 +2426,16 @@ extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int
     }
     CK(cudaMemcpyAsync(h->d_raw, y0.data(), (size_t)2 * L * 8, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(h->d_tmp_b, cant0.data(), (size_t)L * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(h->d_c, lab0.data(), (size_t)n0 * sizeof(int), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(h->ex.d_c, lab0.data(), (size_t)n0 * sizeof(int), cudaMemcpyHostToDevice, s));
     // ---- steps 1 .. T-1 on the device -------------------------------------------------------------------------------
     double* dx = x;
     int64_t ldx = ld_x;
-    if (memspace == ICMSLAM_HOST) { dx = h->d_x; ldx = T; }
+    if (memspace == ICMSLAM_HOST) { dx = h->ds.d_x; ldx = T; }
     Pass0Params P;
-    P.T = T; P.Lcap = L; P.off = h->d_off; P.bx = h->d_bx; P.by = h->d_by; P.d = h->d_d; P.beam = h->d_beam; P.ang = h->d_ang;
-    P.odo = h->d_odo; P.ldo = T; P.u = h->d_u; P.ldu = T; P.cfg = h->dcfg;
+    P.T = T; P.Lcap = L; P.off = h->ex.d_off; P.bx = h->ex.d_bx; P.by = h->ex.d_by; P.d = h->ex.d_d; P.beam = h->ex.d_beam; P.ang = h->ds.d_ang;
+    P.odo = h->ds.d_odo; P.ldo = T; P.u = h->ds.d_u; P.ldu = T; P.cfg = h->dcfg;
     P.x0[0] = x0[0]; P.x0[1] = x0[1]; P.x0[2] = x0[2];
-    P.x = dx; P.ldx = ldx; P.y = h->d_raw; P.cant = h->d_tmp_b; P.lact0 = k0; P.c = h->d_c; P.seen_x = h->d_seen_x; P.seen_y = h->d_seen_y;
+    P.x = dx; P.ldx = ldx; P.y = h->d_raw; P.cant = h->d_tmp_b; P.lact0 = k0; P.c = h->ex.d_c; P.seen_x = h->ex.d_seen_x; P.seen_y = h->ex.d_seen_y;
     P.st = h->d_st; P.nev = &h->d_st->newton_iters;
     k_set_raw_l<<<1, 1, 0, s>>>(h->d_st, k0);                     // (also clears the status word)
     CK(cudaGetLastError());
@@ -2446,7 +2444,7 @@ extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int
     k_pass0<<<1, 256, smem, s>>>(P);
     CK(cudaGetLastError());
     h->n_launch += 2;
-    int rc = sync_state(h);
+    rc = sync_state(h);
     if (rc) return rc;
     if (h->h_st->status & ST_LABEL_CAP) return ICMSLAM_ERR_LABEL_CAP;
     const int lact = h->h_st->lact;
