@@ -1,7 +1,8 @@
-// assoc.cuh -- landmark grid, data association, label assignment, landmark statistics
+// assoc.cuh -- data association, label assignment, landmark statistics
 // (Mapa.actualizar Branch B, ICM_SLAM.py:167-194, for all scans of a sweep at once).
 #pragma once
 #include "common.cuh"
+#include "fastgrid.cuh"
 
 // Device-resident sweep state (no host round trip inside a sweep).
 struct DevState {
@@ -17,100 +18,10 @@ struct DevState {
     int dirty_tiles; // record tiles that went through the association kernel this sweep (runs.cuh; filled on request)
     unsigned long long newton_iters;
     unsigned long long solved;
-    // grid parameters of the association grid / filter grid
-    double gx0, gy0, ginv_h;
-    int gnx, gny;
-    double fx0, fy0, finv_h;
-    int fnx, fny;
-    double f_extent;  // max bbox extent of the kept landmarks
     double cambio[3]; // calc_cambio of the sweep's map against the previous one, accumulated by the fast tail: min, max, sum
     int cambio_unres; // new landmarks whose nearest old landmark the tail could not certify (then cambio[] is not usable)
     int cambio_pad;
 };
-
-// ---- grid construction ---------------------------------------------------------------------
-// bounding box of the first n points -> grid origin / dims (one block).  n is read from the
-// device (pointer) so the whole sweep stays capturable.
-__global__ void k_grid_setup(const double* __restrict__ px, const double* __restrict__ py, const int* __restrict__ n_ptr,
-                             double dist_thr, int max_cells, double* gx0, double* gy0, double* ginv_h, int* gnx, int* gny,
-                             double* extent)
-{
-    __shared__ double sh[4][32];
-    const int n = *n_ptr;
-    double mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        double x = px[i], y = py[i];
-        mnx = fmin(mnx, x); mxx = fmax(mxx, x);
-        mny = fmin(mny, y); mxy = fmax(mxy, y);
-    }
-    mnx = warp_min(mnx); mny = warp_min(mny); mxx = warp_max(mxx); mxy = warp_max(mxy);
-    int w = threadIdx.x / WARP, l = threadIdx.x % WARP;
-    if (l == 0) { sh[0][w] = mnx; sh[1][w] = mny; sh[2][w] = mxx; sh[3][w] = mxy; }
-    __syncthreads();
-    if (w == 0) {
-        int nw = blockDim.x / WARP;
-        mnx = l < nw ? sh[0][l] : INFINITY; mny = l < nw ? sh[1][l] : INFINITY;
-        mxx = l < nw ? sh[2][l] : -INFINITY; mxy = l < nw ? sh[3][l] : -INFINITY;
-        mnx = warp_min(mnx); mny = warp_min(mny); mxx = warp_max(mxx); mxy = warp_max(mxy);
-        if (l == 0) {
-            if (n <= 0) { mnx = mny = 0.0; mxx = mxy = 0.0; }
-            double h = dist_thr * (1.0 + 9.5367431640625e-07);   // 1 + 2^-20
-            if (!(h > 0.0)) h = 1.0;
-            double ex = mxx - mnx, ey = mxy - mny;
-            // grow the cell until the grid fits the fixed cell budget (still >= dist_thr: exact)
-            for (;;) {   // (+1 slack per axis: the two floor() evaluations may differ by one at a boundary)
-                double nxd = floor(ex / h) + 2.0, nyd = floor(ey / h) + 2.0;
-                if (nxd * nyd <= (double)max_cells) break;
-                h *= 1.5;
-            }
-            *gx0 = mnx; *gy0 = mny; *ginv_h = 1.0 / h;
-            *gnx = grid_coord(mxx, mnx, 1.0 / h) + 1;
-            *gny = grid_coord(mxy, mny, 1.0 / h) + 1;
-            if (extent) *extent = fmax(ex, ey);
-        }
-    }
-}
-
-__device__ __forceinline__ int cell_of(double x, double y, double gx0, double gy0, double inv_h, int nx, int ny)
-{
-    int cx = min(max(grid_coord(x, gx0, inv_h), 0), nx - 1);
-    int cy = min(max(grid_coord(y, gy0, inv_h), 0), ny - 1);
-    return cy * nx + cx;
-}
-
-__global__ void k_cell_count(const double* __restrict__ px, const double* __restrict__ py, const int* __restrict__ n_ptr,
-                             const double* gx0, const double* gy0, const double* ginv_h, const int* gnx, const int* gny,
-                             int* __restrict__ cell_cnt, int* __restrict__ cell_id)
-{
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= *n_ptr) return;
-    int c = cell_of(px[i], py[i], *gx0, *gy0, *ginv_h, *gnx, *gny);
-    cell_id[i] = c;
-    atomicAdd(cell_cnt + c, 1);
-}
-
-__global__ void k_cell_fill(const double* __restrict__ px, const double* __restrict__ py, const int* __restrict__ n_ptr,
-                            const int* __restrict__ cell_id, const int* __restrict__ cell_start, int* __restrict__ cell_fill,
-                            double* __restrict__ sx, double* __restrict__ sy, int* __restrict__ sidx)
-{
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= *n_ptr) return;
-    int c = cell_id[i];
-    int p = cell_start[c] + atomicAdd(cell_fill + c, 1);
-    sx[p] = px[i];
-    sy[p] = py[i];
-    sidx[p] = i;
-}
-
-__device__ __forceinline__ Grid load_grid(const double* gx0, const double* gy0, const double* ginv_h, const int* gnx,
-                                          const int* gny, const int* cell_start, const double* lx, const double* ly,
-                                          const int* lidx, int n)
-{
-    Grid g;
-    g.x0 = *gx0; g.y0 = *gy0; g.inv_h = *ginv_h; g.nx = *gnx; g.ny = *gny;
-    g.cell_start = cell_start; g.lx = lx; g.ly = ly; g.lidx = lidx; g.n = n;
-    return g;
-}
 
 // ---- association ---------------------------------------------------------------------------
 // One warp per scan, lanes over the scan's kept observations.  Projects with the sweep's INPUT
@@ -119,14 +30,14 @@ __device__ __forceinline__ Grid load_grid(const double* gx0, const double* gy0, 
 // observations add into the per-label sums; far ones are marked -1 and counted per scan.
 __global__ void __launch_bounds__(256)
 k_assoc(int T, const int* __restrict__ off, const double* __restrict__ bx, const double* __restrict__ by,
-        const double* __restrict__ x, int64_t ldx, double x0x, double x0y, double x0t, DevState* st,
-        const int* __restrict__ cell_start, const double* __restrict__ glx, const double* __restrict__ gly,
-        const int* __restrict__ gidx, double dist_thr, int* __restrict__ c, int* __restrict__ nfar,
-        double* __restrict__ sum_x, double* __restrict__ sum_y, int* __restrict__ cnt)
+        const double* __restrict__ x, int64_t ldx, double x0x, double x0y, double x0t, const FGeom* __restrict__ geom,
+        const int* __restrict__ cell_start, const double2* __restrict__ pts, const int* __restrict__ gidx, double thr2_hi,
+        int* __restrict__ c, int* __restrict__ nfar, double* __restrict__ sum_x, double* __restrict__ sum_y, int* __restrict__ cnt)
 {
     const int lane = threadIdx.x % WARP;
     const int wpb = blockDim.x / WARP;
-    Grid g = load_grid(&st->gx0, &st->gy0, &st->ginv_h, &st->gnx, &st->gny, cell_start, glx, gly, gidx, st->lsearch);
+    FGrid G;
+    G.g = *geom; G.cell_start = cell_start; G.pts = pts; G.idx = gidx;
     for (int t = blockIdx.x * wpb + threadIdx.x / WARP; t < T; t += gridDim.x * wpb) {
         int o = off[t], e = off[t + 1];
         int far = 0;
@@ -136,13 +47,12 @@ k_assoc(int T, const int* __restrict__ off, const double* __restrict__ bx, const
             else { px = x[t]; py = x[ldx + t]; th = x[2 * ldx + t]; }
             Rot r = make_rot(th);
             for (int i = o + lane; i < e; i += WARP) {
-                double wx, wy, best, lxb, lyb;
-                int arg;
+                double wx, wy, best;
                 project(r, px, py, bx[i], by[i], wx, wy);
-                if (g.n > 0) grid_nearest(g, wx, wy, best, arg, lxb, lyb);
-                else { best = INFINITY; arg = 0; }
-                if (best > dist_thr) { c[i] = -1; ++far; }
+                const int bk = fgrid_nearest(G, wx, wy, best);      // (an empty map: no candidate, best = INFINITY)
+                if (best > thr2_hi) { c[i] = -1; ++far; }          // sqrt_rn(best) > dist_thr
                 else {
+                    const int arg = __ldg(gidx + bk);
                     c[i] = arg;
                     atomicAdd(sum_x + arg, wx);
                     atomicAdd(sum_y + arg, wy);

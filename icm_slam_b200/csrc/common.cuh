@@ -127,50 +127,3 @@ __device__ __forceinline__ double warp_max(double v)
     for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(FULLMASK, v, o));
     return v;
 }
-
-// Uniform landmark grid used by the association (ICM_SLAM.py:169-172) and by Mapa.filtrar's
-// nearest-neighbour search (ICM_SLAM.py:241-245).  Cell edge h >= dist_thr*(1+2^-20), so every
-// landmark within dist_thr of a point lies in the 3x3 block of cells around the point's cell.
-struct Grid {
-    double x0, y0, inv_h;
-    int nx, ny;
-    const int* cell_start;   // nx*ny + 1
-    const double* lx;        // landmarks sorted by cell
-    const double* ly;
-    const int* lidx;         // original landmark index
-    int n;
-};
-
-__device__ __forceinline__ int grid_coord(double v, double v0, double inv_h)
-{
-    double f = floor((v - v0) * inv_h);
-    // clamp into int range before converting; callers clamp to the grid afterwards
-    f = fmin(fmax(f, -2.0e9), 2.0e9);
-    return (int)f;
-}
-
-// Nearest landmark of (wx, wy) among those within the 3x3 neighbourhood; ties -> lowest original
-// index (np.argmin picks the first minimum).  Returns the rooted distance in `best` (INFINITY if
-// the neighbourhood is empty) and the original index in `arg`.
-__device__ __forceinline__ void grid_nearest(const Grid& g, double wx, double wy, double& best, int& arg, double& lxb,
-                                             double& lyb)
-{
-    best = INFINITY;
-    arg = 0;
-    lxb = 0.0;
-    lyb = 0.0;
-    int cx = grid_coord(wx, g.x0, g.inv_h), cy = grid_coord(wy, g.y0, g.inv_h);
-    if (cx < -1 || cy < -1 || cx > g.nx || cy > g.ny) return;
-    int c0 = max(cx - 1, 0), c1 = min(cx + 1, g.nx - 1);
-    int r0 = max(cy - 1, 0), r1 = min(cy + 1, g.ny - 1);
-    if (c0 > c1) return;
-    for (int r = r0; r <= r1; ++r) {
-        int s = __ldg(g.cell_start + r * g.nx + c0), e = __ldg(g.cell_start + r * g.nx + c1 + 1);
-        for (int k = s; k < e; ++k) {
-            double lx = __ldg(g.lx + k), ly = __ldg(g.ly + k);
-            double dd = dist_rn(lx - wx, ly - wy);
-            int id = __ldg(g.lidx + k);
-            if (dd < best || (dd == best && id < arg)) { best = dd; arg = id; lxb = lx; lyb = ly; }
-        }
-    }
-}

@@ -1,8 +1,9 @@
-// fastgrid.cuh -- the landmark grid of the fused sweep path.
+// fastgrid.cuh -- the landmark grid: the association (ICM_SLAM.py:169-172), Mapa.filtrar's
+// nearest-neighbour search (ICM_SLAM.py:241-245) and calc_cambio (ICM_SLAM.py:490-495).
 //
-// Same contract as the grid in common.cuh (every landmark within dist_thr of a query point is
-// visited, ties resolved exactly as cdist + np.argmin do, ICM_SLAM.py:169-172) with a layout made
-// for the hot loop:
+// Contract: every landmark within dist_thr of a query point is visited, and ties are resolved
+// exactly as cdist + np.argmin resolve them (the first minimum of the rooted distances).  Layout,
+// made for the hot loop of the fused sweep:
 //   * replicated binning: cell edge h >= 2*thr1 (thr1 = dist_thr*(1+2^-20)) and every landmark is
 //     registered in each of the (at most 2 x 2) cells its thr1-disc overlaps, so a query reads ONE
 //     cell -- the one containing the query point -- instead of a 3 x 3 block;

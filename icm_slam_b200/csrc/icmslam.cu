@@ -23,7 +23,6 @@
 #include "fcluster.h"
 #include "pass0.cuh"
 
-#define MAX_CELLS (1 << 22)
 #define ASSOC_MAX_OBS 4096      // observations of one scan icmslam_associate accepts (a scan has at most B <= 1024 beams)
 
 // ---- owners of the handle's CUDA resources: each is released by exactly one destructor ------------------------------------
@@ -60,6 +59,29 @@ struct Buf : Owner<T*, Release> {
 };
 template <typename T> using DevBuf = Buf<T, cudaFree>;
 template <typename T> using PinnedBuf = Buf<T, cudaFreeHost>;
+
+// A landmark grid (fastgrid.cuh): geometry, per-cell counts (all zero between builds: the fill pass counts them back down) and
+// starts, the cell-sorted entries and the bounding box.  A handle has two.  `grid` indexes the map of the fused sweep's chain
+// (Chain::grid_map) and only the fused sweep writes it; every other reader (the generic sweep's association, Mapa.filtrar,
+// calc_cambio) builds `scratch_grid`.  calc_cambio runs between two fused sweeps of icmslam_iterate_until: were it to rebuild
+// `grid`, the next sweep would find its grid stale, rebuild it and void every run record.
+struct LandmarkGrid {
+    DevBuf<FGeom> geom;
+    DevBuf<int> cnt, start, idx;
+    DevBuf<double2> pts;
+    DevBuf<unsigned long long> bb;
+    cudaError_t alloc(int cells, size_t entries)
+    {
+        cudaError_t e = geom.alloc(1);
+        if (e == cudaSuccess) e = cnt.alloc((size_t)cells + 2);
+        if (e == cudaSuccess) e = start.alloc((size_t)cells + 2);
+        if (e == cudaSuccess) e = idx.alloc(entries);
+        if (e == cudaSuccess) e = pts.alloc(entries);
+        if (e == cudaSuccess) e = bb.alloc(4);
+        if (e == cudaSuccess) e = cudaMemset(cnt, 0, ((size_t)cells + 2) * sizeof(int));
+        return e;
+    }
+};
 
 struct icmslam_handle {
     icmslam_config cfg;
@@ -111,9 +133,6 @@ struct icmslam_handle {
     DevBuf<double> d_kx, d_ky, d_kc, d_ox, d_oy, d_oc, d_acc;
     DevBuf<double> d_map_in /*2 x Lcap*/, d_map_out /*2 x Lcap*/;
     DevBuf<double> d_tmp_a, d_tmp_b; /* 2 x Lcap scratch for filter_map / calc_cambio inputs */
-    // grid
-    DevBuf<int> d_cell_start, d_cell_fill, d_cell_id, d_gidx;
-    DevBuf<double> d_glx, d_gly;
     // state
     DevBuf<DevState> d_st;
     PinnedBuf<DevState> h_st;   // pinned mirror
@@ -157,11 +176,8 @@ struct icmslam_handle {
     int use_runs = 1;            // ICMSLAM_RUNS=0: every tile goes through the association kernel every sweep (no steady-state shortcut)
     int assoc_blocks = 0;        // grid of the (persistent) association kernel
     long long *d_fsum_x = nullptr, *d_fsum_y = nullptr;
-    int fg_cells = 0;            // cell budget of the fast grid (host constant)
-    DevBuf<int> d_fg_cnt, d_fg_start, d_fg_idx;
-    DevBuf<double2> d_fg_pts;
-    DevBuf<FGeom> d_fg_geom;
-    DevBuf<unsigned long long> d_bb;
+    int fg_cells = 0;            // cell budget of the landmark grids (host constant)
+    LandmarkGrid grid, scratch_grid;
     int obs_cap = 0, max_tile_obs = 0;
     // host-memspace sweeps: copy of the map returned by the last one (a caller that feeds it back continues the device-side
     // map chain: grid, hints and labels stay valid, sensors.py:315 `mapa_viejo = mapa_refinado`)
@@ -390,19 +406,9 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
     if (e == cudaSuccess) e = h->d_map_out.alloc(2 * L);
     if (e == cudaSuccess) e = h->d_tmp_a.alloc(2 * L);
     if (e == cudaSuccess) e = h->d_tmp_b.alloc(2 * L);
-    if (e == cudaSuccess) e = h->d_cell_start.alloc((size_t)MAX_CELLS + 2);
-    if (e == cudaSuccess) e = h->d_cell_fill.alloc((size_t)MAX_CELLS + 2);
-    if (e == cudaSuccess) e = h->d_cell_id.alloc(L);
-    if (e == cudaSuccess) e = h->d_gidx.alloc(L);
-    if (e == cudaSuccess) e = h->d_glx.alloc(L);
-    if (e == cudaSuccess) e = h->d_gly.alloc(L);
     h->fg_cells = (int)(4 * L > 4096 ? 4 * L : 4096);
-    if (e == cudaSuccess) e = h->d_fg_cnt.alloc((size_t)h->fg_cells + 2);
-    if (e == cudaSuccess) e = h->d_fg_start.alloc((size_t)h->fg_cells + 2);
-    if (e == cudaSuccess) e = h->d_fg_idx.alloc(4 * L);    // replicated binning: <= 4 cells per landmark
-    if (e == cudaSuccess) e = h->d_fg_pts.alloc(4 * L);
-    if (e == cudaSuccess) e = h->d_fg_geom.alloc(1);
-    if (e == cudaSuccess) e = h->d_bb.alloc(4);
+    if (e == cudaSuccess) e = h->grid.alloc(h->fg_cells, 4 * L);    // replicated binning: <= 4 cells per landmark
+    if (e == cudaSuccess) e = h->scratch_grid.alloc(h->fg_cells, 4 * L);
     if (e == cudaSuccess) e = h->d_ts.alloc(1);
     if (e == cudaSuccess) e = h->d_seg_rec.alloc(SEG_REC);
     if (e == cudaSuccess) e = h->d_seg_rec_pose.alloc(SEG_REC);
@@ -442,7 +448,6 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
         h->assoc_blocks = 2 * (sms > 0 ? sms : 1);
     }
-    if (e == cudaSuccess) e = cudaMemset(h->d_fg_cnt, 0, ((size_t)h->fg_cells + 2) * sizeof(int));
     {   // gate and fixed-point scale of the fused path
         const double thr = cfg->dist_thr;
         double s2 = thr * thr;
@@ -530,8 +535,8 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
     CK(h->ds.d_blk_prefix.alloc((size_t)nblk(T + 1, RT_TILE) + 2));
     {   // scan workspace for the largest scan of a sweep, so that nothing allocates inside a graph capture
         size_t need = 0, b = 0;
-        const int lens[4] = {h->Lcap + 1, h->fg_cells + 2, T + 1, MAX_CELLS + 2};      // (the generic grid scans MAX_CELLS + 1 cells)
-        for (int k = 0; k < 4; ++k) { CK(cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, lens[k], h->stream)); if (b > need) need = b; }
+        const int lens[3] = {h->Lcap + 1, h->fg_cells + 2, T + 1};
+        for (int k = 0; k < 3; ++k) { CK(cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, lens[k], h->stream)); if (b > need) need = b; }
         int rcw = ensure_cub(h, need);
         if (rcw) return rcw;
     }
@@ -747,25 +752,24 @@ extern "C" int icmslam_set_counts(icmslam_handle* h, const double* in, int32_t n
     return ICMSLAM_OK;
 }
 
-// ---- grid over a point set whose size lives on the device --------------------------------------
-static int build_grid(icmslam_handle* h, const double* px, const double* py, const int* n_ptr, int n_cap, bool filter_grid)
+// landmark grid G (fastgrid.cuh) over the first *n_ptr points of (px, py): five kernels (the caller counts them).  G.cnt is all
+// zero on entry and on exit (the fill pass counts it back down), so no per-build memset is needed.
+static int build_fgrid(icmslam_handle* h, LandmarkGrid& G, const double* px, const double* py, const int* n_ptr, int n_cap)
 {
-    DevState* st = h->d_st;
-    double *gx0 = filter_grid ? &st->fx0 : &st->gx0, *gy0 = filter_grid ? &st->fy0 : &st->gy0;
-    double* ginv = filter_grid ? &st->finv_h : &st->ginv_h;
-    int *gnx = filter_grid ? &st->fnx : &st->gnx, *gny = filter_grid ? &st->fny : &st->gny;
-    CK(cudaMemsetAsync(h->d_cell_fill, 0, ((size_t)MAX_CELLS + 2) * sizeof(int), h->stream));
-    k_grid_setup<<<1, 1024, 0, h->stream>>>(px, py, n_ptr, h->dcfg.dist_thr, MAX_CELLS, gx0, gy0, ginv, gnx, gny,
-                                            filter_grid ? &st->f_extent : nullptr);
+    cudaStream_t s = h->stream;
+    k_fgrid_bbox_reset<<<1, 1, 0, s>>>(G.bb);
     CK(cudaGetLastError());
-    // counts go to cell_fill, scanned into cell_start, then cell_fill is reused as the fill cursor
-    k_cell_count<<<nblk(n_cap, 256), 256, 0, h->stream>>>(px, py, n_ptr, gx0, gy0, ginv, gnx, gny, h->d_cell_fill, h->d_cell_id);
+    int nb = nblk(n_cap, 256);
+    if (nb > 148 * 2) nb = 148 * 2;
+    k_fgrid_bbox<<<nb, 256, 0, s>>>(px, py, n_ptr, G.bb);
     CK(cudaGetLastError());
-    int rc = exclusive_sum(h, h->d_cell_fill, h->d_cell_start, MAX_CELLS + 1);
+    k_fgrid_geom<<<1, 1, 0, s>>>(G.bb, n_ptr, h->dcfg.dist_thr, h->fg_cells, G.geom);
+    CK(cudaGetLastError());
+    k_fgrid_count<<<nblk(n_cap, 256), 256, 0, s>>>(px, py, n_ptr, G.geom, G.cnt);
+    CK(cudaGetLastError());
+    int rc = exclusive_sum(h, G.cnt, G.start, h->fg_cells + 1);
     if (rc) return rc;
-    CK(cudaMemsetAsync(h->d_cell_fill, 0, ((size_t)MAX_CELLS + 2) * sizeof(int), h->stream));
-    k_cell_fill<<<nblk(n_cap, 256), 256, 0, h->stream>>>(px, py, n_ptr, h->d_cell_id, h->d_cell_start, h->d_cell_fill, h->d_glx,
-                                                         h->d_gly, h->d_gidx);
+    k_fgrid_fill<<<nblk(n_cap, 256), 256, 0, s>>>(px, py, n_ptr, G.geom, G.start, G.cnt, G.pts, G.idx);
     CK(cudaGetLastError());
     return ICMSLAM_OK;
 }
@@ -782,13 +786,14 @@ static int run_filter(icmslam_handle* h, const double* raw_x, const double* raw_
     k_compact_kept<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_kflag, h->d_kpos, raw_x, raw_y, cnt_i, cnt_d, h->d_kx, h->d_ky,
                                                         h->d_kc, h->d_parent, L);
     CK(cudaGetLastError());
-    rc = build_grid(h, h->d_kx, h->d_ky, &st->kept, L, true);
+    LandmarkGrid& G = h->scratch_grid;
+    rc = build_fgrid(h, G, h->d_kx, h->d_ky, &st->kept, L);
     if (rc) return rc;
     CK(cudaMemsetAsync(h->d_acc, 0, 8 * sizeof(double), h->stream));
-    k_filter_diameter<<<nblk(FILTER_SMALL_K, 128), 128, 0, h->stream>>>(st, h->d_kx, h->d_ky, h->dcfg.dist_thr, h->d_acc);
+    k_filter_diameter<<<nblk(FILTER_SMALL_K, 128), 128, 0, h->stream>>>(st, h->d_kx, h->d_ky, G.bb, h->dcfg.dist_thr, h->d_acc);
     CK(cudaGetLastError());
-    k_filter_nn<<<nblk(L, 128), 128, 0, h->stream>>>(st, h->d_kx, h->d_ky, h->dcfg.dist_thr, h->d_acc, h->d_cell_start, h->d_glx,
-                                                     h->d_gly, h->d_gidx, h->d_nn, h->d_indflag, L);
+    k_filter_nn<<<nblk(L, 128), 128, 0, h->stream>>>(st, h->d_kx, h->d_ky, h->dcfg.dist_thr, h->d_acc, G.bb, G.geom, G.start, G.pts,
+                                                     G.idx, h->d_nn, h->d_indflag, L);
     CK(cudaGetLastError());
     rc = exclusive_sum(h, h->d_indflag, h->d_indpos, L);
     if (rc) return rc;
@@ -838,29 +843,6 @@ static void default_opts(icmslam_sweep_opts& o, const icmslam_sweep_opts* opts)
     if (opts) o = *opts;
     if (o.newton_maxit <= 0) o.newton_maxit = 20;
     if (!(o.newton_tol > 0.0)) o.newton_tol = 1e-7;    // Newton is quadratic: the step after |dtheta| <= 1e-7 is ~1e-14
-}
-
-// fast grid (fastgrid.cuh) over the first *n_ptr points of (px, py).  cell_cnt is all zero on entry and
-// on exit (the fill pass counts it back down), so no per-build memset is needed.
-static int build_fgrid(icmslam_handle* h, const double* px, const double* py, const int* n_ptr, int n_cap)
-{
-    cudaStream_t s = h->stream;
-    k_fgrid_bbox_reset<<<1, 1, 0, s>>>(h->d_bb);
-    CK(cudaGetLastError());
-    int nb = nblk(n_cap, 256);
-    if (nb > 148 * 2) nb = 148 * 2;
-    k_fgrid_bbox<<<nb, 256, 0, s>>>(px, py, n_ptr, h->d_bb);
-    CK(cudaGetLastError());
-    k_fgrid_geom<<<1, 1, 0, s>>>(h->d_bb, n_ptr, h->dcfg.dist_thr, h->fg_cells, h->d_fg_geom);
-    CK(cudaGetLastError());
-    k_fgrid_count<<<nblk(n_cap, 256), 256, 0, s>>>(px, py, n_ptr, h->d_fg_geom, h->d_fg_cnt);
-    CK(cudaGetLastError());
-    int rc = exclusive_sum(h, h->d_fg_cnt, h->d_fg_start, h->fg_cells + 1);
-    if (rc) return rc;
-    k_fgrid_fill<<<nblk(n_cap, 256), 256, 0, s>>>(px, py, n_ptr, h->d_fg_geom, h->d_fg_start, h->d_fg_cnt, h->d_fg_pts, h->d_fg_idx);
-    CK(cudaGetLastError());
-    h->n_launch += 5;
-    return ICMSLAM_OK;
 }
 
 // (a map from outside: run records are void, and so is what the steady tail remembers of the grid the previous chain built)
@@ -930,14 +912,14 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     const double* min_y = h->d_map_in + L;
     const bool timing = (o.reserved & 2) != 0;
     if (h->ch.grid_map != h->d_map_in) {      // the grid of the previous sweep's tail does not index this map: build it
-        int rc = build_fgrid(h, min_x, min_y, &st->lsearch, n_search_cap);
+        int rc = build_fgrid(h, h->grid, min_x, min_y, &st->lsearch, n_search_cap);
         if (rc) return rc;
-        k_lmrec_build<<<nblk(n_search_cap, 256), 256, 0, s>>>(min_x, min_y, &st->lsearch, h->d_fg_geom, h->d_fg_start, h->d_fg_pts, h->d_fg_idx,
+        k_lmrec_build<<<nblk(n_search_cap, 256), 256, 0, s>>>(min_x, min_y, &st->lsearch, h->grid.geom, h->grid.start, h->grid.pts, h->grid.idx,
                                                               h->thr1sq, h->thr2_hi, h->d_lmrec2[h->ch.lm_cur]);
         CK(cudaGetLastError());
         k_epoch_bump<<<1, 1, 0, s>>>(h->d_ts);      // a map from outside: its labels are a new numbering, run records are void
         CK(cudaGetLastError());
-        h->n_launch += 2;
+        h->n_launch += 7;      // the grid (5), k_lmrec_build, k_epoch_bump
         h->ch.hint_map = nullptr;
     }
     double4* pp_in = ppar_for(h, xin);
@@ -953,15 +935,15 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
     R.fsum_x = h->d_fsum_x; R.fsum_y = h->d_fsum_y; R.cnt = h->d_cnt; R.fix_scale = h->fix_scale; R.tile_slots = h->ex.d_tile_slots; R.tile_nslots = h->ex.d_tile_nslots;
     R.far_list = h->ds.d_far_list; R.ts = h->d_ts; R.farbits = h->ex.d_farbits;
     R.scan_dirty = h->ex.d_scan_dirty; R.tile_flag = h->ex.d_tile_flag; R.dirty_list = h->ex.d_dirty_list;
-    R.geom = h->d_fg_geom; R.cell_start = h->d_fg_start; R.gpts = h->d_fg_pts; R.dist_thr = h->dcfg.dist_thr;
+    R.geom = h->grid.geom; R.cell_start = h->grid.start; R.gpts = h->grid.pts; R.dist_thr = h->dcfg.dist_thr;
     R.st = st; R.L_in = h->begin_L; R.slice0 = 0; R.fz = h->fz;
     AssocParams A;
-    A.first_halo = h->seg_first ? 0 : 1; A.T = T; A.off = h->ex.d_off; A.bxy = h->ex.d_bxy; A.cfg = h->dcfg; A.thr2_hi = h->thr2_hi; A.st = st; A.geom = h->d_fg_geom;
-    A.cell_start = h->d_fg_start; A.gpts = h->d_fg_pts; A.gidx = h->d_fg_idx; A.remap = h->d_remap;
+    A.first_halo = h->seg_first ? 0 : 1; A.T = T; A.off = h->ex.d_off; A.bxy = h->ex.d_bxy; A.cfg = h->dcfg; A.thr2_hi = h->thr2_hi; A.st = st; A.geom = h->grid.geom;
+    A.cell_start = h->grid.start; A.gpts = h->grid.pts; A.gidx = h->grid.idx; A.remap = h->d_remap;
     { const char* eh = getenv("ICMSLAM_HINTS"); A.skip_hints = (eh && atoi(eh) == 0) ? 1 : 0; }
     A.hints = (h->ch.hint_map == h->d_map_in) ? 1 : 0;
     A.c = h->ex.d_c; A.obs_cap = h->obs_cap; A.R = R;
-    A.n_tiles = h->n_tiles; A.blk_prefix = h->ds.d_blk_prefix; A.Lcap = L; A.bb = h->d_bb; A.stw = st; A.final = 1; A.p2p = h->p2p;
+    A.n_tiles = h->n_tiles; A.blk_prefix = h->ds.d_blk_prefix; A.Lcap = L; A.bb = h->grid.bb; A.stw = st; A.final = 1; A.p2p = h->p2p;
     const int nb = h->assoc_blocks < h->n_tiles ? h->assoc_blocks : h->n_tiles;      // grid of the association kernel
     SolveParams P;
     P.T = T; P.t_lo = h->seg_lo; P.t_hi = h->seg_hi; P.lay = traj_layout(h, x0);
@@ -1102,7 +1084,7 @@ static int fused_part_c(icmslam_handle* h, const double* xout, double* dmap_out,
         a.fsum_x = h->d_fsum_x; a.fsum_y = h->d_fsum_y; a.cnt = h->d_cnt; a.map_x = min_x; a.map_y = min_y;
         a.inv_scale = 1.0 / h->fix_scale; a.cota = h->dcfg.cota; a.dist_thr = h->dcfg.dist_thr; a.thr1sq = h->thr1sq; a.thr2_hi = h->thr2_hi;
         a.lmrec_old = h->d_lmrec2[h->ch.lm_cur]; a.lmrec_new = h->d_lmrec2[h->ch.lm_cur ^ 1];
-        a.gbuild = h->d_gbuild; a.nnd0 = h->d_nnd0; a.gslots = h->d_gslots; a.gpts = h->d_fg_pts;
+        a.gbuild = h->d_gbuild; a.nnd0 = h->d_nnd0; a.gslots = h->d_gslots; a.gpts = h->grid.pts;
         a.raw_x = raw_x; a.raw_y = raw_y; a.rawcnt = h->d_rawcnt;
         a.map_out = dmap_out; a.cap_out = out_cap; a.ld_out = out_ld; a.counts_state = h->d_counts; a.remap = h->d_remap; a.Lcap = L;
         a.cpart = h->d_cpart; a.fz = h->fz;
@@ -1169,22 +1151,22 @@ static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t 
                                                h->d_cnt, st, h->d_sh_x, h->d_sh_y, h->d_sh_k, h->fz, h->d_counts);
     CK(cudaGetLastError());
     k_tail_compact<<<nblk(L, 256), 256, 0, s>>>(st, h->d_kflag, h->d_blk_kept, h->d_kpos, raw_x, raw_y, h->d_cnt, h->d_kx, h->d_ky, h->d_kc,
-                                                h->d_parent, h->d_bb, L, h->d_klab, h->d_rawcnt, ts);
+                                                h->d_parent, h->grid.bb, L, h->d_klab, h->d_rawcnt, ts);
     CK(cudaGetLastError());
-    k_tail_count<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, st, ts, h->d_bb, h->dcfg.dist_thr, h->fg_cells, h->d_fg_geom, h->d_fg_cnt);
+    k_tail_count<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, st, ts, h->grid.bb, h->dcfg.dist_thr, h->fg_cells, h->grid.geom, h->grid.cnt);
     CK(cudaGetLastError());
-    k_cell_scan<<<nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS), CS_THREADS, 0, s>>>(h->d_fg_cnt, h->d_fg_start, h->fg_cells + 1, h->d_scan_state, ts);
+    k_cell_scan<<<nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS), CS_THREADS, 0, s>>>(h->grid.cnt, h->grid.start, h->fg_cells + 1, h->d_scan_state, ts);
     CK(cudaGetLastError());
-    k_fgrid_fill<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, &st->kept, h->d_fg_geom, h->d_fg_start, h->d_fg_cnt, h->d_fg_pts,
-                                              h->d_fg_idx, h->d_gslots, &ts->steady_ok);
+    k_fgrid_fill<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, &st->kept, h->grid.geom, h->grid.start, h->grid.cnt, h->grid.pts,
+                                              h->grid.idx, h->d_gslots, &ts->steady_ok);
     CK(cudaGetLastError());
     {
         SlowArgs sa;
         sa.dist_thr = h->dcfg.dist_thr; sa.parent = h->d_parent; sa.ind_pos = h->d_indpos; sa.ind = h->d_ind; sa.lab = h->d_lab; sa.used = h->d_used;
-        sa.rank = h->d_rank; sa.ox = h->d_ox; sa.oy = h->d_oy; sa.oc = h->d_oc; sa.max_cells = h->fg_cells; sa.geom = h->d_fg_geom;
-        sa.cell_cnt = h->d_fg_cnt; sa.cell_start = h->d_fg_start; sa.pts = h->d_fg_pts; sa.gidx = h->d_fg_idx;
+        sa.rank = h->d_rank; sa.ox = h->d_ox; sa.oy = h->d_oy; sa.oc = h->d_oc; sa.max_cells = h->fg_cells; sa.geom = h->grid.geom;
+        sa.cell_cnt = h->grid.cnt; sa.cell_start = h->grid.start; sa.pts = h->grid.pts; sa.gidx = h->grid.idx;
         sa.gbuild = h->d_gbuild; sa.nnd0 = h->d_nnd0; sa.steady_enable = h->steady_enable; sa.fz = h->fz;
-        k_tail_nn<<<nblk(L, 256), 256, 0, s>>>(st, ts, h->d_kx, h->d_ky, h->d_kc, h->d_fg_geom, h->d_fg_start, h->d_fg_pts, h->d_fg_idx, h->thr2_lt,
+        k_tail_nn<<<nblk(L, 256), 256, 0, s>>>(st, ts, h->d_kx, h->d_ky, h->d_kc, h->grid.geom, h->grid.start, h->grid.pts, h->grid.idx, h->thr2_lt,
                                                h->d_nn, h->d_indflag, L, h->d_klab, h->d_kflag, h->d_kpos, h->d_lmrec2[h->ch.lm_cur],
                                                h->d_lmrec2[h->ch.lm_cur ^ 1], dmap_out, out_cap, out_ld, h->d_counts, h->thr1sq, h->thr2_hi, h->d_remap, sa);
         CK(cudaGetLastError());
@@ -1277,16 +1259,17 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         const int64_t ldx = ldout;
         CK(cudaMemsetAsync(h->d_sum_x, 0, (size_t)L * 8, s));
         CK(cudaMemsetAsync(h->d_sum_y, 0, (size_t)L * 8, s));
-        rc = build_grid(h, min_x, min_y, &st->lsearch, n_search_cap, false);
+        LandmarkGrid& G = h->scratch_grid;
+        rc = build_fgrid(h, G, min_x, min_y, &st->lsearch, n_search_cap);
         if (rc) return rc;
-        h->n_launch += 3;
+        h->n_launch += 5;
         PoseArrays A;
         A.x = dx; A.ldx = ldx; A.odo = h->ds.d_odo; A.ldo = T; A.u = h->ds.d_u; A.ldu = T;
         A.x0[0] = x0[0]; A.x0[1] = x0[1]; A.x0[2] = x0[2];
         A.off = h->ex.d_off; A.T = T;
         if (timing) CK(cudaEventRecord(h->ev[0], s));
-        k_assoc<<<148 * 8, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, x0[0], x0[1], x0[2], st, h->d_cell_start, h->d_glx,
-                                        h->d_gly, h->d_gidx, h->dcfg.dist_thr, h->ex.d_c, h->ds.d_nfar, h->d_sum_x, h->d_sum_y, h->d_cnt);
+        k_assoc<<<148 * 8, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, x0[0], x0[1], x0[2], G.geom, G.start, G.pts, G.idx,
+                                        h->thr2_hi, h->ex.d_c, h->ds.d_nfar, h->d_sum_x, h->d_sum_y, h->d_cnt);
         CK(cudaGetLastError());
         h->n_launch += 1;
         if (timing) CK(cudaEventRecord(h->ev[1], s));
@@ -1358,7 +1341,7 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
     // Mapa.filtrar (sensors.py:165-166)
     rc = run_filter(h, raw_x, raw_y, h->d_cnt, nullptr, dmap_out, out_cap, out_ld, nullptr, 1);
     if (rc) return rc;
-    h->n_launch += 11;   // filter grid build (3) + filter kernels (8)
+    h->n_launch += 13;   // filter grid build (5) + filter kernels (8)
     h->ch.lact_dirty = true;
     return ICMSLAM_OK;
 }
@@ -2078,12 +2061,13 @@ extern "C" int icmslam_calc_cambio(icmslam_handle* h, const double* map_new, int
     CK(cudaMemcpy2DAsync(h->d_tmp_b, (size_t)L * 8, map_old, (size_t)ld_old * 8, (size_t)L_old * 8, 2, cudaMemcpyDefault, s));
     k_set_lsearch<<<1, 1, 0, s>>>(h->d_st, L_old);
     CK(cudaGetLastError());
-    int rc = build_grid(h, h->d_tmp_b, h->d_tmp_b + L, &h->d_st->lsearch, L_old, false);
+    LandmarkGrid& G = h->scratch_grid;
+    int rc = build_fgrid(h, G, h->d_tmp_b, h->d_tmp_b + L, &h->d_st->lsearch, L_old);
     if (rc) return rc;
     double init[3] = {INFINITY, 0.0, 0.0};
     CK(cudaMemcpyAsync(h->d_acc, init, sizeof init, cudaMemcpyHostToDevice, s));
-    k_cambio<<<nblk(L_new, 128), 128, 0, s>>>(h->d_st, h->d_tmp_a, h->d_tmp_a + L, L_new, h->d_tmp_b, h->d_tmp_b + L, L_old,
-                                              h->d_cell_start, h->d_glx, h->d_gly, h->d_gidx, h->d_acc);
+    k_cambio<<<nblk(L_new, 128), 128, 0, s>>>(h->d_tmp_a, h->d_tmp_a + L, L_new, h->d_tmp_b, h->d_tmp_b + L, L_old, G.geom, G.start, G.pts,
+                                              h->dcfg.dist_thr, h->d_acc);
     CK(cudaGetLastError());
     double res[3];
     CK(cudaMemcpyAsync(res, h->d_acc, sizeof res, cudaMemcpyDeviceToHost, s));

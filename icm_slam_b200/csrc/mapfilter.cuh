@@ -5,13 +5,15 @@
 // that neighbour is renamed to the survivor's class (c[c==c[b[i]]] = c[i]); (3) classes are
 // renumbered densely in ascending order; (4) each class becomes the count-weighted mean of its
 // members.  The reference builds the full K x K distance matrix (O(K^2) memory, impossible at
-// 1e5 landmarks); here the neighbour search uses the uniform grid, and step (2) -- inherently
-// sequential but touching only the few landmarks that do have a close neighbour -- is a directed
-// union-find walked by one thread.  A brute-force path keeps the reference's exact corner cases
-// (zero distances replaced by the map diameter, :242) for small or degenerate maps.
+// 1e5 landmarks); here the neighbour search scans the survivor's own cell of the landmark grid
+// (fastgrid.cuh), and step (2) -- inherently sequential but touching only the few landmarks that
+// do have a close neighbour -- is a directed union-find walked by one thread.  A brute-force path
+// keeps the reference's exact corner cases (zero distances replaced by the map diameter, :242) for
+// small or degenerate maps.
 #pragma once
 #include "common.cuh"
 #include "assoc.cuh"
+#include "fastgrid.cuh"
 
 #define FILTER_SMALL_K 2048
 
@@ -68,16 +70,19 @@ __device__ __forceinline__ void atomic_min_pos(double* addr, double v)   // v >=
     atomicMin((unsigned long long*)addr, (unsigned long long)__double_as_longlong(v));
 }
 
-__device__ __forceinline__ bool filter_small_path(const DevState* st, double dist_thr)
+// bb: bounding box of the survivors (the filter grid's, fastgrid.cuh k_fgrid_bbox)
+__device__ __forceinline__ bool filter_small_path(const DevState* st, const unsigned long long* bb, double dist_thr)
 {
-    return st->kept <= FILTER_SMALL_K || !(st->f_extent >= dist_thr);
+    if (st->kept <= FILTER_SMALL_K) return true;
+    const double extent = fmax(dkey_inv(bb[2]) - dkey_inv(bb[0]), dkey_inv(bb[3]) - dkey_inv(bb[1]));
+    return !(extent >= dist_thr);
 }
 
 // brute-force path, step A: the map diameter amax (:242)
 __global__ void k_filter_diameter(const DevState* st, const double* __restrict__ kx, const double* __restrict__ ky,
-                                  double dist_thr, double* __restrict__ amax)
+                                  const unsigned long long* __restrict__ bb, double dist_thr, double* __restrict__ amax)
 {
-    if (!filter_small_path(st, dist_thr)) return;
+    if (!filter_small_path(st, bb, dist_thr)) return;
     const int K = st->kept;
     double m = 0.0;
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < K; j += gridDim.x * blockDim.x)
@@ -88,9 +93,9 @@ __global__ void k_filter_diameter(const DevState* st, const double* __restrict__
 
 // nearest other survivor: amin / b (:243-245), flag = amin < dist_thr
 __global__ void k_filter_nn(const DevState* st, const double* __restrict__ kx, const double* __restrict__ ky,
-                            double dist_thr, const double* __restrict__ amax_p, const int* __restrict__ cell_start,
-                            const double* __restrict__ glx, const double* __restrict__ gly, const int* __restrict__ gidx,
-                            int* __restrict__ nn, int* __restrict__ ind_flag, int Lcap)
+                            double dist_thr, const double* __restrict__ amax_p, const unsigned long long* __restrict__ bb,
+                            const FGeom* __restrict__ geom, const int* __restrict__ cell_start, const double2* __restrict__ pts,
+                            const int* __restrict__ gidx, int* __restrict__ nn, int* __restrict__ ind_flag, int Lcap)
 {
     int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= Lcap) return;
@@ -99,7 +104,7 @@ __global__ void k_filter_nn(const DevState* st, const double* __restrict__ kx, c
     const double xj = kx[j], yj = ky[j];
     double best = INFINITY;
     int arg = 0;
-    if (filter_small_path(st, dist_thr)) {
+    if (filter_small_path(st, bb, dist_thr)) {
         const double amax = *amax_p;
         for (int i = 0; i < K; ++i) {
             double dd = (i == j) ? 0.0 : dist_rn(kx[i] - xj, ky[i] - yj);
@@ -107,18 +112,16 @@ __global__ void k_filter_nn(const DevState* st, const double* __restrict__ kx, c
             if (dd < best) { best = dd; arg = i; }             // argmin: first minimum
         }
     } else {
-        // diameter >= dist_thr here, so zero distances (replaced by it) can never pass the gate
-        Grid g = load_grid(&st->fx0, &st->fy0, &st->finv_h, &st->fnx, &st->fny, cell_start, glx, gly, gidx, K);
-        int cx = grid_coord(xj, g.x0, g.inv_h), cy = grid_coord(yj, g.y0, g.inv_h);
-        int c0 = max(cx - 1, 0), c1 = min(cx + 1, g.nx - 1), r0 = max(cy - 1, 0), r1 = min(cy + 1, g.ny - 1);
-        for (int r = r0; r <= r1; ++r) {
-            int s = cell_start[r * g.nx + c0], e = cell_start[r * g.nx + c1 + 1];
-            for (int k = s; k < e; ++k) {
-                int id = gidx[k];
-                double dd = dist_rn(glx[k] - xj, gly[k] - yj);
-                if (dd == 0.0) continue;
-                if (dd < best || (dd == best && id < arg)) { best = dd; arg = id; }
-            }
+        // diameter >= dist_thr here, so zero distances (replaced by it) can never pass the gate; the survivor's own cell holds
+        // every survivor within dist_thr of it
+        const FGeom g = *geom;
+        const int c = fgrid_cell(g, xj, yj);
+        for (int k = cell_start[c]; k < cell_start[c + 1]; ++k) {
+            const double2 p = pts[k];
+            const int id = gidx[k];
+            const double dd = dist_rn(p.x - xj, p.y - yj);
+            if (dd == 0.0) continue;
+            if (dd < best || (dd == best && id < arg)) { best = dd; arg = id; }
         }
     }
     nn[j] = arg;
@@ -201,21 +204,28 @@ __global__ void k_filter_finalize(DevState* st, const int* __restrict__ used, co
 }
 
 // ---- calc_cambio ---------------------------------------------------------------------------
-// thread per NEW landmark: nearest OLD landmark (grid first, full scan if nothing is in reach).
-__global__ void k_cambio(DevState* st, const double* __restrict__ nx_, const double* __restrict__ ny_, int Ln,
-                         const double* __restrict__ oldx, const double* __restrict__ oldy, int Lo,
-                         const int* __restrict__ cell_start, const double* __restrict__ glx, const double* __restrict__ gly,
-                         const int* __restrict__ gidx, double* __restrict__ acc /* min,max,sum */)
+// thread per NEW landmark: distance to the nearest OLD landmark.  The new landmark's cell of the grid over the old map holds every
+// old landmark within dist_thr (1 + FG_MARGIN) of it (fastgrid.cuh: landmarks are registered with that radius plus a 2^-20 slack
+// for the rounding of the cell arithmetic), so the nearest candidate within that reach is the nearest old landmark; otherwise,
+// or with no candidate, a full scan.  The minimum of the rooted distances is the root of the minimum squared one (sqrt_rn is
+// monotone), so the result does not depend on the path.
+__global__ void k_cambio(const double* __restrict__ nx_, const double* __restrict__ ny_, int Ln, const double* __restrict__ oldx,
+                         const double* __restrict__ oldy, int Lo, const FGeom* __restrict__ geom, const int* __restrict__ cell_start,
+                         const double2* __restrict__ pts, double dist_thr, double* __restrict__ acc /* min,max,sum */)
 {
     int j = blockIdx.x * blockDim.x + threadIdx.x;
     double best = INFINITY;
     if (j < Ln) {
         const double xj = nx_[j], yj = ny_[j];
-        Grid g = load_grid(&st->gx0, &st->gy0, &st->ginv_h, &st->gnx, &st->gny, cell_start, glx, gly, gidx, Lo);
-        int arg; double lxb, lyb;
-        grid_nearest(g, xj, yj, best, arg, lxb, lyb);
-        // the 3x3 block only guarantees completeness within one cell edge
-        if (!(best * g.inv_h <= 1.0)) {
+        const FGeom g = *geom;
+        const int c = fgrid_cell(g, xj, yj);
+        double s2 = INFINITY;
+        for (int k = cell_start[c]; k < cell_start[c + 1]; ++k) {
+            const double2 p = pts[k];
+            s2 = fmin(s2, dist2_rn(p.x - xj, p.y - yj));
+        }
+        best = __dsqrt_rn(s2);
+        if (!(best <= dist_thr + FG_MARGIN * dist_thr)) {
             best = INFINITY;
             for (int i = 0; i < Lo; ++i) best = fmin(best, dist_rn(oldx[i] - xj, oldy[i] - yj));
         }
