@@ -8,11 +8,20 @@ sweeps of a rank's handles are enqueued back to back on their own streams, so sm
     for i in batch.owned(n_traj):
         batch.add(i, z_i, odo_i, u_i, map_i, x_i)
     batch.finalize()                                  # (ConcatBatch only)
-    batch.iterate(30)                                 # a fixed number of sweeps of every trajectory, or
+    batch.iterate(30)                                 # a fixed number of sweeps of every trajectory (any sweep mode, below), or
     conv = batch.iterate_until(60, tol)               # each trajectory until its own largest landmark change is <= tol (the
                                                       # reference's stop rule, sensors.py:302-315): {i: (n_done, cambios (n_done, 3))}
     res = batch.results()          # {i: (x (3 x T), mapa (2 x L))}
     allres = gather_results(res)   # optional, for output only (torch.distributed all_gather_object)
+
+iterate takes the sweep mode of Engine.iterate: schedule ("redblack" | "sequential"), solver ("newton" | "nm"), view ("prev" |
+"full" | "running"); the default is the fast restated sweep (redblack, newton, prev).  Every mode sweeps each trajectory exactly
+as it would be swept alone, so the reference's own sweep runs a whole batch in one handle:
+
+    batch.iterate(30, schedule="sequential", solver="nm", view="running")      # the reference's ICM, one warp per trajectory
+
+A ConcatBatch numbers new labels over the whole batch (each trajectory's labels keep their order) and its label cap applies to the
+batch; iterate_until runs the default mode only.
 """
 from __future__ import annotations
 
@@ -146,6 +155,8 @@ class ConcatBatch:
         return e.n
 
     def iterate(self, n_sweeps: int = 1, **mode):
+        """n_sweeps sweeps of every trajectory in the sweep mode of Engine.iterate (schedule, solver, view, ...), each trajectory
+        exactly as alone; e.g. iterate(n, schedule="sequential", solver="nm", view="running") for the reference's own ICM."""
         self.engine.iterate(None, self.x0s[:, 0], int(n_sweeps), **mode)
 
     def iterate_until(self, max_sweeps: int, tol: float):

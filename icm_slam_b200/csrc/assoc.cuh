@@ -25,12 +25,12 @@ struct DevState {
 
 // ---- association ---------------------------------------------------------------------------
 // One warp per scan, lanes over the scan's kept observations.  Projects with the sweep's INPUT
-// pose (sensors.py:141,153), finds the nearest of the first `lsearch` previous-map landmarks
+// pose (sensors.py:141,153; each trajectory's first scan with its own x0, TrajLayout), finds the nearest of the first `lsearch` previous-map landmarks
 // (cdist + argmin, ICM_SLAM.py:169-171), gates at dist_thr (strict >, :172).  Matched
 // observations add into the per-label sums; far ones are marked -1 and counted per scan.
 __global__ void __launch_bounds__(256)
 k_assoc(int T, const int* __restrict__ off, const double* __restrict__ bx, const double* __restrict__ by,
-        const double* __restrict__ x, int64_t ldx, double x0x, double x0y, double x0t, const FGeom* __restrict__ geom,
+        const double* __restrict__ x, int64_t ldx, const TrajLayout lay, const FGeom* __restrict__ geom,
         const int* __restrict__ cell_start, const double2* __restrict__ pts, const int* __restrict__ gidx, double thr2_hi,
         int* __restrict__ c, int* __restrict__ nfar, double* __restrict__ sum_x, double* __restrict__ sum_y, int* __restrict__ cnt)
 {
@@ -43,8 +43,7 @@ k_assoc(int T, const int* __restrict__ off, const double* __restrict__ bx, const
         int far = 0;
         if (e > o) {
             double px, py, th;
-            if (t == 0) { px = x0x; py = x0y; th = x0t; }
-            else { px = x[t]; py = x[ldx + t]; th = x[2 * ldx + t]; }
+            lay.scan_pose(x, ldx, t, px, py, th);
             Rot r = make_rot(th);
             for (int i = o + lane; i < e; i += WARP) {
                 double wx, wy, best;
@@ -77,7 +76,7 @@ __global__ void k_flag_positive(const int* __restrict__ v, int n, int* __restric
 // scan that has far observations: rewrite c, and own the new label's statistics (no atomics).
 __global__ void __launch_bounds__(256)
 k_new_labels(int T, const int* __restrict__ off, const double* __restrict__ bx, const double* __restrict__ by,
-             const double* __restrict__ x, int64_t ldx, double x0x, double x0y, double x0t, DevState* st,
+             const double* __restrict__ x, int64_t ldx, const TrajLayout lay, DevState* st,
              const int* __restrict__ nfar, const int* __restrict__ far_prefix, int Lcap, int* __restrict__ c,
              double* __restrict__ sum_x, double* __restrict__ sum_y, int* __restrict__ cnt)
 {
@@ -96,8 +95,7 @@ k_new_labels(int T, const int* __restrict__ off, const double* __restrict__ bx, 
         if (label >= Lcap) continue;
         int o = off[t], e = off[t + 1];
         double px, py, th;
-        if (t == 0) { px = x0x; py = x0y; th = x0t; }
-        else { px = x[t]; py = x[ldx + t]; th = x[2 * ldx + t]; }
+        lay.scan_pose(x, ldx, t, px, py, th);
         Rot r = make_rot(th);
         double sx = 0.0, sy = 0.0;
         for (int i0 = o; i0 < e; i0 += WARP) {       // sequential-in-lane-order sum of the far points
@@ -141,7 +139,7 @@ __global__ void k_means(const DevState* st, const double* __restrict__ sum_x, co
 __global__ void k_running_mean(const DevState* st, const int* __restrict__ seg_start, const int* __restrict__ cnt,
                                const int* __restrict__ sorted_obs, const int* __restrict__ scan_of,
                                const double* __restrict__ bx, const double* __restrict__ by, const double* __restrict__ x,
-                               int64_t ldx, double x0x, double x0y, double x0t, double* __restrict__ seen_x,
+                               int64_t ldx, const TrajLayout lay, double* __restrict__ seen_x,
                                double* __restrict__ seen_y, double* __restrict__ raw_x, double* __restrict__ raw_y, int Lcap)
 {
     int l = blockIdx.x * blockDim.x + threadIdx.x;
@@ -153,8 +151,7 @@ __global__ void k_running_mean(const DevState* st, const int* __restrict__ seg_s
     while (j < e) {
         int t = scan_of[sorted_obs[j]];
         double px, py, th;
-        if (t == 0) { px = x0x; py = x0y; th = x0t; }
-        else { px = x[t]; py = x[ldx + t]; th = x[2 * ldx + t]; }
+        lay.scan_pose(x, ldx, t, px, py, th);
         Rot r = make_rot(th);
         double sx = 0.0, sy = 0.0;
         int k = 0, j2 = j;

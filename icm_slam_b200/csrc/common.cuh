@@ -50,6 +50,28 @@ struct Freeze {
     }
 };
 
+// Which columns are pinned first poses (sensors.py:131: x[:,0] is never updated, scan 0 is projected with self.x0): column 0
+// of the trajectory's first segment, or -- a batch of independent trajectories of traj_T columns each laid end to end in one
+// handle (BASELINE configs[4]) -- the first column of every trajectory, each with its own x0.  A trajectory's last pose has no
+// successor.  The fused solve and the generic kernels both go by these rules.
+struct TrajLayout {
+    int first;                 // column 0 is the trajectory's first pose
+    int traj_T;                // > 0: batch of trajectories of this many columns
+    const double* x0s;         // batch: 3 x K first poses (row-major, leading dimension ldx0s)
+    int64_t ldx0s;
+    double x0[3];              // single trajectory: self.x0
+    __device__ __forceinline__ bool pinned(int t) const { return traj_T > 0 ? (t % traj_T) == 0 : (t == 0 && first); }
+    __device__ __forceinline__ bool after_pinned(int t) const { return traj_T > 0 ? (t % traj_T) == 1 : (t == 1 && first); }
+    __device__ __forceinline__ bool has_next(int t, int T) const { return t + 1 < T && (traj_T == 0 || ((t + 1) % traj_T) != 0); }
+    __device__ __forceinline__ double x0_of(int t, int r) const { return traj_T > 0 ? x0s[r * ldx0s + t / traj_T] : x0[r]; }
+    // the pose scan t is projected with (sensors.py:141,153): its trajectory's x0 for a pinned column, else x[:, t]
+    __device__ __forceinline__ void scan_pose(const double* x, int64_t ldx, int t, double& px, double& py, double& th) const
+    {
+        if (pinned(t)) { px = x0_of(t, 0); py = x0_of(t, 1); th = x0_of(t, 2); }
+        else { px = x[t]; py = x[ldx + t]; th = x[2 * ldx + t]; }
+    }
+};
+
 // Status word written by kernels (checked by the host after the sweep).
 enum { ST_OK = 0, ST_LABEL_CAP = 1, /* 4: empty map */ ST_P2P_TIMEOUT = 8 };
 

@@ -1263,12 +1263,16 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         rc = build_fgrid(h, G, min_x, min_y, &st->lsearch, n_search_cap);
         if (rc) return rc;
         h->n_launch += 5;
+        // (the generic sweep covers the handle's whole trajectory, or the whole batch: column 0 is a first pose either way)
+        TrajLayout lay = traj_layout(h, x0);
+        lay.first = 1;
+        const int traj_K = h->traj_T > 0 ? h->traj_K : 1, traj_cols = h->traj_T > 0 ? h->traj_T : T;
         PoseArrays A;
         A.x = dx; A.ldx = ldx; A.odo = h->ds.d_odo; A.ldo = T; A.u = h->ds.d_u; A.ldu = T;
-        A.x0[0] = x0[0]; A.x0[1] = x0[1]; A.x0[2] = x0[2];
+        A.lay = lay;
         A.off = h->ex.d_off; A.T = T;
         if (timing) CK(cudaEventRecord(h->ev[0], s));
-        k_assoc<<<148 * 8, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, x0[0], x0[1], x0[2], G.geom, G.start, G.pts, G.idx,
+        k_assoc<<<148 * 8, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, lay, G.geom, G.start, G.pts, G.idx,
                                         h->thr2_hi, h->ex.d_c, h->ds.d_nfar, h->d_sum_x, h->d_sum_y, h->d_cnt);
         CK(cudaGetLastError());
         h->n_launch += 1;
@@ -1278,7 +1282,7 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         CK(cudaGetLastError());
         rc = exclusive_sum(h, h->ds.d_flag, h->ds.d_prefix, T);
         if (rc) return rc;
-        k_new_labels<<<148 * 4, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, x0[0], x0[1], x0[2], st, h->ds.d_nfar, h->ds.d_prefix,
+        k_new_labels<<<148 * 4, 256, 0, s>>>(T, h->ex.d_off, h->ex.d_bx, h->ex.d_by, dx, ldx, lay, st, h->ds.d_nfar, h->ds.d_prefix,
                                              L, h->ex.d_c, h->d_sum_x, h->d_sum_y, h->d_cnt);
         CK(cudaGetLastError());
         h->n_launch += 2;
@@ -1306,7 +1310,7 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
             CK(cub::DeviceRadixSort::SortPairs(h->d_sort_ws, bytes, (const unsigned*)h->ex.d_c.p, (unsigned*)h->ex.d_keys_out.p, h->ex.d_iota.p, h->ex.d_sorted.p,
                                                (int)n, 0, end_bit, s));
             k_running_mean<<<nblk(L, 128), 128, 0, s>>>(st, h->d_seg, h->d_cnt, h->ex.d_sorted, h->ex.d_scan_of, h->ex.d_bx, h->ex.d_by, dx, ldx,
-                                                        x0[0], x0[1], x0[2], h->ex.d_seen_x, h->ex.d_seen_y, raw_x, raw_y, L);
+                                                        lay, h->ex.d_seen_x, h->ex.d_seen_y, raw_x, raw_y, L);
             CK(cudaGetLastError());
             h->n_launch += 1;
         }
@@ -1322,14 +1326,14 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         S.lsearch_ptr = &st->lsearch;
         if (timing) CK(cudaEventRecord(h->ev[2], s));
         if (o.schedule == ICMSLAM_SCHED_REDBLACK) {
-            int half = (T + 1) / 2;
-            k_pose_colour<<<nblk(half, 128), 128, 0, s>>>(1, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
+            const int threads = traj_K * ((traj_cols + 1) / 2);
+            k_pose_colour<<<nblk(threads, 128), 128, 0, s>>>(1, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
             CK(cudaGetLastError());
-            k_pose_colour<<<nblk(half, 128), 128, 0, s>>>(0, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
+            k_pose_colour<<<nblk(threads, 128), 128, 0, s>>>(0, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
             CK(cudaGetLastError());
             h->n_launch += 2;
         } else {
-            k_pose_sequential<<<1, 32, 0, s>>>(h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
+            k_pose_walk<<<traj_K, WARP, 0, s>>>(h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
             CK(cudaGetLastError());
             h->n_launch += 1;
         }

@@ -9,7 +9,8 @@
 //                All observation terms enter through 11 moment sums accumulated in ONE pass over
 //                the pose's observations, so the iterations cost O(1) per pose.
 // Two schedules: REDBLACK (odd poses, then even poses; thread per pose) and SEQUENTIAL (the
-// reference's forward Gauss-Seidel; one thread walks the trajectory).
+// reference's forward Gauss-Seidel; one warp walks each trajectory).  Both keep to the batch
+// rules of TrajLayout (common.cuh).
 #pragma once
 #include "common.cuh"
 #include "assoc.cuh"
@@ -64,6 +65,10 @@ __device__ __forceinline__ void rota_mul(double phi, double vx, double vy, doubl
 }
 
 // ---- faithful energy (used by NM) ------------------------------------------------------------
+// WARPED: called by all 32 lanes of a warp with the same arguments (k_pose_walk).  The lanes form the per-observation residuals
+// side by side; every lane then adds them into h in observation order with the scalar loop's expressions, so the energy is the
+// same to the last bit and the same on every lane.
+template <bool WARPED = false>
 __device__ double pose_energy(const DevCfg& cfg, const PoseProblem& P, const ObsArrays& O, const SeenSrc& S, const double x[3])
 {
     double f = 0.0;
@@ -81,15 +86,36 @@ __device__ double pose_energy(const DevCfg& cfg, const PoseProblem& P, const Obs
     g_step(P.a, P.ua[0], P.ua[1], cfg.dt, ga);   // sensors.py:247-255 / 273-281
     double g0 = x[0] - ga[0], g1 = x[1] - ga[1], g2 = entrepi(x[2] - ga[2]);
     double hh = 0.0;                              // h, sensors.py:194-204
-    for (int k = 0; k < P.n; ++k) {
-        int i = P.o + k;
-        double alfa = O.ang[O.beam[i]] + x[2] - ICM_HALFPI;
-        double s, c, sx, sy;
-        sincos(alfa, &s, &c);
-        seen_of(S, i, sx, sy);
-        double dx = (x[0] + O.d[i] * c) - sx, dy = (x[1] + O.d[i] * s) - sy;
-        hh += dx * cfg.q1 * dx;
-        hh += dy * cfg.q2 * dy;
+    if constexpr (WARPED) {
+        const int lane = threadIdx.x & (WARP - 1);
+        for (int k0 = 0; k0 < P.n; k0 += WARP) {
+            double dx = 0.0, dy = 0.0;
+            if (k0 + lane < P.n) {
+                int i = P.o + k0 + lane;
+                double alfa = O.ang[O.beam[i]] + x[2] - ICM_HALFPI;
+                double s, c, sx, sy;
+                sincos(alfa, &s, &c);
+                seen_of(S, i, sx, sy);
+                dx = (x[0] + O.d[i] * c) - sx; dy = (x[1] + O.d[i] * s) - sy;
+            }
+            const int m = min(WARP, P.n - k0);
+            for (int j = 0; j < m; ++j) {
+                const double ex = __shfl_sync(FULLMASK, dx, j), ey = __shfl_sync(FULLMASK, dy, j);
+                hh += ex * cfg.q1 * ex;
+                hh += ey * cfg.q2 * ey;
+            }
+        }
+    } else {
+        for (int k = 0; k < P.n; ++k) {
+            int i = P.o + k;
+            double alfa = O.ang[O.beam[i]] + x[2] - ICM_HALFPI;
+            double s, c, sx, sy;
+            sincos(alfa, &s, &c);
+            seen_of(S, i, sx, sy);
+            double dx = (x[0] + O.d[i] * c) - sx, dy = (x[1] + O.d[i] * s) - sy;
+            hh += dx * cfg.q1 * dx;
+            hh += dy * cfg.q2 * dy;
+        }
     }
     rota_mul(P.o0[2], P.o1[0] - P.o0[0], P.o1[1] - P.o0[1], ox, oy);
     rota_mul(P.a[2], x[0] - P.a[0], x[1] - P.a[1], px, py);
@@ -114,6 +140,7 @@ __device__ __forceinline__ void nm_sort4(double sim[4][3], double fs[4])
     }
 }
 
+template <bool WARPED = false>
 __device__ int nelder_mead(const DevCfg& cfg, const PoseProblem& P, const ObsArrays& O, const SeenSrc& S,
                            const double start[3], double out[3])
 {
@@ -127,7 +154,7 @@ __device__ int nelder_mead(const DevCfg& cfg, const PoseProblem& P, const ObsArr
         if (sim[k + 1][k] != 0.0) sim[k + 1][k] = mul_rn(1 + 0.05, sim[k + 1][k]);
         else sim[k + 1][k] = 0.00025;
     }
-    for (int k = 0; k < 4; ++k) { fs[k] = pose_energy(cfg, P, O, S, sim[k]); ++nev; }
+    for (int k = 0; k < 4; ++k) { fs[k] = pose_energy<WARPED>(cfg, P, O, S, sim[k]); ++nev; }
     nm_sort4(sim, fs);
     int iterations = 1;
     while (nev < maxfun && iterations < maxiter) {
@@ -142,11 +169,11 @@ __device__ int nelder_mead(const DevCfg& cfg, const PoseProblem& P, const ObsArr
             xbar[j] = __ddiv_rn(add_rn(add_rn(sim[0][j], sim[1][j]), sim[2][j]), 3.0);
             xr[j] = sub_rn(mul_rn(2.0, xbar[j]), sim[3][j]);
         }
-        double fxr = pose_energy(cfg, P, O, S, xr); ++nev;
+        double fxr = pose_energy<WARPED>(cfg, P, O, S, xr); ++nev;
         bool doshrink = false;
         if (fxr < fs[0]) {
             for (int j = 0; j < 3; ++j) xe[j] = sub_rn(mul_rn(3.0, xbar[j]), mul_rn(2.0, sim[3][j]));
-            double fxe = pose_energy(cfg, P, O, S, xe); ++nev;
+            double fxe = pose_energy<WARPED>(cfg, P, O, S, xe); ++nev;
             if (fxe < fxr) { for (int j = 0; j < 3; ++j) sim[3][j] = xe[j]; fs[3] = fxe; }
             else { for (int j = 0; j < 3; ++j) sim[3][j] = xr[j]; fs[3] = fxr; }
         } else if (fxr < fs[2]) {
@@ -155,19 +182,19 @@ __device__ int nelder_mead(const DevCfg& cfg, const PoseProblem& P, const ObsArr
         } else {
             if (fxr < fs[3]) {
                 for (int j = 0; j < 3; ++j) xe[j] = sub_rn(mul_rn(1.5, xbar[j]), mul_rn(0.5, sim[3][j]));
-                double fxc = pose_energy(cfg, P, O, S, xe); ++nev;
+                double fxc = pose_energy<WARPED>(cfg, P, O, S, xe); ++nev;
                 if (fxc <= fxr) { for (int j = 0; j < 3; ++j) sim[3][j] = xe[j]; fs[3] = fxc; }
                 else doshrink = true;
             } else {
                 for (int j = 0; j < 3; ++j) xe[j] = add_rn(mul_rn(0.5, xbar[j]), mul_rn(0.5, sim[3][j]));
-                double fxcc = pose_energy(cfg, P, O, S, xe); ++nev;
+                double fxcc = pose_energy<WARPED>(cfg, P, O, S, xe); ++nev;
                 if (fxcc < fs[3]) { for (int j = 0; j < 3; ++j) sim[3][j] = xe[j]; fs[3] = fxcc; }
                 else doshrink = true;
             }
             if (doshrink) {
                 for (int k = 1; k < 4; ++k) {
                     for (int j = 0; j < 3; ++j) sim[k][j] = add_rn(sim[0][j], mul_rn(0.5, sub_rn(sim[k][j], sim[0][j])));
-                    fs[k] = pose_energy(cfg, P, O, S, sim[k]); ++nev;
+                    fs[k] = pose_energy<WARPED>(cfg, P, O, S, sim[k]); ++nev;
                 }
             }
         }
@@ -296,25 +323,32 @@ struct PoseArrays {
     double* x; int64_t ldx;                 // 3 x T poses (in/out)
     const double* odo; int64_t ldo;         // 3 x T
     const double* u; int64_t ldu;           // 2 x T
-    double x0[3];                           // self.x0 (sensors.py:131)
+    TrajLayout lay;                         // self.x0 (sensors.py:131) of the trajectory or of each trajectory of a batch
     const int* off;
     int T;
+    // trajectories and columns per trajectory (one trajectory: 1 and T)
+    __device__ __forceinline__ int traj_cols() const { return lay.traj_T > 0 ? lay.traj_T : T; }
 };
 
+// Pose t (never a pinned one).  WARPED: all 32 lanes of a warp call it for the same t (k_pose_walk) and compute the same
+// result; lane 0 writes it.
+template <bool WARPED = false>
 __device__ __forceinline__ void update_pose(int t, const DevCfg& cfg, const PoseArrays& A, const ObsArrays& O,
                                             const SeenSrc& S, int solver, double tol, int maxit,
                                             unsigned long long* iters)
 {
+    const bool writer = !WARPED || (threadIdx.x & (WARP - 1)) == 0;
     const int o = A.off[t], n = A.off[t + 1] - o;
     double res[3];
     if (n == 0) {   // sensors.py:147-151: average of the previous result and the next (old) pose
+        const bool t1 = A.lay.after_pinned(t);
         for (int j = 0; j < 3; ++j) {
-            double prev = (t == 1) ? A.x0[j] : A.x[j * A.ldx + t - 1];
+            double prev = t1 ? A.lay.x0_of(t - 1, j) : A.x[j * A.ldx + t - 1];
             res[j] = (prev + A.x[j * A.ldx + t + 1]) / 2.0;
         }
     } else {
         PoseProblem P;
-        P.has_next = (t + 1 < A.T) ? 1 : 0;
+        P.has_next = A.lay.has_next(t, A.T) ? 1 : 0;
         P.o = o; P.n = n;
         for (int j = 0; j < 3; ++j) {
             P.a[j] = A.x[j * A.ldx + t - 1];
@@ -336,8 +370,8 @@ __device__ __forceinline__ void update_pose(int t, const DevCfg& cfg, const Pose
             g_step(P.a, P.ua[0], P.ua[1], cfg.dt, start);                // sensors.py:262
         }
         if (solver == ICMSLAM_SOLVER_NM) {
-            int nev = nelder_mead(cfg, P, O, S, start, res);
-            if (iters) atomicAdd(iters, (unsigned long long)nev);
+            int nev = nelder_mead<WARPED>(cfg, P, O, S, start, res);
+            if (iters && writer) atomicAdd(iters, (unsigned long long)nev);
         } else {
             Moments M;
             moments_zero(M);
@@ -347,27 +381,33 @@ __device__ __forceinline__ void update_pose(int t, const DevCfg& cfg, const Pose
                 moments_add(M, O.bx[o + k], O.by[o + k], sx - start[0], sy - start[1]);
             }
             int it = newton_moments(cfg, P, M, start[0], start[1], start[2], tol, maxit, res);
-            if (iters) atomicAdd(iters, (unsigned long long)it);
+            if (iters && writer) atomicAdd(iters, (unsigned long long)it);
         }
     }
-    A.x[t] = res[0]; A.x[A.ldx + t] = res[1]; A.x[2 * A.ldx + t] = res[2];   // sensors.py:162
+    if (writer) { A.x[t] = res[0]; A.x[A.ldx + t] = res[1]; A.x[2 * A.ldx + t] = res[2]; }   // sensors.py:162
+    if (WARPED) __syncwarp();      // (the next pose of the walk reads this one)
 }
 
-// red-black: parity 1 -> t = 1,3,5,... ; parity 0 -> t = 2,4,6,...
+// red-black by trajectory-local time tl = t - k traj_T: parity 1 -> tl = 1,3,5,... ; parity 0 -> tl = 2,4,6,...  (so a
+// trajectory of a batch is swept exactly as it is alone, whatever the parity of traj_T).  (traj_cols + 1) / 2 threads per
+// trajectory.
 __global__ void __launch_bounds__(128)
 k_pose_colour(int parity, DevCfg cfg, PoseArrays A, ObsArrays O, SeenSrc S, int solver, double tol, int maxit,
               unsigned long long* iters)
 {
-    int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    int t = 2 * idx + (parity ? 1 : 2);
-    if (t >= A.T) return;
-    update_pose(t, cfg, A, O, S, solver, tol, maxit, iters);
+    const int Tt = A.traj_cols(), per = (Tt + 1) / 2;
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    const int k = idx / per, tl = 2 * (idx - k * per) + (parity ? 1 : 2);
+    if (k >= A.T / Tt || tl >= Tt) return;
+    update_pose(k * Tt + tl, cfg, A, O, S, solver, tol, maxit, iters);
 }
 
-// the reference's forward Gauss-Seidel (sensors.py:145): one thread walks t = 1..T-1
-__global__ void k_pose_sequential(DevCfg cfg, PoseArrays A, ObsArrays O, SeenSrc S, int solver, double tol, int maxit,
-                                  unsigned long long* iters)
+// the reference's forward Gauss-Seidel (sensors.py:145): the warp of block k walks t = 1 .. traj_T-1 of trajectory k (one
+// block of one warp per trajectory: trajectories take different Nelder-Mead branches).  Its lanes share each energy's
+// observations (pose_energy<true>); everything else runs on every lane alike.
+__global__ void __launch_bounds__(WARP)
+k_pose_walk(DevCfg cfg, PoseArrays A, ObsArrays O, SeenSrc S, int solver, double tol, int maxit, unsigned long long* iters)
 {
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    for (int t = 1; t < A.T; ++t) update_pose(t, cfg, A, O, S, solver, tol, maxit, iters);
+    const int Tt = A.traj_cols(), t0 = blockIdx.x * Tt;
+    for (int t = t0 + 1; t < t0 + Tt; ++t) update_pose<true>(t, cfg, A, O, S, solver, tol, maxit, iters);
 }

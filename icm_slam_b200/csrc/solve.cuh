@@ -63,22 +63,6 @@ __global__ void k_interleave(const double* __restrict__ bx, const double* __rest
     if (i < n) out[i] = make_double2(bx[i], by[i]);
 }
 
-// Which columns are pinned first poses (sensors.py:131: x[:,0] is never updated, scan 0 is projected with self.x0): column 0
-// of the trajectory's first segment, or -- a batch of independent trajectories of traj_T columns each laid end to end in one
-// handle (BASELINE configs[4]) -- the first column of every trajectory, each with its own x0.  A trajectory's last pose has no
-// successor.
-struct TrajLayout {
-    int first;                 // column 0 is the trajectory's first pose
-    int traj_T;                // > 0: batch of trajectories of this many columns
-    const double* x0s;         // batch: 3 x K first poses (row-major, leading dimension ldx0s)
-    int64_t ldx0s;
-    double x0[3];              // single trajectory: self.x0
-    __device__ __forceinline__ bool pinned(int t) const { return traj_T > 0 ? (t % traj_T) == 0 : (t == 0 && first); }
-    __device__ __forceinline__ bool after_pinned(int t) const { return traj_T > 0 ? (t % traj_T) == 1 : (t == 1 && first); }
-    __device__ __forceinline__ bool has_next(int t, int T) const { return t + 1 < T && (traj_T == 0 || ((t + 1) % traj_T) != 0); }
-    __device__ __forceinline__ double x0_of(int t, int r) const { return traj_T > 0 ? x0s[r * ldx0s + t / traj_T] : x0[r]; }
-};
-
 // ppar of poses given from outside (set_poses, host sweeps, halo columns).  A pinned column is projected with its x0
 // (sensors.py:131,141), not with x[:,t].
 __global__ void k_ppar_init(const double* __restrict__ x, int64_t ld, int t_begin, int t_end, const TrajLayout L, double4* __restrict__ ppar)

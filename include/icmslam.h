@@ -154,8 +154,10 @@ int icmslam_get_poses(icmslam_handle* h, double* x, int64_t ld_x, int32_t memspa
  * end to end (T = K * traj_T), each translated to its own region of the plane so that their landmarks are farther apart than
  * any gate (icm_slam_b200/batch.py does both); x0s (HOST, 3 x K) are their pinned first poses.  Every trajectory's first pose is
  * then pinned to its own x0, its last pose has no successor, and one sweep of the handle is one sweep of every trajectory: ONE
- * launch of each kernel for the whole batch.  (REDBLACK, NEWTON, PREV) sweeps only; the x0 argument of icmslam_iterate is
- * ignored.  traj_T <= 0 switches back to a single trajectory. */
+ * launch of each kernel for the whole batch.  Every sweep mode is valid on a batch handle (icmslam_iterate and icmslam_sweep; the
+ * SEQUENTIAL schedule walks each trajectory with its own warp); new labels are numbered over the whole batch and the label cap L
+ * applies to the batch.  The x0 argument of icmslam_iterate / icmslam_sweep is ignored.  traj_T <= 0 switches back to a single
+ * trajectory. */
 int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double* x0s, int64_t ld_x0s, int32_t K);
 
 /* -- time-segment partition over several GPUs (no reference counterpart: the reference sweep is strictly
