@@ -149,3 +149,12 @@ __device__ __forceinline__ double warp_max(double v)
     for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(FULLMASK, v, o));
     return v;
 }
+
+__device__ __forceinline__ void atomic_max_pos(double* addr, double v)   // v >= 0
+{
+    atomicMax((unsigned long long*)addr, (unsigned long long)__double_as_longlong(v));
+}
+__device__ __forceinline__ void atomic_min_pos(double* addr, double v)   // v >= 0
+{
+    atomicMin((unsigned long long*)addr, (unsigned long long)__double_as_longlong(v));
+}

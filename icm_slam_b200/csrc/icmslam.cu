@@ -62,9 +62,10 @@ template <typename T> using PinnedBuf = Buf<T, cudaFreeHost>;
 
 // A landmark grid (fastgrid.cuh): geometry, per-cell counts (all zero between builds: the fill pass counts them back down) and
 // starts, the cell-sorted entries and the bounding box.  A handle has two.  `grid` indexes the map of the fused sweep's chain
-// (Chain::grid_map) and only the fused sweep writes it; every other reader (the generic sweep's association, Mapa.filtrar,
-// calc_cambio) builds `scratch_grid`.  calc_cambio runs between two fused sweeps of icmslam_iterate_until: were it to rebuild
-// `grid`, the next sweep would find its grid stale, rebuild it and void every run record.
+// (Chain::grid_map) and is written by the filter chain; a caller other than the fused sweep invalidates ch.grid_map.  The two
+// other readers (the generic sweep's association, calc_cambio) build `scratch_grid`.  calc_cambio runs between two fused sweeps
+// of icmslam_iterate_until: were it to rebuild `grid`, the next sweep would find its grid stale, rebuild it and void every run
+// record.
 struct LandmarkGrid {
     DevBuf<FGeom> geom;
     DevBuf<int> cnt, start, idx;
@@ -774,47 +775,54 @@ static int build_fgrid(icmslam_handle* h, LandmarkGrid& G, const double* px, con
     return ICMSLAM_OK;
 }
 
-// ---- Mapa.filtrar on device-resident raw map (d_raw, counts from cnt_i or cnt_d) -----------------
-// Expects d_kflag already set.  Writes map_out (device pointer) and the Mapa state.
-static int run_filter(icmslam_handle* h, const double* raw_x, const double* raw_y, const int* cnt_i, const double* cnt_d,
-                      double* map_out, int cap_out, int64_t ld_out, double* counts_out, int update_state)
+// ---- Mapa.filtrar (ICM_SLAM.py:204-265) for every caller: the filter chain of tail.cuh ---------------------------------------
+// k_tail_compact -> k_tail_count -> k_cell_scan -> k_fgrid_fill -> k_tail_nn over the raw map (raw_x, raw_y): the filtered map
+// to map_out, its counts to d_counts, its width to st->new_l and st->lact, and h->grid built over it.  What the chain reads is
+// left by its entry (k_fused_means and far_scan_block in the fused sweep, k_means_flags or k_flags_from_counts otherwise):
+//   * raw_x / raw_y hold the raw means, st->raw_l their number;
+//   * d_kflag holds the keep flags, d_blk_kept the kept landmarks per 256-thread block, counted on a grid of k_tail_compact's
+//     shape (the compaction takes its positions from them);
+//   * d_cnt holds the int observation counts (k_tail_compact moves them to d_rawcnt and clears d_cnt), unless cnt_d gives
+//     double counts, which are taken as they are (d_cnt and d_rawcnt then stay as they were);
+//   * h->grid's bounding box is reset, ts->n_ind is 0, and ts->steady_ok is 0 (otherwise every kernel of the chain returns at
+//     once);
+//   * h->grid's cell counts are all zero (every build leaves them so).
+// `fused` launches k_tail_nn<true>, which also closes the fused sweep's bookkeeping (sequence numbers, epoch, steady tail).  Any
+// other caller invalidates ch.grid_map and ch.hint_map: the grid, d_remap and the landmark records the chain writes then belong
+// to no map chain, and the next fused sweep rebuilds them.
+//
+// Why the chain gives the reference's result (a K x K search) at every map size:
+//   * the grid is searched unless the map is degenerate (extent < dist_thr), where tail_slow_body runs the reference's brute
+//     force.  With an extent >= dist_thr the map diameter is >= dist_thr, and the reference substitutes the diameter for zero
+//     distances, so a substituted value never passes the strict gate.  The nearest neighbour is read only for survivors that pass
+//     the gate, and on those the grid's rule (rooted distances, the lowest index on ties) is argmin's first minimum;
+//   * with no merge the new map is mul_rn(x, c) / c and c, as the reference's count-weighted mean of one member;
+//   * with merges the merged means are accumulated with fp64 atomics in no fixed order: equal up to the rounding of that order.
+static int filter_chain(icmslam_handle* h, const double* raw_x, const double* raw_y, const double* cnt_d, double* dmap_out, int out_cap,
+                        int64_t out_ld, cudaStream_t s, bool fused)
 {
     const int L = h->Lcap;
     DevState* st = h->d_st;
-    int rc = exclusive_sum(h, h->d_kflag, h->d_kpos, L);
-    if (rc) return rc;
-    k_compact_kept<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_kflag, h->d_kpos, raw_x, raw_y, cnt_i, cnt_d, h->d_kx, h->d_ky,
-                                                        h->d_kc, h->d_parent, L);
+    TailState* ts = h->d_ts;
+    k_tail_compact<<<nblk(L, 256), 256, 0, s>>>(st, h->d_kflag, h->d_blk_kept, h->d_kpos, raw_x, raw_y, h->d_cnt, h->d_kx, h->d_ky, h->d_kc,
+                                                h->d_parent, h->grid.bb, L, h->d_klab, h->d_rawcnt, ts, cnt_d);
     CK(cudaGetLastError());
-    LandmarkGrid& G = h->scratch_grid;
-    rc = build_fgrid(h, G, h->d_kx, h->d_ky, &st->kept, L);
-    if (rc) return rc;
-    CK(cudaMemsetAsync(h->d_acc, 0, 8 * sizeof(double), h->stream));
-    k_filter_diameter<<<nblk(FILTER_SMALL_K, 128), 128, 0, h->stream>>>(st, h->d_kx, h->d_ky, G.bb, h->dcfg.dist_thr, h->d_acc);
+    k_tail_count<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, st, ts, h->grid.bb, h->dcfg.dist_thr, h->fg_cells, h->grid.geom, h->grid.cnt);
     CK(cudaGetLastError());
-    k_filter_nn<<<nblk(L, 128), 128, 0, h->stream>>>(st, h->d_kx, h->d_ky, h->dcfg.dist_thr, h->d_acc, G.bb, G.geom, G.start, G.pts,
-                                                     G.idx, h->d_nn, h->d_indflag, L);
+    k_cell_scan<<<nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS), CS_THREADS, 0, s>>>(h->grid.cnt, h->grid.start, h->fg_cells + 1, h->d_scan_state, ts);
     CK(cudaGetLastError());
-    rc = exclusive_sum(h, h->d_indflag, h->d_indpos, L);
-    if (rc) return rc;
-    k_ind_compact<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_indflag, h->d_indpos, h->d_ind, L);
+    k_fgrid_fill<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, &st->kept, h->grid.geom, h->grid.start, h->grid.cnt, h->grid.pts,
+                                              h->grid.idx, h->d_gslots, &ts->steady_ok);
     CK(cudaGetLastError());
-    k_relabel<<<1, 32, 0, h->stream>>>(st, h->d_ind, h->d_nn, h->d_parent);
-    CK(cudaGetLastError());
-    CK(cudaMemsetAsync(h->d_used, 0, (size_t)L * sizeof(int), h->stream));
-    CK(cudaMemsetAsync(h->d_ox, 0, (size_t)L * sizeof(double), h->stream));
-    CK(cudaMemsetAsync(h->d_oy, 0, (size_t)L * sizeof(double), h->stream));
-    CK(cudaMemsetAsync(h->d_oc, 0, (size_t)L * sizeof(double), h->stream));
-    k_roots<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_parent, h->d_lab, h->d_used);
-    CK(cudaGetLastError());
-    rc = exclusive_sum(h, h->d_used, h->d_rank, L);
-    if (rc) return rc;
-    k_merge_accumulate<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_lab, h->d_rank, h->d_kx, h->d_ky, h->d_kc, h->d_ox, h->d_oy,
-                                                            h->d_oc);
-    CK(cudaGetLastError());
-    k_filter_finalize<<<nblk(L, 256), 256, 0, h->stream>>>(st, h->d_used, h->d_rank, h->d_ox, h->d_oy, h->d_oc, map_out, cap_out,
-                                                           ld_out, update_state ? h->d_counts.p : nullptr, counts_out, L,
-                                                           update_state);
+    SlowArgs sa;
+    sa.dist_thr = h->dcfg.dist_thr; sa.parent = h->d_parent; sa.ind_pos = h->d_indpos; sa.ind = h->d_ind; sa.lab = h->d_lab; sa.used = h->d_used;
+    sa.rank = h->d_rank; sa.ox = h->d_ox; sa.oy = h->d_oy; sa.oc = h->d_oc; sa.max_cells = h->fg_cells; sa.geom = h->grid.geom;
+    sa.cell_cnt = h->grid.cnt; sa.cell_start = h->grid.start; sa.pts = h->grid.pts; sa.gidx = h->grid.idx;
+    sa.gbuild = h->d_gbuild; sa.nnd0 = h->d_nnd0; sa.steady_enable = h->steady_enable; sa.fz = h->fz;
+    auto nn = fused ? k_tail_nn<true> : k_tail_nn<false>;
+    nn<<<nblk(L, 256), 256, 0, s>>>(st, ts, h->d_kx, h->d_ky, h->d_kc, h->grid.geom, h->grid.start, h->grid.pts, h->grid.idx, h->thr2_lt,
+                                    h->d_nn, h->d_indflag, L, h->d_klab, h->d_kflag, h->d_kpos, h->d_lmrec2[h->ch.lm_cur],
+                                    h->d_lmrec2[h->ch.lm_cur ^ 1], dmap_out, out_cap, out_ld, h->d_counts, h->thr1sq, h->thr2_hi, h->d_remap, sa);
     CK(cudaGetLastError());
     return ICMSLAM_OK;
 }
@@ -1135,44 +1143,18 @@ static int fused_part_c(icmslam_handle* h, const double* xout, double* dmap_out,
     return ICMSLAM_OK;
 }
 
-// the filter's full chain (tail.cuh): everything after k_tail_steady
+// the full chain (tail.cuh): everything after k_tail_steady -- the fused entry, then the filter chain
 static int full_chain(icmslam_handle* h, double* dmap_out, int out_cap, int64_t out_ld, cudaStream_t s)
 {
     const int L = h->Lcap;
     DevState* st = h->d_st;
-    TailState* ts = h->d_ts;
-    const double* min_x = h->d_map_in;
-    const double* min_y = h->d_map_in + L;
     double* raw_x = h->d_raw;
     double* raw_y = h->d_raw + L;
-    {
-    k_fused_means<<<nblk(L, 256), 256, 0, s>>>(st, h->d_fsum_x, h->d_fsum_y, h->d_cnt, min_x, min_y, 1.0 / h->fix_scale, h->dcfg.cota,
-                                               h->d_newraw, raw_x, raw_y, h->d_kflag, L, h->d_blk_kept, h->ex.d_farbits, h->n_tiles * 4, h->p2p, ts,
+    k_fused_means<<<nblk(L, 256), 256, 0, s>>>(st, h->d_fsum_x, h->d_fsum_y, h->d_cnt, h->d_map_in, h->d_map_in + L, 1.0 / h->fix_scale, h->dcfg.cota,
+                                               h->d_newraw, raw_x, raw_y, h->d_kflag, L, h->d_blk_kept, h->ex.d_farbits, h->n_tiles * 4, h->p2p, h->d_ts,
                                                h->d_cnt, st, h->d_sh_x, h->d_sh_y, h->d_sh_k, h->fz, h->d_counts);
     CK(cudaGetLastError());
-    k_tail_compact<<<nblk(L, 256), 256, 0, s>>>(st, h->d_kflag, h->d_blk_kept, h->d_kpos, raw_x, raw_y, h->d_cnt, h->d_kx, h->d_ky, h->d_kc,
-                                                h->d_parent, h->grid.bb, L, h->d_klab, h->d_rawcnt, ts);
-    CK(cudaGetLastError());
-    k_tail_count<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, st, ts, h->grid.bb, h->dcfg.dist_thr, h->fg_cells, h->grid.geom, h->grid.cnt);
-    CK(cudaGetLastError());
-    k_cell_scan<<<nblk(h->fg_cells + 1, CS_THREADS * CS_ITEMS), CS_THREADS, 0, s>>>(h->grid.cnt, h->grid.start, h->fg_cells + 1, h->d_scan_state, ts);
-    CK(cudaGetLastError());
-    k_fgrid_fill<<<nblk(L, 256), 256, 0, s>>>(h->d_kx, h->d_ky, &st->kept, h->grid.geom, h->grid.start, h->grid.cnt, h->grid.pts,
-                                              h->grid.idx, h->d_gslots, &ts->steady_ok);
-    CK(cudaGetLastError());
-    {
-        SlowArgs sa;
-        sa.dist_thr = h->dcfg.dist_thr; sa.parent = h->d_parent; sa.ind_pos = h->d_indpos; sa.ind = h->d_ind; sa.lab = h->d_lab; sa.used = h->d_used;
-        sa.rank = h->d_rank; sa.ox = h->d_ox; sa.oy = h->d_oy; sa.oc = h->d_oc; sa.max_cells = h->fg_cells; sa.geom = h->grid.geom;
-        sa.cell_cnt = h->grid.cnt; sa.cell_start = h->grid.start; sa.pts = h->grid.pts; sa.gidx = h->grid.idx;
-        sa.gbuild = h->d_gbuild; sa.nnd0 = h->d_nnd0; sa.steady_enable = h->steady_enable; sa.fz = h->fz;
-        k_tail_nn<<<nblk(L, 256), 256, 0, s>>>(st, ts, h->d_kx, h->d_ky, h->d_kc, h->grid.geom, h->grid.start, h->grid.pts, h->grid.idx, h->thr2_lt,
-                                               h->d_nn, h->d_indflag, L, h->d_klab, h->d_kflag, h->d_kpos, h->d_lmrec2[h->ch.lm_cur],
-                                               h->d_lmrec2[h->ch.lm_cur ^ 1], dmap_out, out_cap, out_ld, h->d_counts, h->thr1sq, h->thr2_hi, h->d_remap, sa);
-        CK(cudaGetLastError());
-    }
-    }
-    return ICMSLAM_OK;
+    return filter_chain(h, raw_x, raw_y, nullptr, dmap_out, out_cap, out_ld, s, true);
 }
 
 // streams and events of the chunk-pipelined host sweep, created on first use
@@ -1251,7 +1233,6 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         return ICMSLAM_OK;
     } else {
         h->ch.stats_clean = false;
-        h->ch.rawcnt_valid = false;
         CK(cudaMemsetAsync(h->d_cnt, 0, ((size_t)L + 1) * sizeof(int), s));
         CK(cudaMemsetAsync(h->d_counts, 0, (size_t)L * sizeof(double), s));
         if (xin != xout) CK(cudaMemcpy2DAsync(xout, (size_t)ldout * 8, xin, (size_t)ldin * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToDevice, s));
@@ -1315,7 +1296,7 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
             h->n_launch += 1;
         }
         k_means_flags<<<nblk(L, 256), 256, 0, s>>>(st, h->d_sum_x, h->d_sum_y, h->d_cnt, h->dcfg.cota, running ? 1 : 0, raw_x, raw_y,
-                                                   h->d_kflag, L);
+                                                   h->d_kflag, L, h->d_blk_kept, h->grid.bb, h->d_ts);
         CK(cudaGetLastError());
         h->n_launch += 1;
         ObsArrays O;
@@ -1343,9 +1324,10 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
     h->ch.grid_map = nullptr;
     h->ch.hint_map = nullptr;
     // Mapa.filtrar (sensors.py:165-166)
-    rc = run_filter(h, raw_x, raw_y, h->d_cnt, nullptr, dmap_out, out_cap, out_ld, nullptr, 1);
+    rc = filter_chain(h, raw_x, raw_y, nullptr, dmap_out, out_cap, out_ld, s, false);
     if (rc) return rc;
-    h->n_launch += 13;   // filter grid build (5) + filter kernels (8)
+    h->n_launch += 5;
+    h->ch.rawcnt_valid = true;
     h->ch.lact_dirty = true;
     return ICMSLAM_OK;
 }
@@ -2028,12 +2010,12 @@ extern "C" int icmslam_filter_map(icmslam_handle* h, const double* map_in, int64
     CK(cudaMemcpyAsync(h->d_tmp_b, counts_in, (size_t)L_in * 8, cudaMemcpyDefault, s));
     k_set_raw_l<<<1, 1, 0, s>>>(h->d_st, L_in);
     CK(cudaGetLastError());
-    k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, L_in, h->dcfg.cota, h->d_kflag, L);
+    k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, L_in, h->dcfg.cota, h->d_kflag, L, h->d_blk_kept, h->grid.bb, h->d_ts);
     CK(cudaGetLastError());
     // (the result goes through the handle's spare map buffer and rewrites the Mapa state: whatever map chain the handle was
     //  continuing -- grid, hints, run records, the copy of the last returned map -- no longer describes that buffer)
     h->ch.grid_map = nullptr; h->ch.hint_map = nullptr; h->last_map_L = -1;
-    int rc = run_filter(h, h->d_tmp_a, h->d_tmp_a + L, nullptr, h->d_tmp_b, h->d_map_out, L, L, h->d_tmp_b + L, 1);
+    int rc = filter_chain(h, h->d_tmp_a, h->d_tmp_a + L, h->d_tmp_b, h->d_map_out, L, L, s, false);
     if (rc) return rc;
     rc = sync_state(h);
     if (rc) return rc;
@@ -2440,13 +2422,13 @@ extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int
     h->ch.ppar_of = nullptr;
     // ---- Mapa.filtrar on the map that was built (sensors.py:99-100) ---------------------------------------------------
     h->ch.stats_clean = false;
-    h->ch.rawcnt_valid = false;
     k_counts_to_int<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, L, h->d_cnt);      // (get_raw_map reports integer counts)
     CK(cudaGetLastError());
-    k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, lact, h->dcfg.cota, h->d_kflag, L);
+    k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, lact, h->dcfg.cota, h->d_kflag, L, h->d_blk_kept, h->grid.bb, h->d_ts);
     CK(cudaGetLastError());
-    rc = run_filter(h, h->d_raw, h->d_raw + L, nullptr, h->d_tmp_b, h->d_map_out, L, L, nullptr, 1);
+    rc = filter_chain(h, h->d_raw, h->d_raw + L, nullptr, h->d_map_out, L, L, s, false);
     if (rc) return rc;
+    h->ch.rawcnt_valid = true;
     rc = sync_state(h);
     if (rc) return rc;
     int status = status_from_state(h->h_st);

@@ -1,206 +1,64 @@
-// mapfilter.cuh -- Mapa.filtrar (ICM_SLAM.py:204-265) and calc_cambio (ICM_SLAM.py:490-495).
+// mapfilter.cuh -- the entries of Mapa.filtrar (ICM_SLAM.py:204-265) for the callers other than the fused sweep, and
+// calc_cambio (ICM_SLAM.py:490-495).
 //
-// filtrar: (1) drop labels observed fewer than `cota` times; (2) every survivor whose nearest
-// OTHER survivor is closer than dist_thr is visited in ascending index order and the class of
-// that neighbour is renamed to the survivor's class (c[c==c[b[i]]] = c[i]); (3) classes are
-// renumbered densely in ascending order; (4) each class becomes the count-weighted mean of its
-// members.  The reference builds the full K x K distance matrix (O(K^2) memory, impossible at
-// 1e5 landmarks); here the neighbour search scans the survivor's own cell of the landmark grid
-// (fastgrid.cuh), and step (2) -- inherently sequential but touching only the few landmarks that
-// do have a close neighbour -- is a directed union-find walked by one thread.  A brute-force path
-// keeps the reference's exact corner cases (zero distances replaced by the map diameter, :242) for
-// small or degenerate maps.
+// Mapa.filtrar itself is the fused tail's filter chain (tail.cuh, k_tail_compact .. k_tail_nn); every caller runs it.  The
+// fused sweep enters it through k_fused_means; the generic sweep through k_means_flags, icmslam_filter_map and pass 0 through
+// k_flags_from_counts.  An entry leaves what the chain reads (filter_chain in icmslam.cu lists it): keep flags, kept landmarks
+// per block, and the chain's per-call state reset.
 #pragma once
 #include "common.cuh"
 #include "assoc.cuh"
 #include "fastgrid.cuh"
+#include "tail.cuh"
 
-#define FILTER_SMALL_K 2048
+// The end of an entry, reached by every thread of the block: the block's kept landmarks (k_tail_compact takes its positions from
+// them, so an entry is launched on k_tail_compact's grid, nblk(Lcap, 256) x 256), and the chain's per-call state as far_scan_block
+// leaves it for the fused sweep: the survivors' bounding box empty, the merge counter zero, steady_ok = 0 (the chain runs).
+__device__ __forceinline__ void filter_entry(int keep, int* __restrict__ blk_kept, unsigned long long* bb, TailState* ts)
+{
+    const int total = __syncthreads_count(keep);
+    if (threadIdx.x == 0) {
+        blk_kept[blockIdx.x] = total;
+        if (blockIdx.x == 0) {
+            bb[0] = bb[1] = ~0ull;
+            bb[2] = bb[3] = 0ull;
+            ts->n_ind = 0;
+            ts->steady_ok = 0;
+        }
+    }
+}
 
-// means + keep flag in one pass over the labels
+// generic sweep: means + keep flag in one pass over the labels
 __global__ void k_means_flags(const DevState* st, const double* __restrict__ sum_x, const double* __restrict__ sum_y,
                               const int* __restrict__ cnt, double cota, int running, double* __restrict__ raw_x,
-                              double* __restrict__ raw_y, int* __restrict__ flag, int Lcap)
+                              double* __restrict__ raw_y, int* __restrict__ flag, int Lcap, int* __restrict__ blk_kept,
+                              unsigned long long* bb, TailState* ts)
 {
-    int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l >= Lcap) return;
-    int k = l < st->raw_l ? cnt[l] : 0;
-    if (!running) {   // RUNNING view already wrote the reference-arithmetic means
-        raw_x[l] = k > 0 ? sum_x[l] / (double)k : 0.0;
-        raw_y[l] = k > 0 ? sum_y[l] / (double)k : 0.0;
-    }
-    flag[l] = (l < st->raw_l && !((double)k < cota)) ? 1 : 0;      // :232-236
-}
-
-// generic: flags (double counts) for icmslam_filter_map on caller data
-__global__ void k_flags_from_counts(const double* __restrict__ counts, int n, double cota, int* __restrict__ flag, int Lcap)
-{
-    int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l >= Lcap) return;
-    flag[l] = (l < n && !(counts[l] < cota)) ? 1 : 0;
-}
-
-__global__ void k_compact_kept(DevState* st, const int* __restrict__ flag, const int* __restrict__ pos,
-                               const double* __restrict__ raw_x, const double* __restrict__ raw_y,
-                               const int* __restrict__ cnt_i, const double* __restrict__ cnt_d, double* __restrict__ kx,
-                               double* __restrict__ ky, double* __restrict__ kc, int* __restrict__ parent, int Lcap)
-{
-    int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l >= Lcap) return;
-    if (flag[l]) {
-        int p = pos[l];
-        kx[p] = raw_x[l];
-        ky[p] = raw_y[l];
-        kc[p] = cnt_i ? (double)cnt_i[l] : cnt_d[l];
-        parent[p] = p;
-    }
-    if (l == Lcap - 1) {
-        st->kept = pos[l] + flag[l];
-        st->n_ind = 0;
-        if (st->kept == 0) st->status |= 4;   // ValueError in the reference (ICM_SLAM.py:241-255)
-    }
-}
-
-__device__ __forceinline__ void atomic_max_pos(double* addr, double v)   // v >= 0
-{
-    atomicMax((unsigned long long*)addr, (unsigned long long)__double_as_longlong(v));
-}
-__device__ __forceinline__ void atomic_min_pos(double* addr, double v)   // v >= 0
-{
-    atomicMin((unsigned long long*)addr, (unsigned long long)__double_as_longlong(v));
-}
-
-// bb: bounding box of the survivors (the filter grid's, fastgrid.cuh k_fgrid_bbox)
-__device__ __forceinline__ bool filter_small_path(const DevState* st, const unsigned long long* bb, double dist_thr)
-{
-    if (st->kept <= FILTER_SMALL_K) return true;
-    const double extent = fmax(dkey_inv(bb[2]) - dkey_inv(bb[0]), dkey_inv(bb[3]) - dkey_inv(bb[1]));
-    return !(extent >= dist_thr);
-}
-
-// brute-force path, step A: the map diameter amax (:242)
-__global__ void k_filter_diameter(const DevState* st, const double* __restrict__ kx, const double* __restrict__ ky,
-                                  const unsigned long long* __restrict__ bb, double dist_thr, double* __restrict__ amax)
-{
-    if (!filter_small_path(st, bb, dist_thr)) return;
-    const int K = st->kept;
-    double m = 0.0;
-    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < K; j += gridDim.x * blockDim.x)
-        for (int i = 0; i < K; ++i) m = fmax(m, dist_rn(kx[i] - kx[j], ky[i] - ky[j]));
-    m = warp_max(m);
-    if ((threadIdx.x % WARP) == 0) atomic_max_pos(amax, m);
-}
-
-// nearest other survivor: amin / b (:243-245), flag = amin < dist_thr
-__global__ void k_filter_nn(const DevState* st, const double* __restrict__ kx, const double* __restrict__ ky,
-                            double dist_thr, const double* __restrict__ amax_p, const unsigned long long* __restrict__ bb,
-                            const FGeom* __restrict__ geom, const int* __restrict__ cell_start, const double2* __restrict__ pts,
-                            const int* __restrict__ gidx, int* __restrict__ nn, int* __restrict__ ind_flag, int Lcap)
-{
-    int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= Lcap) return;
-    const int K = st->kept;
-    if (j >= K) { ind_flag[j] = 0; return; }
-    const double xj = kx[j], yj = ky[j];
-    double best = INFINITY;
-    int arg = 0;
-    if (filter_small_path(st, bb, dist_thr)) {
-        const double amax = *amax_p;
-        for (int i = 0; i < K; ++i) {
-            double dd = (i == j) ? 0.0 : dist_rn(kx[i] - xj, ky[i] - yj);
-            if (dd == 0.0) dd = amax;                          // a[a==0] = max(a)
-            if (dd < best) { best = dd; arg = i; }             // argmin: first minimum
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    int keep = 0;
+    if (l < Lcap) {
+        const int k = l < st->raw_l ? cnt[l] : 0;
+        if (!running) {   // RUNNING view already wrote the reference-arithmetic means
+            raw_x[l] = k > 0 ? sum_x[l] / (double)k : 0.0;
+            raw_y[l] = k > 0 ? sum_y[l] / (double)k : 0.0;
         }
-    } else {
-        // diameter >= dist_thr here, so zero distances (replaced by it) can never pass the gate; the survivor's own cell holds
-        // every survivor within dist_thr of it
-        const FGeom g = *geom;
-        const int c = fgrid_cell(g, xj, yj);
-        for (int k = cell_start[c]; k < cell_start[c + 1]; ++k) {
-            const double2 p = pts[k];
-            const int id = gidx[k];
-            const double dd = dist_rn(p.x - xj, p.y - yj);
-            if (dd == 0.0) continue;
-            if (dd < best || (dd == best && id < arg)) { best = dd; arg = id; }
-        }
+        keep = (l < st->raw_l && !((double)k < cota)) ? 1 : 0;      // :232-236
+        flag[l] = keep;
     }
-    nn[j] = arg;
-    ind_flag[j] = best < dist_thr ? 1 : 0;                     // :245 (strict <)
+    filter_entry(keep, blk_kept, bb, ts);
 }
 
-__global__ void k_ind_compact(DevState* st, const int* __restrict__ flag, const int* __restrict__ pos, int* __restrict__ ind,
-                              int Lcap)
+// icmslam_filter_map and pass 0: keep flags from double counts
+__global__ void k_flags_from_counts(const double* __restrict__ counts, int n, double cota, int* __restrict__ flag, int Lcap,
+                                    int* __restrict__ blk_kept, unsigned long long* bb, TailState* ts)
 {
-    int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= Lcap) return;
-    if (flag[j]) ind[pos[j]] = j;
-    if (j == Lcap - 1) st->n_ind = pos[j] + flag[j];
-}
-
-__device__ __forceinline__ int uf_find(const int* parent, int v)
-{
-    while (parent[v] != v) v = parent[v];
-    return v;
-}
-
-// :247-249 -- for i in ind ascending: c[c == c[b[i]]] = c[i]   (class of the neighbour renamed)
-__global__ void k_relabel(const DevState* st, const int* __restrict__ ind, const int* __restrict__ nn, int* parent)
-{
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    const int n = st->n_ind;
-    for (int q = 0; q < n; ++q) {
-        int i = ind[q];
-        int X = uf_find(parent, nn[i]), Y = uf_find(parent, i);
-        if (X != Y) parent[X] = Y;
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    int keep = 0;
+    if (l < Lcap) {
+        keep = (l < n && !(counts[l] < cota)) ? 1 : 0;
+        flag[l] = keep;
     }
-}
-
-__global__ void k_roots(const DevState* st, const int* __restrict__ parent, int* __restrict__ lab, int* __restrict__ used)
-{
-    int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= st->kept) return;
-    int r = uf_find(parent, j);
-    lab[j] = r;
-    used[r] = 1;
-}
-
-// :251-260 -- dense renumbering (rank of the class label) + count-weighted mean
-__global__ void k_merge_accumulate(const DevState* st, const int* __restrict__ lab, const int* __restrict__ rank,
-                                   const double* __restrict__ kx, const double* __restrict__ ky, const double* __restrict__ kc,
-                                   double* __restrict__ ox, double* __restrict__ oy, double* __restrict__ oc)
-{
-    int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= st->kept) return;
-    int r = rank[lab[j]];
-    if (lab[j] == j && st->n_ind == 0) {   // common case: nothing merged
-        ox[r] = mul_rn(kx[j], kc[j]); oy[r] = mul_rn(ky[j], kc[j]); oc[r] = kc[j];
-        return;
-    }
-    atomicAdd(ox + r, mul_rn(kx[j], kc[j]));
-    atomicAdd(oy + r, mul_rn(ky[j], kc[j]));
-    atomicAdd(oc + r, kc[j]);
-}
-
-__global__ void k_filter_finalize(DevState* st, const int* __restrict__ used, const int* __restrict__ rank,
-                                  const double* __restrict__ ox, const double* __restrict__ oy, const double* __restrict__ oc,
-                                  double* __restrict__ map_out, int cap_out, int64_t ld_out, double* __restrict__ counts_state,
-                                  double* __restrict__ counts_out, int Lcap, int update_state)
-{
-    int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= Lcap) return;
-    const int K = st->kept;
-    const int newL = K > 0 ? rank[K - 1] + used[K - 1] : 0;
-    double c = r < newL ? oc[r] : 0.0;
-    if (r < cap_out && map_out) {
-        map_out[r] = r < newL ? ox[r] / c : 0.0;
-        map_out[ld_out + r] = r < newL ? oy[r] / c : 0.0;
-    }
-    if (counts_state) counts_state[r] = c;
-    if (counts_out && r < cap_out) counts_out[r] = c;
-    if (r == 0) {
-        st->new_l = newL;
-        if (update_state) st->lact = newL;
-    }
+    filter_entry(keep, blk_kept, bb, ts);
 }
 
 // ---- calc_cambio ---------------------------------------------------------------------------

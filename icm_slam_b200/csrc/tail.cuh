@@ -17,13 +17,14 @@
 //   k_tail_nn        nearest other survivor of every survivor (:241-245) through the grid; the survivors written as the
 //                    new map on the assumption that nothing merges; the LAST block to finish checks the assumption and
 //                    otherwise runs the reference's sequential relabelling (:247-260) and rebuilds the grid
+// k_tail_compact .. k_tail_nn are Mapa.filtrar for every caller: the generic sweep, icmslam_filter_map and pass 0 enter them
+// through the kernels of mapfilter.cuh instead of k_fused_means, and launch k_tail_nn<false>, without the sweep's bookkeeping.
 // The chain keeps its own inputs clean for the next sweep (statistics, counts, far bits are zeroed by the kernel that
 // consumes them last): a sweep needs no memset.
 #pragma once
 #include "common.cuh"
 #include "assoc.cuh"
 #include "fastgrid.cuh"
-#include "mapfilter.cuh"
 #include "p2p.cuh"
 
 struct __align__(16) FarRec {
@@ -365,13 +366,14 @@ k_fused_means(const DevState* st, long long* fsum_x, long long* fsum_y, const in
 }
 
 // kept landmarks -> dense (kx, ky, kc), union-find parents, bounding box (ordered-key atomics, one set per block).  The position
-// of a kept landmark = kept landmarks of the blocks before this one (blk_kept, from k_fused_means' grid of the same shape) +
-// those before it in the block.  Clears the observation counts for the next sweep.
+// of a kept landmark = kept landmarks of the blocks before this one (blk_kept, from the entry kernel's grid of the same shape) +
+// those before it in the block.  The counts are the observation counts cnt, moved to rawcnt and cleared for the next sweep; or,
+// given cnt_d (icmslam_filter_map: a caller's counts, unrounded), cnt_d, with cnt and rawcnt left as they are.
 __global__ void __launch_bounds__(256)
 k_tail_compact(DevState* st, const int* __restrict__ flag, const int* __restrict__ blk_kept, int* __restrict__ pos,
                const double* __restrict__ raw_x, const double* __restrict__ raw_y, int* __restrict__ cnt, double* __restrict__ kx,
                double* __restrict__ ky, double* __restrict__ kc, int* __restrict__ parent, unsigned long long* bb, int Lcap,
-               int* __restrict__ klab, int* __restrict__ rawcnt, const TailState* ts)
+               int* __restrict__ klab, int* __restrict__ rawcnt, const TailState* ts, const double* __restrict__ cnt_d)
 {
     if (ts->steady_ok) return;
     __shared__ int wpart[8], wcnt[8];
@@ -390,18 +392,24 @@ k_tail_compact(DevState* st, const int* __restrict__ flag, const int* __restrict
     double mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
     if (l < Lcap) {
         pos[l] = p;
-        const int k = cnt[l];
-        rawcnt[l] = k;
+        double c;
+        if (cnt_d) {
+            c = cnt_d[l];
+        } else {
+            const int k = cnt[l];
+            rawcnt[l] = k;
+            cnt[l] = 0;
+            if (l == Lcap - 1) cnt[Lcap] = 0;
+            c = (double)k;
+        }
         if (f) {
             const double x = raw_x[l], y = raw_y[l];
-            kx[p] = x; ky[p] = y; kc[p] = (double)k;
+            kx[p] = x; ky[p] = y; kc[p] = c;
             parent[p] = p;
             klab[p] = l;
             mnx = mxx = x; mny = mxy = y;
         }
-        cnt[l] = 0;
         if (l == Lcap - 1) {
-            cnt[Lcap] = 0;
             st->kept = p + f;
             st->n_ind = 0;
             if (p + f == 0) st->status |= 4;   // ValueError in the reference (ICM_SLAM.py:241-255)
@@ -546,7 +554,9 @@ __device__ void tail_slow_body(DevState* st, TailState* ts, double dist_thr, dou
 // radius r (<= half the distance to any other old landmark: |new - other| >= 2 r - d > d).
 // The survivors are written as the new map (count-weighted mean of one member, :258-260) on the assumption that nothing
 // merges; the last block to finish knows whether that held (n_ind == 0 and the map is not degenerate), closes the sweep's
-// bookkeeping and, if it did not, runs the reference's sequential relabelling over what the other blocks left.
+// bookkeeping (FUSED: the instance the fused sweep launches; the other callers of the filter have no sweep in flight to close)
+// and, if it did not, runs the reference's sequential relabelling over what the other blocks left.
+template <bool FUSED>
 __global__ void __launch_bounds__(256)
 k_tail_nn(DevState* st, TailState* ts, double* __restrict__ kx, double* __restrict__ ky, double* __restrict__ kc, const FGeom* geom,
           const int* cell_start, const double2* pts, const int* idx, double thr2_lt, int* nn, int* ind_flag, int Lcap,
@@ -654,19 +664,22 @@ k_tail_nn(DevState* st, TailState* ts, double* __restrict__ kx, double* __restri
         if (last) {      // every other block's results are in global memory
             __threadfence();
             ts->nn_ticket = 0;
-            ts->far_count = 0; ts->n_dirty = 0;      // (consumed by k_tail_labels / the association kernel: ready for the next sweep)
-            ts->p2p_seq += 1u;
-            ts->sweep_no += 1u;
             const int n_ind = atomicAdd(&ts->n_ind, 0);
             slow = (n_ind != 0 || ts->degenerate) ? 1 : 0;
-            // every old label survived in place (its position among the kept landmarks is its index) and nothing was added
-            const int ls = st->lsearch, e = max(ls - 1, 0);
-            const int identity = (!slow && ls > 0 && K == ls && kflag[e] && kpos[e] == e) ? 1 : 0;
-            // run records (runs.cuh) name landmarks by index: void every one of them when landmark indices changed
-            if (!identity) ts->epoch += 1;
-            if (!slow) { st->new_l = K; st->lact = K; st->n_ind = 0; ts->remap_identity = identity; }
-            ts->steady_armed = (!slow && sa.steady_enable) ? 1 : 0;      // (a merged map is rebuilt by one block without the steady tail's inputs)
-            ts->steady_K = K;
+            if (!slow) { st->new_l = K; st->lact = K; st->n_ind = 0; }
+            if (FUSED) {
+                ts->far_count = 0; ts->n_dirty = 0;      // (consumed by k_tail_labels / the association kernel: ready for the next sweep)
+                ts->p2p_seq += 1u;
+                ts->sweep_no += 1u;
+                // every old label survived in place (its position among the kept landmarks is its index) and nothing was added
+                const int ls = st->lsearch, e = max(ls - 1, 0);
+                const int identity = (!slow && ls > 0 && K == ls && kflag[e] && kpos[e] == e) ? 1 : 0;
+                // run records (runs.cuh) name landmarks by index: void every one of them when landmark indices changed
+                if (!identity) ts->epoch += 1;
+                ts->remap_identity = identity;
+                ts->steady_armed = (!slow && sa.steady_enable) ? 1 : 0;      // (a merged map is rebuilt by one block without the steady tail's inputs)
+                ts->steady_K = K;
+            }
         }
         s_last = last; s_slow = slow;
     }
@@ -869,6 +882,12 @@ k_lmrec_build(const double* __restrict__ mx, const double* __restrict__ my, cons
 }
 
 // ---- the merge path: one block ------------------------------------------------------------------------
+__device__ __forceinline__ int uf_find(const int* parent, int v)
+{
+    while (parent[v] != v) v = parent[v];
+    return v;
+}
+
 // block-wide exclusive scan of v[0..n) (global memory) into out[0..n); returns the total to all threads
 __device__ int block_exclusive_scan(const int* v, int* out, int n, int* wsum /* >= 33 ints of shared memory */)
 {
@@ -977,7 +996,7 @@ __device__ void tail_slow_body(DevState* st, TailState* ts, double dist_thr, dou
         for (int j = tid; j < K; j += nth)
             if (fz.landmark(kx[j], ky[j])) { const int r = rank[lab[j]]; if (r < cap_out) { map_out[r] = kx[j]; map_out[ld_out + r] = ky[j]; } }
     }
-    if (tid == 0) { st->new_l = newL; st->lact = newL; st->n_ind = n_ind; ts->remap_identity = 0; st->cambio_unres += 1; }   // (merged map: calc_cambio needs the full search)
+    if (tid == 0) { st->new_l = newL; st->lact = newL; st->n_ind = n_ind; st->cambio_unres += 1; }   // (merged map: calc_cambio needs the full search)
     __syncthreads();
     // ---- rebuild the landmark grid over the merged map (it is the next sweep's association grid) -------------
     {

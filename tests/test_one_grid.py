@@ -1,6 +1,6 @@
 """The landmark grid outside the fused sweep (the generic sweep's association, Mapa.filtrar's neighbour search, calc_cambio)
-on maps large enough for the grid paths to run, against the CPU oracle or a numpy brute force.  And calc_cambio between two
-fused sweeps leaves the fused chain as it was."""
+on large maps, against the CPU oracle or a numpy brute force.  And calc_cambio between two fused sweeps, and the callers of the
+filter chain other than the fused sweep, leave the fused chain as it was."""
 import numpy as np
 import pytest
 
@@ -10,7 +10,7 @@ pytestmark = pytest.mark.gpu
 
 TOL_XY = 1e-6
 TOL_TH = 1e-8
-FILTER_SMALL_K = 2048       # (mapfilter.cuh) above this many survivors Mapa.filtrar searches the grid
+LARGE_K = 2048              # survivors of the large maps below (the golden fixtures' raw maps have at most 200 landmarks)
 
 
 def _cfg(**kw):
@@ -60,7 +60,7 @@ def test_generic_sweeps_with_a_large_map_vs_oracle(view):
         r = orc.sweep(ocfg, mo, ext, odo, u, odo[:, 0], map_o, xo, "redblack", "newton", view)
         st, Lout, mout = e.sweep(map_g, xg, odo[:, 0], schedule="redblack", solver="newton", view=view, fused=False,
                                  newton_tol=1e-12, newton_maxit=50)
-        assert e.sweep_stats()["kept"] > FILTER_SMALL_K
+        assert e.sweep_stats()["kept"] > LARGE_K
         assert np.array_equal(e.associations(), r["c"])
         assert Lout == r["map"].shape[1]
         dd = np.abs(xg - xo)
@@ -72,8 +72,10 @@ def test_generic_sweeps_with_a_large_map_vs_oracle(view):
 
 
 def test_filter_map_with_merges_vs_oracle():
-    """Mapa.filtrar on 3000 landmarks with planted close pairs, chains and exact ties: the grid branch merges what the
-    reference's K x K search merges."""
+    """Mapa.filtrar with merges, as the reference's K x K search does it: 3070 landmarks with planted close pairs, chains and
+    exact ties (the grid search), and a map whose extent is below dist_thr but whose diameter is not, with coincident
+    landmarks (the brute force of a degenerate map: a zero distance is replaced by the diameter, so a coincident pair with no
+    other landmark within dist_thr stays two landmarks)."""
     from oracle import oracle as orc
     rng = np.random.default_rng(20181 + 32)
     G = 50
@@ -86,24 +88,31 @@ def test_filter_map_with_merges_vs_oracle():
     chain = close[:, :50] + np.array([[0.6], [0.0]])                   # chains of three
     tie = base[:, pick[50:60]] + np.array([[0.0], [0.5]])
     tie2 = base[:, pick[50:60]] + np.array([[0.0], [-0.5]])            # equidistant pairs around the same landmark
-    mapa = np.ascontiguousarray(np.concatenate([base, close, chain, tie, tie2], axis=1)[:, rng.permutation(3070)])
-    counts = rng.integers(1, 60, mapa.shape[1]).astype(np.float64)
+    large = np.ascontiguousarray(np.concatenate([base, close, chain, tie, tie2], axis=1)[:, rng.permutation(3070)])
+    large_counts = rng.integers(1, 60, large.shape[1]).astype(np.float64)
+    assert int((large_counts >= 10.0).sum()) > LARGE_K
+    far = 5.75 + rng.uniform(0.0, 0.15, (2, 20))
+    small = np.concatenate([np.full((2, 2), 5.0), far, far[:, :3], np.full((2, 1), 5.9)], axis=1)
+    small_counts = rng.integers(1, 60, small.shape[1]).astype(np.float64)
+    small_counts[:2] = (20.0, 30.0)
+    assert np.ptp(small, axis=1).max() < 1.0 <= np.hypot(0.9, 0.9)
     cfgd = dict(CONFIG_ROS, L=4096, cota=10.0)
     e = _engine_plain(cfgd)
-    out, cnt, Lout = e.filter_map(mapa, counts)
-    assert int((counts >= 10.0).sum()) > FILTER_SMALL_K
-    mo = orc.Mapa(orc.make_cfg(**cfgd))
-    mo.landmarks_actuales = mapa.shape[1]
-    mo.cant_obs_i[:] = 0.0
-    mo.cant_obs_i[: mapa.shape[1]] = counts
-    full = np.zeros((2, 4096))              # (the oracle's map has L columns)
-    full[:, : mapa.shape[1]] = mapa
-    ref = mo.filtrar(full)
-    Lref = mo.landmarks_actuales
-    assert Lref < int((counts >= 10.0).sum())         # merges happened
-    assert Lout == Lref
-    assert np.array_equal(cnt[:Lout], mo.cant_obs_i[:Lref])
-    assert np.max(np.abs(out[:, :Lout] - ref[:, :Lref])) <= 1e-12
+    for mapa, counts in ((large, large_counts), (small, small_counts)):
+        out, cnt, Lout = e.filter_map(mapa, counts)
+        mo = orc.Mapa(orc.make_cfg(**cfgd))
+        mo.landmarks_actuales = mapa.shape[1]
+        mo.cant_obs_i[:] = 0.0
+        mo.cant_obs_i[: mapa.shape[1]] = counts
+        full = np.zeros((2, 4096))              # (the oracle's map has L columns)
+        full[:, : mapa.shape[1]] = mapa
+        ref = mo.filtrar(full)
+        Lref = mo.landmarks_actuales
+        assert Lref < int((counts >= 10.0).sum())         # merges happened
+        assert Lout == Lref
+        assert np.array_equal(cnt[:Lout], mo.cant_obs_i[:Lref])
+        assert np.max(np.abs(out[:, :Lout] - ref[:, :Lref])) <= 1e-12
+    assert Lout > 2 and np.array_equal(out[:, :2], np.full((2, 2), 5.0))      # (the coincident pair)
     e.close()
 
 
@@ -159,3 +168,30 @@ def test_calc_cambio_between_fused_sweeps_leaves_the_chain():
     (n_a, map_a, x_a, ep_a), (n_b, map_b, x_b, ep_b) = res
     assert n_a == n_b and ep_a == ep_b
     assert np.array_equal(map_a, map_b) and np.array_equal(x_a, x_b)
+
+
+def test_filter_callers_leave_the_fused_sweep_counters():
+    """Pass 0, Mapa.filtrar and a generic sweep run the fused tail's filter chain without closing a fused sweep: the sweep and
+    peer-memory sequence numbers and the label-numbering epoch stay as the last fused sweep left them."""
+    import ctypes as C
+    from helpers import c1_inputs, golden
+    g = golden("c1_ref.npz")
+    z, odo, u = c1_inputs()
+    e = _engine(_cfg(), z, odo, u)
+    e.set_map(g["p0_map"]); e.set_poses(g["p0_x"])
+    e.iterate(None, odo[:, 0], 2)
+
+    def counters():
+        trace, cn = (C.c_uint64 * 256)(), (C.c_uint32 * 3)()
+        assert e.lib.icmslam_get_trace(e._h, trace, cn) == 0
+        return list(cn), e.sweep_stats()["epoch"]
+
+    before = counters()
+    assert before[0][0] >= 2
+    e.pass0(odo[:, 0])
+    e.filter_map(g["p0_map"], np.full(g["p0_map"].shape[1], 400.0))
+    e.landmarks_actuales = g["p0_map"].shape[1]
+    x = np.ascontiguousarray(g["p0_x"].copy())
+    e.sweep(g["p0_map"].copy(), x, odo[:, 0], fused=False)
+    assert counters() == before
+    e.close()
