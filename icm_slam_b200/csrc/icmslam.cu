@@ -905,7 +905,10 @@ static void launch_runs(int blocks, cudaStream_t s, const RunParams& R)
 
 static void launch_solve(int blocks, cudaStream_t s, const SolveParams& P)
 {
-    if (P.fz.frozen) k_solve_tile<true><<<blocks, ST_THREADS, 0, s>>>(P);
+    if (P.lay.traj_T & 1) {      // a batch of odd-length trajectories: colours by trajectory-local time
+        if (P.fz.frozen) k_solve_tile<true, true><<<blocks, ST_THREADS, 0, s>>>(P);
+        else k_solve_tile<false, true><<<blocks, ST_THREADS, 0, s>>>(P);
+    } else if (P.fz.frozen) k_solve_tile<true><<<blocks, ST_THREADS, 0, s>>>(P);
     else k_solve_tile<false><<<blocks, ST_THREADS, 0, s>>>(P);
 }
 

@@ -9,7 +9,7 @@
 // their odometry increments, controls and heading sin/cos in shared memory.  Thread q (a slot) solves the whole odd pose
 // tb-1+2q (q = 0: the halo tb-1, owned by the previous tile, which computes the identical value from the identical inputs),
 // then, after a block barrier, the even pose tb+2q from the new odd poses in shared memory: every warp works in both colour
-// phases.  Every input is read once; the new poses and their projection parameters (x, y, sin/cos of theta - pi/2: what
+// phases.  In a batch of odd-length trajectories the colours follow each trajectory's local time (solve_slot_load).  Every input is read once; the new poses and their projection parameters (x, y, sin/cos of theta - pi/2: what
 // tras_rot_z needs next sweep, ICM_SLAM.py:465-480) are written coalesced.
 #pragma once
 #include "common.cuh"
@@ -228,15 +228,29 @@ struct SlotMom {
     int t, li;
 };
 
-template <bool FZ>
+// LOCAL: a batch of trajectories of odd length (p.lay.traj_T odd), coloured by trajectory-local time t - k traj_T like
+// k_pose_colour.  Trajectory k starts on column k traj_T, whose parity is k's: in an odd-numbered trajectory the slot's pair
+// (tb-1+2q, tb+2q) swaps roles -- phase 0 solves the local-odd tb+2q, phase 1 the local-even tb-1+2q -- and the re-solved halo
+// is tb+ST_OWN right of the tile instead of tb-1 (its neighbour tb+ST_OWN+1 is staged).  The roles go by the trajectory of
+// tb-1+2q: where the pair spans a boundary, tb+2q is the next trajectory's pinned first pose and phase 0 passes it through.
+template <bool FZ, bool LOCAL>
 __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb, int q, int phase)
 {
     SlotMom s;
-    s.t = phase == 0 ? tb - 1 + 2 * q : tb + 2 * q;
-    s.li = s.t - (tb - 2);
-    // (phase 0, slot 0 = the odd pose tb-1 left of the tile: re-solved here because the even pose tb needs its NEW value;
-    //  phase 1, last slot = tb+ST_OWN: the next tile's)
-    s.valid = s.t >= 0 && s.t < p.t_hi && (phase == 0 ? (q == 0 || s.t >= p.t_lo) : (q != ST_SLOTS - 1 && s.t >= p.t_lo));
+    if (LOCAL) {
+        const int a = tb - 1 + 2 * q;
+        const bool swap = a >= 0 && ((a / p.lay.traj_T) & 1);
+        s.t = (phase == 0) != swap ? a : a + 1;
+        s.li = s.t - (tb - 2);
+        // (phase 0 also solves the halo next to the tile: tb-1 or tb+ST_OWN; phase 1 only the owned poses)
+        s.valid = s.t >= 0 && s.t < p.t_hi && (phase == 0 ? (q == 0 || s.t >= p.t_lo) : (s.t >= tb && s.t < tb + ST_OWN && s.t >= p.t_lo));
+    } else {
+        s.t = phase == 0 ? tb - 1 + 2 * q : tb + 2 * q;
+        s.li = s.t - (tb - 2);
+        // (phase 0, slot 0 = the odd pose tb-1 left of the tile: re-solved here because the even pose tb needs its NEW value;
+        //  phase 1, last slot = tb+ST_OWN: the next tile's)
+        s.valid = s.t >= 0 && s.t < p.t_hi && (phase == 0 ? (q == 0 || s.t >= p.t_lo) : (q != ST_SLOTS - 1 && s.t >= p.t_lo));
+    }
     // (a frozen pose is handled like a pinned one: its input value passes through; the trajectory's first pose is pinned and its
     //  last has no successor, so no pose of another trajectory reads it)
     s.pinned = s.valid && (p.lay.pinned(s.t) || (FZ && p.fz.scan(s.t)));
@@ -255,8 +269,9 @@ __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb,
     return s;
 }
 
-// FZ: a batch with frozen trajectories (p.fz); the plain sweep launches the instance without the test
-template <bool FZ>
+// FZ: a batch with frozen trajectories (p.fz); the plain sweep launches the instance without the test.  LOCAL: a batch of
+// odd-length trajectories (solve_slot_load); every other handle launches the instance without it.
+template <bool FZ, bool LOCAL = false>
 __global__ void __launch_bounds__(ST_THREADS, ST_MINB)
 k_solve_tile(const SolveParams p)
 {
@@ -264,8 +279,9 @@ k_solve_tile(const SolveParams p)
     const int q = threadIdx.x;      // the slot
     if (p.trace_row && blockIdx.x == 0 && q == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); p.trace_row[((*p.trace_seq) & 31) * 8 + 5] = t; }
     const int tb = p.t_lo + (p.tile0 + blockIdx.x) * ST_OWN;      // t_lo is even: colours stay aligned with the global time index
+                                                                  // (LOCAL: with each trajectory's local time, solve_slot_load)
     const int T = p.T;
-    SlotMom cur = solve_slot_load<FZ>(p, tb, q, 0);      // (in flight while the tile is staged)
+    SlotMom cur = solve_slot_load<FZ, LOCAL>(p, tb, q, 0);      // (in flight while the tile is staged)
     for (int li = q; li < ST_XT; li += ST_THREADS) {
         const int t = tb - 2 + li;
         const bool ok = t >= 0 && t < T;
@@ -330,7 +346,7 @@ k_solve_tile(const SolveParams p)
             if (solve) { rx = x2; ry = y2; th = th2; my_iters += it; }
         }
         SlotMom nxt = cur;
-        if (phase == 0) nxt = solve_slot_load<FZ>(p, tb, q, 1);      // (the even pose's moments arrive during the barrier)
+        if (phase == 0) nxt = solve_slot_load<FZ, LOCAL>(p, tb, q, 1);      // (the even pose's moments arrive during the barrier)
         if (qvalid && !pinned) {
             // the new heading's sin/cos exactly as next sweep's projection forms them (one sincos per pose per sweep)
             double st, ct;

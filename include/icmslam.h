@@ -155,7 +155,10 @@ int icmslam_get_poses(icmslam_handle* h, double* x, int64_t ld_x, int32_t memspa
  * any gate (icm_slam_b200/batch.py does both); x0s (HOST, 3 x K) are their pinned first poses.  Every trajectory's first pose is
  * then pinned to its own x0, its last pose has no successor, and one sweep of the handle is one sweep of every trajectory: ONE
  * launch of each kernel for the whole batch.  Every sweep mode is valid on a batch handle (icmslam_iterate and icmslam_sweep; the
- * SEQUENTIAL schedule walks each trajectory with its own warp); new labels are numbered over the whole batch and the label cap L
+ * SEQUENTIAL schedule walks each trajectory with its own warp), at any traj_T >= 3: the REDBLACK schedule, fused or not, colours
+ * pose t of trajectory k by the parity of t - k * traj_T, so an odd traj_T sweeps each trajectory as it is swept alone.  Refused:
+ * traj_T < 3 or traj_T * K != T (ICMSLAM_ERR_INVALID), a trajectory whose first or last scan is empty
+ * (ICMSLAM_ERR_UNSUPPORTED); a refused call leaves the handle as it was.  New labels are numbered over the whole batch and the label cap L
  * applies to the batch.  The x0 argument of icmslam_iterate / icmslam_sweep is ignored.  traj_T <= 0 switches back to a single
  * trajectory. */
 int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double* x0s, int64_t ld_x0s, int32_t K);
