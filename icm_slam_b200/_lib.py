@@ -95,6 +95,7 @@ def lib():
     L.icmslam_get_poses.argtypes = [vp, vp, i64, i32]
     L.icmslam_set_segment.argtypes = [vp, i32, i32, i32, i32]
     L.icmslam_set_batch.argtypes = [vp, i32, vp, i64, i32]
+    L.icmslam_set_batch_lengths.argtypes = [vp, vp, i32, vp, i64]
     L.icmslam_device_ptr.argtypes = [vp, i32, C.POINTER(vp), C.POINTER(i64)]
     L.icmslam_seg_begin.argtypes = [vp, vp, C.POINTER(SweepOpts)]
     L.icmslam_seg_exchange.argtypes = [vp, vp, i32, i32]
@@ -135,7 +136,7 @@ EXPORTS = [
     "icmslam_calc_cambio", "icmslam_filtrar_obs", "icmslam_set_map", "icmslam_get_map", "icmslam_iterate",
     "icmslam_get_kernel_ms", "icmslam_get_launch_count", "icmslam_get_transfer_bytes", "icmslam_set_poses", "icmslam_get_poses", "icmslam_set_segment", "icmslam_device_ptr", "icmslam_seg_begin",
     "icmslam_seg_exchange", "icmslam_seg_halo", "icmslam_p2p_export", "icmslam_p2p_import", "icmslam_get_trace", "icmslam_pose_eval", "icmslam_seg_finish", "icmslam_fcluster", "icmslam_pass0", "icmslam_associate", "icmslam_iterate_until", "icmslam_set_counts", "icmslam_set_batch",
-    "icmslam_batch_iterate_until",
+    "icmslam_batch_iterate_until", "icmslam_set_batch_lengths",
 ]
 
 

@@ -20,8 +20,9 @@ as it would be swept alone, so the reference's own sweep runs a whole batch in o
 
     batch.iterate(30, schedule="sequential", solver="nm", view="running")      # the reference's ICM, one warp per trajectory
 
-A ConcatBatch numbers new labels over the whole batch (each trajectory's labels keep their order) and its label cap applies to the
-batch; iterate_until runs the default mode only.
+The trajectories of a ConcatBatch may have any lengths >= 3 (icmslam_set_batch_lengths).  It holds at most 4096 trajectories,
+numbers new labels over the whole batch (each trajectory's labels keep their order) and its label cap applies to the batch;
+iterate_until runs the default mode only.
 """
 from __future__ import annotations
 
@@ -83,11 +84,12 @@ class TrajectoryBatch:
 
 
 class ConcatBatch:
-    """The batch as ONE handle (icmslam_set_batch): the K owned trajectories (equal length) laid end to end and translated to
-    disjoint regions of the plane -- their landmarks are farther apart than any gate, and the energy only sees differences of
-    positions, so every trajectory is solved exactly as it would be alone -- with each trajectory's first pose pinned to its own x0.
-    One sweep of the batch = one launch of each kernel over all K x T columns (TrajectoryBatch, one handle per trajectory, needs
-    K x 15 small launches and is launch-bound).
+    """The batch as ONE handle (icmslam_set_batch_lengths): the K owned trajectories (any lengths >= 3, at most 4096 of them) laid
+    end to end and translated to disjoint regions of the plane -- their landmarks are farther apart than any gate, and the energy
+    only sees differences of positions, so every trajectory is solved exactly as it would be alone -- with each trajectory's first
+    pose pinned to its own x0.
+    One sweep of the batch = one launch of each kernel over all columns of all K trajectories (TrajectoryBatch, one handle per
+    trajectory, needs K x 15 small launches and is launch-bound).
 
         b = ConcatBatch(config_for_one_trajectory, rank, world)
         b.add(i, z_i, odo_i, u_i, map_i, x_i) ...; b.finalize(); b.iterate(30); res = b.results()
@@ -123,31 +125,31 @@ class ConcatBatch:
         K = len(self._items)
         if K == 0:
             raise ValueError("empty batch")
-        Tk = self._items[0][1].shape[1]
-        if any(it[1].shape[1] != Tk for it in self._items):
-            raise ValueError("the trajectories of a ConcatBatch have the same length")
+        lengths = np.array([it[1].shape[1] for it in self._items], np.int64)
+        if lengths.min() < 3:
+            raise ValueError("every trajectory of a ConcatBatch has at least 3 scans")
         if K > 64 * 64:
             raise ValueError("at most 4096 trajectories per handle")
         z = np.concatenate([it[1] for it in self._items], axis=1)
         odo = np.concatenate([it[2] for it in self._items], axis=1)
         u = np.concatenate([it[3] for it in self._items], axis=1)
         x = np.concatenate([it[5] for it in self._items], axis=1)
-        maps, self._nl = [], []
+        starts = np.concatenate([[0], np.cumsum(lengths)])
+        maps = []
         for k, it in enumerate(self._items):
             off = self._offset(k)
-            odo[0:2, k * Tk:(k + 1) * Tk] += off[:, None]
-            x[0:2, k * Tk:(k + 1) * Tk] += off[:, None]
+            odo[0:2, starts[k]:starts[k + 1]] += off[:, None]
+            x[0:2, starts[k]:starts[k + 1]] += off[:, None]
             maps.append(it[4] + off[:, None])
-            self._nl.append(it[4].shape[1])
         mapa = np.concatenate(maps, axis=1)
         cfg = copy(self.config)
         cfg.L = max(int(self.Lper) * K, mapa.shape[1] + K)
-        self.K, self.Tk = K, Tk
+        self.K, self.starts = K, starts      # trajectory k covers columns starts[k] .. starts[k+1]-1
         e = Engine(cfg, device=self.device)
         e.load(z, odo, u, precondition=precondition)
         e.extract()
-        self.x0s = np.ascontiguousarray(np.stack([odo[:, k * Tk] for k in range(K)], axis=1))
-        e.set_batch(Tk, self.x0s)
+        self.x0s = np.ascontiguousarray(odo[:, starts[:-1]])
+        e.set_batch_lengths(lengths, self.x0s)
         e.set_map(mapa)
         e.set_poses(np.ascontiguousarray(x))
         self.engine = e
@@ -175,7 +177,7 @@ class ConcatBatch:
         out = {}
         for k, it in enumerate(self._items):
             off = self._offset(k)
-            xs = x[:, k * self.Tk:(k + 1) * self.Tk].copy()
+            xs = x[:, self.starts[k]:self.starts[k + 1]].copy()
             xs[0:2] -= off[:, None]
             out[it[0]] = (xs, mapa[:, kk == k] - off[:, None])
         return out

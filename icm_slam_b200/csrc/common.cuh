@@ -24,7 +24,7 @@ struct DevCfg {
 #define FZ_SLOTS 5     // per-trajectory results of a sweep: min, max, sum of the resolved changes, new landmarks, unresolved ones
 struct Freeze {
     const unsigned char* frozen;   // K bytes: trajectory k is frozen
-    int traj_T;                    // columns per trajectory: scan t belongs to trajectory t / traj_T
+    const int* traj;               // trajectory of each column (TrajLayout::traj)
     int K, cols;
     double pitch;
     double* slots;                 // FZ_SLOTS x K (row r, trajectory k): calc_cambio of each trajectory's landmarks
@@ -33,7 +33,7 @@ struct Freeze {
         const double k = rint(y / pitch) * (double)cols + rint(x / pitch);
         return (k >= 0.0 && k < (double)K) ? (int)k : -1;
     }
-    __device__ __forceinline__ bool scan(int t) const { return frozen != nullptr && frozen[t / traj_T] != 0; }
+    __device__ __forceinline__ bool scan(int t) const { return frozen != nullptr && frozen[__ldg(traj + t)] != 0; }
     __device__ __forceinline__ bool landmark(double x, double y) const
     {
         if (frozen == nullptr) return false;
@@ -51,19 +51,24 @@ struct Freeze {
 };
 
 // Which columns are pinned first poses (sensors.py:131: x[:,0] is never updated, scan 0 is projected with self.x0): column 0
-// of the trajectory's first segment, or -- a batch of independent trajectories of traj_T columns each laid end to end in one
-// handle (BASELINE configs[4]) -- the first column of every trajectory, each with its own x0.  A trajectory's last pose has no
-// successor.  The fused solve and the generic kernels both go by these rules.
+// of the trajectory's first segment, or -- a batch of K independent trajectories of any lengths laid end to end in one handle
+// (BASELINE configs[4]) -- the first column of every trajectory, each with its own x0.  Trajectory k covers columns
+// start[k] .. start[k+1]-1; traj[t] is the trajectory of column t.  A trajectory's last pose has no successor.  The fused solve
+// and the generic kernels both go by these rules.
 struct TrajLayout {
     int first;                 // column 0 is the trajectory's first pose
-    int traj_T;                // > 0: batch of trajectories of this many columns
+    int K;                     // > 0: batch of K trajectories
+    const int* start;          // batch: K + 1 column starts (start[K] = T)
+    const int* traj;           // batch: T trajectory indices
     const double* x0s;         // batch: 3 x K first poses (row-major, leading dimension ldx0s)
     int64_t ldx0s;
     double x0[3];              // single trajectory: self.x0
-    __device__ __forceinline__ bool pinned(int t) const { return traj_T > 0 ? (t % traj_T) == 0 : (t == 0 && first); }
-    __device__ __forceinline__ bool after_pinned(int t) const { return traj_T > 0 ? (t % traj_T) == 1 : (t == 1 && first); }
-    __device__ __forceinline__ bool has_next(int t, int T) const { return t + 1 < T && (traj_T == 0 || ((t + 1) % traj_T) != 0); }
-    __device__ __forceinline__ double x0_of(int t, int r) const { return traj_T > 0 ? x0s[r * ldx0s + t / traj_T] : x0[r]; }
+    __device__ __forceinline__ int traj_of(int t) const { return __ldg(traj + t); }
+    __device__ __forceinline__ int begin(int t) const { return __ldg(start + traj_of(t)); }   // (batch) first column of t's trajectory
+    __device__ __forceinline__ bool pinned(int t) const { return K > 0 ? t == begin(t) : (t == 0 && first); }
+    __device__ __forceinline__ bool after_pinned(int t) const { return K > 0 ? t - begin(t) == 1 : (t == 1 && first); }
+    __device__ __forceinline__ bool has_next(int t, int T) const { return t + 1 < T && (K == 0 || t + 1 < __ldg(start + traj_of(t) + 1)); }
+    __device__ __forceinline__ double x0_of(int t, int r) const { return K > 0 ? x0s[r * ldx0s + traj_of(t)] : x0[r]; }
     // the pose scan t is projected with (sensors.py:141,153): its trajectory's x0 for a pinned column, else x[:, t]
     __device__ __forceinline__ void scan_pose(const double* x, int64_t ldx, int t, double& px, double& py, double& th) const
     {

@@ -5,6 +5,7 @@
 
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <new>
 #include <utility>
@@ -163,7 +164,9 @@ struct icmslam_handle {
     DevBuf<unsigned long long> d_scan_state;   // block totals of k_cell_scan
     DevBuf<int> d_remap;                // label of the last sweep -> label in the current map
     DevBuf<int> d_klab;                 // raw label of each kept landmark (fast tail)
-    int traj_T = 0, traj_K = 0; DevBuf<double> d_x0s;   // batch of independent trajectories laid end to end (icmslam_set_batch)
+    // batch of independent trajectories laid end to end (icmslam_set_batch / icmslam_set_batch_lengths): K + 1 column starts,
+    // the trajectory of each column, 3 x K first poses; traj_odd: some trajectory starts on an odd column
+    int traj_K = 0; bool traj_odd = false; DevBuf<int> d_traj_start, d_traj_of; DevBuf<double> d_x0s;
     // per-trajectory freezing (icmslam_batch_iterate_until): fz.frozen is null outside that call
     Freeze fz = {};
     DevBuf<unsigned char> d_fz_mask, d_fz_need; DevBuf<double> d_fz_slots; DevBuf<int> d_fz_reg; int fz_K = 0;
@@ -288,7 +291,7 @@ extern "C" const char* icmslam_last_error(const icmslam_handle* h) { return h ? 
 // (a captured sweep holds the freeze arguments it was captured with)
 static bool same_freeze(const Freeze& a, const Freeze& b)
 {
-    return a.frozen == b.frozen && a.traj_T == b.traj_T && a.K == b.K && a.cols == b.cols && a.pitch == b.pitch && a.slots == b.slots;
+    return a.frozen == b.frozen && a.traj == b.traj && a.K == b.K && a.cols == b.cols && a.pitch == b.pitch && a.slots == b.slots;
 }
 
 static void drop_graphs(icmslam_handle* h)
@@ -313,8 +316,8 @@ static void free_dataset(icmslam_handle* h)
     reset_extraction(h);
     h->ds = icmslam_handle::Dataset();
     h->last_map_L = -1;
-    h->traj_T = 0; h->traj_K = 0;
-    h->d_x0s.reset();
+    h->traj_K = 0; h->traj_odd = false;
+    h->d_traj_start.reset(); h->d_traj_of.reset(); h->d_x0s.reset();
     h->d_fz_mask.reset(); h->d_fz_need.reset(); h->d_fz_slots.reset(); h->d_fz_reg.reset(); h->fz_K = 0;
     h->n = 0;
 }
@@ -860,7 +863,7 @@ __global__ void k_note_dirty(DevState* st, const TailState* ts) { st->dirty_tile
 static TrajLayout traj_layout(const icmslam_handle* h, const double* x0)
 {
     TrajLayout L;
-    L.first = h->seg_first; L.traj_T = h->traj_T; L.x0s = h->d_x0s; L.ldx0s = h->traj_K;
+    L.first = h->seg_first; L.K = h->traj_K; L.start = h->d_traj_start; L.traj = h->d_traj_of; L.x0s = h->d_x0s; L.ldx0s = h->traj_K;
     L.x0[0] = x0[0]; L.x0[1] = x0[1]; L.x0[2] = x0[2];
     return L;
 }
@@ -903,9 +906,9 @@ static void launch_runs(int blocks, cudaStream_t s, const RunParams& R)
     else k_runs<false><<<blocks, RUNS_THREADS, 0, s>>>(R);
 }
 
-static void launch_solve(int blocks, cudaStream_t s, const SolveParams& P)
+static void launch_solve(const icmslam_handle* h, int blocks, cudaStream_t s, const SolveParams& P)
 {
-    if (P.lay.traj_T & 1) {      // a batch of odd-length trajectories: colours by trajectory-local time
+    if (h->traj_odd) {      // a batch with a trajectory that starts on an odd column: colours by trajectory-local time
         if (P.fz.frozen) k_solve_tile<true, true><<<blocks, ST_THREADS, 0, s>>>(P);
         else k_solve_tile<false, true><<<blocks, ST_THREADS, 0, s>>>(P);
     } else if (P.fz.frozen) k_solve_tile<true><<<blocks, ST_THREADS, 0, s>>>(P);
@@ -999,7 +1002,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
             if (ready > h->n_solve_tiles) ready = h->n_solve_tiles;
             if (ready > solved) {
                 P.tile0 = solved;
-                launch_solve(ready - solved, s, P);
+                launch_solve(h, ready - solved, s, P);
                 CK(cudaGetLastError());
                 h->n_launch += 1;
                 CK(cudaEventRecord(h->ev_out[c], s));
@@ -1035,7 +1038,7 @@ static int fused_part_a(icmslam_handle* h, const double* xin, int64_t ldin, doub
         CK(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
         ss = h->side_stream;
     }
-    launch_solve(h->n_solve_tiles, ss, P);
+    launch_solve(h, h->n_solve_tiles, ss, P);
     CK(cudaGetLastError());
     if (h->d2h_x) {      // a host-memory caller: its poses start their way back as soon as they are solved, beside the tail
         CK(cudaMemcpy2DAsync(h->d2h_x, (size_t)h->d2h_ld * 8, kout, (size_t)kld * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, ss));
@@ -1250,7 +1253,6 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         // (the generic sweep covers the handle's whole trajectory, or the whole batch: column 0 is a first pose either way)
         TrajLayout lay = traj_layout(h, x0);
         lay.first = 1;
-        const int traj_K = h->traj_T > 0 ? h->traj_K : 1, traj_cols = h->traj_T > 0 ? h->traj_T : T;
         PoseArrays A;
         A.x = dx; A.ldx = ldx; A.odo = h->ds.d_odo; A.ldo = T; A.u = h->ds.d_u; A.ldu = T;
         A.lay = lay;
@@ -1310,14 +1312,13 @@ static int sweep_core(icmslam_handle* h, const double* xin, int64_t ldin, double
         S.lsearch_ptr = &st->lsearch;
         if (timing) CK(cudaEventRecord(h->ev[2], s));
         if (o.schedule == ICMSLAM_SCHED_REDBLACK) {
-            const int threads = traj_K * ((traj_cols + 1) / 2);
-            k_pose_colour<<<nblk(threads, 128), 128, 0, s>>>(1, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
+            k_pose_colour<<<nblk(T, 128), 128, 0, s>>>(1, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
             CK(cudaGetLastError());
-            k_pose_colour<<<nblk(threads, 128), 128, 0, s>>>(0, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
+            k_pose_colour<<<nblk(T, 128), 128, 0, s>>>(0, h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
             CK(cudaGetLastError());
             h->n_launch += 2;
         } else {
-            k_pose_walk<<<traj_K, WARP, 0, s>>>(h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
+            k_pose_walk<<<h->traj_K > 0 ? h->traj_K : 1, WARP, 0, s>>>(h->dcfg, A, O, S, o.solver, o.newton_tol, o.newton_maxit, iters);
             CK(cudaGetLastError());
             h->n_launch += 1;
         }
@@ -1579,28 +1580,68 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
 }
 
 // ---- a batch of independent trajectories in one handle (BASELINE configs[4]) ---------------------------------------------
-extern "C" int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double* x0s, int64_t ld_x0s, int32_t K)
+// Trajectory k covers columns start[k] .. start[k+1]-1 (start[0] = 0, start[K] = T).  The caller has checked the arguments; this
+// checks the scans and changes the handle only when it accepts the layout.
+static int set_layout(icmslam_handle* h, const std::vector<int>& start, const double* x0s, int64_t ld_x0s)
 {
-    if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
-    CK(cudaSetDevice(h->cfg.device));
-    if (traj_T <= 0) { drop_graphs(h); h->traj_T = 0; h->traj_K = 0; h->d_x0s.reset(); h->ch.ppar_of = nullptr; return ICMSLAM_OK; }
-    if (!x0s || K <= 0 || ld_x0s < K || (int64_t)traj_T * K != h->T || traj_T < 3 || !h->fused_ok) return ICMSLAM_ERR_INVALID;
+    const int K = (int)start.size() - 1;
     // every trajectory needs a non-empty first and last scan (the reference returns early / raises otherwise, sensors.py:137, :148)
     std::vector<int> off((size_t)h->T + 1);
     CK(cudaMemcpyAsync(off.data(), h->ex.d_off, ((size_t)h->T + 1) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
+    bool odd = false;
+    std::vector<int> traj((size_t)h->T);
     for (int k = 0; k < K; ++k) {
-        const int a = k * traj_T, b = (k + 1) * traj_T - 1;
+        const int a = start[k], b = start[k + 1] - 1;
         if (off[a + 1] == off[a] || off[b + 1] == off[b]) return ICMSLAM_ERR_UNSUPPORTED;
+        odd = odd || (a & 1);
+        std::fill(traj.begin() + a, traj.begin() + b + 1, k);
     }
-    drop_graphs(h);      // (before the old buffer goes: graphs hold it)
-    CK(h->d_x0s.alloc((size_t)3 * K));
-    CK(cudaMemcpy2DAsync(h->d_x0s, (size_t)K * 8, x0s, (size_t)ld_x0s * 8, (size_t)K * 8, 3, cudaMemcpyHostToDevice, h->stream));
+    DevBuf<int> d_start, d_traj; DevBuf<double> d_x0;
+    CK(d_start.alloc((size_t)K + 1)); CK(d_traj.alloc((size_t)h->T)); CK(d_x0.alloc((size_t)3 * K));
+    CK(cudaMemcpyAsync(d_start, start.data(), ((size_t)K + 1) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(d_traj, traj.data(), (size_t)h->T * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpy2DAsync(d_x0, (size_t)K * 8, x0s, (size_t)ld_x0s * 8, (size_t)K * 8, 3, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    h->traj_T = traj_T; h->traj_K = K;
+    drop_graphs(h);      // (before the old buffers go: graphs hold them)
+    h->d_traj_start = std::move(d_start); h->d_traj_of = std::move(d_traj); h->d_x0s = std::move(d_x0);
+    h->traj_K = K; h->traj_odd = odd;
     h->first_empty = false; h->last_empty = false;
     h->ch.ppar_of = nullptr;
     return ICMSLAM_OK;
+}
+
+extern "C" int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double* x0s, int64_t ld_x0s, int32_t K)
+{
+    if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
+    CK(cudaSetDevice(h->cfg.device));
+    if (traj_T <= 0) {
+        drop_graphs(h);
+        h->traj_K = 0; h->traj_odd = false; h->d_traj_start.reset(); h->d_traj_of.reset(); h->d_x0s.reset();
+        h->ch.ppar_of = nullptr;
+        return ICMSLAM_OK;
+    }
+    if (!x0s || K <= 0 || ld_x0s < K || (int64_t)traj_T * K != h->T || traj_T < 3 || !h->fused_ok) return ICMSLAM_ERR_INVALID;
+    std::vector<int> start((size_t)K + 1);
+    for (int k = 0; k <= K; ++k) start[k] = k * traj_T;
+    return set_layout(h, start, x0s, ld_x0s);
+}
+
+extern "C" int icmslam_set_batch_lengths(icmslam_handle* h, const int32_t* lengths, int32_t K, const double* x0s, int64_t ld_x0s)
+{
+    if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
+    CK(cudaSetDevice(h->cfg.device));
+    if (!lengths || !x0s || K <= 0 || ld_x0s < K || !h->fused_ok) return ICMSLAM_ERR_INVALID;
+    std::vector<int> start((size_t)K + 1, 0);
+    int64_t sum = 0;
+    for (int k = 0; k < K; ++k) {
+        if (lengths[k] < 3) return ICMSLAM_ERR_INVALID;
+        sum += lengths[k];
+        if (sum > h->T) return ICMSLAM_ERR_INVALID;
+        start[k + 1] = (int)sum;
+    }
+    if (sum != h->T) return ICMSLAM_ERR_INVALID;
+    return set_layout(h, start, x0s, ld_x0s);
 }
 
 // ---- time-segment partition: one handle per GPU owns columns [t_lo, t_hi) of the T columns it loaded ------
@@ -2289,7 +2330,7 @@ extern "C" int icmslam_batch_iterate_until(icmslam_handle* h, int32_t max_sweeps
                                            int32_t region_cols, const icmslam_sweep_opts* opts, double* cambios, int32_t* n_done,
                                            int32_t* n_run)
 {
-    if (!h || !n_done || !n_run || max_sweeps < 0 || !(region_pitch > 0.0) || region_cols <= 0 || h->traj_T <= 0 || !h->d_x0s)
+    if (!h || !n_done || !n_run || max_sweeps < 0 || !(region_pitch > 0.0) || region_cols <= 0 || h->traj_K <= 0)
         return ICMSLAM_ERR_INVALID;
     icmslam_sweep_opts o;
     default_opts(o, opts);
@@ -2323,7 +2364,7 @@ extern "C" int icmslam_batch_iterate_until(icmslam_handle* h, int32_t max_sweeps
         h->fz_K = K;
     }
     CK(cudaMemsetAsync(h->d_fz_mask, 0, (size_t)K, s));
-    h->fz.frozen = h->d_fz_mask; h->fz.traj_T = h->traj_T; h->fz.K = K; h->fz.cols = region_cols; h->fz.pitch = region_pitch;
+    h->fz.frozen = h->d_fz_mask; h->fz.traj = h->d_traj_of; h->fz.K = K; h->fz.cols = region_cols; h->fz.pitch = region_pitch;
     h->fz.slots = h->d_fz_slots;
     h->fz_fallbacks = 0;
     const int rc = batch_until_loop(h, max_sweeps, tol_max_change, o, cambios, n_done, n_run);

@@ -326,8 +326,6 @@ struct PoseArrays {
     TrajLayout lay;                         // self.x0 (sensors.py:131) of the trajectory or of each trajectory of a batch
     const int* off;
     int T;
-    // trajectories and columns per trajectory (one trajectory: 1 and T)
-    __device__ __forceinline__ int traj_cols() const { return lay.traj_T > 0 ? lay.traj_T : T; }
 };
 
 // Pose t (never a pinned one).  WARPED: all 32 lanes of a warp call it for the same t (k_pose_walk) and compute the same
@@ -388,26 +386,25 @@ __device__ __forceinline__ void update_pose(int t, const DevCfg& cfg, const Pose
     if (WARPED) __syncwarp();      // (the next pose of the walk reads this one)
 }
 
-// red-black by trajectory-local time tl = t - k traj_T: parity 1 -> tl = 1,3,5,... ; parity 0 -> tl = 2,4,6,...  (so a
-// trajectory of a batch is swept exactly as it is alone, whatever the parity of traj_T).  (traj_cols + 1) / 2 threads per
-// trajectory.
+// red-black by trajectory-local time tl = t - start[k]: parity 1 -> tl = 1,3,5,... ; parity 0 -> tl = 2,4,6,...  (so a
+// trajectory of a batch is swept exactly as it is alone, wherever it starts).  One thread per column.
 __global__ void __launch_bounds__(128)
 k_pose_colour(int parity, DevCfg cfg, PoseArrays A, ObsArrays O, SeenSrc S, int solver, double tol, int maxit,
               unsigned long long* iters)
 {
-    const int Tt = A.traj_cols(), per = (Tt + 1) / 2;
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    const int k = idx / per, tl = 2 * (idx - k * per) + (parity ? 1 : 2);
-    if (k >= A.T / Tt || tl >= Tt) return;
-    update_pose(k * Tt + tl, cfg, A, O, S, solver, tol, maxit, iters);
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= A.T) return;
+    const int tl = A.lay.K > 0 ? t - A.lay.begin(t) : t;
+    if (tl == 0 || (tl & 1) != parity) return;
+    update_pose(t, cfg, A, O, S, solver, tol, maxit, iters);
 }
 
-// the reference's forward Gauss-Seidel (sensors.py:145): the warp of block k walks t = 1 .. traj_T-1 of trajectory k (one
-// block of one warp per trajectory: trajectories take different Nelder-Mead branches).  Its lanes share each energy's
+// the reference's forward Gauss-Seidel (sensors.py:145): the warp of block k walks t = start[k]+1 .. start[k+1]-1 of trajectory
+// k (one block of one warp per trajectory: trajectories take different Nelder-Mead branches).  Its lanes share each energy's
 // observations (pose_energy<true>); everything else runs on every lane alike.
 __global__ void __launch_bounds__(WARP)
 k_pose_walk(DevCfg cfg, PoseArrays A, ObsArrays O, SeenSrc S, int solver, double tol, int maxit, unsigned long long* iters)
 {
-    const int Tt = A.traj_cols(), t0 = blockIdx.x * Tt;
-    for (int t = t0 + 1; t < t0 + Tt; ++t) update_pose<true>(t, cfg, A, O, S, solver, tol, maxit, iters);
+    const int t0 = A.lay.K > 0 ? A.lay.start[blockIdx.x] : 0, t1 = A.lay.K > 0 ? A.lay.start[blockIdx.x + 1] : A.T;
+    for (int t = t0 + 1; t < t1; ++t) update_pose<true>(t, cfg, A, O, S, solver, tol, maxit, iters);
 }

@@ -9,7 +9,7 @@
 // their odometry increments, controls and heading sin/cos in shared memory.  Thread q (a slot) solves the whole odd pose
 // tb-1+2q (q = 0: the halo tb-1, owned by the previous tile, which computes the identical value from the identical inputs),
 // then, after a block barrier, the even pose tb+2q from the new odd poses in shared memory: every warp works in both colour
-// phases.  In a batch of odd-length trajectories the colours follow each trajectory's local time (solve_slot_load).  Every input is read once; the new poses and their projection parameters (x, y, sin/cos of theta - pi/2: what
+// phases.  In a batch whose trajectories do not all start on even columns the colours follow each trajectory's local time (solve_slot_load).  Every input is read once; the new poses and their projection parameters (x, y, sin/cos of theta - pi/2: what
 // tras_rot_z needs next sweep, ICM_SLAM.py:465-480) are written coalesced.
 #pragma once
 #include "common.cuh"
@@ -228,18 +228,18 @@ struct SlotMom {
     int t, li;
 };
 
-// LOCAL: a batch of trajectories of odd length (p.lay.traj_T odd), coloured by trajectory-local time t - k traj_T like
-// k_pose_colour.  Trajectory k starts on column k traj_T, whose parity is k's: in an odd-numbered trajectory the slot's pair
-// (tb-1+2q, tb+2q) swaps roles -- phase 0 solves the local-odd tb+2q, phase 1 the local-even tb-1+2q -- and the re-solved halo
-// is tb+ST_OWN right of the tile instead of tb-1 (its neighbour tb+ST_OWN+1 is staged).  The roles go by the trajectory of
-// tb-1+2q: where the pair spans a boundary, tb+2q is the next trajectory's pinned first pose and phase 0 passes it through.
+// LOCAL: a batch in which some trajectory starts on an odd column, coloured by trajectory-local time t - start[k] like
+// k_pose_colour.  In a trajectory that starts on an odd column the slot's pair (tb-1+2q, tb+2q) swaps roles -- phase 0 solves
+// the local-odd tb+2q, phase 1 the local-even tb-1+2q -- and the re-solved halo is tb+ST_OWN right of the tile instead of tb-1
+// (its neighbour tb+ST_OWN+1 is staged).  The roles go by the trajectory of tb-1+2q: where the pair spans a boundary, tb+2q is
+// the next trajectory's pinned first pose and phase 0 passes it through.
 template <bool FZ, bool LOCAL>
 __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb, int q, int phase)
 {
     SlotMom s;
     if (LOCAL) {
         const int a = tb - 1 + 2 * q;
-        const bool swap = a >= 0 && ((a / p.lay.traj_T) & 1);
+        const bool swap = a >= 0 && a < p.T && (p.lay.begin(a) & 1);      // (a >= T: neither pose of the pair is valid)
         s.t = (phase == 0) != swap ? a : a + 1;
         s.li = s.t - (tb - 2);
         // (phase 0 also solves the halo next to the tile: tb-1 or tb+ST_OWN; phase 1 only the owned poses)
@@ -269,8 +269,8 @@ __device__ __forceinline__ SlotMom solve_slot_load(const SolveParams& p, int tb,
     return s;
 }
 
-// FZ: a batch with frozen trajectories (p.fz); the plain sweep launches the instance without the test.  LOCAL: a batch of
-// odd-length trajectories (solve_slot_load); every other handle launches the instance without it.
+// FZ: a batch with frozen trajectories (p.fz); the plain sweep launches the instance without the test.  LOCAL: a batch with a
+// trajectory that starts on an odd column (solve_slot_load); every other handle launches the instance without it.
 template <bool FZ, bool LOCAL = false>
 __global__ void __launch_bounds__(ST_THREADS, ST_MINB)
 k_solve_tile(const SolveParams p)

@@ -975,11 +975,32 @@ __device__ void tail_slow_body(DevState* st, TailState* ts, double dist_thr, dou
     }
     __syncthreads();
     const int newL = block_exclusive_scan(used, rank, K, wsum);   // :251-253 dense renumbering in ascending order
-    for (int j = tid; j < K; j += nth) {                           // :258-260 count-weighted means
+    // :258-260 count-weighted means, each class summed in ascending landmark order like the reference, so the result does not
+    // depend on the order in which threads arrive: a class of one landmark by its own thread, the landmarks of merged classes
+    // (at most 2 n_ind of them) by one thread in order.  used[] becomes the class sizes, parent[] (no longer needed) the flags
+    // of the landmarks in merged classes, ind[] their ordered list.
+    for (int j = tid; j < K; j += nth) used[j] = 0;
+    __syncthreads();
+    for (int j = tid; j < K; j += nth) atomicAdd(used + rank[lab[j]], 1);
+    __syncthreads();
+    for (int j = tid; j < K; j += nth) {
         const int r = rank[lab[j]];
-        atomicAdd(ox + r, mul_rn(kx[j], kc[j]));
-        atomicAdd(oy + r, mul_rn(ky[j], kc[j]));
-        atomicAdd(oc + r, kc[j]);
+        const bool single = used[r] == 1;
+        if (single) { ox[r] = add_rn(0.0, mul_rn(kx[j], kc[j])); oy[r] = add_rn(0.0, mul_rn(ky[j], kc[j])); oc[r] = add_rn(0.0, kc[j]); }
+        parent[j] = single ? 0 : 1;
+    }
+    __syncthreads();
+    const int n_mem = block_exclusive_scan(parent, ind_pos, K, wsum);
+    for (int j = tid; j < K; j += nth)
+        if (parent[j]) ind[ind_pos[j]] = j;
+    __syncthreads();
+    if (tid == 0) {
+        for (int q = 0; q < n_mem; ++q) {
+            const int j = ind[q], r = rank[lab[j]];
+            ox[r] = add_rn(ox[r], mul_rn(kx[j], kc[j]));
+            oy[r] = add_rn(oy[r], mul_rn(ky[j], kc[j]));
+            oc[r] = add_rn(oc[r], kc[j]);
+        }
     }
     __syncthreads();
     for (int r = tid; r < Lcap; r += nth) {

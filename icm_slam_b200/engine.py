@@ -147,6 +147,17 @@ class Engine:
         check(self.lib.icmslam_set_batch(self._h, int(traj_T), _ptr(x0s)[0], _rows(x0s, 3), int(x0s.shape[1])), self._h)
         self.batch_K = int(x0s.shape[1])
 
+    def set_batch_lengths(self, lengths, x0s):
+        """The loaded columns are K independent trajectories of lengths[k] >= 3 columns each, laid end to end (sum = T; x0s: 3 x K
+        pinned first poses).  set_batch(0, None) switches back to one trajectory."""
+        lengths = np.ascontiguousarray(lengths, dtype=np.int32)
+        x0s = np.ascontiguousarray(x0s, dtype=np.float64)
+        K = int(lengths.shape[0])
+        if x0s.ndim != 2 or x0s.shape != (3, K):
+            raise ValueError("x0s must be 3 x K")
+        check(self.lib.icmslam_set_batch_lengths(self._h, C.c_void_p(lengths.ctypes.data), K, _ptr(x0s)[0], K), self._h)
+        self.batch_K = K
+
     def set_counts(self, counts=None):
         """cant_obs_i <- counts (rest zero); None: Mapa.clear_obs."""
         c = np.zeros(0) if counts is None else np.ascontiguousarray(counts, dtype=np.float64)

@@ -156,12 +156,18 @@ int icmslam_get_poses(icmslam_handle* h, double* x, int64_t ld_x, int32_t memspa
  * then pinned to its own x0, its last pose has no successor, and one sweep of the handle is one sweep of every trajectory: ONE
  * launch of each kernel for the whole batch.  Every sweep mode is valid on a batch handle (icmslam_iterate and icmslam_sweep; the
  * SEQUENTIAL schedule walks each trajectory with its own warp), at any traj_T >= 3: the REDBLACK schedule, fused or not, colours
- * pose t of trajectory k by the parity of t - k * traj_T, so an odd traj_T sweeps each trajectory as it is swept alone.  Refused:
- * traj_T < 3 or traj_T * K != T (ICMSLAM_ERR_INVALID), a trajectory whose first or last scan is empty
- * (ICMSLAM_ERR_UNSUPPORTED); a refused call leaves the handle as it was.  New labels are numbered over the whole batch and the label cap L
- * applies to the batch.  The x0 argument of icmslam_iterate / icmslam_sweep is ignored.  traj_T <= 0 switches back to a single
- * trajectory. */
+ * pose t of trajectory k by the parity of t minus the trajectory's first column, so every trajectory is swept as it is swept
+ * alone.  Refused: traj_T < 3 or traj_T * K != T (ICMSLAM_ERR_INVALID), a trajectory whose first or last scan is empty
+ * (ICMSLAM_ERR_UNSUPPORTED); a refused call leaves the handle as it was and a successful one drops the cached graphs.  New labels
+ * are numbered over the whole batch and the label cap L applies to the batch.  The x0 argument of icmslam_iterate /
+ * icmslam_sweep is ignored.  traj_T <= 0 switches back to a single trajectory (from either kind of batch). */
 int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double* x0s, int64_t ld_x0s, int32_t K);
+
+/* K trajectories of lengths[k] columns each, laid end to end (sum = T); x0s as in icmslam_set_batch.  Everything said of
+ * icmslam_set_batch holds, with trajectory k on columns lengths[0] + ... + lengths[k-1] onwards.  Refused with
+ * ICMSLAM_ERR_INVALID: K <= 0, ld_x0s < K, a length below 3, lengths whose sum is not T; with ICMSLAM_ERR_UNSUPPORTED: a
+ * trajectory whose first or last scan is empty. */
+int icmslam_set_batch_lengths(icmslam_handle* h, const int32_t* lengths, int32_t K, const double* x0s, int64_t ld_x0s);
 
 /* -- time-segment partition over several GPUs (no reference counterpart: the reference sweep is strictly
  * sequential in time, sensors.py:145-162; only the restated (REDBLACK, NEWTON, PREV) sweep partitions).
