@@ -108,6 +108,10 @@ def lib():
     L.icmslam_seg_finish.argtypes = [vp]
     L.icmslam_fcluster.argtypes = [vp, vp, i32, dbl, vp, _ip]
     L.icmslam_pass0.argtypes = [vp, vp, vp, i64, vp, i32, i64, _ip, i32]
+    L.icmslam_append.argtypes = [vp, vp, i32, i64, vp, i64, vp, i64, i32]
+    L.icmslam_pass0_begin.argtypes = [vp, vp]
+    L.icmslam_pass0_advance.argtypes = [vp, _ip]
+    L.icmslam_pass0_finish.argtypes = [vp, vp, i64, vp, i32, i64, _ip, i32]
     L.icmslam_get_kernel_ms.argtypes = [vp, vp]
     L.icmslam_get_launch_count.argtypes = [vp, C.POINTER(i64)]
     L.icmslam_get_transfer_bytes.argtypes = [vp, C.POINTER(i64), C.POINTER(i64)]
@@ -136,7 +140,8 @@ EXPORTS = [
     "icmslam_calc_cambio", "icmslam_filtrar_obs", "icmslam_set_map", "icmslam_get_map", "icmslam_iterate",
     "icmslam_get_kernel_ms", "icmslam_get_launch_count", "icmslam_get_transfer_bytes", "icmslam_set_poses", "icmslam_get_poses", "icmslam_set_segment", "icmslam_device_ptr", "icmslam_seg_begin",
     "icmslam_seg_exchange", "icmslam_seg_halo", "icmslam_p2p_export", "icmslam_p2p_import", "icmslam_get_trace", "icmslam_pose_eval", "icmslam_seg_finish", "icmslam_fcluster", "icmslam_pass0", "icmslam_associate", "icmslam_iterate_until", "icmslam_set_counts", "icmslam_set_batch",
-    "icmslam_batch_iterate_until", "icmslam_set_batch_lengths",
+    "icmslam_batch_iterate_until", "icmslam_set_batch_lengths", "icmslam_append", "icmslam_pass0_begin", "icmslam_pass0_advance",
+    "icmslam_pass0_finish",
 ]
 
 

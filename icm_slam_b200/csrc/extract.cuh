@@ -2,7 +2,9 @@
 // range pre-conditioning (sensors_definitions.py:21-22) and filtrar_obs.m (scripts/filtrar_obs.m).
 //
 // Layout: `scans` is the reference's B x T array (row = beam, column = scan), so one scan is a
-// strided column.  A block stages a [B][32 scans] tile through shared memory with coalesced row
+// strided column.  Every scan is filtered on its own, so the kernels take a window [t_lo, t_hi) of columns: the whole log, or
+// the columns an append brought (the CSR offsets of the window continue those before it).  `masks` and `counts` are indexed
+// from t_lo; `off`, `scan_of` and the observation arrays are global.  A block stages a [B][32 scans] tile through shared memory with coalesced row
 // reads (32 consecutive scans = 256 B per beam row), then each warp owns whole scans.
 #pragma once
 #include "common.cuh"
@@ -27,10 +29,10 @@ __device__ __forceinline__ double median3(double a, double b, double c)
 // smem layout: tile[B][EX_TILE+1] | per warp: vpx[B], vpy[B], vb[B](int)
 template <int PASS>
 __global__ void __launch_bounds__(EX_THREADS)
-k_extract(const double* __restrict__ scans, int B, int T, int64_t ld, const double* __restrict__ cosb,
+k_extract(const double* __restrict__ scans, int B, int t_lo, int T, int64_t ld, const double* __restrict__ cosb,
           const double* __restrict__ sinb, DevCfg cfg, int precondition, int nwords,
-          uint32_t* __restrict__ masks,      // T * nwords keep bitmasks
-          int* __restrict__ counts,          // PASS 1: kept beams per scan
+          uint32_t* __restrict__ masks,      // (T - t_lo) * nwords keep bitmasks
+          int* __restrict__ counts,          // PASS 1: kept beams per scan of the window
           const int* __restrict__ off,       // PASS 2: CSR offsets
           int* __restrict__ beam, double* __restrict__ d, double* __restrict__ bx, double* __restrict__ by,
           int* __restrict__ scan_of)
@@ -42,7 +44,7 @@ k_extract(const double* __restrict__ scans, int B, int T, int64_t ld, const doub
     double* vpx = tile + (size_t)B * TP + (size_t)warp * 3 * B;
     double* vpy = vpx + B;
     int* vb = (int*)(vpy + B);
-    const int t0 = blockIdx.x * EX_TILE;
+    const int t0 = t_lo + blockIdx.x * EX_TILE;
     // coalesced tile load: thread -> (beam row, scan column)
     for (int e = threadIdx.x; e < B * EX_TILE; e += EX_THREADS) {
         int b = e / EX_TILE, c = e % EX_TILE;
@@ -82,7 +84,7 @@ k_extract(const double* __restrict__ scans, int B, int T, int64_t ld, const doub
             }
             __syncwarp();
             // zero the mask words of this scan
-            for (int w = lane; w < nwords; w += WARP) masks[(int64_t)t * nwords + w] = 0u;
+            for (int w = lane; w < nwords; w += WARP) masks[(int64_t)(t - t_lo) * nwords + w] = 0u;
             __syncwarp();
             int kept = 0;
             if (k > 1) {                                          // :42
@@ -99,19 +101,19 @@ k_extract(const double* __restrict__ scans, int B, int T, int64_t ld, const doub
                         // sqrt is monotone and correctly rounded: min_i sqrt(s_i) == sqrt(min_i s_i)
                         double m = fmin(100.0, __dsqrt_rn(m2));
                         keep = m <= cfg.dist_thr;               // :50
-                        if (keep) atomicOr(&masks[(int64_t)t * nwords + (vb[j] >> 5)], 1u << (vb[j] & 31));
+                        if (keep) atomicOr(&masks[(int64_t)(t - t_lo) * nwords + (vb[j] >> 5)], 1u << (vb[j] & 31));
                     }
                     kept += __popc(__ballot_sync(FULLMASK, keep));
                 }
             }
-            if (lane == 0) counts[t] = kept;
+            if (lane == 0) counts[t - t_lo] = kept;
             __syncwarp();
         } else {
             int base = off[t];
             if (off[t + 1] == base) continue;
             for (int b0 = 0; b0 < B; b0 += WARP) {
                 int b = b0 + lane;
-                uint32_t word = masks[(int64_t)t * nwords + (b0 >> 5)];
+                uint32_t word = masks[(int64_t)(t - t_lo) * nwords + (b0 >> 5)];
                 bool keep = (b < B) && ((word >> lane) & 1u);
                 if (keep) {
                     double a = b > 0 ? tile[(b - 1) * TP + c] : 0.0;

@@ -96,19 +96,23 @@ struct icmslam_handle {
     char err[512];
     // dataset
     int B = 0, T = 0, precondition = 0;
-    struct Dataset {      // what icmslam_load allocates, sized by T and B
+    int cap_T = 0;        // columns d_scans, d_odo, d_u and d_x have room for (their leading dimension): T after icmslam_load
+                          // and after ensure_layout, grown by doubling when icmslam_append brings more
+    struct Dataset {      // what icmslam_load allocates (B x cap_T, 3 x cap_T, ...) and ensure_layout sizes by T
         DevBuf<double> d_scans, d_odo, d_u, d_cos, d_sin, d_ang;
         DevBuf<int> d_nfar, d_flag, d_prefix;       // per scan workspace
-        DevBuf<double> d_x /*3 x T*/, d_x2 /*3 x T, pose double buffer*/, d_inc /*3 x T odometry increments*/;
+        DevBuf<double> d_x /*3 x cap_T*/, d_x2 /*3 x T, pose double buffer*/, d_inc /*3 x T odometry increments*/;
         DevBuf<FarRec> d_far_list;
         DevBuf<int> d_blk_prefix;
     } ds;
-    // extraction
-    bool extracted = false;
-    int64_t n = 0;
+    // extraction: the CSR arrays cover all T columns once `extracted`; what only the sweeps read follows on demand
+    // (ensure_layout: `laid_out`)
+    bool extracted = false, laid_out = false;
+    int64_t n = 0, n_cap = 0;           // observations, and the room of the per-observation arrays (d_off has cap_T + 1 entries)
+    std::vector<int> off_h;             // host copy of the T + 1 offsets
     int n_empty = 0, max_per_scan = 0;
     bool first_empty = false, last_empty = false;
-    struct Extraction {   // what icmslam_extract allocates (some of it on first use), sized by n and the tile count
+    struct Extraction {   // what icmslam_extract / icmslam_append and ensure_layout allocate (some of it on first use)
         DevBuf<int> d_off, d_beam, d_scan_of;
         DevBuf<double> d_d, d_bx, d_by;
         DevBuf<double2> d_bxy;               // interleaved (bx, by) records for the TMA staging
@@ -135,6 +139,15 @@ struct icmslam_handle {
     DevBuf<double> d_kx, d_ky, d_kc, d_ox, d_oy, d_oc, d_acc;
     DevBuf<double> d_map_in /*2 x Lcap*/, d_map_out /*2 x Lcap*/;
     DevBuf<double> d_tmp_a, d_tmp_b; /* 2 x Lcap scratch for filter_map / calc_cambio inputs */
+    // pass 0 as a resumable walk (icmslam_pass0_begin / _advance / _finish): its own map under construction (2 x Lcap) and
+    // counts, which no other call writes, and the carried state; on the host the columns walked and x0
+    struct Walk {
+        DevBuf<double> y, cant;
+        DevBuf<Pass0Carry> carry;
+        bool on = false;
+        int t = 0, lact = 0;
+        double x0[3] = {0, 0, 0};
+    } walk;
     // state
     DevBuf<DevState> d_st;
     PinnedBuf<DevState> h_st;   // pinned mirror
@@ -299,7 +312,8 @@ static void drop_graphs(icmslam_handle* h)
     for (auto& g : h->graphs) g.exec.reset();
 }
 
-// a fresh extraction: graphs that hold the old buffers go first, and nothing the host knew of the old observations stays
+// a fresh extraction: graphs that hold the old buffers go first, and nothing the host knew of the old observations stays (a
+// pass-0 walk over them included)
 static void reset_extraction(icmslam_handle* h)
 {
     drop_graphs(h);
@@ -309,17 +323,23 @@ static void reset_extraction(icmslam_handle* h)
     h->ch.hint_map = nullptr;
     h->fused_ok = false;
     h->extracted = false;
+    h->laid_out = false;
+    h->n = 0; h->n_cap = 0;
+    h->off_h.clear();
+    h->n_empty = 0; h->max_per_scan = 0;
+    h->walk.on = false;
 }
 
 static void free_dataset(icmslam_handle* h)
 {
     reset_extraction(h);
     h->ds = icmslam_handle::Dataset();
+    h->cap_T = 0;
+    h->ch.x_cur = 0;
     h->last_map_L = -1;
     h->traj_K = 0; h->traj_odd = false;
     h->d_traj_start.reset(); h->d_traj_of.reset(); h->d_x0s.reset();
     h->d_fz_mask.reset(); h->d_fz_need.reset(); h->d_fz_slots.reset(); h->d_fz_reg.reset(); h->fz_K = 0;
-    h->n = 0;
 }
 
 extern "C" int icmslam_destroy(icmslam_handle* h)
@@ -410,6 +430,9 @@ extern "C" int icmslam_create(const icmslam_config* cfg, icmslam_handle** out)
     if (e == cudaSuccess) e = h->d_map_out.alloc(2 * L);
     if (e == cudaSuccess) e = h->d_tmp_a.alloc(2 * L);
     if (e == cudaSuccess) e = h->d_tmp_b.alloc(2 * L);
+    if (e == cudaSuccess) e = h->walk.y.alloc(2 * L);
+    if (e == cudaSuccess) e = h->walk.cant.alloc(L);
+    if (e == cudaSuccess) e = h->walk.carry.alloc(1);
     h->fg_cells = (int)(4 * L > 4096 ? 4 * L : 4096);
     if (e == cudaSuccess) e = h->grid.alloc(h->fg_cells, 4 * L);    // replicated binning: <= 4 cells per landmark
     if (e == cudaSuccess) e = h->scratch_grid.alloc(h->fg_cells, 4 * L);
@@ -510,6 +533,28 @@ extern "C" int icmslam_synchronize(icmslam_handle* h)
     return ICMSLAM_OK;
 }
 
+// the scans' workspace for the largest scan of a sweep, so that nothing allocates inside a graph capture
+static int size_cub(icmslam_handle* h)
+{
+    size_t need = 0, b = 0;
+    const int lens[3] = {h->Lcap + 1, h->fg_cells + 2, h->T + 1};
+    for (int k = 0; k < 3; ++k) { CK(cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, lens[k], h->stream)); if (b > need) need = b; }
+    return ensure_cub(h, need);
+}
+
+// a rows x new_ld buffer in place of `b`, with the first `cols` columns of each row of b (leading dimension ld) copied over
+template <typename E>
+static cudaError_t regrow(icmslam_handle* h, DevBuf<E>& b, int rows, int64_t ld, int64_t cols, int64_t new_ld)
+{
+    DevBuf<E> nb;
+    cudaError_t e = nb.alloc((size_t)rows * new_ld);
+    if (e == cudaSuccess && cols > 0 && b)
+        e = cudaMemcpy2DAsync(nb, (size_t)new_ld * sizeof(E), b, (size_t)ld * sizeof(E), (size_t)cols * sizeof(E), rows, cudaMemcpyDeviceToDevice,
+                              h->stream);
+    if (e == cudaSuccess) b = std::move(nb);      // (cudaFree waits for the copy out of the old buffer)
+    return e;
+}
+
 extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, int32_t T, int64_t ld_scans,
                             const double* odo, int64_t ld_odo, const double* u, int64_t ld_u, const double* cos_tab,
                             const double* sin_tab, int32_t precondition, int32_t memspace)
@@ -519,7 +564,7 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
     (void)memspace;   // cudaMemcpyDefault resolves host / device pointers (UVA)
     CK(cudaSetDevice(h->cfg.device));
     free_dataset(h);
-    h->B = B; h->T = T; h->precondition = precondition;
+    h->B = B; h->T = T; h->cap_T = T; h->precondition = precondition;
     CK(h->ds.d_scans.alloc((size_t)B * T));
     CK(h->ds.d_odo.alloc((size_t)3 * T));
     CK(h->ds.d_u.alloc((size_t)2 * T));
@@ -527,23 +572,9 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
     CK(h->ds.d_sin.alloc((size_t)B));
     CK(h->ds.d_ang.alloc((size_t)B));
     CK(h->ds.d_x.alloc((size_t)3 * T));
-    CK(h->ds.d_nfar.alloc((size_t)T + 1));
-    CK(h->ds.d_flag.alloc((size_t)T + 1));
-    CK(h->ds.d_prefix.alloc((size_t)T + 1));
-    CK(h->ds.d_inc.alloc((size_t)3 * T));
-    CK(h->ds.d_x2.alloc((size_t)3 * T));
     h->seg_lo = 0; h->seg_hi = T; h->seg_first = 1; h->seg_last = 1;
-    h->n_tiles = nblk(T, RT_TILE);
-    h->n_solve_tiles = nblk(T, ST_OWN);
-    CK(h->ds.d_far_list.alloc((size_t)T));
-    CK(h->ds.d_blk_prefix.alloc((size_t)nblk(T + 1, RT_TILE) + 2));
-    {   // scan workspace for the largest scan of a sweep, so that nothing allocates inside a graph capture
-        size_t need = 0, b = 0;
-        const int lens[3] = {h->Lcap + 1, h->fg_cells + 2, T + 1};
-        for (int k = 0; k < 3; ++k) { CK(cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, lens[k], h->stream)); if (b > need) need = b; }
-        int rcw = ensure_cub(h, need);
-        if (rcw) return rcw;
-    }
+    int rc = size_cub(h);
+    if (rc) return rc;
     const size_t w = (size_t)T * sizeof(double);
     CK(cudaMemcpy2DAsync(h->ds.d_scans, w, scans, (size_t)ld_scans * sizeof(double), w, B, cudaMemcpyDefault, h->stream));
     CK(cudaMemcpy2DAsync(h->ds.d_odo, w, odo, (size_t)ld_odo * sizeof(double), w, 3, cudaMemcpyDefault, h->stream));
@@ -554,8 +585,6 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
         cb[i] = cos_tab ? cos_tab[i] : cos(ang[i]);
         sb[i] = sin_tab ? sin_tab[i] : sin(ang[i]);
     }
-    k_odo_increments<<<nblk(T, 256), 256, 0, h->stream>>>(h->ds.d_odo, T, T, h->ds.d_inc, T);
-    CK(cudaGetLastError());
     CK(cudaMemcpyAsync(h->ds.d_ang, ang.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->ds.d_cos, cb.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->ds.d_sin, sb.data(), B * sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -563,52 +592,109 @@ extern "C" int icmslam_load(icmslam_handle* h, const double* scans, int32_t B, i
     return ICMSLAM_OK;
 }
 
-extern "C" int icmslam_extract(icmslam_handle* h)
+// filtrar_z of the columns [t_lo, T): all of them after reset_extraction, or those an append brought.  The offsets of the
+// window continue from the h->n observations before it, and the per-observation arrays grow (by doubling) to hold the new ones.
+static int extract_window(icmslam_handle* h, int t_lo)
 {
-    if (!h || !h->ds.d_scans) return ICMSLAM_ERR_INVALID;
-    CK(cudaSetDevice(h->cfg.device));
-    reset_extraction(h);
-    const int B = h->B, T = h->T;
+    const int B = h->B, T = h->T, W = T - t_lo;
     const int nwords = (B + 31) / 32;
+    cudaStream_t s = h->stream;
     DevBuf<uint32_t> d_masks;
     DevBuf<int> d_counts;
-    CK(d_masks.alloc((size_t)T * nwords));
-    CK(d_counts.alloc((size_t)T + 1));
-    CK(h->ex.d_off.alloc((size_t)T + 1));
-    CK(cudaMemsetAsync(d_counts, 0, ((size_t)T + 1) * sizeof(int), h->stream));
+    CK(d_masks.alloc((size_t)W * nwords));
+    CK(d_counts.alloc((size_t)W + 1));
+    if (!h->ex.d_off) CK(h->ex.d_off.alloc((size_t)h->cap_T + 1));
+    CK(cudaMemsetAsync(d_counts, 0, ((size_t)W + 1) * sizeof(int), s));
     const size_t smem = extract_smem_bytes(B);
     CK(cudaFuncSetAttribute(k_extract<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaFuncSetAttribute(k_extract<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int blocks = nblk(T, EX_TILE);
-    k_extract<1><<<blocks, EX_THREADS, smem, h->stream>>>(h->ds.d_scans, B, T, T, h->ds.d_cos, h->ds.d_sin, h->dcfg, h->precondition,
-                                                          nwords, d_masks, d_counts, nullptr, nullptr, nullptr, nullptr,
-                                                          nullptr, nullptr);
+    const int blocks = nblk(W, EX_TILE);
+    k_extract<1><<<blocks, EX_THREADS, smem, s>>>(h->ds.d_scans, B, t_lo, T, h->cap_T, h->ds.d_cos, h->ds.d_sin, h->dcfg, h->precondition,
+                                                  nwords, d_masks, d_counts, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
     CK(cudaGetLastError());
-    int rc = exclusive_sum(h, d_counts, h->ex.d_off, T + 1);
-    if (rc) return rc;
-    std::vector<int> off((size_t)T + 1);
-    CK(cudaMemcpyAsync(off.data(), h->ex.d_off, ((size_t)T + 1) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    h->n = off[T];
-    h->n_empty = 0; h->max_per_scan = 0;
-    for (int t = 0; t < T; ++t) {
+    {   // off[t_lo .. T] = n + exclusive sum of the window's counts
+        size_t bytes = 0;
+        CK(cub::DeviceScan::ExclusiveScan(nullptr, bytes, (const int*)d_counts, h->ex.d_off + t_lo, cub::Sum(), (int)h->n, W + 1, s));
+        int rc = ensure_cub(h, bytes);
+        if (rc) return rc;
+        CK(cub::DeviceScan::ExclusiveScan(h->d_cub, bytes, (const int*)d_counts, h->ex.d_off + t_lo, cub::Sum(), (int)h->n, W + 1, s));
+    }
+    std::vector<int>& off = h->off_h;
+    off.resize((size_t)T + 1);
+    CK(cudaMemcpyAsync(off.data() + t_lo, h->ex.d_off + t_lo, ((size_t)W + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    for (int t = t_lo; t < T; ++t) {
         int k = off[t + 1] - off[t];
         if (k == 0) ++h->n_empty;
         if (k > h->max_per_scan) h->max_per_scan = k;
     }
     h->first_empty = off[1] == off[0];
     h->last_empty = off[T] == off[T - 1];
-    const size_t n = (size_t)h->n;
-    CK(h->ex.d_beam.alloc(n)); CK(h->ex.d_scan_of.alloc(n)); CK(h->ex.d_d.alloc(n)); CK(h->ex.d_bx.alloc(n + 2)); CK(h->ex.d_by.alloc(n + 2));
-    CK(cudaMemsetAsync(h->ex.d_bx, 0, (n + 2) * sizeof(double), h->stream));
-    CK(cudaMemsetAsync(h->ex.d_by, 0, (n + 2) * sizeof(double), h->stream));
-    CK(h->ex.d_c.alloc(n + 8));      // (+ slack: the fused kernel stages 16-byte aligned slices of it)
-    k_extract<2><<<blocks, EX_THREADS, smem, h->stream>>>(h->ds.d_scans, B, T, T, h->ds.d_cos, h->ds.d_sin, h->dcfg, h->precondition,
-                                                          nwords, d_masks, nullptr, h->ex.d_off, h->ex.d_beam, h->ex.d_d, h->ex.d_bx,
-                                                          h->ex.d_by, h->ex.d_scan_of);
+    const int64_t n0 = h->n, n = off[T];
+    if (n > h->n_cap || !h->ex.d_beam) {
+        const int64_t cap = std::max(2 * h->n_cap, n);
+        CK(regrow(h, h->ex.d_beam, 1, n0, n0, cap)); CK(regrow(h, h->ex.d_scan_of, 1, n0, n0, cap)); CK(regrow(h, h->ex.d_d, 1, n0, n0, cap));
+        CK(regrow(h, h->ex.d_bx, 1, n0, n0, cap + 2)); CK(regrow(h, h->ex.d_by, 1, n0, n0, cap + 2));
+        CK(regrow(h, h->ex.d_c, 1, n0, n0, cap + 8));      // (+ slack: the fused kernel stages 16-byte aligned slices of it)
+        if (h->ex.d_seen_x) { CK(regrow(h, h->ex.d_seen_x, 1, n0, n0, cap)); CK(regrow(h, h->ex.d_seen_y, 1, n0, n0, cap)); }
+        h->n_cap = cap;
+    }
+    CK(cudaMemsetAsync(h->ex.d_bx + n, 0, 2 * sizeof(double), s));
+    CK(cudaMemsetAsync(h->ex.d_by + n, 0, 2 * sizeof(double), s));
+    k_extract<2><<<blocks, EX_THREADS, smem, s>>>(h->ds.d_scans, B, t_lo, T, h->cap_T, h->ds.d_cos, h->ds.d_sin, h->dcfg, h->precondition,
+                                                  nwords, d_masks, nullptr, h->ex.d_off, h->ex.d_beam, h->ex.d_d, h->ex.d_bx, h->ex.d_by,
+                                                  h->ex.d_scan_of);
     CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(s));      // (the masks and counts go when this returns)
+    h->n = n;
+    h->extracted = true;
+    h->laid_out = false;
+    return ICMSLAM_OK;
+}
+
+// the resident poses into d_x (a sweep may have left them in the double buffer)
+static int poses_home(icmslam_handle* h)
+{
+    if (h->ch.x_cur) CK(cudaMemcpyAsync(h->ds.d_x, h->ds.d_x2, (size_t)3 * h->cap_T * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+    h->ch.x_cur = 0;
+    h->ch.ppar_of = nullptr;
+    return ICMSLAM_OK;
+}
+
+// What the sweeps read beyond the extraction, laid out for the T columns loaded: the pose, odometry and control arrays with
+// leading dimension T, the odometry increments, the per-scan workspaces, run records and tiles, projection parameters, body
+// moments and the association kernel's shared-memory budget.  Done by icmslam_extract, and by the first call after an append
+// that sweeps or sets what a sweep reads (a walk of pass 0 needs none of it).
+static int ensure_layout(icmslam_handle* h)
+{
+    if (!h->extracted || h->laid_out) return ICMSLAM_OK;
+    drop_graphs(h);
+    const int T = h->T;
+    cudaStream_t s = h->stream;
+    int rc = poses_home(h);
+    if (rc) return rc;
+    if (h->cap_T != T) {      // (an append left the columns in larger buffers)
+        CK(regrow(h, h->ds.d_scans, h->B, h->cap_T, T, T));
+        CK(regrow(h, h->ds.d_odo, 3, h->cap_T, T, T));
+        CK(regrow(h, h->ds.d_u, 2, h->cap_T, T, T));
+        CK(regrow(h, h->ds.d_x, 3, h->cap_T, T, T));
+        h->cap_T = T;
+    }
+    CK(h->ds.d_x2.alloc((size_t)3 * T));
+    CK(h->ds.d_inc.alloc((size_t)3 * T));
+    k_odo_increments<<<nblk(T, 256), 256, 0, s>>>(h->ds.d_odo, T, T, h->ds.d_inc, T);
+    CK(cudaGetLastError());
+    CK(h->ds.d_nfar.alloc((size_t)T + 1));
+    CK(h->ds.d_flag.alloc((size_t)T + 1));
+    CK(h->ds.d_prefix.alloc((size_t)T + 1));
+    CK(h->ds.d_far_list.alloc((size_t)T));
+    CK(h->ds.d_blk_prefix.alloc((size_t)nblk(T + 1, RT_TILE) + 2));
+    h->n_tiles = nblk(h->seg_hi - (h->seg_lo - (h->seg_first ? 0 : 1)), RT_TILE);
+    h->n_solve_tiles = nblk(h->seg_hi - h->seg_lo, ST_OWN);
+    h->ex.d_keys_out.reset(); h->ex.d_iota.reset(); h->ex.d_sorted.reset();      // (the running view sizes them by n on first use)
+    const size_t n = (size_t)h->n;
     CK(h->ex.d_bxy.alloc(n + 2));
-    k_interleave<<<nblk((int64_t)n, 256), 256, 0, h->stream>>>(h->ex.d_bx, h->ex.d_by, (int64_t)n, h->ex.d_bxy);
+    k_interleave<<<nblk((int64_t)n, 256), 256, 0, s>>>(h->ex.d_bx, h->ex.d_by, (int64_t)n, h->ex.d_bxy);
     CK(cudaGetLastError());
     {   // run records and their bookkeeping (runs.cuh): slice s (32 scans) owns slots [s * maxr * 32, (s + 1) * maxr * 32)
         const size_t nt = (size_t)nblk(T + 1, RT_TILE) + 2;      // (+1 scan: a segment's tiling may start one scan earlier)
@@ -620,28 +706,28 @@ extern "C" int icmslam_extract(icmslam_handle* h)
         CK(h->ex.d_nruns.alloc(nt * RT_TILE));
         CK(h->ex.d_tile_perm.alloc(nt * RT_TILE));
         CK(h->ex.d_pos_nruns.alloc(nt * RT_TILE));
-        CK(cudaMemsetAsync(h->ex.d_pos_nruns, 0, nt * RT_TILE * sizeof(unsigned short), h->stream));
-        CK(cudaMemsetAsync(h->ex.d_tile_perm, 0, nt * RT_TILE, h->stream));      // (rewritten with every tile's records; never read before)
+        CK(cudaMemsetAsync(h->ex.d_pos_nruns, 0, nt * RT_TILE * sizeof(unsigned short), s));
+        CK(cudaMemsetAsync(h->ex.d_tile_perm, 0, nt * RT_TILE, s));      // (rewritten with every tile's records; never read before)
         CK(h->ex.d_ppar[0].alloc((size_t)T)); CK(h->ex.d_ppar[1].alloc((size_t)T));
         CK(h->ex.d_farbits.alloc(nt * 4)); CK(h->ex.d_tile_epoch.alloc(nt));
         CK(h->ex.d_tile_flag.alloc(nt)); CK(h->ex.d_dirty_list.alloc(nt)); CK(h->ex.d_tile_slots.alloc(nt * RS_SLOTS)); CK(h->ex.d_tile_nslots.alloc(nt));
-        CK(cudaMemsetAsync(h->ex.d_tile_nslots, 0, nt * sizeof(int), h->stream));
+        CK(cudaMemsetAsync(h->ex.d_tile_nslots, 0, nt * sizeof(int), s));
         CK(h->ex.d_scan_dirty.alloc(nt * RT_TILE));
-        CK(cudaMemsetAsync(h->ex.d_nruns, 0, nt * RT_TILE * sizeof(unsigned short), h->stream));
-        CK(cudaMemsetAsync(h->ex.d_tile_epoch, 0xff, nt * sizeof(int), h->stream));       // epoch -1: no tile holds records
-        CK(cudaMemsetAsync(h->ex.d_tile_flag, 0, nt * sizeof(int), h->stream));
-        CK(cudaMemsetAsync(h->ex.d_farbits, 0, nt * 4 * sizeof(unsigned), h->stream));
-        CK(cudaMemsetAsync(h->ex.d_scan_dirty, 0, nt * RT_TILE * sizeof(int), h->stream));
+        CK(cudaMemsetAsync(h->ex.d_nruns, 0, nt * RT_TILE * sizeof(unsigned short), s));
+        CK(cudaMemsetAsync(h->ex.d_tile_epoch, 0xff, nt * sizeof(int), s));       // epoch -1: no tile holds records
+        CK(cudaMemsetAsync(h->ex.d_tile_flag, 0, nt * sizeof(int), s));
+        CK(cudaMemsetAsync(h->ex.d_farbits, 0, nt * 4 * sizeof(unsigned), s));
+        CK(cudaMemsetAsync(h->ex.d_scan_dirty, 0, nt * RT_TILE * sizeof(int), s));
     }
     CK(h->ex.d_bm.alloc((size_t)6 * T));
     CK(h->ex.d_dyn.alloc((size_t)6 * T));
-    CK(cudaMemsetAsync(h->ex.d_dyn, 0, (size_t)6 * T * sizeof(double), h->stream));
-    k_body_moments<<<nblk(T, 128), 128, 0, h->stream>>>(h->ex.d_off, h->ex.d_bxy, T, h->ex.d_bm, T);
+    CK(cudaMemsetAsync(h->ex.d_dyn, 0, (size_t)6 * T * sizeof(double), s));
+    k_body_moments<<<nblk(T, 128), 128, 0, s>>>(h->ex.d_off, h->ex.d_bxy, T, h->ex.d_bm, T);
     CK(cudaGetLastError());
-    CK(cudaStreamSynchronize(h->stream));
-    h->extracted = true;
+    CK(cudaStreamSynchronize(s));
     {   // shared-memory budget of the association kernel: observations of one tile of RT_TILE scans
         int mx = 0;
+        const std::vector<int>& off = h->off_h;
         for (int tb = 0; tb < T; ++tb) {   // (any tile origin: a later icmslam_set_segment may shift the tiling)
             int t1 = tb + RT_TILE < T ? tb + RT_TILE : T;
             int m = off[t1] - off[tb];
@@ -667,7 +753,56 @@ extern "C" int icmslam_extract(icmslam_handle* h)
         CK(cudaFuncSetAttribute(k_assoc_tiles, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
         h->fused_ok = h->max_per_scan <= 65535 && h->Lcap <= RUN_MAX_LABEL;
     }
+    h->laid_out = true;
     return ICMSLAM_OK;
+}
+
+extern "C" int icmslam_extract(icmslam_handle* h)
+{
+    if (!h || !h->ds.d_scans) return ICMSLAM_ERR_INVALID;
+    CK(cudaSetDevice(h->cfg.device));
+    reset_extraction(h);
+    int rc = extract_window(h, 0);
+    if (rc) return rc;
+    return ensure_layout(h);
+}
+
+extern "C" int icmslam_append(icmslam_handle* h, const double* scans, int32_t n_new, int64_t ld_scans, const double* odometry,
+                              int64_t ld_odo, const double* controls, int64_t ld_u, int32_t memspace)
+{
+    if (!h || !h->ds.d_scans || !scans || !odometry || !controls || n_new <= 0 || ld_scans < n_new || ld_odo < n_new || ld_u < n_new)
+        return ICMSLAM_ERR_INVALID;
+    if ((int64_t)h->T + n_new > INT32_MAX) return ICMSLAM_ERR_INVALID;
+    if (h->traj_K > 0 || h->seg_lo != 0 || h->seg_hi != h->T || !h->seg_first || !h->seg_last || h->p2p.on) return ICMSLAM_ERR_UNSUPPORTED;
+    (void)memspace;
+    CK(cudaSetDevice(h->cfg.device));
+    // captured graphs, the map chain and the projection parameters hold buffers that move or columns that change (the odometry
+    // increment of the old last column reads the new first one)
+    drop_graphs(h);
+    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr;
+    int rc = poses_home(h);
+    if (rc) return rc;
+    const int T0 = h->T, T = T0 + n_new;
+    const int t_lo = h->extracted ? T0 : 0;      // (a log loaded but not extracted yet is extracted whole)
+    if (T > h->cap_T) {
+        const int cap = std::max(2 * h->cap_T, T);
+        CK(regrow(h, h->ds.d_scans, h->B, h->cap_T, T0, cap));
+        CK(regrow(h, h->ds.d_odo, 3, h->cap_T, T0, cap));
+        CK(regrow(h, h->ds.d_u, 2, h->cap_T, T0, cap));
+        CK(regrow(h, h->ds.d_x, 3, h->cap_T, T0, cap));
+        if (h->ex.d_off) CK(regrow(h, h->ex.d_off, 1, (int64_t)T0 + 1, h->extracted ? (int64_t)T0 + 1 : 0, (int64_t)cap + 1));
+        h->cap_T = cap;
+    }
+    const size_t ld = (size_t)h->cap_T * sizeof(double), w = (size_t)n_new * sizeof(double);
+    CK(cudaMemcpy2DAsync(h->ds.d_scans + T0, ld, scans, (size_t)ld_scans * sizeof(double), w, h->B, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(h->ds.d_odo + T0, ld, odometry, (size_t)ld_odo * sizeof(double), w, 3, cudaMemcpyDefault, h->stream));
+    CK(cudaMemcpy2DAsync(h->ds.d_u + T0, ld, controls, (size_t)ld_u * sizeof(double), w, 2, cudaMemcpyDefault, h->stream));
+    h->T = T;
+    h->seg_hi = T;
+    h->laid_out = false;
+    rc = size_cub(h);
+    if (rc) return rc;
+    return extract_window(h, t_lo);      // (ends in a stream synchronise: the caller's buffers may go away)
 }
 
 extern "C" int icmslam_extraction_size(const icmslam_handle* h, int64_t* n_obs, int32_t* n_empty, int32_t* max_per_scan)
@@ -1179,8 +1314,8 @@ static bool pipe_ready(icmslam_handle* h)
 static int ensure_seen(icmslam_handle* h)
 {
     if (h->ex.d_seen_x && h->ex.d_seen_y) return ICMSLAM_OK;
-    CK(h->ex.d_seen_x.alloc((size_t)h->n));
-    CK(h->ex.d_seen_y.alloc((size_t)h->n));
+    CK(h->ex.d_seen_x.alloc((size_t)h->n_cap));      // (the room of the per-observation arrays: an append grows them together)
+    CK(h->ex.d_seen_y.alloc((size_t)h->n_cap));
     return ICMSLAM_OK;
 }
 
@@ -1346,6 +1481,10 @@ extern "C" int icmslam_sweep(icmslam_handle* h, const double* map_in, int32_t L_
     icmslam_sweep_opts o;
     default_opts(o, opts);
     CK(cudaSetDevice(h->cfg.device));
+    {
+        int rc = ensure_layout(h);
+        if (rc) return rc;
+    }
     const int T = h->T, L = h->Lcap;
     cudaStream_t s = h->stream;
     if (h->first_empty) {   // sensors.py:137-139: inputs returned unchanged
@@ -1444,6 +1583,8 @@ extern "C" int icmslam_set_map(icmslam_handle* h, const double* map, int32_t L_m
     if (!h || L_map < 0 || L_map > h->Lcap || (L_map > 0 && (!map || ld < L_map))) return ICMSLAM_ERR_INVALID;
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
+    int rc = ensure_layout(h);
+    if (rc) return rc;
     if (L_map > 0)
         CK(cudaMemcpy2DAsync(h->d_map_in, (size_t)h->Lcap * 8, map, (size_t)ld * 8, (size_t)L_map * 8, 2, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -1478,6 +1619,8 @@ extern "C" int icmslam_set_poses(icmslam_handle* h, const double* x, int64_t ld_
     if (!h || !h->ds.d_x || !x || ld_x < h->T) return ICMSLAM_ERR_INVALID;
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
+    int rc = ensure_layout(h);
+    if (rc) return rc;
     const int T = h->T;
     CK(cudaMemcpy2DAsync(h->ds.d_x, (size_t)T * 8, x, (size_t)ld_x * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -1491,8 +1634,8 @@ extern "C" int icmslam_get_poses(icmslam_handle* h, double* x, int64_t ld_x, int
     if (!h || !h->ds.d_x || !x || ld_x < h->T) return ICMSLAM_ERR_INVALID;
     (void)memspace;
     CK(cudaSetDevice(h->cfg.device));
-    const int T = h->T;
-    CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, cur_x(h), (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
+    const int T = h->T;      // (the resident poses have leading dimension cap_T, which is T unless an append grew the log)
+    CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, cur_x(h), (size_t)h->cap_T * 8, (size_t)T * 8, 3, cudaMemcpyDefault, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return ICMSLAM_OK;
 }
@@ -1504,6 +1647,10 @@ extern "C" int icmslam_iterate(icmslam_handle* h, double* x, int64_t ld_x, const
     icmslam_sweep_opts o;
     default_opts(o, opts);
     CK(cudaSetDevice(h->cfg.device));
+    {
+        int rc = ensure_layout(h);
+        if (rc) return rc;
+    }
     const int T = h->T, L = h->Lcap;
     cudaStream_t s = h->stream;
     h->last_map_L = -1;
@@ -1615,6 +1762,8 @@ extern "C" int icmslam_set_batch(icmslam_handle* h, int32_t traj_T, const double
 {
     if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
+    int rc = ensure_layout(h);
+    if (rc) return rc;
     if (traj_T <= 0) {
         drop_graphs(h);
         h->traj_K = 0; h->traj_odd = false; h->d_traj_start.reset(); h->d_traj_of.reset(); h->d_x0s.reset();
@@ -1631,6 +1780,8 @@ extern "C" int icmslam_set_batch_lengths(icmslam_handle* h, const int32_t* lengt
 {
     if (!h || !h->extracted) return ICMSLAM_ERR_INVALID;
     CK(cudaSetDevice(h->cfg.device));
+    int rc = ensure_layout(h);
+    if (rc) return rc;
     if (!lengths || !x0s || K <= 0 || ld_x0s < K || !h->fused_ok) return ICMSLAM_ERR_INVALID;
     std::vector<int> start((size_t)K + 1, 0);
     int64_t sum = 0;
@@ -1649,6 +1800,8 @@ extern "C" int icmslam_set_segment(icmslam_handle* h, int32_t t_lo, int32_t t_hi
 {
     if (!h || !h->extracted || t_lo < 0 || t_hi > h->T || t_lo >= t_hi || (t_lo & 1)) return ICMSLAM_ERR_INVALID;
     if ((!is_first && t_lo < 2) || (!is_last && t_hi > h->T - 1)) return ICMSLAM_ERR_INVALID;   // halo columns must exist
+    int rc = ensure_layout(h);
+    if (rc) return rc;
     h->seg_lo = t_lo; h->seg_hi = t_hi; h->seg_first = is_first ? 1 : 0; h->seg_last = is_last ? 1 : 0;
     h->n_tiles = nblk(t_hi - (t_lo - (is_first ? 0 : 1)), RT_TILE);
     h->n_solve_tiles = nblk(t_hi - t_lo, ST_OWN);
@@ -1661,6 +1814,8 @@ extern "C" int icmslam_set_segment(icmslam_handle* h, int32_t t_lo, int32_t t_hi
 extern "C" int icmslam_device_ptr(icmslam_handle* h, int32_t which, void** ptr, int64_t* count)
 {
     if (!h || !ptr || !count) return ICMSLAM_ERR_INVALID;
+    int rc = ensure_layout(h);      // (the poses with leading dimension T)
+    if (rc) return rc;
     const int64_t L = h->Lcap;
     switch (which) {
     case ICMSLAM_PTR_SEG_REC: *ptr = h->d_seg_rec; *count = SEG_REC; break;
@@ -1738,7 +1893,13 @@ extern "C" int icmslam_p2p_import(icmslam_handle* h, int32_t rank, int32_t world
 // (boundary poses, far-scan count) in the ICMSLAM_PTR_SEG_REC buffer for the all-gather.
 extern "C" int icmslam_seg_begin(icmslam_handle* h, const double* x0, const icmslam_sweep_opts* opts)
 {
-    if (!h || !h->extracted || !x0 || !h->fused_ok) return ICMSLAM_ERR_INVALID;
+    if (!h || !h->extracted || !x0) return ICMSLAM_ERR_INVALID;
+    {
+        CK(cudaSetDevice(h->cfg.device));
+        int rc = ensure_layout(h);
+        if (rc) return rc;
+    }
+    if (!h->fused_ok) return ICMSLAM_ERR_INVALID;
     icmslam_sweep_opts o;
     default_opts(o, opts);
     if (!fused_mode(h, o)) return ICMSLAM_ERR_UNSUPPORTED;     // only the restated parallel sweep partitions in time (DESIGN.md)
@@ -2400,92 +2561,162 @@ extern "C" int icmslam_filtrar_obs(icmslam_handle* h, const double* obs, int32_t
     return err ? ICMSLAM_ERR_INVALID : ICMSLAM_OK;
 }
 
-// ---- pass 0: inicializar_online replayed on the loaded log (sensors.py:51-123) ---------------------------------
-// x (3 x T) receives the causal pose estimates (x[:,0] = x0), map_out the filtered map (`mapa_viejo`,
-// sensors.py:99-102), *L_out its width; landmarks_actuales / cant_obs_i are left as the reference leaves them.
-extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int64_t ld_x, double* map_out, int32_t cap_out,
-                             int64_t ld_map_out, int32_t* L_out, int32_t memspace)
+// ---- pass 0: inicializar_online on the loaded log (sensors.py:51-123), as a walk that can stop and resume ---------------------
+// begin: x0 and an empty walk.  advance: the steps of every loaded column the walk has not taken (Branch A / fcluster on the host
+// at column 0, then k_pass0); the poses go to the resident pose buffer, the labels and running means to the per-observation
+// arrays, the map under construction and its counts to the walk's own buffers, published as the handle's raw map.  finish:
+// Mapa.filtrar of the map built so far (sensors.py:99-102).
+// the walk's map under construction becomes the handle's raw map (d_raw, d_rawcnt, raw_l), as icmslam_pass0 leaves it
+static int publish_walk(icmslam_handle* h)
 {
-    if (!h || !h->extracted || !x0 || !x || ld_x < h->T || !L_out) return ICMSLAM_ERR_INVALID;
-    if (map_out && (cap_out <= 0 || ld_map_out < cap_out)) return ICMSLAM_ERR_INVALID;
-    if (h->max_per_scan > 1024) return ICMSLAM_ERR_UNSUPPORTED;
-    CK(cudaSetDevice(h->cfg.device));
-    const int T = h->T, L = h->Lcap;
-    cudaStream_t s = h->stream;
+    const int L = h->Lcap;
+    CK(cudaMemcpyAsync(h->d_raw, h->walk.y, (size_t)2 * L * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+    k_walk_publish<<<nblk(L, 256), 256, 0, h->stream>>>(h->walk.carry, h->walk.cant, L, h->d_rawcnt, h->d_st);
+    CK(cudaGetLastError());
+    h->n_launch += 1;
+    h->ch.rawcnt_valid = true;
+    h->ch.lact_dirty = true;
+    return ICMSLAM_OK;
+}
+
+extern "C" int icmslam_pass0_begin(icmslam_handle* h, const double* x0)
+{
+    if (!h || !h->extracted || !x0) return ICMSLAM_ERR_INVALID;
+    h->walk.on = false;
     if (h->first_empty) return ICMSLAM_EMPTY_FIRST_SCAN;        // (the reference would fail inside tras_rot_z / linkage)
-    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr;
+    CK(cudaSetDevice(h->cfg.device));
     int rc = ensure_seen(h);
     if (rc) return rc;
-    // ---- step 0: Branch A of Mapa.actualizar on the first scan (ICM_SLAM.py:160-165), on the host ------------------
-    std::vector<int> off2(2);
-    CK(cudaMemcpyAsync(off2.data(), h->ex.d_off, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    const int n0 = off2[1] - off2[0];
-    DevBuf<double> d_w;
-    CK(d_w.alloc((size_t)2 * n0));
-    k_project_scan<<<nblk(n0, 128), 128, 0, s>>>(h->ex.d_off, 0, h->ex.d_bx, h->ex.d_by, x0[0], x0[1], x0[2], d_w, d_w + n0);
-    CK(cudaGetLastError());
-    std::vector<double> w((size_t)2 * n0);
-    CK(cudaMemcpyAsync(w.data(), d_w, (size_t)2 * n0 * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    std::vector<int> lab0(n0);
-    const int k0 = icm_fcluster::fcluster_inconsistent(w.data(), w.data() + n0, n0, h->cfg.dist_thr, lab0.data());
-    if (k0 > L) return ICMSLAM_ERR_LABEL_CAP;
-    std::vector<double> y0((size_t)2 * L, 0.0), cant0((size_t)L, 0.0);
-    for (int i = 0; i < k0; ++i) {                                // np.mean(obs[c==i,:], axis=0): row-order sum / count
-        double sx = 0.0, sy = 0.0;
-        int k = 0;
-        for (int j = 0; j < n0; ++j) if (lab0[j] == i) { sx += w[j]; sy += w[n0 + j]; ++k; }
-        y0[i] = sx / (double)k; y0[L + i] = sy / (double)k; cant0[i] = (double)k;
-    }
-    CK(cudaMemcpyAsync(h->d_raw, y0.data(), (size_t)2 * L * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(h->d_tmp_b, cant0.data(), (size_t)L * 8, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(h->ex.d_c, lab0.data(), (size_t)n0 * sizeof(int), cudaMemcpyHostToDevice, s));
-    // ---- steps 1 .. T-1 on the device -------------------------------------------------------------------------------
-    double* dx = x;
-    int64_t ldx = ld_x;
-    if (memspace == ICMSLAM_HOST) { dx = h->ds.d_x; ldx = T; }
-    Pass0Params P;
-    P.T = T; P.Lcap = L; P.off = h->ex.d_off; P.bx = h->ex.d_bx; P.by = h->ex.d_by; P.d = h->ex.d_d; P.beam = h->ex.d_beam; P.ang = h->ds.d_ang;
-    P.odo = h->ds.d_odo; P.ldo = T; P.u = h->ds.d_u; P.ldu = T; P.cfg = h->dcfg;
-    P.x0[0] = x0[0]; P.x0[1] = x0[1]; P.x0[2] = x0[2];
-    P.x = dx; P.ldx = ldx; P.y = h->d_raw; P.cant = h->d_tmp_b; P.lact0 = k0; P.c = h->ex.d_c; P.seen_x = h->ex.d_seen_x; P.seen_y = h->ex.d_seen_y;
-    P.st = h->d_st; P.nev = &h->d_st->newton_iters;
-    k_set_raw_l<<<1, 1, 0, s>>>(h->d_st, k0);                     // (also clears the status word)
-    CK(cudaGetLastError());
-    CK(cudaMemsetAsync(&h->d_st->newton_iters, 0, sizeof(unsigned long long), s));
-    const size_t smem = (size_t)2 * 1024 * 8 + 1024 * 4;
-    k_pass0<<<1, 256, smem, s>>>(P);
-    CK(cudaGetLastError());
-    h->n_launch += 2;
-    rc = sync_state(h);
+    h->walk.on = true;
+    h->walk.t = 0; h->walk.lact = 0;
+    h->walk.x0[0] = x0[0]; h->walk.x0[1] = x0[1]; h->walk.x0[2] = x0[2];
+    return ICMSLAM_OK;
+}
+
+extern "C" int icmslam_pass0_advance(icmslam_handle* h, int32_t* t_done)
+{
+    if (!h || !h->walk.on || !t_done) return ICMSLAM_ERR_INVALID;
+    const int T = h->T, L = h->Lcap;
+    int t_lo = h->walk.t;
+    *t_done = t_lo;
+    for (int t = t_lo; t < T; ++t)
+        if (h->off_h[t + 1] - h->off_h[t] > 1024) return ICMSLAM_ERR_UNSUPPORTED;      // (k_pass0 stages one scan in shared memory)
+    CK(cudaSetDevice(h->cfg.device));
+    cudaStream_t s = h->stream;
+    int rc = ensure_seen(h);
     if (rc) return rc;
-    if (h->h_st->status & ST_LABEL_CAP) return ICMSLAM_ERR_LABEL_CAP;
-    const int lact = h->h_st->lact;
-    h->ch.x_cur = 0;
-    h->ch.ppar_of = nullptr;
-    // ---- Mapa.filtrar on the map that was built (sensors.py:99-100) ---------------------------------------------------
+    // the walk rewrites labels (the map chain's hints), the resident poses and the raw map
+    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr;
+    rc = poses_home(h);
+    if (rc) return rc;
+    const double* x0 = h->walk.x0;
+    int k0 = 0;
+    if (t_lo == 0) {    // ---- step 0: Branch A of Mapa.actualizar on the first scan (ICM_SLAM.py:160-165), on the host ------------
+        const int n0 = h->off_h[1] - h->off_h[0];
+        DevBuf<double> d_w;
+        CK(d_w.alloc((size_t)2 * n0));
+        k_project_scan<<<nblk(n0, 128), 128, 0, s>>>(h->ex.d_off, 0, h->ex.d_bx, h->ex.d_by, x0[0], x0[1], x0[2], d_w, d_w + n0);
+        CK(cudaGetLastError());
+        std::vector<double> w((size_t)2 * n0);
+        CK(cudaMemcpyAsync(w.data(), d_w, (size_t)2 * n0 * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        std::vector<int> lab0(n0);
+        k0 = icm_fcluster::fcluster_inconsistent(w.data(), w.data() + n0, n0, h->cfg.dist_thr, lab0.data());
+        if (k0 > L) { h->walk.on = false; return ICMSLAM_ERR_LABEL_CAP; }
+        std::vector<double> y0((size_t)2 * L, 0.0), cant0((size_t)L, 0.0);
+        for (int i = 0; i < k0; ++i) {                                // np.mean(obs[c==i,:], axis=0): row-order sum / count
+            double sx = 0.0, sy = 0.0;
+            int k = 0;
+            for (int j = 0; j < n0; ++j) if (lab0[j] == i) { sx += w[j]; sy += w[n0 + j]; ++k; }
+            y0[i] = sx / (double)k; y0[L + i] = sy / (double)k; cant0[i] = (double)k;
+        }
+        CK(cudaMemcpyAsync(h->walk.y, y0.data(), (size_t)2 * L * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(h->walk.cant, cant0.data(), (size_t)L * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(h->ex.d_c, lab0.data(), (size_t)n0 * sizeof(int), cudaMemcpyHostToDevice, s));
+        CK(cudaMemsetAsync(&h->d_st->newton_iters, 0, sizeof(unsigned long long), s));
+        t_lo = 1;
+    }
+    // ---- steps t_lo .. T-1 on the device ----------------------------------------------------------------------------------
+    if (h->walk.t == 0 || t_lo < T) {      // (after step 0 even at T = 1: the launch starts the carry)
+        Pass0Params P;
+        P.t_lo = t_lo; P.t_hi = T; P.Lcap = L;
+        P.off = h->ex.d_off; P.bx = h->ex.d_bx; P.by = h->ex.d_by; P.d = h->ex.d_d; P.beam = h->ex.d_beam; P.ang = h->ds.d_ang;
+        P.odo = h->ds.d_odo; P.ldo = h->cap_T; P.u = h->ds.d_u; P.ldu = h->cap_T; P.cfg = h->dcfg;
+        P.first = h->walk.t == 0 ? 1 : 0;
+        P.x0[0] = x0[0]; P.x0[1] = x0[1]; P.x0[2] = x0[2]; P.lact0 = k0; P.carry = h->walk.carry;
+        P.x = h->ds.d_x; P.ldx = h->cap_T; P.y = h->walk.y; P.cant = h->walk.cant;
+        P.c = h->ex.d_c; P.seen_x = h->ex.d_seen_x; P.seen_y = h->ex.d_seen_y;
+        P.st = h->d_st; P.nev = &h->d_st->newton_iters;
+        const size_t smem = (size_t)2 * 1024 * 8 + 1024 * 4;
+        k_pass0<<<1, 256, smem, s>>>(P);
+        CK(cudaGetLastError());
+        h->n_launch += 1;
+        Pass0Carry c;
+        CK(cudaMemcpyAsync(&c, h->walk.carry, sizeof c, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        h->walk.lact = c.lact;
+        *t_done = c.t;
+        if (c.t < T) {      // the label cap: the walk stops at the column that needed a label beyond L (begin it again)
+            h->walk.on = false;
+            h->ch.lact_dirty = true;
+            return ICMSLAM_ERR_LABEL_CAP;
+        }
+    }
+    h->walk.t = T;
+    *t_done = T;
+    return publish_walk(h);
+}
+
+extern "C" int icmslam_pass0_finish(icmslam_handle* h, double* x, int64_t ld_x, double* map_out, int32_t cap_out, int64_t ld_map_out,
+                                    int32_t* L_out, int32_t memspace)
+{
+    if (!h || !h->walk.on || !x || ld_x < h->walk.t || !L_out) return ICMSLAM_ERR_INVALID;
+    if (map_out && (cap_out <= 0 || ld_map_out < cap_out)) return ICMSLAM_ERR_INVALID;
+    (void)memspace;
+    CK(cudaSetDevice(h->cfg.device));
+    const int L = h->Lcap, tw = h->walk.t, lact = h->walk.lact;
+    cudaStream_t s = h->stream;
+    int rc = ensure_layout(h);
+    if (rc) return rc;
+    rc = publish_walk(h);
+    if (rc) return rc;
+    // ---- Mapa.filtrar on the map that was built (sensors.py:99-100) ---------------------------------------------------------
+    h->ch.grid_map = nullptr; h->ch.hint_map = nullptr;
     h->ch.stats_clean = false;
-    k_counts_to_int<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, L, h->d_cnt);      // (get_raw_map reports integer counts)
+    k_counts_to_int<<<nblk(L, 256), 256, 0, s>>>(h->walk.cant, L, h->d_cnt);      // (get_raw_map reports integer counts)
     CK(cudaGetLastError());
-    k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->d_tmp_b, lact, h->dcfg.cota, h->d_kflag, L, h->d_blk_kept, h->grid.bb, h->d_ts);
+    k_flags_from_counts<<<nblk(L, 256), 256, 0, s>>>(h->walk.cant, lact, h->dcfg.cota, h->d_kflag, L, h->d_blk_kept, h->grid.bb, h->d_ts);
     CK(cudaGetLastError());
     rc = filter_chain(h, h->d_raw, h->d_raw + L, nullptr, h->d_map_out, L, L, s, false);
     if (rc) return rc;
-    h->ch.rawcnt_valid = true;
     rc = sync_state(h);
     if (rc) return rc;
     int status = status_from_state(h->h_st);
     if (status) return status;
     const int newL = h->h_st->new_l;
     *L_out = newL;
-    if (memspace == ICMSLAM_HOST)
-        CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, dx, (size_t)T * 8, (size_t)T * 8, 3, cudaMemcpyDeviceToHost, s));
+    if (tw > 0) CK(cudaMemcpy2DAsync(x, (size_t)ld_x * 8, h->ds.d_x, (size_t)h->cap_T * 8, (size_t)tw * 8, 3, cudaMemcpyDefault, s));
     const int wd = newL < cap_out ? newL : cap_out;
     if (map_out && wd > 0)
         CK(cudaMemcpy2DAsync(map_out, (size_t)ld_map_out * 8, h->d_map_out, (size_t)L * 8, (size_t)wd * 8, 2, cudaMemcpyDefault, s));
     CK(cudaStreamSynchronize(s));
     return ICMSLAM_OK;
+}
+
+// x (3 x T) receives the causal pose estimates (x[:,0] = x0), map_out the filtered map (`mapa_viejo`, sensors.py:99-102), *L_out
+// its width; landmarks_actuales / cant_obs_i are left as the reference leaves them.  One walk over the whole log.
+extern "C" int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int64_t ld_x, double* map_out, int32_t cap_out,
+                             int64_t ld_map_out, int32_t* L_out, int32_t memspace)
+{
+    if (!h || !h->extracted || !x0 || !x || ld_x < h->T || !L_out) return ICMSLAM_ERR_INVALID;
+    if (map_out && (cap_out <= 0 || ld_map_out < cap_out)) return ICMSLAM_ERR_INVALID;
+    if (h->max_per_scan > 1024) return ICMSLAM_ERR_UNSUPPORTED;
+    int rc = icmslam_pass0_begin(h, x0);
+    if (rc) return rc;
+    int32_t t_done = 0;
+    rc = icmslam_pass0_advance(h, &t_done);
+    if (rc) return rc;
+    return icmslam_pass0_finish(h, x, ld_x, map_out, cap_out, ld_map_out, L_out, memspace);
 }
 
 // ---- pass 0 helpers ---------------------------------------------------------------------------------------------

@@ -8,24 +8,32 @@
 // ICM_SLAM.py:167-194) and ONE thread runs the reference's Nelder-Mead on fun_x (sensors.py:258-282)
 // operation for operation, so the poses match the reference to 1e-6 m / 1e-8 rad.  Step 0 (Branch A of
 // Mapa.actualizar, scipy's fcluster) runs on the host (fcluster.h) before the kernel.
-// Not a hot path: it runs once per log and is not part of the sweeps/s metric.
+// The walk can stop and resume: one launch takes the columns [t_lo, t_hi) and carries the last pose and landmarks_actuales
+// in device memory (Pass0Carry) to the next launch, beside the map under construction and its counts, so that columns appended
+// to a loaded log are walked as they arrive (icmslam_pass0_advance).
+// Not a hot path: it runs once per column and is not part of the sweeps/s metric.
 #pragma once
 #include "common.cuh"
 #include "assoc.cuh"
 #include "pose.cuh"
 
+// what the walk carries from one launch to the next: the pose of the last column walked, landmarks_actuales, columns walked
+struct Pass0Carry { double x[3]; int lact; int t; };
+
 struct Pass0Params {
-    int T, Lcap;
+    int t_lo, t_hi, Lcap;            // the columns this launch walks (t_lo >= 1)
     const int* off;
     const double *bx, *by, *d; const int* beam; const double* ang;
     const double* odo; int64_t ldo;
     const double* u; int64_t ldu;
     DevCfg cfg;
+    int first;                       // t_lo == 1 after step 0: the carry starts from x0 / lact0 and x[:,0] = x0
     double x0[3];
-    double* x; int64_t ldx;          // 3 x T poses (out); x[:,0] = x0
-    double* y;                       // 2 x Lcap map under construction (in: clusters of scan 0)
-    double* cant;                    // Lcap observation counts (in: cluster sizes)
     int lact0;                       // landmarks after scan 0
+    Pass0Carry* carry;               // in (unless first) and out
+    double* x; int64_t ldx;          // 3 x T poses (out: columns [t_lo, t_hi))
+    double* y;                       // 2 x Lcap map under construction (in / out; after step 0: clusters of scan 0)
+    double* cant;                    // Lcap observation counts (in / out; after step 0: cluster sizes)
     int* c;                          // labels per observation (out; scan 0 filled by the host)
     double *seen_x, *seen_y;         // per observation: its landmark's running mean after the scan
     DevState* st;
@@ -56,15 +64,21 @@ k_pass0(const Pass0Params p)
     int* cl = reinterpret_cast<int*>(wy + 1024);
     double* yx = p.y;
     double* yy = p.y + cap;
-    if (tid == 0) { xt[0] = p.x0[0]; xt[1] = p.x0[1]; xt[2] = p.x0[2]; s_lact = p.lact0; s_abort = 0; }
-    if (tid < 3) p.x[tid * p.ldx] = p.x0[tid];
+    if (tid == 0) {
+        const double* x_last = p.first ? p.x0 : p.carry->x;
+        xt[0] = x_last[0]; xt[1] = x_last[1]; xt[2] = x_last[2];
+        s_lact = p.first ? p.lact0 : p.carry->lact;
+        s_abort = 0;
+    }
+    if (p.first && tid < 3) p.x[tid * p.ldx] = p.x0[tid];
     __syncthreads();
     ObsArrays O;
     O.bx = p.bx; O.by = p.by; O.d = p.d; O.beam = p.beam; O.ang = p.ang;
     SeenSrc S;
     S.view = ICMSLAM_VIEW_RUNNING; S.c = p.c; S.seen_x = p.seen_x; S.seen_y = p.seen_y;
     S.raw_x = nullptr; S.raw_y = nullptr; S.min_x = nullptr; S.min_y = nullptr; S.lsearch_ptr = nullptr;
-    for (int t = 1; t < p.T; ++t) {
+    int t = p.t_lo;
+    for (; t < p.t_hi; ++t) {
         if (tid == 0) {
             const double ua[2] = {p.u[t - 1], p.u[p.ldu + t - 1]};
             g_step(xt, ua[0], ua[1], p.cfg.dt, xtc);               // sensors.py:111
@@ -141,5 +155,19 @@ k_pass0(const Pass0Params p)
         }
         __syncthreads();
     }
-    if (tid == 0) { p.st->lact = s_lact; p.st->raw_l = s_lact; }
+    if (tid == 0) {      // (on the label cap t is the column that could not be walked)
+        p.carry->x[0] = xt[0]; p.carry->x[1] = xt[1]; p.carry->x[2] = xt[2];
+        p.carry->lact = s_lact; p.carry->t = t;
+        p.st->lact = s_lact; p.st->raw_l = s_lact;
+    }
+}
+
+// the walk's construction becomes the handle's raw map (icmslam_get_raw_map): counts, width and landmarks_actuales (the map
+// itself is copied beside this launch); the status word is cleared as a fresh pass 0 clears it
+__global__ void k_walk_publish(const Pass0Carry* __restrict__ carry, const double* __restrict__ cant, int Lcap, int* __restrict__ rawcnt,
+                               DevState* st)
+{
+    const int l = blockIdx.x * blockDim.x + threadIdx.x;
+    if (l < Lcap) rawcnt[l] = (int)cant[l];
+    if (l == 0) { st->lact = carry->lact; st->raw_l = carry->lact; st->status = 0; }
 }

@@ -46,7 +46,9 @@ def _rows(a, nrows):
         import torch
         assert a.dtype == torch.float64 and a.dim() == 2 and a.shape[0] == nrows and a.stride(1) == 1, "need fp64 (%d, n) row-major" % nrows
         return int(a.stride(0)) if a.shape[0] > 1 else int(a.shape[1])
-    assert a.dtype == np.float64 and a.ndim == 2 and a.shape[0] == nrows and a.strides[1] == 8, "need fp64 (%d, n) row-major" % nrows
+    # (the stride of a dimension of size 1 is arbitrary in numpy: one column is row-major whatever its column stride says)
+    assert a.dtype == np.float64 and a.ndim == 2 and a.shape[0] == nrows and (a.strides[1] == 8 or a.shape[1] == 1), \
+        "need fp64 (%d, n) row-major" % nrows
     return int(a.strides[0] // 8) if a.shape[0] > 1 else int(a.shape[1])
 
 
@@ -100,14 +102,38 @@ class Engine:
         self.B, self.T = B, T
         self.n = 0
 
-    def extract(self):
-        check(self.lib.icmslam_extract(self._h), self._h)
+    def _extraction_size(self):
         n = C.c_int64()
         ne = C.c_int32()
         mx = C.c_int32()
         check(self.lib.icmslam_extraction_size(self._h, C.byref(n), C.byref(ne), C.byref(mx)), self._h)
         self.n, self.n_empty, self.max_per_scan = int(n.value), int(ne.value), int(mx.value)
         return self.n
+
+    def extract(self):
+        check(self.lib.icmslam_extract(self._h), self._h)
+        return self._extraction_size()
+
+    def append(self, scans, odometry, controls):
+        """More columns of the loaded log (scans B x n_new, odometry 3 x n_new, controls 2 x n_new; pre-conditioned as `load`
+        was told), extracted on arrival: the handle then holds what load + extract of the whole log give.  Returns n_obs."""
+        if not _is_torch(scans):
+            scans = np.asarray(scans, dtype=np.float64)
+            odometry = np.asarray(odometry, dtype=np.float64)
+            controls = np.asarray(controls, dtype=np.float64)
+            if scans.ndim != 2 or scans.strides[1] != 8:
+                scans = np.ascontiguousarray(scans)
+            if odometry.ndim != 2 or odometry.strides[1] != 8:
+                odometry = np.ascontiguousarray(odometry)
+            if controls.ndim != 2 or controls.strides[1] != 8:
+                controls = np.ascontiguousarray(controls)
+        n_new = int(scans.shape[1])
+        ps, ms = _ptr(scans)
+        po, _ = _ptr(odometry)
+        pu, _ = _ptr(controls)
+        check(self.lib.icmslam_append(self._h, ps, n_new, _rows(scans, self.B), po, _rows(odometry, 3), pu, _rows(controls, 2), ms), self._h)
+        self.T += n_new
+        return self._extraction_size()
 
     def get_extraction(self):
         off = np.empty(self.T + 1, np.int32)
@@ -328,6 +354,30 @@ class Engine:
         Lout = C.c_int32()
         st = self.lib.icmslam_pass0(self._h, C.c_void_p(x0.ctypes.data), _ptr(x)[0], self.T, _ptr(out)[0], self.L, self.L, C.byref(Lout), HOST)
         check(st, self._h)
+        return x, out[:, : Lout.value].copy()
+
+    def pass0_begin(self, x0):
+        """Starts pass 0 as a walk that resumes as the log grows (append).  Returns the status: EMPTY_FIRST_SCAN (1) when
+        column 0 has no observation (the walk does not start), else OK."""
+        x0 = np.ascontiguousarray(np.asarray(x0, dtype=np.float64).reshape(3))
+        return check(self.lib.icmslam_pass0_begin(self._h, C.c_void_p(x0.ctypes.data)), self._h)
+
+    def pass0_advance(self) -> int:
+        """Walks every loaded column not walked yet; returns the columns walked.  Poses, labels and the raw map then equal
+        pass0 of the log cut there."""
+        t = C.c_int32(0)
+        check(self.lib.icmslam_pass0_advance(self._h, C.byref(t)), self._h)
+        self.t_walked = int(t.value)
+        return self.t_walked
+
+    def pass0_finish(self):
+        """Mapa.filtrar of the map the walk built (sensors.py:99-102): (positions 3 x columns walked, mapa_viejo 2 x L'), as
+        pass0 of the log cut there returns them.  The walk goes on: later appends and advances extend it."""
+        t = int(getattr(self, "t_walked", 0))
+        x = np.zeros((3, t))
+        out = np.zeros((2, self.L))
+        Lout = C.c_int32()
+        check(self.lib.icmslam_pass0_finish(self._h, _ptr(x)[0], max(t, 1), _ptr(out)[0], self.L, self.L, C.byref(Lout), HOST), self._h)
         return x, out[:, : Lout.value].copy()
 
     def associations(self):

@@ -8,10 +8,13 @@ within one sampling period of t0 + k * deltat, searched from a guess that follow
 column per aligned pair to `mediciones` (B x T), `odometria` (3 x T), `u` (2 x T); a `std_srvs/SetBool` service raises
 `iterations_flag`, after which the offline sweeps run on what has arrived.
 
-Here the arrays grow in preallocated host buffers (amortised doubling instead of one np.hstack per message) and are handed to
-the device in one piece when the solver needs them: pass 0 is causal, so running it after the log has arrived
-(`ICM_SLAM.inicializar`, native) gives what the reference computes message by message.  `OnlineICM` = `ICM_ROS` of the reference:
-the solver façade + this transport.
+Here the arrays grow in preallocated host buffers (amortised doubling instead of one np.hstack per message), and the columns
+that arrived are handed to the device after every `pump` call (`ROS.feed`): the first through `Engine.load`, later ones through
+`Engine.append`, which extracts them on arrival, and pass 0 advances over them (`Engine.pass0_advance`), so `positions` and the
+map under construction exist while the robot is still driving, as in the reference.  When the iterations flag is raised,
+`Engine.pass0_finish` filters the map built so far and the sweeps start on the data already on the device.  The feeding runs on
+the thread that runs `inicializar_online`, never inside a transport callback (a handle is not thread-safe).  `OnlineICM` =
+`ICM_ROS` of the reference: the solver façade + this transport.
 
 The fake transport (`FakeRos`, `publish_log`) restates matlab2ros/createbag.py:35-153: `sensor_msgs/LaserScan` and
 `nav_msgs/Odometry` dictionaries with a running header (seq, stamp = seq * 0.1 s), delivered to the subscribed callbacks in
@@ -153,6 +156,8 @@ class ROS:
         self.lidar = Lidar(name="lidar", topic=config.topic_laser, topic_msg=config.topic_laser_msg, **D)
         self.odom = Odometria(name="odometria", topic=config.topic_odometry, topic_msg=config.topic_odometry_msg, **D)
         self.client = None
+        self._fed = 0            # aligned columns handed to the solver's engine
+        self._walking = False    # pass 0 walks them (False: nothing fed yet, or column 0 has no observation)
 
     def connect_ros(self, client=None):
         self.client = client if client is not None else RoslibpyClient()
@@ -194,6 +199,29 @@ class ROS:
             self.new_data += 1
         self.mediciones, self.odometria, self.u = self._med.view(), self._odo.view(), self._u.view()
 
+    def feed(self, engine):
+        """Hands every aligned column that arrived since the last call to `engine` -- the first ones through `load` + `extract`,
+        later ones through `append` -- and advances pass 0 over them (x0 = odometria[:, 0], sensors.py:61): `positions` is then
+        the causal estimate of every column walked (sensors.py:104).  Each column goes to the engine once, in order.  Returns the
+        columns fed so far."""
+        T = self._u.n                       # (principal_callback appends to the laser log first and to the controls last)
+        if T == self._fed:
+            return T
+        cols = slice(self._fed, T)
+        z, odo, u = self._med.buf[:, cols], self._odo.buf[:, cols], self._u.buf[:, cols]
+        if self._fed == 0:
+            engine.load(z, odo, u, precondition=False)
+            engine.extract()
+            self.x0 = np.array([odo[:, 0]]).T
+            self._walking = engine.pass0_begin(self.x0.reshape(3)) == 0
+        else:
+            engine.append(z, odo, u)
+        self._fed = T
+        if self._walking:
+            t = engine.pass0_advance()
+            self.positions = engine.get_poses()[:, :t]
+        return T
+
 
 class OnlineICM(ICM_SLAM, ROS):
     """`ICM_ROS` of the reference (sensors.py:15-104): the solver with the ROS transport attached."""
@@ -206,18 +234,30 @@ class OnlineICM(ICM_SLAM, ROS):
     def inicializar_online(self, client=None, pump=None):
         """sensors.py:51-104.  Connects, lets the messages arrive -- `pump(self)` is called until it returns False or the
         iterations service has been called (a fake publisher delivers its log there; with a real bridge the callbacks run on
-        the client's thread and `pump` only has to wait) -- then x0 = odometria[:, 0] (:61) and pass 0 over what arrived."""
+        the client's thread and `pump` only has to wait) -- and after every `pump` call feeds what arrived to the engine and
+        advances pass 0 over it (`feed`: x0 = odometria[:, 0], :61; `positions` follows).  Then Mapa.filtrar of the map built
+        (:99-102): returns (mapa_viejo, positions) as `inicializar` does on the same log."""
         self.connect_ros(client)
         try:
-            while pump is not None and pump(self) and not self.iterations_flag:
-                pass
+            while pump is not None:
+                more = pump(self)
+                self.feed(self._engine)
+                if not more or self.iterations_flag:
+                    break
+            self.feed(self._engine)
         finally:
             self.disconnect_ros()
         if self.new_data == 0:
             raise RuntimeError("no aligned laser / odometry message pair arrived")
-        self.x0 = np.array([np.asarray(self.odometria)[:, 0]]).T
-        self.invalidate()                       # (the logs grew in place)
-        return self.inicializar()
+        self.adopt_engine(self._engine)         # (the engine holds the log: iterar does not upload it again)
+        if self._walking:
+            xs, mapa = self._engine.pass0_finish()
+        else:                                   # an empty first scan: what pass 0 returns then (sensors.py:137-139)
+            xs, mapa = self._engine.pass0(self.x0.reshape(3))
+        self.mapa_viejo = mapa.copy()
+        self.positions = xs.copy()
+        self.iterations_flag = True
+        return mapa, xs
 
 
 # ---- clients -----------------------------------------------------------------------------------------------------------------

@@ -117,6 +117,15 @@ int icmslam_extraction_size(const icmslam_handle* h, int64_t* n_obs, int32_t* n_
 int icmslam_get_extraction(icmslam_handle* h, int32_t* off, int32_t* beam, double* d, double* bx,
                            double* by, int32_t memspace);
 
+/* -- a log that grows while the robot drives (ICM_ROS.principal_callback, ICM_SLAM.py:301-341): n_new more columns of the log
+ * loaded with icmslam_load (same B, same precondition flag and beam tables), HOST or DEVICE pointers, extracted on arrival.  The
+ * handle then holds exactly what icmslam_load + icmslam_extract of the whole log leave.  ICMSLAM_ERR_INVALID before icmslam_load
+ * / with n_new <= 0; ICMSLAM_ERR_UNSUPPORTED on a batch or segment handle.  A refused call leaves the handle as it was.  The
+ * buffers grow by doubling; what only the sweeps read is laid out again by the next call that sweeps or sets their inputs
+ * (icmslam_sweep / _iterate*, _set_map, _set_poses, _set_batch*, _set_segment, _device_ptr, icmslam_pass0_finish). */
+int icmslam_append(icmslam_handle* h, const double* scans, int32_t n_new, int64_t ld_scans, const double* odometry,
+                   int64_t ld_odo, const double* controls, int64_t ld_u, int32_t memspace);
+
 /* -- Mapa state (ICM_SLAM.py:115, :119-126): landmarks_actuales and cant_obs_i. */
 int icmslam_set_landmarks_actuales(icmslam_handle* h, int32_t lact);
 int icmslam_get_landmarks_actuales(const icmslam_handle* h, int32_t* lact);
@@ -217,6 +226,22 @@ int icmslam_fcluster(const double* px, const double* py, int32_t n, double t, in
  * Sequential by construction; the inner solver is the reference's Nelder-Mead on fun_x. */
 int icmslam_pass0(icmslam_handle* h, const double* x0, double* x, int64_t ld_x, double* map_out, int32_t cap_out,
                   int64_t ld_map_out, int32_t* L_out, int32_t memspace);
+/* pass 0 as a walk that can be resumed, so that the poses and the map under construction exist while the log grows
+ * (icmslam_pass0 = begin + advance + finish over the loaded log).
+ * begin: x0 (HOST, 3 doubles) and an empty walk; ICMSLAM_EMPTY_FIRST_SCAN when column 0 has no observation.
+ * advance: the steps of every loaded column the walk has not taken yet (Branch A / fcluster when it reaches column 0); *t_done =
+ *   columns walked.  Then the resident poses of columns < t_done (icmslam_get_poses), the labels of their scans
+ *   (icmslam_get_associations) and the map under construction with its counts (icmslam_get_raw_map) are bit for bit what
+ *   icmslam_pass0 gives on the log cut at t_done.  The walk keeps its map in buffers of its own: icmslam_filter_map,
+ *   _calc_cambio, _associate and the sweeps may come between two advances.  ICMSLAM_ERR_LABEL_CAP from the advance that crosses
+ *   L (the walk must then be begun again); ICMSLAM_ERR_UNSUPPORTED from an advance that would walk a scan of more than 1024
+ *   kept beams; ICMSLAM_ERR_INVALID before begin.
+ * finish: Mapa.filtrar of the map built so far (sensors.py:99-102), with the outputs of icmslam_pass0 (x: the t_done columns
+ *   walked).  It does not end the walk: more appends and advances may follow, and a later finish includes them. */
+int icmslam_pass0_begin(icmslam_handle* h, const double* x0);
+int icmslam_pass0_advance(icmslam_handle* h, int32_t* t_done);
+int icmslam_pass0_finish(icmslam_handle* h, double* x, int64_t ld_x, double* map_out, int32_t cap_out, int64_t ld_map_out,
+                         int32_t* L_out, int32_t memspace);
 
 /* -- the model functions the reference leaves to the user (sensors.py:170-282) for ONE pose, on the device: `op` selects
  * g(x_ant, u_ant) (:206-211), h(x, z) against the matched landmarks `seen` (:175-204), the energy fun_xn / fun_x at x (:224-282;
